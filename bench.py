@@ -9,6 +9,12 @@
     python bench.py --workload poisson1080 [--impl reference]   row f-3: one screened-Poisson reconstruction per step; the
                                                              reference arm is the reference's own solver (OpenMP backend),
                                                              the GPU line also times its CUDA backend on the same device
+    python bench.py ... --dump-outputs DIR                   also writes what the timed path computed in its last step
+                                                             as DIR/<name>.npy (one GPU; the inputs are seeded, so two
+                                                             builds can be compared output for output)
+
+The bench writes nothing into the tree it runs from (which may be read-only): no bytecode caches, and the CPU
+baseline's -march=native oracle build goes to a temporary directory.
 
 Workload "cfg5": synthetic 1920x1080 homogeneous-medium Cornell scene, 10 M photons per iteration,
 G-BRE 3D kernel, mixed shift (useShiftNull), area MIS, pathSet; radius = bsphereR * scale * 0.01.
@@ -40,6 +46,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 
 WORKLOADS = {
     # name: (w, h, photons, default scale)
@@ -70,10 +77,52 @@ def parse():
     ap.add_argument("--photons", type=int, default=None)
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="target CPU-baseline sample time")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path computed in its last step as DIR/<name>.npy "
+                         "(a fixed, seeded sample of the rays where the whole output exceeds 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 # --------------------------------------------------------------------------------------------
+DUMP_MAX_BYTES = 64 << 20
+DUMP_MAX_RAYS = 1 << 18     # 27 floats per ray: 28 MB of gather output
+
+
+def dump_rows(n):
+    """--dump-outputs: the rays whose results are written, a fixed seeded sample (sorted) when there are too many"""
+    if n <= DUMP_MAX_RAYS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0xD0).choice(n, DUMP_MAX_RAYS, replace=False))
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: every array as <path>/<name>.npy (float32 / float64 only, 64 MB at most in all)"""
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def dump_gather(path, out_dev, rays, mvol_dev=None):
+    """--dump-outputs of a gather: the 27 output floats per ray (mediumFlux[3], shiftedMediumFlux[4][3],
+    weightedMediumFlux[4][3]) of the sampled rays, with their index in the ray set and their pixel; for G-VPM also MVol
+    (int32 view of the uint32 photon count per ray that drives the host's radius update)"""
+    import torch
+    rows = dump_rows(rays.n)
+    idx = torch.from_numpy(rows).to(out_dev.device)
+    arrays = {"gather_out": out_dev[:rays.n * 27].view(rays.n, 27)[idx].cpu().numpy(), "ray_index": rows.astype(np.float64),
+              "ray_pixel": np.stack([rays.px[rows], rays.py[rows]], axis=1).astype(np.float64)}
+    if mvol_dev is not None:
+        arrays["gather_mvol"] = mvol_dev[:rays.n][idx].cpu().numpy().view(np.uint32).astype(np.float64)
+    dump_outputs(path, arrays)
+
+
 def pinned(n, dtype):
     import torch
     t = torch.empty(n, dtype=dtype, pin_memory=torch.cuda.is_available())
@@ -821,6 +870,8 @@ def technique_main(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: gvpm_b200 has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of a one-GPU run")
     torch.cuda.set_device(local)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
@@ -867,11 +918,12 @@ def technique_main(args):
             ctx.build_planes()
 
     def gather_device():
+        """-> device pointers (out [n_rays*27] float32, G-VPM: mvol [n_rays] uint32, else None)"""
         if tech == "vpm":
-            return ctx.gather_vpm_device(d["nb"])[0]
+            return ctx.gather_vpm_device(d["nb"])
         if tech == "beams":
-            return ctx.gather_beams_device(False)[0]
-        return ctx.gather_planes_device(False)[0]
+            return ctx.gather_beams_device(False)[0], None
+        return ctx.gather_planes_device(False)[0], None
 
     def collect(ptr):
         if world == 1:
@@ -881,11 +933,14 @@ def technique_main(args):
             send[:n_local * 27].copy_(view)
             dist.gather(send, gathered, dst=0)
 
+    last_out = [None]     # device pointers of the last resident gather's outputs
+
     def step_resident(k):
         with torch.cuda.stream(stream):
             flush.fill_(k & 255)          # L2 flush between timed steps (untimed work would be nicer; it is 256 MB at HBM speed: ~40 us)
         build()
-        collect(gather_device())
+        last_out[0] = gather_device()
+        collect(last_out[0][0])
 
     def step_e2e(k):
         upload_prims()
@@ -936,6 +991,11 @@ def technique_main(args):
         sampler.start()
     W = max(3, args.warmup)
     ms_total, launches = timed(step_resident, args.steps, W)
+    if args.dump_outputs:   # before the untimed gathers below overwrite the output buffers
+        out_ptr, mvol_ptr = last_out[0]
+        dump_gather(args.dump_outputs, torch.as_tensor(DevView(out_ptr, n_local * 27 * 4), device="cuda").view(torch.float32),
+                    rays, None if mvol_ptr is None else
+                    torch.as_tensor(DevView(mvol_ptr, n_local * 4), device="cuda").view(torch.int32))
     ms_e2e, _ = timed(step_e2e, args.steps, W)
     clocks = sampler.stop() if rank == 0 else None
     # phases + the roofline numerator H (neighbour pairs) from untimed runs
@@ -1056,8 +1116,9 @@ def poisson_main(args):
         if not pr.available():
             print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/libgvpm_poisson_ref.so absent"}))
             return
-        reference_cpu(min(1, args.warmup))
-        ms, _ = reference_cpu(max(1, min(args.steps, 5)))
+        if args.warmup:
+            reference_cpu(args.warmup)
+        ms, _ = reference_cpu(args.steps)
         value = w * h / (ms * 1e-3)
         cb = {"value": value, "unit": "pixels/s", "cores": os.cpu_count(), "kind": "reference",
               "sample": f"whole {w}x{h} reconstruction, the reference's own poisson::Solver (OpenMP backend), {ms:.0f} ms"}
@@ -1066,7 +1127,8 @@ def poisson_main(args):
         return
     from gvpm_b200.api import Context
     ctx = Context(0)
-    for _ in range(max(3, args.warmup)):
+    W = max(3, args.warmup)
+    for _ in range(W):
         rec = ctx.poisson_solve(tp, dx, dy, direct, preset=preset)
     clocks = ClockSampler(0)
     clocks.start()
@@ -1077,9 +1139,11 @@ def poisson_main(args):
         wall.append((time.perf_counter() - t0) * 1e3)
         dev_ms.append(ctx.last_poisson_ms())
     ck = clocks.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"reconstruction": rec})
     ms, wall_ms = float(np.mean(dev_ms)), float(np.mean(wall))
     nbytes = int(tp.nbytes + dx.nbytes + dy.nbytes + direct.nbytes)
-    line = dict(base, value=w * h / (ms * 1e-3), ms_per_step=ms, clocks=ck,
+    line = dict(base, value=w * h / (ms * 1e-3), ms_per_step=ms, warmup=W, clocks=ck,
                 e2e={"value": w * h / (wall_ms * 1e-3), "unit": "pixels/s", "h2d_bytes_per_step": nbytes,
                      "d2h_bytes_per_step": int(rec.nbytes), "ms_per_step": wall_ms},
                 timing="value: CUDA events inside gvpm_poisson_solve (copies included); e2e: wall clock around the call")
@@ -1092,7 +1156,7 @@ def poisson_main(args):
     if pr.cuda_available():
         pr.solve(tp, dx, dy, direct, backend="CUDA", **pr.preset(preset))       # warm-up (context, allocations)
         ts = []
-        for _ in range(max(1, min(args.steps, 5))):
+        for _ in range(args.steps):
             t0 = time.perf_counter()
             got = pr.solve(tp, dx, dy, direct, backend="CUDA", **pr.preset(preset))
             ts.append((time.perf_counter() - t0) * 1e3)
@@ -1125,6 +1189,8 @@ def main():
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: gvpm_b200 has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of a one-GPU run")
     torch.cuda.set_device(local)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
@@ -1516,6 +1582,8 @@ def main():
         sampler.start()
     W = max(3, args.warmup)
     ms_total, launches, build_ms, gather_ms = timed(step_resident, args.steps, W, False)
+    if args.dump_outputs:   # the last timed step's result buffer, before the legs below reuse it
+        dump_gather(args.dump_outputs, out_bufs[(W + args.steps - 1) & 1], rays)
     collect_ok = None
     if peer_collect:   # what rank 0 holds after the run = what the ranks gathered in their last two steps
         sums = torch.stack([out_bufs[b][:n_local * 27].double().sum() for b in (0, 1)])

@@ -6,6 +6,7 @@ legs.  The product package gvpm_b200 never imports this module.
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -14,6 +15,7 @@ from gvpm_b200 import _native as N
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libgvpm_oracle.so")
 _lib = None
+_native_dir = None
 
 
 def build():
@@ -21,13 +23,15 @@ def build():
 
 
 def prefer_native():
-    """bench.py's CPU legs: build the oracle with -march=native on THIS machine (untimed) and load that build; falls back to
-    the portable build.  Must be called before the first load().  -> the flags in use"""
-    global LIB_PATH
+    """bench.py's CPU legs: build the oracle with -march=native on THIS machine (untimed) into a temporary directory, which
+    goes when the process ends, and load that build; falls back to the portable build.  Must be called before the first
+    load().  -> the flags in use"""
+    global LIB_PATH, _native_dir
     assert _lib is None, "prefer_native() after load()"
     try:
-        subprocess.check_call(["make", "-s", "-B", "-C", _HERE, "native"])
-        LIB_PATH = os.path.join(_HERE, "_native", "libgvpm_oracle.so")
+        _native_dir = tempfile.TemporaryDirectory(prefix="gvpm_oracle_native_")
+        subprocess.check_call(["make", "-s", "-B", "-C", _HERE, "native", "NATIVE_DIR=" + _native_dir.name])
+        LIB_PATH = os.path.join(_native_dir.name, "libgvpm_oracle.so")
         return "-O3 -march=native -ffp-contract=off"
     except Exception:  # noqa: BLE001 - no compiler on the box: the shipped portable build
         return "-O3 -ffp-contract=off (portable build: native rebuild failed)"

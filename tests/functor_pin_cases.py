@@ -2,6 +2,7 @@
 flattened inputs of the C ABI, evaluated by the reference's own compiled functors (oracle/functor_binding.py) or by the
 oracle restatement (oracle/binding.py).  Camera segments are first medium edges (edge_id = 1), the case the reference
 harness rebuilds (oracle/ref_functor.cpp)."""
+import os
 import zlib
 
 import numpy as np
@@ -9,6 +10,31 @@ import numpy as np
 import gvpm_b200 as g
 import gvpm_testlib as H
 from gvpm_b200 import _native as N
+
+
+# The reference's outputs on these cases (tests/golden/make_functor_golden.py), stored in parts of under 1 MB each: the point
+# functors, the beam / plane functors and the whole passes.
+GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+GOLDEN_PARTS = ("functor_pins.npz", "functor_pins_beams_planes.npz", "functor_pins_passes.npz")
+
+
+def golden_part(key):
+    """the file of GOLDEN_PARTS that holds a golden key"""
+    if key.startswith("pass"):
+        return GOLDEN_PARTS[2]
+    if key.split("_")[0] in ("beams", "planes", "sppmbeams", "sppmplanes"):
+        return GOLDEN_PARTS[1]
+    return GOLDEN_PARTS[0]
+
+
+def load_golden():
+    """every golden key of the functor pins, read from its part"""
+    out = {}
+    for part in GOLDEN_PARTS:
+        z = dict(np.load(os.path.join(GOLDEN_DIR, part)))
+        assert all(golden_part(k) == part and k not in out for k in z), part
+        out.update(z)
+    return out
 
 
 def _invalid_offsets(c):

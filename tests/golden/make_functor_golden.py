@@ -1,4 +1,4 @@
-"""Regenerates tests/golden/functor_pins.npz from the REFERENCE'S OWN shift functors (oracle/_ref/libgvpm_functor_ref.so:
+"""Regenerates tests/golden/functor_pins*.npz from the REFERENCE'S OWN shift functors (oracle/_ref/libgvpm_functor_ref.so:
 VolumeGradientBREQuery::operator() and VolumeGradientPositionQuery::operator(), shift_volume_photon.cpp,
 BeamGradRadianceQuery::operator(), shift_volume_beams.cpp, PlaneGradRadianceQuery::operator(), shift_volume_planes.h, sppm's BeamRadianceQuery::operator(), beams.h, and BeamRadianceEstimator::query, bre.cpp,
 compiled from
@@ -104,6 +104,7 @@ if __name__ == "__main__":
         res, _ = fb.planes_pass(c.planes, c.rays, c.medium, c.config, threads=2)
         out[f"passplanes_{name}_bits"] = cases.bits(res)
     print("whole passes of VPM / beams / planes written")
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "functor_pins.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path), "bytes")
+    for part in cases.GOLDEN_PARTS:
+        path = os.path.join(cases.GOLDEN_DIR, part)
+        np.savez_compressed(path, **{k: v for k, v in out.items() if cases.golden_part(k) == part})
+        print("wrote", path, os.path.getsize(path), "bytes")

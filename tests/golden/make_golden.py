@@ -3,7 +3,7 @@
 
 A regression pin of OUR restatement on camera edge 2 (the synthetic camera outside the medium), not reference output: the
 reference ships no fixture for the path.  The vectors that ARE reference output - from the reference's own compiled functors -
-are tests/golden/functor_pins.npz (tests/golden/make_functor_golden.py, DESIGN.md §5).
+are tests/golden/functor_pins*.npz (tests/golden/make_functor_golden.py, DESIGN.md §5).
 Run from the repo root:  python tests/golden/make_golden.py
 """
 import os

@@ -426,3 +426,100 @@ def test_bench_poisson_reference_arm_on_cpu():
     line = json.loads(p.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "pixels/s" and line["cpu_baseline"]["kind"] == "reference"
     assert line["value"] > 0 and line["config"]["pixels"] == 1280 * 720
+
+
+def test_bench_rejects_arguments_it_cannot_honour():
+    """No timed step, or outputs of a path that has none on the device: refused before anything runs."""
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                           timeout=120)
+        assert p.returncode == 2 and "error:" in p.stderr, (extra, p.stderr[-2000:])
+
+
+def _bench_dump(tmp_path, *args):
+    """run bench.py with --dump-outputs on one GPU -> (its JSON line, the dumped arrays by name)"""
+    import json
+    d = tmp_path / "dump"
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--no-cpu-baseline",
+                        "--dump-outputs", str(d)] + list(args), capture_output=True, text=True, timeout=600)
+    assert p.returncode == 0, p.stderr[-2000:]
+    line = json.loads(p.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2
+    z = {f.stem: np.load(f) for f in d.glob("*.npy")}
+    assert all(a.dtype in (np.float32, np.float64) for a in z.values())
+    assert sum(a.nbytes for a in z.values()) <= 64 << 20
+    return line, z
+
+
+def _check_gather_dump(z, rays, out, mvol=None):
+    """the dumped rows are the gather output of the rays they name (index and pixel), all rays where there are few"""
+    assert sorted(z) == sorted(["gather_out", "ray_index", "ray_pixel"] + (["gather_mvol"] if mvol is not None else []))
+    np.testing.assert_array_equal(z["ray_index"], np.arange(rays.n))
+    np.testing.assert_array_equal(z["ray_pixel"], np.stack([rays.px, rays.py], axis=1))
+    assert z["gather_out"].dtype == np.float32 and np.count_nonzero(z["gather_out"][:, :3]) > rays.n // 10
+    import gvpm_testlib as H
+    H.assert_radiance_close(z["gather_out"], out, 1e-4, "bench dump")
+    if mvol is not None:
+        np.testing.assert_array_equal(z["gather_mvol"], mvol)
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_of_the_point_gather(tmp_path, built):
+    """`bench.py --dump-outputs DIR` (cfg1, resident G-BRE path): the dump equals the same gather run directly through
+    the C ABI on the bench's seeded inputs, row by row (27 floats per ray, float32), with each ray's index and pixel."""
+    import types
+    import bench
+    from gvpm_b200.api import Context
+    _, z = _bench_dump(tmp_path, "--workload", "cfg1")
+    inp = bench.make_inputs(types.SimpleNamespace(workload="cfg1", photons=None, scale=None, impl="ours"), 0, 1, pin=False)
+    ctx = Context(0)
+    ctx.set_medium(inp["medium"])
+    ctx.set_config(inp["cfg"])
+    ctx.set_occluders(inp["tri"])
+    ctx.upload_photons(inp["photons"])
+    ctx.upload_rays(inp["rays"])
+    ctx.build_points_for_rays(inp["radius"], want_kept=False)
+    out, _ = ctx.gather_bre(counts=False)
+    ctx.close()
+    _check_gather_dump(z, inp["rays"], out)
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_of_the_vpm_gather(tmp_path, built):
+    """The technique path (cfg2, G-VPM, device pointers of the last gather): radiance and MVol, the per-ray photon count
+    that drives the radius update, equal the same gather run directly through the C ABI on the bench's inputs."""
+    import types
+    import bench
+    from gvpm_b200.api import Context
+    _, z = _bench_dump(tmp_path, "--workload", "cfg2", "--photons", "20000")
+    d = bench.technique_inputs(types.SimpleNamespace(workload="cfg2", photons=20000, scale=None), 0, 1)
+    ctx = Context(0)
+    ctx.set_medium(d["medium"])
+    ctx.set_config(d["cfg"])
+    ctx.set_occluders(d["tri"])
+    ctx.upload_photons(d["photons"])
+    ctx.build_points(d["radius"])
+    ctx.upload_rays(d["rays"])
+    ctx.upload_vpm_samples(d["samples"])
+    out, mvol, _ = ctx.gather_vpm(d["nb"], sample_counts=False)
+    ctx.close()
+    assert mvol.max() > 0
+    _check_gather_dump(z, d["rays"], out, mvol)
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_of_the_poisson_solve(tmp_path, built):
+    """The Poisson path (poisson720): the dumped reconstruction is the solve of the bench's seeded image set."""
+    import importlib.util
+    from gvpm_b200.api import Context
+    line, z = _bench_dump(tmp_path, "--workload", "poisson720")
+    assert line["warmup"] == 3 and sorted(z) == ["reconstruction"]
+    spec = importlib.util.spec_from_file_location("make_poisson_golden", os.path.join(ROOT, "tests", "golden", "make_poisson_golden.py"))
+    G = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(G)
+    _, tp, dx, dy, direct = G.images(720, 1280, 11)
+    ctx = Context(0)
+    want = ctx.poisson_solve(tp, dx, dy, direct, preset="L2D")
+    ctx.close()
+    assert z["reconstruction"].shape == (720, 1280, 3) and z["reconstruction"].dtype == np.float32
+    np.testing.assert_allclose(z["reconstruction"], want, rtol=0, atol=1e-6 * np.abs(want).max())

@@ -1,11 +1,10 @@
-"""The CUDA gathers against REFERENCE OUTPUT directly: tests/golden/functor_pins.npz holds what the reference's own compiled
+"""The CUDA gathers against REFERENCE OUTPUT directly: tests/golden/functor_pins*.npz hold what the reference's own compiled
 shift functors (oracle/_ref/libgvpm_functor_ref.so, built from /root/reference; tests/golden/make_functor_golden.py)
 compute on the seeded cases of tests/functor_pin_cases.py.  Here the same inputs go through the C ABI and the result is
 compared with those vectors - no oracle in between.  Bar (BASELINE.json north_star): primal and the four gradient
 contributions within 1e-4 relative (fp32), globally floored and per ray; the accepted-pair counts exact.
 
 The oracle restatement matches the same vectors bit for bit (tests/test_oracle_functor_pin.py, CPU)."""
-import os
 
 import numpy as np
 import pytest
@@ -14,13 +13,12 @@ import functor_pin_cases as cases
 import gvpm_testlib as H
 
 pytestmark = pytest.mark.gpu
-GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "functor_pins.npz")
 RTOL = 1e-4
 
 
 @pytest.fixture(scope="module")
 def golden():
-    return dict(np.load(GOLDEN))
+    return cases.load_golden()
 
 
 def _close(got, want_bits, what, rows=None):

@@ -9,7 +9,7 @@ filters, the 3-D kernel's random chord position, shiftNull (:119-158), getTypeSh
 heuristic) and the accumulation.
 
 oracle/_ref/libgvpm_functor_ref.so is built from /root/reference (oracle/Makefile, target `functor_ref`) and driven on the
-flattened C-ABI inputs by oracle/ref_functor.cpp; tests/golden/functor_pins.npz holds its outputs on the seeded cases of
+flattened C-ABI inputs by oracle/ref_functor.cpp; tests/golden/functor_pins*.npz hold its outputs on the seeded cases of
 tests/functor_pin_cases.py (tests/golden/make_functor_golden.py), so the pin also holds where the reference tree is
 absent.  Radiance is compared BIT-EXACTLY (floats as integer bits, sums over the neighbour set in photon order)."""
 import os
@@ -22,12 +22,11 @@ import gvpm_testlib as H
 from oracle import binding as ob
 from oracle import functor_binding as fb
 
-GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "functor_pins.npz")
 
 
 @pytest.fixture(scope="module")
 def golden():
-    return dict(np.load(GOLDEN))
+    return cases.load_golden()
 
 
 def _same_rows(got, want, what, rows=None):
