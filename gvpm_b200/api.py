@@ -236,14 +236,12 @@ class Context:
         n = self.n_rays
         ptr, _ = self.ray_staging_peek()
         rs = R.RaySet(n)
-        sizes = [a * n for a in (12, 12, 4, 4, 4, 12, 4, 4, 4, 4, 4, 48, 48, 16, 48, 16)]
         o = 0
-        for (name, dt, wd), sz in zip(R._RAY_FIELDS, sizes):
+        for name, _, _ in R._RAY_FIELDS:   # the field arrays back to back, each starting on a 256-byte boundary
             a = getattr(rs, name)
-            assert a.nbytes == sz, (name, a.nbytes, sz)
-            self._ck(self.lib.gvpm_read_device(self.h, C.c_void_p(ptr + o), a.ctypes.data_as(C.c_void_p), sz),
+            self._ck(self.lib.gvpm_read_device(self.h, C.c_void_p(ptr + o), a.ctypes.data_as(C.c_void_p), a.nbytes),
                      "gvpm_read_device")
-            o += (sz + 255) & ~255
+            o += (a.nbytes + 255) & ~255
         return rs
 
     # ---- rays
@@ -302,26 +300,24 @@ class Context:
                  "gvpm_gather_bre_host")
         return out.reshape(rays.n, N.GVPM_OUT_FLOATS)
 
-    def dump_neighbours_bre(self):
-        """-> (offsets [n_rays+1] uint64, idx uint32 with bit 31 = contributes), per-ray sorted."""
-        n = self.n_rays
-        offsets = np.zeros(n + 1, dtype=np.uint64)
-        rc = self.lib.gvpm_dump_neighbours_bre(self.h, offsets.ctypes.data_as(N.u64p), None, 0)
-        total = int(offsets[n])
+    def _dump_neighbours(self, name, rows, *args):
+        """gvpm_dump_neighbours_<name>: size query, then fill -> (offsets [rows+1] uint64, idx uint32 with bit 31 =
+        contributes), every row's segment in ascending index order."""
+        fn = getattr(self.lib, "gvpm_dump_neighbours_" + name)
+        offsets = np.zeros(rows + 1, dtype=np.uint64)
+        rc = fn(self.h, *args, offsets.ctypes.data_as(N.u64p), None, 0)
+        total = int(offsets[rows])
         if rc != 0 and total == 0:
-            self._ck(rc, "gvpm_dump_neighbours_bre")
+            self._ck(rc, "gvpm_dump_neighbours_" + name)
         idx = np.zeros(max(total, 1), dtype=np.uint32)
         if total:
-            self._ck(self.lib.gvpm_dump_neighbours_bre(self.h, offsets.ctypes.data_as(N.u64p),
-                                                       idx.ctypes.data_as(N.u32p), total),
-                     "gvpm_dump_neighbours_bre")
-        idx = idx[:total]
-        # traversal order -> ascending photon index inside every ray's segment
-        if total:
-            seg = np.repeat(np.arange(n, dtype=np.uint64), np.diff(offsets).astype(np.int64))
-            order = np.lexsort((idx & np.uint32(0x7FFFFFFF), seg))
-            idx = idx[order]
-        return offsets, idx
+            self._ck(fn(self.h, *args, offsets.ctypes.data_as(N.u64p), idx.ctypes.data_as(N.u32p), total),
+                     "gvpm_dump_neighbours_" + name)
+        return offsets, idx[:total]
+
+    def dump_neighbours_bre(self):
+        """-> (offsets [n_rays+1] uint64, idx uint32 with bit 31 = contributes), per-ray sorted."""
+        return self._dump_neighbours("bre", self.n_rays)
 
     # ---- G-Beams 3D
     def upload_beams(self, beams):
@@ -351,18 +347,7 @@ class Context:
         return out.reshape(n, N.GVPM_OUT_FLOATS), (cnt.reshape(n, 2) if counts else None)
 
     def dump_neighbours_beams(self):
-        n = self.n_rays
-        offsets = np.zeros(n + 1, dtype=np.uint64)
-        rc = self.lib.gvpm_dump_neighbours_beams(self.h, offsets.ctypes.data_as(N.u64p), None, 0)
-        total = int(offsets[n])
-        if rc != 0 and total == 0:
-            self._ck(rc, "gvpm_dump_neighbours_beams")
-        idx = np.zeros(max(total, 1), dtype=np.uint32)
-        if total:
-            self._ck(self.lib.gvpm_dump_neighbours_beams(self.h, offsets.ctypes.data_as(N.u64p),
-                                                         idx.ctypes.data_as(N.u32p), total),
-                     "gvpm_dump_neighbours_beams")
-        return offsets, idx[:total]
+        return self._dump_neighbours("beams", self.n_rays)
 
     # ---- sppm primal photon beams
     def gather_sppm_beams(self, technique, counts=True):
@@ -379,18 +364,7 @@ class Context:
 
     def dump_neighbours_sppm_beams(self, technique):
         tech = N.BEAM_TECHNIQUES[technique] if isinstance(technique, str) else int(technique)
-        n = self.n_rays
-        offsets = np.zeros(n + 1, dtype=np.uint64)
-        rc = self.lib.gvpm_dump_neighbours_sppm_beams(self.h, tech, offsets.ctypes.data_as(N.u64p), None, 0)
-        total = int(offsets[n])
-        if rc != 0 and total == 0:
-            self._ck(rc, "gvpm_dump_neighbours_sppm_beams")
-        idx = np.zeros(max(total, 1), dtype=np.uint32)
-        if total:
-            self._ck(self.lib.gvpm_dump_neighbours_sppm_beams(self.h, tech, offsets.ctypes.data_as(N.u64p),
-                                                              idx.ctypes.data_as(N.u32p), total),
-                     "gvpm_dump_neighbours_sppm_beams")
-        return offsets, idx[:total]
+        return self._dump_neighbours("sppm_beams", self.n_rays, tech)
 
     # ---- G-Planes 0D
     def upload_planes(self, planes):
@@ -415,18 +389,7 @@ class Context:
         return out.reshape(n, N.GVPM_OUT_FLOATS), (cnt.reshape(n, 2) if counts else None)
 
     def dump_neighbours_planes(self):
-        n = self.n_rays
-        offsets = np.zeros(n + 1, dtype=np.uint64)
-        rc = self.lib.gvpm_dump_neighbours_planes(self.h, offsets.ctypes.data_as(N.u64p), None, 0)
-        total = int(offsets[n])
-        if rc != 0 and total == 0:
-            self._ck(rc, "gvpm_dump_neighbours_planes")
-        idx = np.zeros(max(total, 1), dtype=np.uint32)
-        if total:
-            self._ck(self.lib.gvpm_dump_neighbours_planes(self.h, offsets.ctypes.data_as(N.u64p),
-                                                          idx.ctypes.data_as(N.u32p), total),
-                     "gvpm_dump_neighbours_planes")
-        return offsets, idx[:total]
+        return self._dump_neighbours("planes", self.n_rays)
 
     # ---- G-VPM
     def upload_vpm_samples(self, samples):
@@ -452,21 +415,7 @@ class Context:
         return out.reshape(n, N.GVPM_OUT_FLOATS), mvol, (sc.reshape(ns, 2) if sample_counts else None)
 
     def dump_neighbours_vpm(self, nb_camera_samples):
-        ns = self.n_samples
-        offsets = np.zeros(ns + 1, dtype=np.uint64)
-        rc = self.lib.gvpm_dump_neighbours_vpm(self.h, nb_camera_samples, offsets.ctypes.data_as(N.u64p), None, 0)
-        total = int(offsets[ns])
-        if rc != 0 and total == 0:
-            self._ck(rc, "gvpm_dump_neighbours_vpm")
-        idx = np.zeros(max(total, 1), dtype=np.uint32)
-        if total:
-            self._ck(self.lib.gvpm_dump_neighbours_vpm(self.h, nb_camera_samples, offsets.ctypes.data_as(N.u64p),
-                                                       idx.ctypes.data_as(N.u32p), total), "gvpm_dump_neighbours_vpm")
-        idx = idx[:total]
-        if total:
-            seg = np.repeat(np.arange(ns, dtype=np.uint64), np.diff(offsets).astype(np.int64))
-            idx = idx[np.lexsort((idx & np.uint32(0x7FFFFFFF), seg))]
-        return offsets, idx
+        return self._dump_neighbours("vpm", self.n_samples, nb_camera_samples)
 
     def compute_gradient(self, acc, w, h, use_abs=False, reuse_primal=False, inv_emitted=1.0):
         """computeGradient (gvpm.cpp:1205-1306); reuse_primal: throughput by gvpm.cpp:503-532 (inv_emitted = 1 for the

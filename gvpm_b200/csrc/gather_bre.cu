@@ -424,7 +424,7 @@ k_bre_grid_traverse(const __grid_constant__ GatherParams P) {
   // with the pathSet prefilter a ray only ever pairs with photons of its pixel's parity: it scans that grid alone
   const bool onlyMine = G.parity_split && prefilter && P.cfg.path_set;
   const uint32_t nPass = onlyMine ? 1u : nGridsBuilt;
-  if (P.build_ovf && __ldg(P.build_ovf)) {   // incomplete grid (gvpm_capi.cu build_frustum): report it instead of gathering
+  if (P.build_ovf && __ldg(P.build_ovf)) {   // incomplete grid (capi_points.cu build_frustum): report it instead of gathering
     if (blockIdx.x == 0 && threadIdx.x == 0) *P.pair_counter = 1ull << 62;
     return;
   }
@@ -600,7 +600,7 @@ k_bre_shade(const __grid_constant__ GatherParams P) {
   }
 }
 
-// ---- host-side launchers (called from gvpm_capi.cu) -------------------------------------------
+// ---- host-side launchers (called from the capi_*.cu units) -------------------------------------------
 static int g_trav_blocks[4] = {0, 0, 0, 0}, g_grid_blocks[4] = {0, 0, 0, 0}, g_shade_blocks[2] = {0, 0};
 
 template <int MODE> static void launch_traverse_mode(const GatherParams &P, int &bps, int sm_count, cudaStream_t stream) {

@@ -405,7 +405,8 @@ int gvpm_dump_neighbours_sppm_beams(gvpm_ctx *ctx, int technique, uint64_t *offs
 
 /* Parity aid: neighbour index sets in CSR form.  offsets: [n_rays+1]; idx: capacity `cap`
  * entries, original photon index with bit 31 set when the photon also passes the depth /
- * interaction-mode / pathSet filters.  Returns GVPM_ERR_INVALID when cap is too small
+ * interaction-mode / pathSet filters; every ray's entries in ascending photon index order (this and the
+ * other gvpm_dump_neighbours_* calls).  Returns GVPM_ERR_INVALID when cap is too small
  * (offsets[n_rays] then holds the needed size). */
 int gvpm_dump_neighbours_bre(gvpm_ctx *ctx, uint64_t *offsets, uint32_t *idx, size_t cap);
 
