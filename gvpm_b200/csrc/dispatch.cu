@@ -144,19 +144,8 @@ __global__ void __launch_bounds__(256) k_dispatch_emit(const __grid_constant__ D
   }
   float4 *t = tile[w];
   if (bits) {
-    const size_t s = (size_t)P.begin + i, s3 = 3 * s;
-    const PhotonStaging &S = P.S;
-    auto ld3 = [&](const float *p, float ww) { return make_float4(__ldg(p + s3), __ldg(p + s3 + 1), __ldg(p + s3 + 2), ww); };
-    const uint32_t meta = pack_meta(S.parent_type[s], S.depth[s], S.path_id[s]);
-    float4 *r = t + lane * 9;
-    r[0] = ld3(S.pos, __uint_as_float(meta));
-    r[1] = ld3(S.flux, __ldg(S.parent_pdf + s));
-    r[2] = ld3(S.parent_pos, __ldg(S.edge_pdf + s));
-    r[3] = ld3(S.pred_pos, __ldg(S.rr_weight + s));
-    r[4] = ld3(S.parent_n, 0.f);
-    r[5] = ld3(S.prefix_flux, 0.f);
-    r[6] = ld3(S.parent_albedo, 0.f);
-    r[7] = make_float4(__uint_as_float((uint32_t)s), 0.f, 0.f, 0.f);   // the photon's index in the whole set (parity dumps)
+    const size_t s = (size_t)P.begin + i;
+    photon_record(t + lane * 9, P.S, s, (uint32_t)s);   // A7.x: the photon's index in the whole set (parity dumps)
   }
   __syncthreads();
   for (int d = 0; d < P.n_dst; ++d) {

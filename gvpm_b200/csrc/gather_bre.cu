@@ -31,7 +31,10 @@ namespace gvpm {
 #define GVPM_SHADE_THREADS 128
 #endif
 #ifndef GVPM_SHADE_MIN_BLOCKS
-#define GVPM_SHADE_MIN_BLOCKS 5   // 96 registers; tuned on cfg5: 4: 2.90 ms, 5: 2.63, 6: 2.69, 8: 2.82
+// 96 registers, no spills.  Tuned on cfg5 (B200, 1000 W): 4: 2.90 ms, 5: 2.63, 6: 2.69, 8: 2.82.  A phase A/B hand-off
+// that re-reads the photon record in phase B instead of carrying it through shared memory fits 80 / 72 registers at 6 / 7
+// (with spills) but shades slower at every bound, 5 / 6 / 7: 2.75 / 2.75 / 2.78 ms against 2.44 (profiles/r3_shade_records.md)
+#define GVPM_SHADE_MIN_BLOCKS 5
 #endif
 #ifndef GVPM_TILE_QUEUE
 #define GVPM_TILE_QUEUE 32

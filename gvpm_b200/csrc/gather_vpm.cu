@@ -148,7 +148,7 @@ __device__ __forceinline__ void vpm_photon(const GatherParams &P, const float4 *
   const v3 Tbase(s1.x, s1.y, s1.z);
   const v3 sigS(P.sigma_s[0], P.sigma_s[1], P.sigma_s[2]);
   const v3 q = R.o + t * R.d;
-  const v3 wi = normalize(ph.parent - ph.p);
+  const v3 wi = ph.wi;
   const v3 photonContrib = (sigS * ph.flux) * phase_eval(P, wi, -R.d);
   const v3 baseContrib = (R.eye * Tbase) * photonContrib;  // :529
   // Float kernelVol = (4.0/3.0) * M_PI * pow(searchRadius, 3) in double (:530)
@@ -157,7 +157,7 @@ __device__ __forceinline__ void vpm_photon(const GatherParams &P, const float4 *
   const sf pdfBase = pdfSuccess * pdfSel;
   const sf recip = sf(1.f) / (kernelVol * pdfBase);
   acc_add(a, 0, baseContrib * recip);
-  const PairCtx C = make_pair_ctx(P, ph, wi);
+  const OccluderNear near = pair_occluders(P, ph.parent, ph.lBase);
 
   float Sx[4], Sy[4], Sz[4], Wk[4];
 #pragma unroll 1
@@ -179,10 +179,10 @@ __device__ __forceinline__ void vpm_photon(const GatherParams &P, const float4 *
       if (Tk.v < 1e-20f) Tk = sf(0.f);
       const v3 zShift = ok + t * dk;
       if (P.cfg.use_shift_null && length_sq(ph.p - zShift) < rr2) {  // :584-602
-        shift_null(P, ph, wi, dk, eyeK, sensor, Tk, pdfBase, pdfShift, S, weight);
+        shift_null(P, ph.flux, wi, dk, eyeK, sensor, Tk, pdfBase, pdfShift, S, weight);
       } else {  // :604-639
         const v3 offsetPos = get_shift_pos(P, rr2, ph.p, q, zShift, R.d, dk, false);
-        shift_photon_diffuse(P, ph, C, offsetPos, dk, eyeK, sensor, Tk, pdfBase, pdfShift, S, weight);
+        shift_photon_diffuse(P, ph, near, offsetPos, dk, eyeK, sensor, Tk, pdfBase, pdfShift, S, weight);
       }
     }
     if ((k == 1 && R.px == P.cfg.film_w - 1) || (k == 2 && R.py == P.cfg.film_h - 1)) weight = sf(1.f);

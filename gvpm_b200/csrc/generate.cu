@@ -303,17 +303,9 @@ __device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned lon
       if (EMIT) {
         const unsigned long long slot = first + appended;
         if (slot < P.n_total && P.aos != nullptr) {
-          // the record the gather reads (gvpm_device.cuh: A0 pos, meta | A1 flux, parent pdf | A2 parent, edge pdf |
-          // A3 predecessor, rr | A4 parent normal | A5 prefix flux | A6 parent albedo)
-          float4 *r = P.aos + slot * 8;
-          const v3 pred = ni >= 3 ? prevPos : v3(1.f, 1.f, 1.f);
-          r[0] = make_float4(nvPos.x.v, nvPos.y.v, nvPos.z.v, __uint_as_float(pack_meta((uint32_t)curType, (uint32_t)(ni - 1), pid)));
-          r[1] = make_float4(flux.x.v, flux.y.v, flux.z.v, pdfArea.v);
-          r[2] = make_float4(curPos.x.v, curPos.y.v, curPos.z.v, edgePdf.v);
-          r[3] = make_float4(pred.x.v, pred.y.v, pred.z.v, curRr.v);
-          r[4] = make_float4(curN.x.v, curN.y.v, curN.z.v, 0.f);
-          r[5] = make_float4(prefix.x.v, prefix.y.v, prefix.z.v, 0.f);
-          r[6] = make_float4(curAlbedo.x.v, curAlbedo.y.v, curAlbedo.z.v, 0.f);
+          // the record the gather reads (gvpm_device.cuh photon_record)
+          photon_record(P.aos + slot * 8, nvPos, pack_meta((uint32_t)curType, (uint32_t)(ni - 1), pid), flux, pdfArea,
+                        curPos, edgePdf, ni >= 3 ? prevPos : v3(1.f, 1.f, 1.f), curRr, curN, prefix, curAlbedo, 0u);
         } else if (slot < P.n_total) {
           put3(P.pos, slot, nvPos); put3(P.flux, slot, flux); put3(P.parent_pos, slot, curPos);
           put3(P.pred_pos, slot, ni >= 3 ? prevPos : v3(1.f, 1.f, 1.f));

@@ -71,16 +71,37 @@ __device__ __forceinline__ sf max3(v3 a) { return smax(a.x, smax(a.y, a.z)); }
 //   A0 = pos.xyz,           meta bits   (P0 is the sorted copy of this field)
 //   A1 = flux.xyz,          parent_pdf
 //   A2 = parent_pos.xyz,    edge_pdf
-//   A3 = pred_pos.xyz,      rr_weight
-//   A4 = parent_n.xyz,      -
-//   A5 = prefix_flux.xyz,   -
-//   A6 = parent_albedo.xyz, -
-//   A7 = unused (keeps the record one aligned 128-byte line = 4 sectors)
+//   A3 = wiW.xyz,           rr_weight   wiW = normalize(pred_pos - parent_pos)
+//   A4 = parent_n.xyz,      cosI        cosI = dot(parent_n, wiW)
+//   A5 = prefix_flux.xyz,   nEdge       nEdge = dot(parent_n, -wi)
+//   A6 = parent_albedo.xyz, lBase       lBase = length(pos - parent_pos)
+//   A7 = whole-set index (bits; dispatched records only, else 0), wi.xyz   wi = normalize(parent_pos - pos)
+// wiW, cosI, nEdge, lBase and wi depend on the photon alone: photon_record computes them once, so the shading does
+// not repeat them for every (ray, photon) pair.  The predecessor position itself is not kept.
 // meta: bits 0-1 parent type, bits 2-9 depth, bit 10 pathID & 1.
-#define GVPM_PHOTON_PLANES 7
 #define GVPM_PLANE_PLANES 6  // float4 planes per photon-plane record (plane_device.cuh)
 __host__ __device__ inline uint32_t pack_meta(uint32_t type, uint32_t depth, uint32_t path_id) {
   return (type & 3u) | ((depth & 255u) << 2) | ((path_id & 1u) << 10);
+}
+// Writes the record of one photon to r[0..7] (shared or global memory), from its fields.  The derived terms use the
+// strictly rounded operations, in the order the shading evaluated them per pair, so the stored bits are those values.
+__device__ __forceinline__ void photon_record(float4 *r, v3 pos, uint32_t meta, v3 flux, sf parentPdf, v3 parent,
+                                              sf edgePdf, v3 pred, sf rrW, v3 pn, v3 prefix, v3 albedo,
+                                              uint32_t wholeIndex) {
+  const v3 wiW = normalize(pred - parent);
+  const sf cosI = dot(pn, wiW);
+  const v3 wi = normalize(parent - pos);
+  // normalize(pos - parent) == -wi bit for bit (negation commutes with every rounding involved)
+  const sf nEdge = dot(pn, -wi);
+  const sf lBase = length(pos - parent);
+  r[0] = make_float4(pos.x.v, pos.y.v, pos.z.v, __uint_as_float(meta));
+  r[1] = make_float4(flux.x.v, flux.y.v, flux.z.v, parentPdf.v);
+  r[2] = make_float4(parent.x.v, parent.y.v, parent.z.v, edgePdf.v);
+  r[3] = make_float4(wiW.x.v, wiW.y.v, wiW.z.v, rrW.v);
+  r[4] = make_float4(pn.x.v, pn.y.v, pn.z.v, cosI.v);
+  r[5] = make_float4(prefix.x.v, prefix.y.v, prefix.z.v, nEdge.v);
+  r[6] = make_float4(albedo.x.v, albedo.y.v, albedo.z.v, lBase.v);
+  r[7] = make_float4(__uint_as_float(wholeIndex), wi.x.v, wi.y.v, wi.z.v);
 }
 
 // Rays: 5 records of 64 B per ray (4 float4 each): base + offsets L,R,T,B.
@@ -95,6 +116,14 @@ struct PhotonStaging {
   const uint8_t *parent_type, *depth;
   const uint32_t *path_id;
 };
+// photon_record of photon s of the staging arrays
+__device__ __forceinline__ void photon_record(float4 *r, const PhotonStaging &S, size_t s, uint32_t wholeIndex) {
+  const size_t s3 = 3 * s;
+  auto ld3 = [&](const float *p) { return v3(__ldg(p + s3), __ldg(p + s3 + 1), __ldg(p + s3 + 2)); };
+  photon_record(r, ld3(S.pos), pack_meta(S.parent_type[s], S.depth[s], S.path_id[s]), ld3(S.flux),
+                sf(__ldg(S.parent_pdf + s)), ld3(S.parent_pos), sf(__ldg(S.edge_pdf + s)), ld3(S.pred_pos),
+                sf(__ldg(S.rr_weight + s)), ld3(S.parent_n), ld3(S.prefix_flux), ld3(S.parent_albedo), wholeIndex);
+}
 struct RayStaging {
   const float *o, *d, *mint, *maxt, *edge_len, *eye_contrib, *xi;
   const int32_t *px, *py, *edge_id;

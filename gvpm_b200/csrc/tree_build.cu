@@ -133,9 +133,8 @@ __global__ void k_morton(const float *__restrict__ pos, uint32_t stride, uint32_
   vals[i] = i;
 }
 
-// raw SoA -> 128-byte records in the caller's order (streaming reads, each thread writes its own record)
-//   A0 pos, meta | A1 flux, parent_pdf | A2 parent_pos, edge_pdf | A3 pred_pos, rr_weight | A4 parent_n
-//   A5 prefix_flux | A6 parent_albedo | A7 unused
+// raw SoA -> 128-byte records in the caller's order (streaming reads, each thread writes its own record; layout and
+// derived terms: gvpm_device.cuh photon_record)
 #define GVPM_AOS_FLOAT4 8
 // Each thread assembles its photon's record in registers; the warp then transposes through a padded shared tile so
 // that every store instruction writes 512 contiguous bytes (4 whole records) instead of 32 scattered 16-byte pieces.
@@ -145,20 +144,7 @@ __global__ void __launch_bounds__(256) k_pack_aos(const PhotonStaging S, uint32_
   const uint32_t warpBase = blockIdx.x * blockDim.x + (w << 5);
   const uint32_t s = warpBase + lane;
   float4 *t = tile[w];
-  if (s < n) {
-    const size_t s3 = 3 * (size_t)s;
-    auto ld3 = [&](const float *p, float ww) { return make_float4(__ldg(p + s3), __ldg(p + s3 + 1), __ldg(p + s3 + 2), ww); };
-    const uint32_t meta = pack_meta(S.parent_type[s], S.depth[s], S.path_id[s]);
-    float4 *r = t + lane * 9;
-    r[0] = ld3(S.pos, __uint_as_float(meta));
-    r[1] = ld3(S.flux, __ldg(S.parent_pdf + s));
-    r[2] = ld3(S.parent_pos, __ldg(S.edge_pdf + s));
-    r[3] = ld3(S.pred_pos, __ldg(S.rr_weight + s));
-    r[4] = ld3(S.parent_n, 0.f);
-    r[5] = ld3(S.prefix_flux, 0.f);
-    r[6] = ld3(S.parent_albedo, 0.f);
-    r[7] = make_float4(0.f, 0.f, 0.f, 0.f);
-  }
+  if (s < n) photon_record(t + lane * 9, S, s, 0u);
   __syncwarp();
   if (warpBase >= n) return;
   const uint32_t nRec = min(32u, n - warpBase);
@@ -437,20 +423,7 @@ __global__ void __launch_bounds__(256) k_pack_aos_kept(const PhotonStaging S, ui
   if (km == 0u) return;
   const uint32_t s = warpBase + lane;
   float4 *t = tile[w];
-  if (km >> lane & 1u) {
-    const size_t s3 = 3 * (size_t)s;
-    auto ld3 = [&](const float *p, float ww) { return make_float4(__ldg(p + s3), __ldg(p + s3 + 1), __ldg(p + s3 + 2), ww); };
-    const uint32_t meta = pack_meta(S.parent_type[s], S.depth[s], S.path_id[s]);
-    float4 *r = t + lane * 9;
-    r[0] = ld3(S.pos, __uint_as_float(meta));
-    r[1] = ld3(S.flux, __ldg(S.parent_pdf + s));
-    r[2] = ld3(S.parent_pos, __ldg(S.edge_pdf + s));
-    r[3] = ld3(S.pred_pos, __ldg(S.rr_weight + s));
-    r[4] = ld3(S.parent_n, 0.f);
-    r[5] = ld3(S.prefix_flux, 0.f);
-    r[6] = ld3(S.parent_albedo, 0.f);
-    r[7] = make_float4(0.f, 0.f, 0.f, 0.f);
-  }
+  if (km >> lane & 1u) photon_record(t + lane * 9, S, s, 0u);
   __syncwarp();
   float4 *dst = aos + (size_t)warpBase * GVPM_AOS_FLOAT4;
 #pragma unroll
