@@ -17,8 +17,9 @@
 
 namespace gvpm {
 size_t sort_temp_bytes(uint32_t n);
-cudaError_t run_sort(void *temp, size_t temp_bytes, const uint32_t *kin, uint32_t *kout, const uint32_t *vin,
-                     uint32_t *vout, uint32_t n, cudaStream_t st);
+cudaError_t run_sort_bits(void *temp, size_t temp_bytes, const uint32_t *kin, uint32_t *kout, const uint32_t *vin,
+                          uint32_t *vout, uint32_t n, int bits, cudaStream_t st);
+constexpr int kHilbertBits = 30;   // width of the keys of launch_morton / launch_keys_kept (and of sort_temp_bytes' sort)
 int bounds_blocks(uint32_t n);
 void launch_bounds(const float *pos, uint32_t n, float *partial, float *bounds, cudaStream_t st, uint32_t stride = 3);
 void launch_morton(const float *pos, uint32_t n, const float *bounds, uint32_t *keys, uint32_t *vals,
@@ -37,7 +38,7 @@ cudaError_t launch_cell_scan(void *temp, size_t temp_bytes, const uint32_t *cell
                              cudaStream_t st);
 void launch_pack_scatter(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *keys, const uint32_t *rank,
                          const uint32_t *cell_start, float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st,
-                         bool records_ready, const uint32_t *kept_dev);
+                         bool records_ready, const uint32_t *kept_dev, int sm_count);
 void launch_frustum_mark(const float4 *rays, uint32_t n_rays, const FrustumGrid &G, uint32_t *occ, int sm_count, cudaStream_t st);
 void launch_dispatch(const DispatchParams &P, cudaStream_t st, int ctas);
 void launch_dispatch_signal(const SignalParams &P, cudaStream_t st);
@@ -55,8 +56,6 @@ void launch_scan_u32(uint32_t *vals, uint32_t nb, uint32_t *total, cudaStream_t 
 size_t cell_starts_scratch_bytes(uint32_t n_keys);
 void launch_cell_starts(const uint32_t *sorted_keys, uint32_t n, uint32_t n_keys, uint32_t *cell_start, void *scratch,
                         int sm_count, cudaStream_t st);
-cudaError_t run_sort_bits(void *temp, size_t temp_bytes, const uint32_t *kin, uint32_t *kout, const uint32_t *vin,
-                          uint32_t *vout, uint32_t n, int bits, cudaStream_t st);
 size_t ray_grid_bytes();
 size_t ray_mask_bytes();
 void launch_ray_region(const float4 *rays, uint32_t nRays, float radius, float *box, void *grid, uint32_t *mask,
@@ -64,8 +63,6 @@ void launch_ray_region(const float4 *rays, uint32_t nRays, float radius, float *
 void launch_keep_pruned(const float *pos, uint32_t n, const void *grid, const uint32_t *mask, uint32_t *keepmask,
                         uint32_t *block_kept, cudaStream_t st);
 void launch_keys_kept(const float *pos, const uint32_t *vals, uint32_t m, const void *grid, uint32_t *keys, cudaStream_t st);
-void launch_pack_pruned(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *sorted, uint32_t m,
-                        float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st);
 void launch_pack_sorted(const PhotonStaging &S, float4 *aos, const uint32_t *sorted, uint32_t n, float4 *planes,
                         uint32_t *orig, cudaStream_t st, bool records_ready = false);
 void launch_leaf_boxes(const float4 *p0, uint32_t n, uint32_t nLeaves, float radius, float4 *lo, float4 *hi,

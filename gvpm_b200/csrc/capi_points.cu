@@ -101,10 +101,10 @@ int build_pruned_bvh(gvpm_ctx *ctx, float radius, uint32_t *n_kept) {
     CK(ctx->box_hi.reserve(16 * (size_t)total));
     const PhotonStaging S = staging_ptrs<PhotonSoA>(ctx->ph_staging.p, n);
     launch_keys_kept(S.pos, ctx->vals_in.as<uint32_t>(), kept, rr + gridOff, ctx->keys_in.as<uint32_t>(), st);
-    CK(run_sort(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
-                ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), kept, st));
-    launch_pack_pruned(S, n, keepmask, ctx->vals_out.as<uint32_t>(), kept, ctx->aos.as<float4>(),
-                       ctx->planes.as<float4>(), ctx->orig.as<uint32_t>(), st);
+    CK(run_sort_bits(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
+                     ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), kept, kHilbertBits, st));
+    launch_pack_sorted_kept(S, n, keepmask, ctx->vals_out.as<uint32_t>(), kept, ctx->aos.as<float4>(),
+                            ctx->planes.as<float4>(), ctx->orig.as<uint32_t>(), st, false);
     float4 *lo = ctx->box_lo.as<float4>(), *hi = ctx->box_hi.as<float4>();
     launch_leaf_boxes(ctx->planes.as<float4>(), kept, T.cnt[0], radius, lo, hi, st);
     for (int l = 1; l < levels; ++l)
@@ -251,7 +251,7 @@ int build_frustum(gvpm_ctx *ctx, float radius, uint32_t *n_kept) {
       CK(launch_cell_scan(ctx->sort_temp.p, ctx->sort_temp.cap, cell_count, ctx->cell_start.as<uint32_t>(), n_keys, st));
       launch_pack_scatter(S, n, keepmask, ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), ctx->cell_start.as<uint32_t>(),
                           ctx->records(), ctx->planes.as<float4>(), ctx->orig.as<uint32_t>(), st, direct,
-                          ctx->cell_start.as<uint32_t>() + n_keys - 1);
+                          ctx->cell_start.as<uint32_t>() + n_keys - 1, ctx->sm_count);
       sortedKeys = sortedVals = nullptr;
       ctx->launches += 4;
     } else if (ctx->kept_fraction_hint < 0.5) {
@@ -359,8 +359,8 @@ int gvpm_build_points(gvpm_ctx *ctx, float radius) {
     CK(ctx->bounds_partial.reserve((size_t)bounds_blocks(n) * 6 * sizeof(float)));
     launch_bounds(pos, n, ctx->bounds_partial.as<float>(), ctx->bounds.as<float>(), st, stride);
     launch_morton(pos, n, ctx->bounds.as<float>(), ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), st, stride);
-    CK(run_sort(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
-                ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), n, st));
+    CK(run_sort_bits(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
+                     ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), n, kHilbertBits, st));
     if (!direct) CK(ctx->aos.reserve(128 * (size_t)n));
     launch_pack_sorted(S, ctx->records(), ctx->vals_out.as<uint32_t>(), n, ctx->planes.as<float4>(),
                        ctx->orig.as<uint32_t>(), st, direct);

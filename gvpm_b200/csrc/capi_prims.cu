@@ -53,8 +53,8 @@ int gvpm_build_planes(gvpm_ctx *ctx) {
     launch_bounds(ctx->plane_pos.as<float>(), n, ctx->bounds_partial.as<float>(), ctx->plane_bounds.as<float>(), st);
     launch_morton(ctx->plane_pos.as<float>(), n, ctx->plane_bounds.as<float>(), ctx->keys_in.as<uint32_t>(),
                   ctx->vals_in.as<uint32_t>(), st);
-    CK(run_sort(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
-                ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), n, st));
+    CK(run_sort_bits(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
+                     ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), n, kHilbertBits, st));
     launch_plane_pack_sorted(ctx->plane_raw.as<float4>(), ctx->vals_out.as<uint32_t>(), n, ctx->plane_rec.as<float4>(),
                              ctx->plane_orig.as<uint32_t>(), st);
     launch_plane_leaf_boxes(ctx->plane_rec.as<float4>(), n, nLeaves, ctx->plane_box_lo.as<float4>(),
@@ -212,8 +212,8 @@ int gvpm_build_beams(gvpm_ctx *ctx, float radius) {
     launch_bounds(ctx->sub_pos.as<float>(), n, ctx->bounds_partial.as<float>(), ctx->beam_bounds.as<float>(), st);
     launch_morton(ctx->sub_pos.as<float>(), n, ctx->beam_bounds.as<float>(), ctx->keys_in.as<uint32_t>(),
                   ctx->vals_in.as<uint32_t>(), st);
-    CK(run_sort(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
-                ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), n, st));
+    CK(run_sort_bits(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
+                     ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), n, kHilbertBits, st));
     launch_sub_gather(ctx->sub_raw.as<float4>(), ctx->vals_out.as<uint32_t>(), n, ctx->subs.as<float4>(), st);
     float4 *lo = ctx->beam_box_lo.as<float4>(), *hi = ctx->beam_box_hi.as<float4>();
     launch_subbeam_leaf_boxes(ctx->subs.as<float4>(), ctx->beams.as<float4>(), n, T.cnt[0], radius, lo, hi, st);

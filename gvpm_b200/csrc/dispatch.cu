@@ -10,7 +10,7 @@
 // (~1.1 times), and a receiver builds its grid over the records it was sent, nothing else.
 //
 //   k_dispatch_classify   thread per photon: one keep bit per receiver, per-CTA counts per receiver
-//   k_dispatch_scan       one CTA per receiver: exclusive scan of the CTA counts (slot of a CTA's first record)
+//   k_scan_exclusive      one CTA per receiver: exclusive scan of the CTA counts (slot of a CTA's first record)
 //   k_dispatch_emit       warp per 32 photons: records staged in shared memory (as k_pack_aos), then for every receiver
 //                         the warp's kept records go out as ONE contiguous run of 16-byte stores (slots follow the photon
 //                         order: deterministic, independent of scheduling)
@@ -21,6 +21,7 @@
 #include <cstdint>
 
 #include "frustum_device.cuh"
+#include "warp_ops.cuh"
 
 namespace gvpm {
 
@@ -79,69 +80,22 @@ __global__ void __launch_bounds__(256) k_dispatch_classify(const __grid_constant
     }
     P.keepbits[i] = (uint8_t)bits;
   }
-  __shared__ uint32_t wcnt[8][GVPM_MAX_PEERS];
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  for (int d = 0; d < P.n_dst; ++d) {
-    const uint32_t m = __ballot_sync(0xffffffffu, (bits >> d) & 1u);
-    if (lane == 0) wcnt[w][d] = __popc(m);
-  }
+  __shared__ BallotCounts<8, GVPM_MAX_PEERS> kept;
+  for (int d = 0; d < P.n_dst; ++d) kept.put(__ballot_sync(0xffffffffu, (bits >> d) & 1u), d);
   __syncthreads();
-  if (threadIdx.x < (unsigned)P.n_dst) {
-    uint32_t t = 0;
-    for (int k = 0; k < 8; ++k) t += wcnt[k][threadIdx.x];
-    P.block_cnt[(size_t)threadIdx.x * (P.nb + 1) + blk] = t;
-  }
+  if (threadIdx.x < (unsigned)P.n_dst) P.block_cnt[(size_t)threadIdx.x * (P.nb + 1) + blk] = kept.total(threadIdx.x);
   __syncthreads();
   }
-}
-
-// one CTA per receiver: exclusive scan of nb counts in place, total at [nb]
-__global__ void __launch_bounds__(1024) k_dispatch_scan(uint32_t *__restrict__ block_cnt, uint32_t nb) {
-  uint32_t *v = block_cnt + (size_t)blockIdx.x * (nb + 1);
-  __shared__ uint32_t wsum[32];
-  __shared__ uint32_t carry;
-  if (threadIdx.x == 0) carry = 0u;
-  __syncthreads();
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  for (uint32_t base = 0; base < nb; base += 1024) {
-    const uint32_t i = base + threadIdx.x;
-    const uint32_t x = i < nb ? v[i] : 0u;
-    uint32_t s = x;
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t y = __shfl_up_sync(0xffffffffu, s, o);
-      if (lane >= o) s += y;
-    }
-    if (lane == 31) wsum[w] = s;
-    __syncthreads();
-    if (w == 0) {
-      uint32_t t = wsum[lane];
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, t, o);
-        if (lane >= o) t += y;
-      }
-      wsum[lane] = t;
-    }
-    __syncthreads();
-    const uint32_t pre = carry + (w ? wsum[w - 1] : 0u) + (s - x);
-    if (i < nb) v[i] = pre;
-    __syncthreads();
-    if (threadIdx.x == 1023) carry = pre + x;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) v[nb] = carry;
 }
 
 __global__ void __launch_bounds__(256) k_dispatch_emit(const __grid_constant__ DispatchParams P) {
   __shared__ float4 tile[8][32 * 9];   // per warp: 32 records x 8 float4, row stride 9 float4 (as k_pack_aos)
-  __shared__ uint32_t wcnt[8][GVPM_MAX_PEERS];
+  __shared__ BallotCounts<8, GVPM_MAX_PEERS> kept;
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   for (uint32_t blk = blockIdx.x; blk < P.nb; blk += gridDim.x) {
   const uint32_t i = blk * blockDim.x + threadIdx.x;
   const uint32_t bits = i < P.count ? P.keepbits[i] : 0u;
-  for (int d = 0; d < P.n_dst; ++d) {
-    const uint32_t m = __ballot_sync(0xffffffffu, (bits >> d) & 1u);
-    if (lane == 0) wcnt[w][d] = __popc(m);
-  }
+  for (int d = 0; d < P.n_dst; ++d) kept.put(__ballot_sync(0xffffffffu, (bits >> d) & 1u), d);
   float4 *t = tile[w];
   if (bits) {
     const size_t s = (size_t)P.begin + i;
@@ -151,8 +105,7 @@ __global__ void __launch_bounds__(256) k_dispatch_emit(const __grid_constant__ D
   for (int d = 0; d < P.n_dst; ++d) {
     const uint32_t m = __ballot_sync(0xffffffffu, (bits >> d) & 1u);
     if (m == 0u) continue;
-    uint32_t slot = P.block_cnt[(size_t)d * (P.nb + 1) + blk];
-    for (int k = 0; k < w; ++k) slot += wcnt[k][d];
+    const uint32_t slot = P.block_cnt[(size_t)d * (P.nb + 1) + blk] + kept.before(d);
     const uint32_t cnt = __popc(m);
     if (slot + cnt > P.region_cap) {
       if (lane == 0) atomicOr(P.overflow, 1u);
@@ -219,7 +172,7 @@ void launch_dispatch(const DispatchParams &P, cudaStream_t st, int ctas) {
   }
   const uint32_t grid = ctas > 0 ? (uint32_t)ctas < P.nb ? (uint32_t)ctas : P.nb : P.nb;
   k_dispatch_classify<<<grid, 256, 0, st>>>(P);
-  k_dispatch_scan<<<P.n_dst, 1024, 0, st>>>(P.block_cnt, P.nb);
+  k_scan_exclusive<uint32_t, 1><<<P.n_dst, 1024, 0, st>>>(P.block_cnt, P.nb, P.block_cnt + P.nb, P.nb + 1);
   k_dispatch_emit<<<grid, 256, 0, st>>>(P);
 }
 void launch_dispatch_signal(const SignalParams &P, cudaStream_t st) { k_dispatch_signal<<<1, 32, 0, st>>>(P); }

@@ -15,6 +15,8 @@
 //   is counted once whatever the tree.  Then the functor with its 4 offsets, a segmented warp scan by ray,
 //   and 27 float atomics per run.
 #include "beam_device.cuh"
+#include "launch_sizing.cuh"
+#include "warp_ops.cuh"
 
 namespace gvpm {
 
@@ -46,12 +48,7 @@ __global__ void k_subbeam_leaf_boxes(const float4 *__restrict__ subs, const floa
       h[a] = fmaxf(p1, p2);
     }
   }
-#pragma unroll
-  for (int a = 0; a < 3; ++a)
-    for (int o = 16; o > 0; o >>= 1) {
-      l[a] = fminf(l[a], __shfl_xor_sync(0xffffffffu, l[a], o));
-      h[a] = fmaxf(h[a], __shfl_xor_sync(0xffffffffu, h[a], o));
-    }
+  warp_box(l, h);
   if (lane == 0) {
     const float pad = radius * 1.0001f;
     lo[leaf] = make_float4(l[0] - pad, l[1] - pad, l[2] - pad, 0.f);
@@ -500,24 +497,7 @@ __global__ void __launch_bounds__(128, 4) k_beam_shade_sppm(const __grid_constan
       }
     }
     if (P.dump_pairs) continue;
-    const uint32_t kprev = __shfl_up_sync(0xffffffffu, key, 1);
-    const uint32_t heads = __ballot_sync(0xffffffffu, lane == 0 || kprev != key);
-    const int start = 31 - __clz(heads & (0xffffffffu >> (31 - lane)));
-#pragma unroll
-    for (int off = 1; off < 32; off <<= 1) {
-      const bool same = lane - off >= start;
-#pragma unroll
-      for (int j = 0; j < 3; ++j) {
-        const float vu = __shfl_up_sync(0xffffffffu, a[j], off);
-        if (same) a[j] += vu;
-      }
-    }
-    if (valid && (lane == 31 || (heads >> (lane + 1) & 1u))) {
-      float *o = P.out + (size_t)key * 3;
-#pragma unroll
-      for (int j = 0; j < 3; ++j)
-        if (a[j] != 0.f) atomicAdd(o + j, a[j]);
-    }
+    warp_run_sum<3, true>(key, a, valid, P.out, lane);
   }
 }
 
@@ -530,45 +510,23 @@ void launch_subbeam_leaf_boxes(const float4 *subs, const float4 *beams, uint32_t
   if (nLeaves) k_subbeam_leaf_boxes<<<(nLeaves + 7) / 8, 256, 0, st>>>(subs, beams, n, nLeaves, radius, lo, hi);
 }
 
-static int g_bt_blocks = 0, g_bs_blocks = 0;
 cudaError_t launch_beam_traverse(const GatherParams &P, int sm_count, cudaStream_t stream) {
   if (P.ray_end <= P.ray_begin) return cudaSuccess;
-  if (g_bt_blocks == 0) {
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&g_bt_blocks, k_beam_traverse, kBeamWarps * 32, 0);
-    if (g_bt_blocks < 1) g_bt_blocks = 1;
-  }
-  unsigned grid = (unsigned)(sm_count * g_bt_blocks);
   const unsigned packets = (P.ray_end - P.ray_begin + BPK - 1) / BPK;
-  const unsigned need = (packets + kBeamWarps - 1) / kBeamWarps;
-  if (grid > need) grid = need;
-  k_beam_traverse<<<grid, kBeamWarps * 32, 0, stream>>>(P);
+  const unsigned need = (packets + kBeamWarps - 1) / kBeamWarps;   // persistent: warps pull packets from a counter
+  k_beam_traverse<<<persistent_grid<k_beam_traverse>(sm_count, kBeamWarps * 32, need), kBeamWarps * 32, 0, stream>>>(P);
   return cudaGetLastError();
 }
 cudaError_t launch_beam_shade(const GatherParams &P, unsigned long long total, int sm_count, cudaStream_t stream) {
   if (total == 0) return cudaSuccess;
-  if (g_bs_blocks == 0) {
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&g_bs_blocks, k_beam_shade<false>, 128, 0);
-    if (g_bs_blocks < 1) g_bs_blocks = 1;
-  }
-  unsigned long long need = (total + 127) / 128;
-  unsigned long long grid = (unsigned long long)sm_count * g_bs_blocks * 4;
-  if (grid > need) grid = need;
-  if (P.cfg.beam_kernel_1d) k_beam_shade<true><<<(unsigned)grid, 128, 0, stream>>>(P);
-  else k_beam_shade<false><<<(unsigned)grid, 128, 0, stream>>>(P);
+  if (P.cfg.beam_kernel_1d) k_beam_shade<true><<<stride_grid<k_beam_shade<true>>(sm_count, 128, total), 128, 0, stream>>>(P);
+  else k_beam_shade<false><<<stride_grid<k_beam_shade<false>>(sm_count, 128, total), 128, 0, stream>>>(P);
   return cudaGetLastError();
 }
 
 cudaError_t launch_beam_shade_sppm(const GatherParams &P, unsigned long long total, int sm_count, cudaStream_t stream) {
   if (total == 0) return cudaSuccess;
-  static int blocks = 0;
-  if (blocks == 0) {
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_beam_shade_sppm, 128, 0);
-    if (blocks < 1) blocks = 1;
-  }
-  unsigned long long need = (total + 127) / 128;
-  unsigned long long grid = (unsigned long long)sm_count * blocks * 4;
-  if (grid > need) grid = need;
-  k_beam_shade_sppm<<<(unsigned)grid, 128, 0, stream>>>(P);
+  k_beam_shade_sppm<<<stride_grid<k_beam_shade_sppm>(sm_count, 128, total), 128, 0, stream>>>(P);
   return cudaGetLastError();
 }
 

@@ -18,6 +18,8 @@
 //   (shuffles) folds the lanes of one ray, and the last lane of each run adds 27 floats to the ray's
 //   output row.
 #include "bre_device.cuh"
+#include "launch_sizing.cuh"
+#include "warp_ops.cuh"
 
 namespace gvpm {
 
@@ -58,21 +60,6 @@ struct TileShared {
   uint32_t base[GVPM_MAX_LEVELS];
 };
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
-__device__ __forceinline__ float warp_min(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fminf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
 __device__ __forceinline__ float quad_sum(float v) {
   v += __shfl_xor_sync(0xffffffffu, v, 1);
   return v + __shfl_xor_sync(0xffffffffu, v, 2);
@@ -118,12 +105,7 @@ __device__ __forceinline__ void flush_candidates(const GatherParams &P, uint32_t
   }
   qn = 0;
   if (!DUMP) {
-    uint32_t incl = keep;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += v;
-    }
+    const uint32_t incl = warp_inclusive_scan(keep, lane);
     const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
     if (total) {
       unsigned long long base = 0;
@@ -580,95 +562,45 @@ k_bre_shade(const __grid_constant__ GatherParams P) {
     } else {
       bre_pairs_warp(P, pr, valid, a, shade_sh[threadIdx.x >> 5], lane);
     }
-    // segmented inclusive scan over RUNS of equal ray id (a ray's pairs arrive in contiguous runs,
-    // one per flush; the same ray may own several runs, each adds its own partial sum)
-    const uint32_t key = pr.x;
-    const uint32_t kprev = __shfl_up_sync(0xffffffffu, key, 1);
-    const uint32_t heads = __ballot_sync(0xffffffffu, lane == 0 || kprev != key);
-    const int start = 31 - __clz(heads & (0xffffffffu >> (31 - lane)));  // first lane of my run
-#pragma unroll
-    for (int off = 1; off < 32; off <<= 1) {
-      const bool same = lane - off >= start;
-#pragma unroll
-      for (int j = 0; j < GVPM_OUT_FLOATS; ++j) {
-        const float vu = __shfl_up_sync(0xffffffffu, a[j], off);
-        if (same) a[j] += vu;
-      }
-    }
-    if (valid && (lane == 31 || (heads >> (lane + 1) & 1u))) {
-      float *o = P.out + (size_t)key * GVPM_OUT_FLOATS;
-#pragma unroll
-      for (int j = 0; j < GVPM_OUT_FLOATS; ++j) atomicAdd(o + j, a[j]);
-    }
+    // per-ray sums over RUNS of equal ray id (a ray's pairs arrive in contiguous runs, one per flush; the same ray
+    // may own several runs, each adds its own partial sum)
+    warp_run_sum(pr.x, a, valid, P.out, lane);
   }
 }
 
 // ---- host-side launchers (called from the capi_*.cu units) -------------------------------------------
-static int g_trav_blocks[4] = {0, 0, 0, 0}, g_grid_blocks[4] = {0, 0, 0, 0}, g_shade_blocks[2] = {0, 0};
-
-template <int MODE> static void launch_traverse_mode(const GatherParams &P, int &bps, int sm_count, cudaStream_t stream) {
-  if (bps == 0) {
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_bre_traverse<MODE>, kTravWarps * 32, 0);
-    if (bps < 1) bps = 1;
-  }
-  // persistent grid: a whole number of resident CTAs per SM; warps pull tiles from a counter
-  unsigned grid = (unsigned)(sm_count * bps);
+// persistent grids: warps pull tiles of 32 rays from a counter
+template <int MODE> static void launch_traverse_mode(const GatherParams &P, int sm_count, cudaStream_t stream) {
   const unsigned tiles = (P.ray_end - P.ray_begin + 31) / 32;
   const unsigned need = (tiles + kTravWarps - 1) / kTravWarps;
-  if (grid > need) grid = need;
-  k_bre_traverse<MODE><<<grid, kTravWarps * 32, 0, stream>>>(P);
-}
-template <int MODE> static void launch_grid_mode(const GatherParams &P, int &bps, int sm_count, cudaStream_t stream) {
-  if (bps == 0) {
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_bre_grid_traverse<MODE>, kTravWarps * 32, 0);
-    if (bps < 1) bps = 1;
+  if (P.cell_start != nullptr) {   // frustum grid built for this ray set
+    const unsigned grid = persistent_grid<k_bre_grid_traverse<MODE>>(sm_count, kTravWarps * 32, need);
+    k_bre_grid_traverse<MODE><<<grid, kTravWarps * 32, 0, stream>>>(P);
+  } else {
+    const unsigned grid = persistent_grid<k_bre_traverse<MODE>>(sm_count, kTravWarps * 32, need);
+    k_bre_traverse<MODE><<<grid, kTravWarps * 32, 0, stream>>>(P);
   }
-  unsigned grid = (unsigned)(sm_count * bps);
-  const unsigned tiles = (P.ray_end - P.ray_begin + 31) / 32;
-  const unsigned need = (tiles + kTravWarps - 1) / kTravWarps;
-  if (grid > need) grid = need;
-  k_bre_grid_traverse<MODE><<<grid, kTravWarps * 32, 0, stream>>>(P);
 }
-template <bool SPPM> static void launch_shade_mode(const GatherParams &P, unsigned long long total, int &blocks,
-                                                   int sm_count, cudaStream_t stream) {
-  if (blocks == 0) {
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_bre_shade<SPPM>, GVPM_SHADE_THREADS, 0);
-    if (blocks < 1) blocks = 1;
-  }
+template <bool SPPM> static void launch_shade_mode(const GatherParams &P, unsigned long long total, int sm_count,
+                                                   cudaStream_t stream) {
   // total == ~0: the count is only known on the device (the kernel reads it): size the grid for a full pair list
   if (total == ~0ull || total > P.pair_cap) total = P.pair_cap;
-  unsigned long long need = (total + GVPM_SHADE_THREADS - 1) / GVPM_SHADE_THREADS;
-  if (need == 0) need = 1;
-  unsigned long long grid = (unsigned long long)sm_count * blocks * 4;  // a few waves, grid-stride
-  if (grid > need) grid = need;
-  k_bre_shade<SPPM><<<(unsigned)grid, GVPM_SHADE_THREADS, 0, stream>>>(P);
+  const unsigned grid = stride_grid<k_bre_shade<SPPM>>(sm_count, GVPM_SHADE_THREADS, total);
+  k_bre_shade<SPPM><<<grid, GVPM_SHADE_THREADS, 0, stream>>>(P);
 }
 
 cudaError_t launch_bre_traverse(const GatherParams &P, bool dump, int sm_count, cudaStream_t stream) {
   if (P.ray_end <= P.ray_begin) return cudaSuccess;
-  const int mode = (dump ? 1 : 0) | (P.cfg.sppm_primal ? 2 : 0);
-  if (P.cell_start != nullptr) {   // frustum grid built for this ray set
-    switch (mode) {
-      case 0: launch_grid_mode<0>(P, g_grid_blocks[0], sm_count, stream); break;
-      case 1: launch_grid_mode<1>(P, g_grid_blocks[1], sm_count, stream); break;
-      case 2: launch_grid_mode<2>(P, g_grid_blocks[2], sm_count, stream); break;
-      default: launch_grid_mode<3>(P, g_grid_blocks[3], sm_count, stream); break;
-    }
-    return cudaGetLastError();
-  }
-  switch (mode) {
-    case 0: launch_traverse_mode<0>(P, g_trav_blocks[0], sm_count, stream); break;
-    case 1: launch_traverse_mode<1>(P, g_trav_blocks[1], sm_count, stream); break;
-    case 2: launch_traverse_mode<2>(P, g_trav_blocks[2], sm_count, stream); break;
-    default: launch_traverse_mode<3>(P, g_trav_blocks[3], sm_count, stream); break;
-  }
+  static void (*const kByMode[4])(const GatherParams &, int, cudaStream_t) = {
+      launch_traverse_mode<0>, launch_traverse_mode<1>, launch_traverse_mode<2>, launch_traverse_mode<3>};
+  kByMode[(dump ? 1 : 0) | (P.cfg.sppm_primal ? 2 : 0)](P, sm_count, stream);
   return cudaGetLastError();
 }
 
 cudaError_t launch_bre_shade(const GatherParams &P, unsigned long long total, int sm_count, cudaStream_t stream) {
   if (total == 0) return cudaSuccess;
-  if (P.cfg.sppm_primal) launch_shade_mode<true>(P, total, g_shade_blocks[1], sm_count, stream);
-  else launch_shade_mode<false>(P, total, g_shade_blocks[0], sm_count, stream);
+  if (P.cfg.sppm_primal) launch_shade_mode<true>(P, total, sm_count, stream);
+  else launch_shade_mode<false>(P, total, sm_count, stream);
   return cudaGetLastError();
 }
 

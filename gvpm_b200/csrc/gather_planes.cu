@@ -16,7 +16,9 @@
 //           shared-memory queue.  Phase B: lanes pop their queues and run the strictly rounded intersection + the
 //           functor with its 4 specular shifts, so the divergent, transcendental-heavy shading runs with (nearly)
 //           full lanes although only ~1 in 10 tests hits.
+#include "launch_sizing.cuh"
 #include "plane_device.cuh"
+#include "warp_ops.cuh"
 
 namespace gvpm {
 
@@ -50,12 +52,7 @@ __global__ void k_plane_leaf_boxes(const float4 *__restrict__ planes, uint32_t n
       h[c] = fmaxf(fmaxf(p0, p1), fmaxf(p2, p3));
     }
   }
-#pragma unroll
-  for (int c = 0; c < 3; ++c)
-    for (int o = 16; o > 0; o >>= 1) {
-      l[c] = fminf(l[c], __shfl_xor_sync(0xffffffffu, l[c], o));
-      h[c] = fmaxf(h[c], __shfl_xor_sync(0xffffffffu, h[c], o));
-    }
+  warp_box(l, h);
   if (lane == 0) {
     lo[leaf] = make_float4(l[0], l[1], l[2], 0.f);
     hi[leaf] = make_float4(h[0], h[1], h[2], 0.f);
@@ -187,12 +184,7 @@ __global__ void __launch_bounds__(kPlWarps * 32, 4) k_plane_gather(const __grid_
           h[c] = fmaxf(pa, pb);
         }
       }
-#pragma unroll
-      for (int c = 0; c < 3; ++c)
-        for (int o = 16; o > 0; o >>= 1) {
-          l[c] = fminf(l[c], __shfl_xor_sync(0xffffffffu, l[c], o));
-          h[c] = fmaxf(h[c], __shfl_xor_sync(0xffffffffu, h[c], o));
-        }
+      warp_box(l, h);
       if (lane == 0) {
 #pragma unroll
         for (int c = 0; c < 3; ++c) { S.red[w][c] = l[c]; S.red[w][3 + c] = h[c]; }
@@ -246,11 +238,7 @@ __global__ void __launch_bounds__(kPlWarps * 32, 4) k_plane_gather(const __grid_
         r8[5] = mint; r8[6] = maxt; r8[7] = z;
       }
 #pragma unroll
-      for (int k = 0; k < 8; ++k)
-        for (int o = 16; o > 0; o >>= 1) {
-          const float v = __shfl_xor_sync(0xffffffffu, r8[k], o);
-          r8[k] = (k == 0 || k == 2 || k == 5 || k == 7) ? fminf(r8[k], v) : fmaxf(r8[k], v);
-        }
+      for (int k = 0; k < 8; ++k) r8[k] = (k == 0 || k == 2 || k == 5 || k == 7) ? warp_min(r8[k]) : warp_max(r8[k]);
       if (lane == 0) {
 #pragma unroll
         for (int k = 0; k < 8; ++k) S.tred[w][k] = r8[k];
@@ -410,23 +398,13 @@ void launch_plane_leaf_boxes(const float4 *planes, uint32_t n, uint32_t nLeaves,
   if (nLeaves) k_plane_leaf_boxes<<<(nLeaves + 7) / 8, 256, 0, st>>>(planes, n, nLeaves, lo, hi);
 }
 
-static int g_pl_blocks[2] = {0, 0};
 cudaError_t launch_plane_gather(const GatherParams &P, bool dump, int sm_count, cudaStream_t stream) {
   if (P.n_rays == 0) return cudaSuccess;
   const size_t smem = sizeof(PlaneShared);
-  const int which = dump ? 1 : 0;
-  if (g_pl_blocks[which] == 0) {
-    cudaError_t e = dump ? cudaFuncSetAttribute(k_plane_gather<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                         : cudaFuncSetAttribute(k_plane_gather<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    int nb = 0;
-    if (dump) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_plane_gather<true>, kPlWarps * 32, smem);
-    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_plane_gather<false>, kPlWarps * 32, smem);
-    g_pl_blocks[which] = nb < 1 ? 1 : nb;
-  }
-  unsigned grid = (unsigned)(sm_count * g_pl_blocks[which]);
-  const unsigned need = (P.n_rays + kPlWarps * 32 - 1) / (kPlWarps * 32);
-  if (grid > need) grid = need;
+  const unsigned need = (P.n_rays + kPlWarps * 32 - 1) / (kPlWarps * 32);   // persistent: CTAs pull ray blocks
+  const unsigned grid = dump ? persistent_grid<k_plane_gather<true>>(sm_count, kPlWarps * 32, need, smem)
+                             : persistent_grid<k_plane_gather<false>>(sm_count, kPlWarps * 32, need, smem);
+  if (grid == 0) return cudaGetLastError();   // the shared-memory attribute was refused
   if (dump) k_plane_gather<true><<<grid, kPlWarps * 32, smem, stream>>>(P);
   else k_plane_gather<false><<<grid, kPlWarps * 32, smem, stream>>>(P);
   return cudaGetLastError();

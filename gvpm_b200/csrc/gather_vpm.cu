@@ -13,6 +13,8 @@
 // k_vpm_shade: one thread per pair, same structure as k_bre_shade; the per-sample results are scaled by
 //   1/nbCameraSamples and folded into the ray's 27 accumulators.
 #include "bre_device.cuh"
+#include "launch_sizing.cuh"
+#include "warp_ops.cuh"
 
 namespace gvpm {
 
@@ -218,55 +220,22 @@ __global__ void __launch_bounds__(128, 4) k_vpm_shade(const __grid_constant__ Ga
 #pragma unroll
       for (int j = 0; j < GVPM_OUT_FLOATS; ++j) a[j] *= normalization;
     }
-    // segmented inclusive scan over runs of equal ray index (samples of a ray are adjacent)
-    const uint32_t kprev = __shfl_up_sync(0xffffffffu, key, 1);
-    const uint32_t heads = __ballot_sync(0xffffffffu, lane == 0 || kprev != key);
-    const int start = 31 - __clz(heads & (0xffffffffu >> (31 - lane)));
-#pragma unroll
-    for (int off = 1; off < 32; off <<= 1) {
-      const bool same = lane - off >= start;
-#pragma unroll
-      for (int j = 0; j < GVPM_OUT_FLOATS; ++j) {
-        const float vu = __shfl_up_sync(0xffffffffu, a[j], off);
-        if (same) a[j] += vu;
-      }
-    }
-    if (valid && (lane == 31 || (heads >> (lane + 1) & 1u))) {
-      float *o = P.out + (size_t)key * GVPM_OUT_FLOATS;
-#pragma unroll
-      for (int j = 0; j < GVPM_OUT_FLOATS; ++j) atomicAdd(o + j, a[j]);
-    }
+    // per-ray sums over runs of equal ray index (samples of a ray are adjacent)
+    warp_run_sum(key, a, valid, P.out, lane);
   }
 }
 
-static int g_vt_blocks[2] = {0, 0}, g_vs_blocks = 0;
-
 cudaError_t launch_vpm_traverse(const GatherParams &P, bool dump, int sm_count, cudaStream_t stream) {
   if (P.n_samples == 0) return cudaSuccess;
-  int &bps = g_vt_blocks[dump ? 1 : 0];
-  if (bps == 0) {
-    if (dump) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_vpm_traverse<true>, kVpmWarps * 32, 0);
-    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_vpm_traverse<false>, kVpmWarps * 32, 0);
-    if (bps < 1) bps = 1;
-  }
-  unsigned grid = (unsigned)(sm_count * bps);
-  const unsigned need = (P.n_samples + kVpmWarps - 1) / kVpmWarps;
-  if (grid > need) grid = need;
-  if (dump) k_vpm_traverse<true><<<grid, kVpmWarps * 32, 0, stream>>>(P);
-  else k_vpm_traverse<false><<<grid, kVpmWarps * 32, 0, stream>>>(P);
+  const unsigned need = (P.n_samples + kVpmWarps - 1) / kVpmWarps;   // persistent: warps pull samples from a counter
+  if (dump) k_vpm_traverse<true><<<persistent_grid<k_vpm_traverse<true>>(sm_count, kVpmWarps * 32, need), kVpmWarps * 32, 0, stream>>>(P);
+  else k_vpm_traverse<false><<<persistent_grid<k_vpm_traverse<false>>(sm_count, kVpmWarps * 32, need), kVpmWarps * 32, 0, stream>>>(P);
   return cudaGetLastError();
 }
 
 cudaError_t launch_vpm_shade(const GatherParams &P, unsigned long long total, int sm_count, cudaStream_t stream) {
   if (total == 0) return cudaSuccess;
-  if (g_vs_blocks == 0) {
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&g_vs_blocks, k_vpm_shade, 128, 0);
-    if (g_vs_blocks < 1) g_vs_blocks = 1;
-  }
-  unsigned long long need = (total + 127) / 128;
-  unsigned long long grid = (unsigned long long)sm_count * g_vs_blocks * 4;
-  if (grid > need) grid = need;
-  k_vpm_shade<<<(unsigned)grid, 128, 0, stream>>>(P);
+  k_vpm_shade<<<stride_grid<k_vpm_shade>(sm_count, 128, total), 128, 0, stream>>>(P);
   return cudaGetLastError();
 }
 

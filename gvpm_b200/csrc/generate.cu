@@ -13,6 +13,7 @@
 // operation order; log, exp, sin and cos are polynomial routines (pm_*) built from +, -, *, / only, so a CPU
 // restatement compiled without FMA contraction reproduces every record bit for bit (tests/test_gpu_generate.py).
 #include "gvpm_device.cuh"
+#include "warp_ops.cuh"
 
 namespace gvpm {
 
@@ -359,77 +360,23 @@ __device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned lon
 // pass 1: photons per path; block totals of (photons, contributing paths) packed as (paths << 40 | photons)
 __global__ void __launch_bounds__(256) k_trace_count(const __grid_constant__ TraceParams P, uint8_t *__restrict__ counts,
                                                       unsigned long long *__restrict__ block_tot) {
-  __shared__ unsigned long long ws[8];
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
   uint32_t c = 0;
   if (k < P.n_paths) {
     c = walk_path<false>(P, P.path_base + k, 0ull, 0u);
     counts[k] = (uint8_t)c;
   }
-  unsigned long long v = (unsigned long long)c | ((unsigned long long)(c ? 1u : 0u) << 40);
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = v;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned long long t = 0;
-    for (int i = 0; i < 8; ++i) t += ws[i];
-    block_tot[blockIdx.x] = t;
-  }
-}
-// exclusive scan of the block totals by one block; total -> total_out[0]
-__global__ void __launch_bounds__(1024) k_trace_scan(unsigned long long *__restrict__ block_tot, uint32_t nb,
-                                                      unsigned long long *__restrict__ total_out) {
-  __shared__ unsigned long long ws[32];
-  __shared__ unsigned long long carry;
-  if (threadIdx.x == 0) carry = 0;
-  __syncthreads();
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  for (uint32_t base = 0; base < nb; base += 1024) {
-    const uint32_t i = base + threadIdx.x;
-    const unsigned long long v = i < nb ? block_tot[i] : 0ull;
-    unsigned long long inc = v;
-    for (int o = 1; o < 32; o <<= 1) {
-      const unsigned long long u = __shfl_up_sync(0xffffffffu, inc, o);
-      if (lane >= o) inc += u;
-    }
-    if (lane == 31) ws[w] = inc;
-    __syncthreads();
-    if (w == 0) {
-      const unsigned long long x = ws[lane];
-      unsigned long long xi = x;
-      for (int o = 1; o < 32; o <<= 1) {
-        const unsigned long long u = __shfl_up_sync(0xffffffffu, xi, o);
-        if (lane >= o) xi += u;
-      }
-      ws[lane] = xi - x;
-    }
-    __syncthreads();
-    const unsigned long long excl = carry + ws[w] + (inc - v);
-    if (i < nb) block_tot[i] = excl;
-    __syncthreads();
-    if (threadIdx.x == 1023) carry = excl + v;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) total_out[0] = carry;
+  const unsigned long long t = block_total<8>((unsigned long long)c | ((unsigned long long)(c ? 1u : 0u) << 40));
+  if (threadIdx.x == 0) block_tot[blockIdx.x] = t;
 }
 // pass 2: the same walks, stored.  last_path[0] = 1 + index of the path that stored photon n_total - 1.
 __global__ void __launch_bounds__(256) k_trace_emit(const __grid_constant__ TraceParams P, const uint8_t *__restrict__ counts,
                                                      const unsigned long long *__restrict__ block_off,
                                                      unsigned long long *__restrict__ last_path) {
-  __shared__ unsigned long long ws[8];
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const uint32_t c = k < P.n_paths ? counts[k] : 0u;
-  const unsigned long long v = (unsigned long long)c | ((unsigned long long)(c ? 1u : 0u) << 40);
-  unsigned long long inc = v;
-  for (int o = 1; o < 32; o <<= 1) {
-    const unsigned long long u = __shfl_up_sync(0xffffffffu, inc, o);
-    if (lane >= o) inc += u;
-  }
-  if (lane == 31) ws[w] = inc;
-  __syncthreads();
-  unsigned long long excl = block_off[blockIdx.x] + (inc - v);
-  for (int i = 0; i < w; ++i) excl += ws[i];
+  const unsigned long long excl =
+      block_off[blockIdx.x] + block_exclusive<8>((unsigned long long)c | ((unsigned long long)(c ? 1u : 0u) << 40));
   if (c == 0) return;
   const unsigned long long first = P.slot_base + (excl & ((1ull << 40) - 1ull));
   const uint32_t pid = P.path_id_base + (uint32_t)(excl >> 40);
@@ -449,7 +396,7 @@ void launch_trace_count(const TraceParams &P, uint8_t *counts, unsigned long lon
                         cudaStream_t st) {
   const uint32_t nb = (P.n_paths + 255) / 256;
   if (nb) k_trace_count<<<nb, 256, 0, st>>>(P, counts, block_tot);
-  k_trace_scan<<<1, 1024, 0, st>>>(block_tot, nb, totals);
+  k_scan_exclusive<unsigned long long, 1><<<1, 1024, 0, st>>>(block_tot, nb, totals, 0);
 }
 void launch_trace_emit(const TraceParams &P, const uint8_t *counts, const unsigned long long *block_off,
                        unsigned long long *last_path, cudaStream_t st) {

@@ -8,6 +8,7 @@
 //   SubBeamBVH constructor (sub-beam cuts)          photonmapper/beams_accel.h:98-124
 //   PhotonPlane edges / getCenter                   photonmapper/plane_struct.h:45-74,107-108
 #include "gvpm_device.cuh"
+#include "warp_ops.cuh"
 
 namespace gvpm {
 
@@ -71,86 +72,23 @@ __device__ __forceinline__ int beam_nsub(float len, float subbeamSize) {
   return nSub < 1 ? 1 : nSub;
 }
 
-// per-beam sub-beam count -> exclusive offsets: block totals (k_sub_count), one-block scan of them (k_sub_scan), and the
-// emit pass re-scans inside each block
+// per-beam sub-beam count -> exclusive offsets: block totals (k_sub_count), one-block scan of them (k_scan_exclusive), and
+// the emit pass re-scans inside each block
 __global__ void __launch_bounds__(256) k_sub_count(const float *__restrict__ len, uint32_t n, const float *__restrict__ subsize,
                                                     uint32_t *__restrict__ block_tot) {
-  __shared__ uint32_t ws[8];
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  uint32_t c = i < n ? (uint32_t)beam_nsub(len[i], subsize[0]) : 0u;
-  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-  if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    uint32_t t = 0;
-    for (int k = 0; k < 8; ++k) t += ws[k];
-    block_tot[blockIdx.x] = t;
-  }
-}
-// exclusive scan of nb block totals in place by ONE block (a few thousand to a few ten thousand entries: every thread
-// owns 8 consecutive ones, 8192 per round); total -> total_out[0]
-__global__ void __launch_bounds__(1024) k_sub_scan(uint32_t *__restrict__ block_tot, uint32_t nb, uint32_t *__restrict__ total_out) {
-  __shared__ uint32_t ws[32];
-  __shared__ uint32_t carry;
-  if (threadIdx.x == 0) carry = 0;
-  __syncthreads();
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  constexpr uint32_t kPer = 8;
-  for (uint32_t base = 0; base < nb; base += 1024 * kPer) {
-    const uint32_t i0 = base + threadIdx.x * kPer;
-    uint32_t v[kPer], sum = 0u;
-#pragma unroll
-    for (uint32_t k = 0; k < kPer; ++k) {
-      v[k] = i0 + k < nb ? block_tot[i0 + k] : 0u;
-      sum += v[k];
-    }
-    uint32_t inc = sum;
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t u = __shfl_up_sync(0xffffffffu, inc, o);
-      if (lane >= o) inc += u;
-    }
-    if (lane == 31) ws[w] = inc;
-    __syncthreads();
-    if (w == 0) {
-      uint32_t x = ws[lane], xi = x;
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t u = __shfl_up_sync(0xffffffffu, xi, o);
-        if (lane >= o) xi += u;
-      }
-      ws[lane] = xi - x;   // exclusive prefix of the warp totals
-    }
-    __syncthreads();
-    uint32_t excl = carry + ws[w] + (inc - sum);
-#pragma unroll
-    for (uint32_t k = 0; k < kPer; ++k) {
-      if (i0 + k < nb) block_tot[i0 + k] = excl;
-      excl += v[k];
-    }
-    __syncthreads();
-    if (threadIdx.x == 1023) carry = excl;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) total_out[0] = carry;
+  const uint32_t t = block_total<8>(i < n ? (uint32_t)beam_nsub(len[i], subsize[0]) : 0u);
+  if (threadIdx.x == 0) block_tot[blockIdx.x] = t;
 }
 // sub-beam records in beam order: pos = midpoint (Hilbert key input), raw = (t1, t2, beam index, flags)
 //   flags: bit 0 first, bit 1 last sub-beam of its beam, bits 2.. ordinal (the naive sppm technique's RNG dimension)
 __global__ void __launch_bounds__(256) k_sub_emit(const float4 *__restrict__ rec, const float *__restrict__ len, uint32_t n,
                                                    const float *__restrict__ subsize, const uint32_t *__restrict__ block_off,
                                                    uint32_t cap, float *__restrict__ sub_pos, float4 *__restrict__ sub_raw) {
-  __shared__ uint32_t ws[8];
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const float L = i < n ? len[i] : 0.f;
   const int nSub = i < n ? beam_nsub(L, subsize[0]) : 0;
-  uint32_t inc = (uint32_t)nSub;
-  for (int o = 1; o < 32; o <<= 1) {
-    const uint32_t u = __shfl_up_sync(0xffffffffu, inc, o);
-    if (lane >= o) inc += u;
-  }
-  if (lane == 31) ws[w] = inc;
-  __syncthreads();
-  uint32_t off = block_off[blockIdx.x] + inc - (uint32_t)nSub;
-  for (int k = 0; k < w; ++k) off += ws[k];
+  const uint32_t off = block_off[blockIdx.x] + block_exclusive<8>((uint32_t)nSub);
   if (i >= n) return;
   const float4 b0 = rec[(size_t)i * 8], b1 = rec[(size_t)i * 8 + 1];
   const float lengthSub = __fdiv_rn(L, (float)nSub);
@@ -210,7 +148,7 @@ __global__ void __launch_bounds__(256) k_pack_samples(const SampleStaging S, uin
                                             S.transmittance[3 * (size_t)i + 2], __uint_as_float(rb));
   }
   rad = fmaxf(rad, 0.f);
-  for (int o = 16; o > 0; o >>= 1) rad = fmaxf(rad, __shfl_xor_sync(0xffffffffu, rad, o));
+  rad = warp_max(rad);
   const uint32_t anyBad = __ballot_sync(0xffffffffu, bad);
   if ((threadIdx.x & 31) == 0) {
     atomicMax(stats, __float_as_uint(rad));
@@ -250,10 +188,8 @@ void launch_beam_subsize_seq(const float *len, uint32_t n, float *subsize, cudaS
 void launch_sub_count(const float *len, uint32_t n, const float *subsize, uint32_t *block_tot, uint32_t *total, cudaStream_t st) {
   const uint32_t nb = (n + 255) / 256;
   if (n) k_sub_count<<<nb, 256, 0, st>>>(len, n, subsize, block_tot);
-  k_sub_scan<<<1, 1024, 0, st>>>(block_tot, n ? nb : 0u, total);
+  k_scan_exclusive<uint32_t, 8><<<1, 1024, 0, st>>>(block_tot, n ? nb : 0u, total, 0);   // 8 per thread: tens of thousands
 }
-// in-place exclusive scan of nb words by one block (a few thousand entries); total -> total[0]
-void launch_scan_u32(uint32_t *vals, uint32_t nb, uint32_t *total, cudaStream_t st) { k_sub_scan<<<1, 1024, 0, st>>>(vals, nb, total); }
 void launch_sub_emit(const float4 *rec, const float *len, uint32_t n, const float *subsize, const uint32_t *block_off,
                      uint32_t cap, float *sub_pos, float4 *sub_raw, cudaStream_t st) {
   if (n) k_sub_emit<<<(n + 255) / 256, 256, 0, st>>>(rec, len, n, subsize, block_off, cap, sub_pos, sub_raw);

@@ -17,6 +17,7 @@
 #include <cfloat>
 
 #include "gvpm_device.cuh"
+#include "warp_ops.cuh"
 
 namespace gvpm {
 
@@ -46,7 +47,7 @@ __device__ __forceinline__ void reduce3_finish(f3 v, float *partial, unsigned *t
   float c[3] = {v.x, v.y, v.z};
 #pragma unroll
   for (int a = 0; a < 3; ++a) {
-    for (int o = 16; o > 0; o >>= 1) c[a] += __shfl_xor_sync(0xffffffffu, c[a], o);
+    c[a] = warp_sum(c[a]);
     if (lane == 0) sh[a][w] = c[a];
   }
   __syncthreads();
@@ -67,7 +68,7 @@ __device__ __forceinline__ void reduce3_finish(f3 v, float *partial, unsigned *t
     for (int a = 0; a < 3; ++a) t[a] += ((volatile float *)partial)[3 * b + a];
 #pragma unroll
   for (int a = 0; a < 3; ++a) {
-    for (int o = 16; o > 0; o >>= 1) t[a] += __shfl_xor_sync(0xffffffffu, t[a], o);
+    t[a] = warp_sum(t[a]);
     if (lane == 0) sh[a][w] = t[a];
   }
   __syncthreads();

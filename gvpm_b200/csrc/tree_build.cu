@@ -13,6 +13,7 @@
 
 #include "gvpm_device.cuh"
 #include "frustum_device.cuh"
+#include "warp_ops.cuh"
 
 namespace gvpm {
 
@@ -29,26 +30,22 @@ __global__ void k_bounds_partial(const float *__restrict__ pos, uint32_t stride,
   }
   __shared__ float s[6][32];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  warp_box(lo, hi);
+  if (lane == 0)
 #pragma unroll
-  for (int a = 0; a < 3; ++a) {
-    for (int o = 16; o > 0; o >>= 1) {
-      lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
-      hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
-    }
-    if (lane == 0) { s[a][w] = lo[a]; s[3 + a][w] = hi[a]; }
-  }
+    for (int a = 0; a < 3; ++a) { s[a][w] = lo[a]; s[3 + a][w] = hi[a]; }
   __syncthreads();
   if (w == 0) {
     const int nw = blockDim.x >> 5;
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
-      float l = lane < nw ? s[a][lane] : INFINITY, h = lane < nw ? s[3 + a][lane] : -INFINITY;
-      for (int o = 16; o > 0; o >>= 1) {
-        l = fminf(l, __shfl_xor_sync(0xffffffffu, l, o));
-        h = fmaxf(h, __shfl_xor_sync(0xffffffffu, h, o));
-      }
-      if (lane == 0) { partial[6 * blockIdx.x + a] = l; partial[6 * blockIdx.x + 3 + a] = h; }
+      lo[a] = lane < nw ? s[a][lane] : INFINITY;
+      hi[a] = lane < nw ? s[3 + a][lane] : -INFINITY;
     }
+    warp_box(lo, hi);
+    if (lane == 0)
+#pragma unroll
+      for (int a = 0; a < 3; ++a) { partial[6 * blockIdx.x + a] = lo[a]; partial[6 * blockIdx.x + 3 + a] = hi[a]; }
   }
 }
 // bounds[0..2] = min, [3..5] = max, [6] = max |coordinate|
@@ -61,15 +58,10 @@ __global__ void k_bounds_final(const float *__restrict__ partial, int nblocks, f
       lo[a] = fminf(lo[a], partial[6 * b + a]);
       hi[a] = fmaxf(hi[a], partial[6 * b + 3 + a]);
     }
+  warp_box(lo, hi);
   float mag = 0.f;
 #pragma unroll
-  for (int a = 0; a < 3; ++a) {
-    for (int o = 16; o > 0; o >>= 1) {
-      lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
-      hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
-    }
-    mag = fmaxf(mag, fmaxf(fabsf(lo[a]), fabsf(hi[a])));
-  }
+  for (int a = 0; a < 3; ++a) mag = fmaxf(mag, fmaxf(fabsf(lo[a]), fabsf(hi[a])));
   if (lane == 0) {
     for (int a = 0; a < 3; ++a) { bounds[a] = lo[a]; bounds[3 + a] = hi[a]; }
     bounds[6] = mag;
@@ -178,12 +170,7 @@ __global__ void k_leaf_boxes(const float4 *__restrict__ p0, uint32_t n, uint32_t
     const float4 p = p0[i];
     l[0] = h[0] = p.x; l[1] = h[1] = p.y; l[2] = h[2] = p.z;
   }
-#pragma unroll
-  for (int a = 0; a < 3; ++a)
-    for (int o = 16; o > 0; o >>= 1) {
-      l[a] = fminf(l[a], __shfl_xor_sync(0xffffffffu, l[a], o));
-      h[a] = fmaxf(h[a], __shfl_xor_sync(0xffffffffu, h[a], o));
-    }
+  warp_box(l, h);
   if (lane == 0) {
     lo[leaf] = make_float4(l[0] - radius, l[1] - radius, l[2] - radius, 0.f);
     hi[leaf] = make_float4(h[0] + radius, h[1] + radius, h[2] + radius, 0.f);
@@ -202,12 +189,7 @@ __global__ void k_level_boxes(const float4 *__restrict__ clo, const float4 *__re
     const float4 a = clo[i], b = chi[i];
     l[0] = a.x; l[1] = a.y; l[2] = a.z; h[0] = b.x; h[1] = b.y; h[2] = b.z;
   }
-#pragma unroll
-  for (int a = 0; a < 3; ++a)
-    for (int o = 16; o > 0; o >>= 1) {
-      l[a] = fminf(l[a], __shfl_xor_sync(0xffffffffu, l[a], o));
-      h[a] = fmaxf(h[a], __shfl_xor_sync(0xffffffffu, h[a], o));
-    }
+  warp_box(l, h);
   if (lane == 0) {
     plo[node] = make_float4(l[0], l[1], l[2], 0.f);
     phi[node] = make_float4(h[0], h[1], h[2], 0.f);
@@ -259,16 +241,11 @@ __global__ void k_ray_box(const float4 *__restrict__ rays, uint32_t n, float r, 
       hi[a] = fmaxf(hi[a], fmaxf(p0[a], p1[a]));
     }
   }
+  warp_box(lo, hi);
+  if ((threadIdx.x & 31) == 0)
 #pragma unroll
-  for (int a = 0; a < 3; ++a) {
-    for (int o = 16; o > 0; o >>= 1) {
-      lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
-      hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
-    }
-    if ((threadIdx.x & 31) == 0) {
+    for (int a = 0; a < 3; ++a)
       if (lo[a] <= hi[a]) { atomic_min_float(box + a, lo[a]); atomic_max_float(box + 3 + a, hi[a]); }
-    }
-  }
 }
 // box[0..5] -> grid parameters + the 7-float bounds block the traversal reads (min, max, max |coordinate|)
 __global__ void k_ray_box_final(const float *__restrict__ box, float r, RayGrid *__restrict__ g, float *__restrict__ bounds) {
@@ -338,7 +315,7 @@ __global__ void __launch_bounds__(256) k_ray_mask(const float4 *__restrict__ ray
       const float bx = p1[0] - c1[0], by = p1[1] - c1[1], bz = p1[2] - c1[2];
       spread = fmaxf(sqrtf(ax * ax + ay * ay + az * az), sqrtf(bx * bx + by * by + bz * bz));
     }
-    for (int o = 16; o > 0; o >>= 1) spread = fmaxf(spread, __shfl_xor_sync(0xffffffffu, spread, o));
+    spread = warp_max(spread);
     // (a bundle a few cells wide: the rays of a pixel patch fill the dilated region anyway, so nothing is over-marked)
     const bool coherent = spread <= 4.f * G.cmax;
     if (coherent) {  // all lanes work on the first segment
@@ -369,9 +346,8 @@ __global__ void __launch_bounds__(256) k_ray_mask(const float4 *__restrict__ ray
 __global__ void __launch_bounds__(256) k_keep_pruned(const float *__restrict__ pos, uint32_t n, const RayGrid *__restrict__ gp,
                               const uint32_t *__restrict__ gmask, uint32_t *__restrict__ keepmask,
                               uint32_t *__restrict__ block_kept) {
-  __shared__ uint32_t warpCount[8];
+  __shared__ BallotCounts<8> kept;
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   bool keep = false;
   if (i < n) {
     const RayGrid &G = *gp;
@@ -383,17 +359,10 @@ __global__ void __launch_bounds__(256) k_keep_pruned(const float *__restrict__ p
     }
   }
   const uint32_t km = __ballot_sync(0xffffffffu, keep);
-  if (lane == 0) {
-    warpCount[w] = __popc(km);
-    if (i < n) keepmask[i >> 5] = km;
-  }
+  if ((threadIdx.x & 31) == 0 && i < n) keepmask[i >> 5] = km;
+  kept.put(km);
   __syncthreads();
-  if (threadIdx.x == 0) {
-    uint32_t tot = 0;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) tot += warpCount[k];
-    block_kept[blockIdx.x] = tot;
-  }
+  if (threadIdx.x == 0) block_kept[blockIdx.x] = kept.total();
 }
 // Pass 2 over the m kept photons: 30-bit Hilbert key, quantised in the grid box
 __global__ void k_keys_kept(const float *__restrict__ pos, const uint32_t *__restrict__ vals, uint32_t m,
@@ -461,8 +430,7 @@ __global__ void __launch_bounds__(256) k_pinhole_accum(const float4 *__restrict_
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
 #pragma unroll
   for (int k = 0; k < 13; ++k) {
-    double v = acc[k];
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    const double v = warp_sum(acc[k]);
     if (lane == 0) sh[w][k] = v;
   }
   __syncthreads();
@@ -535,8 +503,7 @@ __global__ void __launch_bounds__(256) k_pinhole_check(const float4 *__restrict_
   }
 #pragma unroll
   for (int k = 0; k < 6; ++k) {
-    float vv = mx[k];
-    for (int o = 16; o > 0; o >>= 1) vv = fmaxf(vv, __shfl_xor_sync(0xffffffffu, vv, o));
+    const float vv = warp_max(mx[k]);
     // monotone map float -> unsigned (handles negatives)
     const unsigned b = __float_as_uint(vv);
     const unsigned key = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
@@ -611,7 +578,7 @@ __global__ void __launch_bounds__(256) k_frustum_keys(const float *__restrict__ 
   // one atomic per CTA, and only while the CTA's maximum beats what is already there (a single hot address otherwise
   // serialises hundreds of thousands of atomics)
   __shared__ float wmag[8];
-  for (int o = 16; o > 0; o >>= 1) mag = fmaxf(mag, __shfl_xor_sync(0xffffffffu, mag, o));
+  mag = warp_max(mag);
   if ((threadIdx.x & 31) == 0) wmag[threadIdx.x >> 5] = mag;
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -645,15 +612,14 @@ __global__ void __launch_bounds__(256) k_compact_kept(const uint32_t *__restrict
                                                        const uint32_t *__restrict__ block_off, uint32_t n,
                                                        uint32_t *__restrict__ keys_c, uint32_t *__restrict__ vals_c,
                                                        uint32_t limit, uint32_t *__restrict__ overflow) {
-  __shared__ uint32_t wcnt[8];
+  __shared__ BallotCounts<8> kept;
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const uint32_t km = i < n ? __ldg(keepmask + (i >> 5)) : 0u;   // i and its warp share the word (blockDim = 256, aligned)
-  if (lane == 0) wcnt[w] = __popc(km);
+  kept.put(km);
   __syncthreads();
+  const int lane = threadIdx.x & 31;
   if (!(km >> lane & 1u)) return;
-  uint32_t pos = block_off[blockIdx.x] + __popc(km & ((1u << lane) - 1u));
-  for (int k = 0; k < w; ++k) pos += wcnt[k];
+  const uint32_t pos = block_off[blockIdx.x] + kept.before() + __popc(km & ((1u << lane) - 1u));
   if (pos >= limit) {   // more kept photons than the (bounded) sort was sized for: the build is incomplete, say so
     *overflow = 1u;
     return;
@@ -736,9 +702,9 @@ size_t sort_temp_bytes(uint32_t n) {
   return bytes;
 }
 
-cudaError_t run_sort(void *temp, size_t temp_bytes, const uint32_t *kin, uint32_t *kout, const uint32_t *vin,
-                     uint32_t *vout, uint32_t n, cudaStream_t st) {
-  return cub::DeviceRadixSort::SortPairs(temp, temp_bytes, kin, kout, vin, vout, (int)n, 0, 30, st);
+cudaError_t run_sort_bits(void *temp, size_t temp_bytes, const uint32_t *kin, uint32_t *kout, const uint32_t *vin,
+                          uint32_t *vout, uint32_t n, int bits, cudaStream_t st) {
+  return cub::DeviceRadixSort::SortPairs(temp, temp_bytes, kin, kout, vin, vout, (int)n, 0, bits, st);
 }
 
 int bounds_blocks(uint32_t n) {
@@ -779,12 +745,16 @@ void launch_keep_pruned(const float *pos, uint32_t n, const void *grid, const ui
 void launch_keys_kept(const float *pos, const uint32_t *vals, uint32_t m, const void *grid, uint32_t *keys, cudaStream_t st) {
   if (m) k_keys_kept<<<(m + 255) / 256, 256, 0, st>>>(pos, vals, m, (const RayGrid *)grid, keys);
 }
-// records of the kept photons (caller's order) + sorted position plane / index map of the m kept ones
-void launch_pack_pruned(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *sorted, uint32_t m,
-                        float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st) {
-  if (!m) return;
-  k_pack_aos_kept<<<(n + 255) / 256, 256, 0, st>>>(S, n, keepmask, aos);
-  k_gather_sorted<<<(m + 255) / 256, 256, 0, st>>>(aos, sorted, m, planes, orig);
+// records of the kept photons only (keepmask; skipped when they exist already), then the sorted position plane / index
+// map of the first m sorted slots
+void launch_pack_sorted_kept(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *sorted, uint32_t m,
+                             float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st, bool records_ready) {
+  if (!records_ready && n) k_pack_aos_kept<<<(n + 255) / 256, 256, 0, st>>>(S, n, keepmask, aos);
+  if (m) k_gather_sorted<<<(m + 255) / 256, 256, 0, st>>>(aos, sorted, m, planes, orig);
+}
+// in-place exclusive scan of nb words by one CTA (a few thousand entries, 8 per thread); total -> total[0]
+void launch_scan_u32(uint32_t *vals, uint32_t nb, uint32_t *total, cudaStream_t st) {
+  k_scan_exclusive<uint32_t, 8><<<1, 1024, 0, st>>>(vals, nb, total, 0);
 }
 
 // ---- frustum grid launchers ----
@@ -807,9 +777,6 @@ void launch_compact_kept(const uint32_t *keys, const uint32_t *keepmask, const u
 void launch_fill_u32(uint32_t *p, uint32_t n, uint32_t value, cudaStream_t st) {
   if (n) k_fill_u32<<<std::min<uint32_t>((n + 255) / 256, 2048u), 256, 0, st>>>(p, n, value);
 }
-// records of the kept photons only (keepmask), then the sorted position plane / index map of the first m sorted slots
-void launch_pack_sorted_kept(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *sorted, uint32_t m,
-                             float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st, bool records_ready);
 // occ: frustum_occ_bytes() (zeroed here); coord_mag: one word (zeroed here)
 // pos / stride: photon positions (stride in floats: 3 for the staged SoA plane, 32 for 128-byte records); parity of the
 // photon's path id = (par_src[par_stride * i] >> par_shift) & 1
@@ -836,11 +803,11 @@ cudaError_t launch_cell_scan(void *temp, size_t temp_bytes, const uint32_t *cell
 // records of the kept photons, index map at cell_start[key] + rank, position plane gathered from it (kept_dev: slots in use)
 void launch_pack_scatter(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *keys, const uint32_t *rank,
                          const uint32_t *cell_start, float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st,
-                         bool records_ready, const uint32_t *kept_dev) {
+                         bool records_ready, const uint32_t *kept_dev, int sm_count) {
   if (!n) return;
   if (!records_ready) k_pack_aos_kept<<<(n + 255) / 256, 256, 0, st>>>(S, n, keepmask, aos);
   k_scatter_index<<<(n + 255) / 256, 256, 0, st>>>(keys, rank, keepmask, cell_start, n, orig);
-  k_gather_by_index<<<std::min<uint32_t>((n + 255) / 256, 148u * 16u), 256, 0, st>>>(aos, orig, kept_dev, planes);
+  k_gather_by_index<<<std::min<uint32_t>((n + 255) / 256, 16u * (uint32_t)sm_count), 256, 0, st>>>(aos, orig, kept_dev, planes);
 }
 // the occupancy mask alone (what a rank publishes to the ranks that send it photons)
 void launch_frustum_mark(const float4 *rays, uint32_t n_rays, const FrustumGrid &G, uint32_t *occ, int sm_count, cudaStream_t st) {
@@ -857,15 +824,6 @@ void launch_cell_starts(const uint32_t *sorted_keys, uint32_t n, uint32_t n_keys
   cudaMemsetAsync(n_big, 0, 4, st);
   k_cell_starts<<<(n + 1 + 255) / 256, 256, 0, st>>>(sorted_keys, n, n_keys, cell_start, big, n_big, cap);
   k_cell_starts_big<<<2 * sm_count, 256, 0, st>>>(cell_start, big, n_big, cap);
-}
-cudaError_t run_sort_bits(void *temp, size_t temp_bytes, const uint32_t *kin, uint32_t *kout, const uint32_t *vin,
-                          uint32_t *vout, uint32_t n, int bits, cudaStream_t st) {
-  return cub::DeviceRadixSort::SortPairs(temp, temp_bytes, kin, kout, vin, vout, (int)n, 0, bits, st);
-}
-void launch_pack_sorted_kept(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *sorted, uint32_t m,
-                             float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st, bool records_ready) {
-  if (!records_ready && n) k_pack_aos_kept<<<(n + 255) / 256, 256, 0, st>>>(S, n, keepmask, aos);
-  if (m) k_gather_sorted<<<(m + 255) / 256, 256, 0, st>>>(aos, sorted, m, planes, orig);
 }
 void launch_leaf_boxes(const float4 *p0, uint32_t n, uint32_t nLeaves, float radius, float4 *lo, float4 *hi,
                        cudaStream_t st) {
