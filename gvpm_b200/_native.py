@@ -114,7 +114,7 @@ ABI_SYMBOLS = [
     "gvpm_upload_vpm_samples", "gvpm_gather_vpm", "gvpm_gather_vpm_device", "gvpm_dump_neighbours_vpm",
     "gvpm_upload_beams", "gvpm_build_beams", "gvpm_gather_beams", "gvpm_gather_beams_device", "gvpm_dump_neighbours_beams", "gvpm_beam_subbeam_count",
     "gvpm_gather_sppm_beams", "gvpm_dump_neighbours_sppm_beams",
-    "gvpm_box_scene_default", "gvpm_generate_rays", "gvpm_trace_photons", "gvpm_trace_photons_direct", "gvpm_read_device", "gvpm_measure_read_bandwidth", "gvpm_staging_peek",
+    "gvpm_box_scene_default", "gvpm_generate_rays", "gvpm_trace_photons", "gvpm_trace_photons_direct", "gvpm_trace_beams", "gvpm_planes_from_beams", "gvpm_read_device", "gvpm_measure_read_bandwidth", "gvpm_staging_peek",
     "gvpm_upload_planes", "gvpm_build_planes", "gvpm_gather_planes", "gvpm_gather_planes_device", "gvpm_dump_neighbours_planes",
 ]
 
@@ -154,6 +154,8 @@ def load_lib():
                                        C.c_int, C.c_float]
     lib.gvpm_trace_photons.argtypes = [vp, C.POINTER(BoxScene), C.c_size_t, C.c_uint64, C.c_int, C.c_int, C.c_int, u64p]
     lib.gvpm_trace_photons_direct.argtypes = [vp, C.POINTER(BoxScene), C.c_size_t, C.c_uint64, C.c_int, C.c_int, C.c_int, u64p]
+    lib.gvpm_trace_beams.argtypes = [vp, C.POINTER(BoxScene), C.c_size_t, C.c_uint64, C.c_int, C.c_int, C.c_int, u64p]
+    lib.gvpm_planes_from_beams.argtypes = [vp, C.c_uint64]
     lib.gvpm_read_device.argtypes = [vp, vp, vp, C.c_size_t]
     lib.gvpm_measure_read_bandwidth.argtypes = [vp, C.c_size_t, C.c_int, C.POINTER(C.c_double)]
     lib.gvpm_staging_peek.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(C.c_size_t)]

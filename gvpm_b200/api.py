@@ -208,6 +208,18 @@ class Context:
         self.n_photons = n
         return int(paths.value)
 
+    def trace_beams(self, scene, n, seed, max_depth=12, rr_depth=1, min_depth=0):
+        """the iteration's photon beams traced on the device, committed as gvpm_upload_beams commits them (call
+        build_beams next); -> light paths traced (nbPathBeams)"""
+        paths = C.c_uint64(0)
+        self._ck(self.lib.gvpm_trace_beams(self.h, C.byref(scene), n, C.c_uint64(seed), max_depth, rr_depth, min_depth,
+                                           C.byref(paths)), "gvpm_trace_beams")
+        return int(paths.value)
+
+    def planes_from_beams(self, seed):
+        """one photon plane per beam of the current beam set, made on the device (call build_planes next)"""
+        self._ck(self.lib.gvpm_planes_from_beams(self.h, C.c_uint64(seed)), "gvpm_planes_from_beams")
+
     def photon_staging_peek(self, n=None):
         dev, cnt = C.c_void_p(), C.c_size_t()
         self._ck(self.lib.gvpm_staging_peek(self.h, 0, C.byref(dev), C.byref(cnt)), "gvpm_staging_peek")
@@ -243,6 +255,30 @@ class Context:
                      "gvpm_read_device")
             o += (a.nbytes + 255) & ~255
         return rs
+
+    def _download_staged(self, which, cls, fields):
+        """the staging buffer `which` of gvpm_staging_peek as a `cls` set (arrays back to back, 256-byte aligned)"""
+        dev, cnt = C.c_void_p(), C.c_size_t()
+        self._ck(self.lib.gvpm_staging_peek(self.h, which, C.byref(dev), C.byref(cnt)), "gvpm_staging_peek")
+        out = cls(cnt.value)
+        o = 0
+        for name, _, _ in fields:
+            a = getattr(out, name)
+            if a.nbytes:
+                self._ck(self.lib.gvpm_read_device(self.h, C.c_void_p(dev.value + o), a.ctypes.data_as(C.c_void_p),
+                                                   a.nbytes), "gvpm_read_device")
+            o += (a.nbytes + 255) & ~255
+        return out
+
+    def download_beams(self):
+        """parity aid: the current beam set (uploaded or traced) as a BeamSet"""
+        from . import records as R
+        return self._download_staged(2, R.BeamSet, R._BEAM_FIELDS)
+
+    def download_planes(self):
+        """parity aid: the current plane set (uploaded or made from beams) as a PlaneSet"""
+        from . import records as R
+        return self._download_staged(3, R.PlaneSet, R._PLANE_FIELDS)
 
     # ---- rays
     def upload_rays(self, rays):

@@ -219,9 +219,11 @@ int gvpm_read_device(gvpm_ctx *ctx, const void *dev, void *host, size_t bytes) {
 }
 
 int gvpm_staging_peek(gvpm_ctx *ctx, int which, void **dev, size_t *count) {
-  if (!ctx || !dev || (which != 0 && which != 1)) return GVPM_ERR_INVALID;
-  *dev = which == 0 ? ctx->ph_staging.p : ctx->ray_staging.p;
-  if (count) *count = which == 0 ? ctx->n_photons : ctx->n_rays;
+  if (!ctx || !dev || which < 0 || which > 3) return GVPM_ERR_INVALID;
+  const DevBuf *buf[4] = {&ctx->ph_staging, &ctx->ray_staging, &ctx->beam_staging, &ctx->plane_staging};
+  const size_t n[4] = {ctx->n_photons, ctx->n_rays, ctx->n_beams, ctx->n_planes};
+  *dev = buf[which]->p;
+  if (count) *count = n[which];
   return GVPM_OK;
 }
 

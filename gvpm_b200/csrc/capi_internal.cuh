@@ -88,10 +88,11 @@ cudaError_t launch_vpm_shade(const GatherParams &P, unsigned long long total, in
 void launch_gradient(const float *acc, int w, int h, int use_abs, float *thr, float *gx, float *gy,
                      cudaStream_t st, int reuse = 0, float inv_emitted = 1.f);
 void launch_generate_rays(const RayGenParams &P, cudaStream_t st);
-void launch_trace_count(const TraceParams &P, uint8_t *counts, unsigned long long *block_tot, unsigned long long *totals,
-                        cudaStream_t st);
-void launch_trace_emit(const TraceParams &P, const uint8_t *counts, const unsigned long long *block_off,
+void launch_trace_count(const TraceParams &P, bool beams, uint8_t *counts, unsigned long long *block_tot,
+                        unsigned long long *totals, cudaStream_t st);
+void launch_trace_emit(const TraceParams &P, bool beams, const uint8_t *counts, const unsigned long long *block_off,
                        unsigned long long *last_path, cudaStream_t st);
+void launch_planes_from_beams(const PlaneGenParams &P, cudaStream_t st);
 void launch_pack_beams(const BeamStaging &S, uint32_t n, float4 *rec, float *len, cudaStream_t st);
 void launch_beam_subsize_seq(const float *len, uint32_t n, float *subsize, cudaStream_t st);
 void launch_sub_count(const float *len, uint32_t n, const float *subsize, uint32_t *block_tot, uint32_t *total, cudaStream_t st);
@@ -229,6 +230,7 @@ struct gvpm_ctx {
   uint32_t hint_n = 0;
   uint32_t hint_rays = 0xffffffffu;   // ray count the hint belongs to
   double trace_photons_per_path = 0.0;   // running estimate (sizes the first batch of gvpm_trace_photons)
+  double trace_beams_per_path = 0.0;     // the same for gvpm_trace_beams
   // pin_scratch: [0,64) fit floats, [64,96) stats words, [128,..) block partials (doubles)
   uint64_t pin_gen = ~0ull;          // rays_gen the ray analysis below belongs to
   int dispatch_ctas = 0;             // side-stream dispatch: CTAs of its persistent grids (GVPM_DISPATCH_CTAS; 0 = one per chunk)
@@ -254,7 +256,7 @@ struct gvpm_ctx {
   // G-Beams
   DevBuf beams, beam_bounds, sub_pos, sub_raw, subs, beam_box_lo, beam_box_hi;
   DevBuf beam_staging, beam_len, beam_aux;  // raw gvpm_beam_soa arrays; beam lengths; [0] subbeamSize, [1] sub-beam total, [16..] block offsets
-  float beam_subsize = 0.f;                 // avgLength / 10 (host copy when the beams came through gvpm_upload_beams)
+  float beam_subsize = 0.f;                 // avgLength / 10 (summed on the host by gvpm_upload_beams, read back by gvpm_trace_beams)
   uint32_t n_subs = 0;                      // sub-beams of the uploaded beam set
   uint32_t n_beams = 0;
   bool beams_loaded = false, beams_built = false;
@@ -266,7 +268,8 @@ struct gvpm_ctx {
   uint32_t n_planes = 0;
   bool planes_loaded = false, planes_built = false;
   DevBuf samples, sample_counts, mvol, sample_staging;  // G-VPM distance samples (+ their raw SoA arrays)
-  uint32_t *sample_stats_host = nullptr;  // pinned: [0] max sample radius (float bits), [1] bad ray index seen; [2] plane flag
+  uint32_t *sample_stats_host = nullptr;  // pinned: [0] max sample radius (float bits), [1] bad ray index seen; [2] plane flag;
+                                          // [4] sub-beam size (float bits), [5] sub-beam count of traced beams
   uint32_t n_samples = 0;
   bool samples_loaded = false;
   float sample_radius_max = 0.f;
@@ -356,9 +359,12 @@ template <class S> typename S::Staging staging_ptrs(const void *base, size_t n) 
 }
 
 // The writable view of a staging buffer a generator kernel fills (RayGenParams o .. off_sensor, TraceParams pos ..
-// path_id): the Staging pointers, in their order, without const.
+// path_id and b_origin .. b_path_id, PlaneGenParams origin .. edge_id): the Staging pointers, in their order, without
+// const.
 static_assert(offsetof(RayGenParams, off_sensor) - offsetof(RayGenParams, o) == (RaySoA::N - 1) * sizeof(void *), "view");
 static_assert(offsetof(TraceParams, path_id) - offsetof(TraceParams, pos) == (PhotonSoA::N - 1) * sizeof(void *), "view");
+static_assert(offsetof(TraceParams, b_path_id) - offsetof(TraceParams, b_origin) == (BeamSoA::N - 1) * sizeof(void *), "view");
+static_assert(offsetof(PlaneGenParams, edge_id) - offsetof(PlaneGenParams, origin) == (PlaneSoA::N - 1) * sizeof(void *), "view");
 template <class S, class Field> void writable_view(Field *&first, const typename S::Staging &st) { memcpy(&first, &st, sizeof(st)); }
 
 // Copies elements [src_first, src_first + count) of every array of `h` to elements [dst_first, dst_first + count) of
@@ -405,3 +411,8 @@ FrustumGrid make_frustum_grid(const gvpm_ctx::RayFit &F, float radius, bool pari
 int build_frustum(gvpm_ctx *ctx, float radius, uint32_t *n_kept);
 int build_pruned_bvh(gvpm_ctx *ctx, float radius, uint32_t *n_kept);
 int check_scene(gvpm_ctx *ctx, const gvpm_box_scene *s);
+// a new beam set of n beams (staging sized, the old set and its build dropped); then fill the staging arrays and
+// commit_beams: records packed, sub-beam size and count known (host: the caller's arrays, for the host-side length sum;
+// nullptr: the beams exist on the device only and the sum runs there)
+int begin_beam_set(gvpm_ctx *ctx, size_t n);
+int commit_beams(gvpm_ctx *ctx, const gvpm_beam_soa *host);

@@ -1,4 +1,4 @@
-// capi_photons.cu — photon staging and upload, peer exchange of photon slices, on-device photon tracing.
+// capi_photons.cu — photon staging and upload, peer exchange of photon slices, on-device photon and beam tracing.
 #include "capi_internal.cuh"
 
 // A new photon set replaces the old one: staged (direct = false), traced straight into the gather records, or
@@ -243,12 +243,75 @@ int gvpm_box_scene_default(gvpm_box_scene *s) {
   return GVPM_OK;
 }
 
-static int trace_impl(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
-                      int min_depth, uint64_t *n_paths, bool direct) {
+// The checks every tracer shares and the walk parameters of the medium: a non-zero return is the error to report.
+static int trace_setup(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
+                       int min_depth, TraceParams &P) {
   if (!ctx || !scene || n > 0xfffffff0u) return GVPM_ERR_INVALID;
   if (!ctx->have_medium) return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_medium first");
   cudaSetDevice(ctx->device);
   int rc = check_scene(ctx, scene);
+  if (rc) return rc;
+  P = TraceParams{};
+  P.scene = *scene;
+  P.sigma_s = ctx->medium.sigma_s[0];
+  P.sigma_a = ctx->medium.sigma_a[0];
+  P.hg_g = ctx->medium.hg_g;
+  P.phase_type = ctx->medium.phase_type;
+  P.max_depth = max_depth > 0 ? max_depth : 64;
+  P.rr_depth = rr_depth;
+  P.min_depth = min_depth;
+  P.seed = seed;
+  P.n_total = n;
+  return GVPM_OK;
+}
+
+// Batches of light paths (count -> scan -> emit, in path order) until P.n_total records exist.  The first batch is
+// sized from the records-per-path ratio seen so far (`per_path`, updated); `barren` is the error when 64 batches do not
+// fill the set.  n_paths: paths up to and including the
+// one that stored the last record.
+static int trace_batches(gvpm_ctx *ctx, TraceParams &P, bool beams, double &per_path, const char *barren,
+                         uint64_t *n_paths) {
+  const unsigned long long n = P.n_total;
+  cudaStream_t st = ctx->stream;
+  unsigned long long filled = 0, pathBase = 0, *host = ctx->pair_count_host;   // host[0] batch total, host[1] last path
+  uint32_t pidBase = 0;
+  host[1] = 0;
+  for (int batch = 0; filled < n; ++batch) {
+    if (batch > 64) return fail(ctx, GVPM_ERR_INVALID, barren);
+    const double ratio = per_path > 0.0 ? per_path : 1.0;
+    double want = (double)(n - filled) / ratio * 1.03 + 4096.0;
+    if (want > 2.0e9) want = 2.0e9;
+    const uint32_t np = (uint32_t)want;
+    const uint32_t nb = (np + 255) / 256;
+    const size_t offCounts = 64, offBlocks = align256(offCounts + np);
+    CK(ctx->trace_scratch.reserve(offBlocks + ((size_t)nb + 1) * 8));
+    char *sc = ctx->trace_scratch.as<char>();
+    unsigned long long *totals = (unsigned long long *)sc;   // [0] batch total, [1] last path
+    if (batch == 0) CK(cudaMemsetAsync(sc, 0, 64, st));
+    P.path_base = pathBase;
+    P.n_paths = np;
+    P.slot_base = filled;
+    P.path_id_base = pidBase;
+    launch_trace_count(P, beams, (uint8_t *)(sc + offCounts), (unsigned long long *)(sc + offBlocks), totals, st);
+    launch_trace_emit(P, beams, (const uint8_t *)(sc + offCounts), (const unsigned long long *)(sc + offBlocks), totals + 1, st);
+    ctx->launches += 3;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(host, totals, 16, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    const unsigned long long records = host[0] & ((1ull << 40) - 1ull), paths = host[0] >> 40;
+    filled += records;
+    pidBase += (uint32_t)paths;
+    pathBase += np;
+    per_path = (double)filled / (double)pathBase;
+  }
+  if (n_paths) *n_paths = host[1];
+  return GVPM_OK;
+}
+
+static int trace_impl(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
+                      int min_depth, uint64_t *n_paths, bool direct) {
+  TraceParams P;
+  int rc = trace_setup(ctx, scene, n, seed, max_depth, rr_depth, min_depth, P);
   if (rc) return rc;
   void *dev = nullptr;
   PhotonStaging S{};
@@ -263,54 +326,10 @@ static int trace_impl(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint
   }
   if (n_paths) *n_paths = 0;
   if (n == 0) return GVPM_OK;
-  cudaStream_t st = ctx->stream;
-  TraceParams P{};
   P.aos = direct ? ctx->aos.as<float4>() : nullptr;
-  P.scene = *scene;
-  P.sigma_s = ctx->medium.sigma_s[0];
-  P.sigma_a = ctx->medium.sigma_a[0];
-  P.hg_g = ctx->medium.hg_g;
-  P.phase_type = ctx->medium.phase_type;
-  P.max_depth = max_depth > 0 ? max_depth : 64;
-  P.rr_depth = rr_depth;
-  P.min_depth = min_depth;
-  P.seed = seed;
-  P.n_total = n;
   writable_view<PhotonSoA>(P.pos, S);
-  // batches of paths until n photons exist; the first one is sized from the photons-per-path ratio seen so far
-  unsigned long long filled = 0, pathBase = 0, *host = ctx->pair_count_host;   // host[0] batch total, host[1] last path
-  uint32_t pidBase = 0;
-  host[1] = 0;
-  for (int batch = 0; filled < n; ++batch) {
-    if (batch > 64) return fail(ctx, GVPM_ERR_INVALID, "gvpm_trace_photons: the light paths store (almost) no photon in this scene");
-    const double ratio = ctx->trace_photons_per_path > 0.0 ? ctx->trace_photons_per_path : 1.0;
-    double want = (double)(n - filled) / ratio * 1.03 + 4096.0;
-    if (want > 2.0e9) want = 2.0e9;
-    const uint32_t np = (uint32_t)want;
-    const uint32_t nb = (np + 255) / 256;
-    const size_t offCounts = 64, offBlocks = align256(offCounts + np);
-    CK(ctx->trace_scratch.reserve(offBlocks + ((size_t)nb + 1) * 8));
-    char *sc = ctx->trace_scratch.as<char>();
-    unsigned long long *totals = (unsigned long long *)sc;   // [0] batch total, [1] last path
-    if (batch == 0) CK(cudaMemsetAsync(sc, 0, 64, st));
-    P.path_base = pathBase;
-    P.n_paths = np;
-    P.slot_base = filled;
-    P.path_id_base = pidBase;
-    launch_trace_count(P, (uint8_t *)(sc + offCounts), (unsigned long long *)(sc + offBlocks), totals, st);
-    launch_trace_emit(P, (const uint8_t *)(sc + offCounts), (const unsigned long long *)(sc + offBlocks), totals + 1, st);
-    ctx->launches += 3;
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(host, totals, 16, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    const unsigned long long photons = host[0] & ((1ull << 40) - 1ull), paths = host[0] >> 40;
-    filled += photons;
-    pidBase += (uint32_t)paths;
-    pathBase += np;
-    ctx->trace_photons_per_path = (double)filled / (double)pathBase;
-  }
-  if (n_paths) *n_paths = host[1];
-  return GVPM_OK;
+  return trace_batches(ctx, P, false, ctx->trace_photons_per_path,
+                       "gvpm_trace_photons: the light paths store (almost) no photon in this scene", n_paths);
 }
 
 int gvpm_trace_photons(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
@@ -320,6 +339,26 @@ int gvpm_trace_photons(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uin
 int gvpm_trace_photons_direct(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth,
                               int rr_depth, int min_depth, uint64_t *n_paths) {
   return trace_impl(ctx, scene, n, seed, max_depth, rr_depth, min_depth, n_paths, true);
+}
+
+int gvpm_trace_beams(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
+                     int min_depth, uint64_t *n_paths) {
+  if (ctx && max_depth > 255)   // per-path counts are bytes: a path stores at most max_depth - 1 beams
+    return fail(ctx, GVPM_ERR_INVALID, "gvpm_trace_beams: max_depth must be <= 255");
+  if (n > 0x0ffffff0u) return GVPM_ERR_INVALID;   // the bound of gvpm_upload_beams
+  TraceParams P;
+  int rc = trace_setup(ctx, scene, n, seed, max_depth, rr_depth, min_depth, P);
+  if (rc) return rc;
+  rc = begin_beam_set(ctx, n);
+  if (rc) return rc;
+  if (n_paths) *n_paths = 0;
+  if (n == 0) return GVPM_OK;
+  const BeamStaging S = staging_ptrs<BeamSoA>(ctx->beam_staging.p, n);
+  writable_view<BeamSoA>(P.b_origin, S);
+  rc = trace_batches(ctx, P, true, ctx->trace_beams_per_path,
+                     "gvpm_trace_beams: the light paths store (almost) no beam in this scene", n_paths);
+  if (rc) return rc;
+  return commit_beams(ctx, nullptr);
 }
 
 }  // extern "C"

@@ -8,8 +8,11 @@
 //                     + GPhotonMap::tryAppend (gvpm_accel.h:119-199): one thread per light path, two passes (count,
 //                     exclusive scan over the paths, emit), so the photons land in path order whatever the launch
 //                     geometry and the set is bit-reproducible; photon flux / pdf bookkeeping as libbidir's
-//                     (SURVEY.md §9.1).
-// Random numbers: PCG32 keyed by (seed, pixel index) / (seed, path index).  Arithmetic: strictly rounded fp32 in a fixed
+//                     (SURVEY.md §9.1).  The same walk emits photon beams instead (EmitKind::Beams): every edge
+//                     that does not escape, LTBeamMap::tryAppendLT (gvpm_beams.h:54-84).
+//   k_planes_from_beams   LTPhotonPlane::transformBeam (gvpm_plane.h:53-73) of every beam of the current set: one
+//                     thread per beam, photon planes written into the plane staging arrays.
+// Random numbers: PCG32 keyed by (seed, pixel index) / (seed, path index) / (seed ^ constant, beam index).  Arithmetic: strictly rounded fp32 in a fixed
 // operation order; log, exp, sin and cos are polynomial routines (pm_*) built from +, -, *, / only, so a CPU
 // restatement compiled without FMA contraction reproduces every record bit for bit (tests/test_gpu_generate.py).
 #include "gvpm_device.cuh"
@@ -245,9 +248,13 @@ __device__ __forceinline__ sf hg_eval(sf g, sf cosWiWo) {   // phase/hg.cpp:107-
   return (sf(GVPM_INV_FOURPI) * (sf(1.f) - g * g)) / (temp * ssqrt(temp));
 }
 
-// The walk of light path `pathIdx`.  EMIT = false: returns the number of photons it would store.  EMIT = true: stores
-// them at slots first, first + 1, ... (< n_total) with path id `pid`.
-template <bool EMIT>
+// What a light path stores: volume photons (GPhotonMap::tryAppend) or photon beams (LTBeamMap::tryAppendLT).
+enum class EmitKind { Photons, Beams };
+
+// The walk of light path `pathIdx`.  EMIT = false: returns the number of records it would store.  EMIT = true: stores
+// them at slots first, first + 1, ... (< n_total) with path id `pid`.  The RNG draws, the arithmetic and the
+// termination do not depend on KIND; only which records are written does.
+template <EmitKind KIND, bool EMIT>
 __device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned long long pathIdx, unsigned long long first,
                                               uint32_t pid) {
   const gvpm_box_scene &S = P.scene;
@@ -271,7 +278,7 @@ __device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned lon
   v3 thr(S.light_power, S.light_power, S.light_power);
   int ci = 1;
   uint32_t appended = 0;
-  const int firstStored = max(2, P.min_depth + 1);
+  const int firstStored = max(2, P.min_depth + 1), firstBeam = max(1, P.min_depth);
   for (;;) {
     const SceneHit h = intersect_scene(S, curPos, dir);
     const sf t = (-sf(pm_log((sf(1.0f) - sf(rng.uniform())).v))) / sigT;
@@ -300,7 +307,23 @@ __device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned lon
     const v3 step((curWeight.x * curRr) * ew, (curWeight.y * curRr) * ew, (curWeight.z * curRr) * ew);
     const v3 flux = thr * step;
     const int ni = ci + 1;
-    if (inMedium && ni >= firstStored) {
+    if (KIND == EmitKind::Beams && ci >= firstBeam) {
+      // beam = edge ci -> ci + 1; its flux stops before the edge's own transmittance (gvpm_beams.h:29-35)
+      if (EMIT) {
+        const unsigned long long slot = first + appended;
+        if (slot < P.n_total) {
+          put3(P.b_origin, slot, curPos); put3(P.b_end, slot, nvPos);
+          put3(P.b_flux, slot, v3((thr.x * curWeight.x) * curRr, (thr.y * curWeight.y) * curRr, (thr.z * curWeight.z) * curRr));
+          put3(P.b_prefix_flux, slot, prefix); put3(P.b_parent_n, slot, curN); put3(P.b_parent_albedo, slot, curAlbedo);
+          put3(P.b_pred_pos, slot, ci >= 2 ? prevPos : v3(1.f, 1.f, 1.f)); put3(P.b_end_n, slot, nvN);
+          P.b_parent_pdf[slot] = pdfArea.v; P.b_rr_weight[slot] = curRr.v;
+          P.b_parent_type[slot] = (uint8_t)curType; P.b_end_on_surface[slot] = inMedium ? 0 : 1;
+          P.b_depth[slot] = (uint8_t)ci; P.b_path_id[slot] = pid;
+        }
+      }
+      ++appended;
+    }
+    if (KIND == EmitKind::Photons && inMedium && ni >= firstStored) {
       if (EMIT) {
         const unsigned long long slot = first + appended;
         if (slot < P.n_total && P.aos != nullptr) {
@@ -357,19 +380,21 @@ __device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned lon
   return appended;
 }
 
-// pass 1: photons per path; block totals of (photons, contributing paths) packed as (paths << 40 | photons)
+// pass 1: records per path; block totals of (records, contributing paths) packed as (paths << 40 | records)
+template <EmitKind KIND>
 __global__ void __launch_bounds__(256) k_trace_count(const __grid_constant__ TraceParams P, uint8_t *__restrict__ counts,
                                                       unsigned long long *__restrict__ block_tot) {
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
   uint32_t c = 0;
   if (k < P.n_paths) {
-    c = walk_path<false>(P, P.path_base + k, 0ull, 0u);
+    c = walk_path<KIND, false>(P, P.path_base + k, 0ull, 0u);
     counts[k] = (uint8_t)c;
   }
   const unsigned long long t = block_total<8>((unsigned long long)c | ((unsigned long long)(c ? 1u : 0u) << 40));
   if (threadIdx.x == 0) block_tot[blockIdx.x] = t;
 }
-// pass 2: the same walks, stored.  last_path[0] = 1 + index of the path that stored photon n_total - 1.
+// pass 2: the same walks, stored.  last_path[0] = 1 + index of the path that stored record n_total - 1.
+template <EmitKind KIND>
 __global__ void __launch_bounds__(256) k_trace_emit(const __grid_constant__ TraceParams P, const uint8_t *__restrict__ counts,
                                                      const unsigned long long *__restrict__ block_off,
                                                      unsigned long long *__restrict__ last_path) {
@@ -381,8 +406,72 @@ __global__ void __launch_bounds__(256) k_trace_emit(const __grid_constant__ Trac
   const unsigned long long first = P.slot_base + (excl & ((1ull << 40) - 1ull));
   const uint32_t pid = P.path_id_base + (uint32_t)(excl >> 40);
   if (first >= P.n_total) return;
-  walk_path<true>(P, P.path_base + k, first, pid);
+  walk_path<KIND, true>(P, P.path_base + k, first, pid);
   if (first + c >= P.n_total) last_path[0] = P.path_base + k + 1ull;   // exactly one path crosses the end of the set
+}
+
+// ---- photon planes from photon beams ------------------------------------------------------------------------------------
+// One thread per beam.  w0 / length0 are PhotonBeam::setEndPoint's (as k_pack_beams forms them); length1 and w1 are
+// LTPhotonPlane::transformBeam's free-flight distance and phase-function direction (host mirror
+// gvpm_host::transformBeam), drawn from PCG32(seed ^ kPlaneSeed, beam index) instead of the integrator's one sequential
+// sampler (DESIGN.md §6).  kPlaneSeed is the constant of gvpm_synth_planes' sampler: a caller that passes the seed of
+// the light paths again does not get the light paths' random numbers.
+constexpr unsigned long long kPlaneSeed = 0xA0761D6478BD642FULL;
+__global__ void __launch_bounds__(256) k_planes_from_beams(const __grid_constant__ PlaneGenParams P) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.n) return;
+  const size_t i3 = 3 * (size_t)i;
+  const float o0 = P.beams.origin[i3], o1 = P.beams.origin[i3 + 1], o2 = P.beams.origin[i3 + 2];
+  // PhotonBeam::setEndPoint (beams_struct.h:73-81), operation for operation as k_pack_beams
+  float d0 = __fsub_rn(P.beams.end[i3], o0), d1 = __fsub_rn(P.beams.end[i3 + 1], o1), d2 = __fsub_rn(P.beams.end[i3 + 2], o2);
+  const float len = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(d0, d0), __fmul_rn(d1, d1)), __fmul_rn(d2, d2)));
+  const float rcp = __fdiv_rn(1.0f, len);
+  d0 = __fmul_rn(d0, rcp); d1 = __fmul_rn(d1, rcp); d2 = __fmul_rn(d2, rcp);
+  const v3 dir(d0, d1, d2);
+  Pcg32 rng(P.seed ^ kPlaneSeed, i);
+  // sampleDistance, EDistanceNormal, mint = Epsilon (homogeneous.cpp:293-352); sampling_weight is 1 (checked by the caller)
+  const sf eps(1e-4f);
+  const sf rand(rng.uniform());
+  const sf length1 = (-sf(pm_log((sf(1.f) - rand).v))) / sf(P.sigma_t1) + eps;
+  v3 w1;
+  for (;;) {
+    const float sx = rng.uniform(), sy = rng.uniform();
+    if (P.phase_type == GVPM_PHASE_ISOTROPIC) {   // squareToUniformSphere (warp.cpp:25-31)
+      const sf z = sf(1.f) - sf(2.f) * sf(sy);
+      const sf r = safe_sqrt(sf(1.f) - z * z);
+      float sn, cs;
+      pm_sincos2pi(sx, sn, cs);
+      w1 = v3(r * sf(cs), r * sf(sn), z);
+    } else {                                      // hg.cpp:73-96 in FrameCoherent(dir)
+      const sf g(P.hg_g);
+      sf cosTheta;
+      if (fabsf(g.v) < eps.v) {
+        cosTheta = sf(1.f) - sf(2.f) * sf(sx);
+      } else {
+        const sf sq = (sf(1.f) - g * g) / ((sf(1.f) - g) + (sf(2.f) * g) * sf(sx));
+        cosTheta = ((sf(1.f) + g * g) - sq * sq) / (sf(2.f) * g);
+      }
+      const sf sinTheta = safe_sqrt(sf(1.f) - cosTheta * cosTheta);
+      float sn, cs;
+      pm_sincos2pi(sy, sn, cs);
+      const sf lx = sinTheta * sf(cs), ly = sinTheta * sf(sn), lz = cosTheta;
+      // coordinateSystemCoherent (util.cpp:592-599)
+      const sf sign(copysignf(1.0f, d2));
+      const sf a = sf(-1.0f) / (sign + dir.z);
+      const sf b = (dir.x * dir.y) * a;
+      const v3 s(sf(1.f) + ((sign * dir.x) * dir.x) * a, sign * b, (-sign) * dir.x);
+      const v3 t(b, sign + (dir.y * dir.y) * a, -dir.y);
+      w1 = (s * lx + t * ly) + dir * lz;
+    }
+    if (fabsf(dot(dir, w1).v) != 1.0f) break;   // a direction parallel to the beam spans no plane
+  }
+  put3(P.origin, i, v3(o0, o1, o2));
+  put3(P.w0, i, dir);
+  P.length0[i] = len;
+  put3(P.w1, i, w1);
+  P.length1[i] = length1.v;
+  P.flux[i3] = P.beams.flux[i3]; P.flux[i3 + 1] = P.beams.flux[i3 + 1]; P.flux[i3 + 2] = P.beams.flux[i3 + 2];
+  P.edge_id[i] = (int32_t)P.beams.depth[i];
 }
 
 // ---- launchers ------------------------------------------------------------------------------------------------------
@@ -392,16 +481,25 @@ void launch_generate_rays(const RayGenParams &P, cudaStream_t st) {
   if (blocksX > 0 && blocksY > 0) k_generate_rays<<<blocksX * blocksY, 1024, 0, st>>>(P);
 }
 // counts: [n_paths] bytes; block_tot: [(n_paths + 255) / 256 + 1] words; totals: [0] batch total (paths << 40 | photons)
-void launch_trace_count(const TraceParams &P, uint8_t *counts, unsigned long long *block_tot, unsigned long long *totals,
-                        cudaStream_t st) {
+// beams: the beam emission kind (b_* arrays) instead of photons
+void launch_trace_count(const TraceParams &P, bool beams, uint8_t *counts, unsigned long long *block_tot,
+                        unsigned long long *totals, cudaStream_t st) {
   const uint32_t nb = (P.n_paths + 255) / 256;
-  if (nb) k_trace_count<<<nb, 256, 0, st>>>(P, counts, block_tot);
+  if (nb) {
+    if (beams) k_trace_count<EmitKind::Beams><<<nb, 256, 0, st>>>(P, counts, block_tot);
+    else k_trace_count<EmitKind::Photons><<<nb, 256, 0, st>>>(P, counts, block_tot);
+  }
   k_scan_exclusive<unsigned long long, 1><<<1, 1024, 0, st>>>(block_tot, nb, totals, 0);
 }
-void launch_trace_emit(const TraceParams &P, const uint8_t *counts, const unsigned long long *block_off,
+void launch_trace_emit(const TraceParams &P, bool beams, const uint8_t *counts, const unsigned long long *block_off,
                        unsigned long long *last_path, cudaStream_t st) {
   const uint32_t nb = (P.n_paths + 255) / 256;
-  if (nb) k_trace_emit<<<nb, 256, 0, st>>>(P, counts, block_off, last_path);
+  if (!nb) return;
+  if (beams) k_trace_emit<EmitKind::Beams><<<nb, 256, 0, st>>>(P, counts, block_off, last_path);
+  else k_trace_emit<EmitKind::Photons><<<nb, 256, 0, st>>>(P, counts, block_off, last_path);
+}
+void launch_planes_from_beams(const PlaneGenParams &P, cudaStream_t st) {
+  if (P.n) k_planes_from_beams<<<(P.n + 255) / 256, 256, 0, st>>>(P);
 }
 
 }  // namespace gvpm

@@ -300,6 +300,22 @@ struct TraceParams {
   uint8_t *parent_type, *depth;
   uint32_t *path_id;
   float4 *aos;                  // not null: write 128-byte gather records (layout above) instead of the staging arrays
+  // beam staging arrays (gvpm_beam_soa order), written by the beam emission kind
+  float *b_origin, *b_end, *b_flux, *b_prefix_flux, *b_parent_n, *b_parent_albedo, *b_pred_pos, *b_end_n, *b_parent_pdf,
+      *b_rr_weight;
+  uint8_t *b_parent_type, *b_end_on_surface, *b_depth;
+  uint32_t *b_path_id;
+};
+// photon planes from the current beam set (generate.cu k_planes_from_beams): one PCG32 stream per beam
+struct PlaneGenParams {
+  BeamStaging beams;
+  uint32_t n;
+  unsigned long long seed;
+  float sigma_t1, hg_g;         // sampling density sigma_s[1] + sigma_a[1] (balance strategy); HG asymmetry
+  int phase_type;
+  // plane staging arrays (gvpm_plane_soa order)
+  float *origin, *w0, *length0, *w1, *length1, *flux;
+  int32_t *edge_id;
 };
 // ---- strictly rounded double (the reference's fp64 island: cylinderIntersection / solveQuadraticDouble,
 // photonmapper/beams_3d_intersections.h:100-137, src/libcore/util.cpp:487-525) ----------------------------

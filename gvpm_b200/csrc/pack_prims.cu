@@ -40,9 +40,9 @@ __global__ void __launch_bounds__(256) k_pack_beams(const BeamStaging S, uint32_
 
 // `Float avgSize = 0; for (b : beams) avgSize += b.getLength();` is a SEQUENTIAL fp32 sum (beams_accel.h:98-102): its
 // rounding depends on the order, and the sub-beam size derived from it decides how every beam is cut.  One warp
-// streams the lengths through shared memory and lane 0 adds them in index order (a ~4-cycle dependent chain per beam:
-// 1 ms for 500 k beams on one SM; gvpm_upload_beams has the host do this sum while the DMA runs and this kernel is
-// only used for beams that were produced on the device).  out[0] = subbeamSize = avg / 10.
+// streams the lengths through shared memory and lane 0 adds them in index order (a ~4-cycle dependent chain per beam).
+// gvpm_upload_beams has the host do this sum while the DMA runs; this kernel serves the beams gvpm_trace_beams makes
+// on the device (capi_prims.cu commit_beams).  out[0] = subbeamSize = avg / 10.
 __global__ void __launch_bounds__(32) k_beam_subsize_seq(const float *__restrict__ len, uint32_t n, float *__restrict__ out) {
   __shared__ float buf[2][32 * 8];
   const int lane = threadIdx.x;

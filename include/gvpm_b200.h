@@ -546,6 +546,25 @@ int gvpm_trace_photons(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uin
  * (gvpm_photon_staging, peer exchange) do not see them. */
 int gvpm_trace_photons_direct(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth,
                               int rr_depth, int min_depth, uint64_t *n_paths);
+/* f-1, beams: the iteration's photon beams traced on the device by the same light-path walk as gvpm_trace_photons
+ * (same random numbers, arithmetic and termination), storing instead every edge vertex(i) -> vertex(i+1) that does not
+ * escape, for i >= max(1, min_depth) - LTBeamMap::tryAppendLT (gvpm/gvpm_beams.h:54-84) with the fields of
+ * gvpm_beam_soa; path_id counts the paths that store at least one beam.  Paths are taken in index order until n beams
+ * exist.  The context is left exactly as gvpm_upload_beams of the same arrays leaves it (records packed, sub-beam
+ * size = the in-order fp32 mean length / 10 summed on the device, gvpm_beam_subbeam_count known): call
+ * gvpm_build_beams next.  n_paths = nbPathBeams (light paths up to and including the one that completed the set).
+ * max_depth <= 255; n <= 0x0ffffff0. */
+int gvpm_trace_beams(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
+                     int min_depth, uint64_t *n_paths);
+/* G-Planes 0D inputs made on the device: one photon plane per beam of the current beam set (uploaded or traced),
+ * as LTPhotonPlane::transformBeam (gvpm/gvpm_plane.h:53-73) extends it - origin, w0, length0 = the beam's
+ * setEndPoint, length1 = a free-flight distance + Epsilon, w1 = a phase-function direction (isotropic or HG in the
+ * coherent frame of the beam; directions parallel to the beam are drawn again), flux and edge_id = depth copied.
+ * Beam i draws from PCG32(seed ^ 0xA0761D6478BD642F, i) instead of the integrator's single sequential sampler
+ * (DESIGN.md §6); log / sin / cos are the polynomial routines of the tracers, so the planes are bit-reproducible.
+ * The context is left as gvpm_upload_planes of the same arrays leaves it: call gvpm_build_planes next.  Fails when
+ * there is no beam set, no medium, or the medium's sampling_weight is not 1. */
+int gvpm_planes_from_beams(gvpm_ctx *ctx, uint64_t seed);
 /* parity aid: copy `bytes` bytes at `dev` (a pointer handed out by this library, e.g. gvpm_photon_staging /
  * gvpm_ray_staging) to host memory, after the work queued on the context's stream */
 int gvpm_read_device(gvpm_ctx *ctx, const void *dev, void *host, size_t bytes);
@@ -554,8 +573,10 @@ int gvpm_read_device(gvpm_ctx *ctx, const void *dev, void *host, size_t bytes);
  * gb_per_s = bytes * reps / time.  A buffer well below the 126 MB L2 gives the L2 read bandwidth, one far above it the
  * HBM read bandwidth. */
 int gvpm_measure_read_bandwidth(gvpm_ctx *ctx, size_t bytes, int reps, double *gb_per_s);
-/* parity aid: the selected photon staging buffer (which = 0) or the ray staging buffer (which = 1) as they are, without
- * the side effects of gvpm_photon_staging / gvpm_ray_staging (which invalidate the build / the committed rays) */
+/* parity aid: the selected photon staging buffer (which = 0), the ray staging buffer (1), the beam staging buffer (2)
+ * or the plane staging buffer (3) as they are, without the side effects of gvpm_photon_staging / gvpm_ray_staging
+ * (which invalidate the build / the committed rays).  Each holds its SoA's arrays back to back, every array starting
+ * on a 256-byte boundary; count = the number of elements of the current set. */
 int gvpm_staging_peek(gvpm_ctx *ctx, int which, void **dev, size_t *count);
 
 /* ---- timing of the last build / gather on the context's stream (CUDA events, ms) ----- */
