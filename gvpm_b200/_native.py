@@ -116,6 +116,8 @@ ABI_SYMBOLS = [
     "gvpm_gather_sppm_beams", "gvpm_dump_neighbours_sppm_beams",
     "gvpm_box_scene_default", "gvpm_generate_rays", "gvpm_trace_photons", "gvpm_trace_photons_direct", "gvpm_trace_beams", "gvpm_planes_from_beams", "gvpm_read_device", "gvpm_measure_read_bandwidth", "gvpm_staging_peek",
     "gvpm_upload_planes", "gvpm_build_planes", "gvpm_gather_planes", "gvpm_gather_planes_device", "gvpm_dump_neighbours_planes",
+    "gvpm_accum_reset", "gvpm_accum_add", "gvpm_accum_fold", "gvpm_accum_read", "gvpm_accum_device",
+    "gvpm_compute_gradient_accum", "gvpm_reconstruct_accum",
 ]
 
 _lib = None
@@ -193,6 +195,13 @@ def load_lib():
     lib.gvpm_poisson_preset.argtypes = [C.c_char_p, C.POINTER(PoissonParams)]
     lib.gvpm_poisson_solve.argtypes = [vp, C.c_int, C.c_int, f32p, f32p, f32p, f32p, C.POINTER(PoissonParams), f32p]
     lib.gvpm_reconstruct.argtypes = [vp, f32p, C.c_int, C.c_int, C.c_int, f32p, C.POINTER(PoissonParams), f32p, f32p, f32p, f32p]
+    lib.gvpm_accum_reset.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.gvpm_accum_add.argtypes = [vp]
+    lib.gvpm_accum_fold.argtypes = [vp, C.c_int, C.c_uint64]
+    lib.gvpm_accum_read.argtypes = [vp, C.c_int, f32p, u8p, u64p]
+    lib.gvpm_accum_device.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
+    lib.gvpm_compute_gradient_accum.argtypes = [vp, C.c_int, C.c_int, C.c_float, f32p, f32p, f32p]
+    lib.gvpm_reconstruct_accum.argtypes = [vp, C.c_int, f32p, C.POINTER(PoissonParams), f32p, f32p, f32p, f32p]
     lib.gvpm_last_poisson_ms.argtypes = [vp]
     lib.gvpm_last_poisson_ms.restype = C.c_float
     lib.gvpm_last_timings.argtypes = [vp, f32p, f32p]

@@ -495,6 +495,57 @@ class Context:
                                            gy.ctypes.data_as(N.f32p), rec.ctypes.data_as(N.f32p)), "gvpm_reconstruct")
         return thr, gx, gy, rec
 
+    # ---- per-pixel accumulators on the device (gvpm_accum_*)
+    def accum_reset(self, w, h, channels=N.GVPM_OUT_FLOATS, apa=True):
+        """zeroed accumulators of w x h pixels: channels 27 (gvpm) or 3 (sppm); apa=False for G-VPM's plain sum"""
+        self._ck(self.lib.gvpm_accum_reset(self.h, int(w), int(h), int(channels), int(bool(apa))), "gvpm_accum_reset")
+        self._accum_shape = (int(h), int(w), int(channels))
+
+    def accum_add(self):
+        """add the per-ray results of the last gather on the current ray set to their pixels"""
+        self._ck(self.lib.gvpm_accum_add(self.h), "gvpm_accum_add")
+
+    def accum_fold(self, it, n_paths):
+        """end of iteration `it` (from 1) of n_paths light paths: APA running mean, or the emitted total (G-VPM)"""
+        self._ck(self.lib.gvpm_accum_fold(self.h, int(it), C.c_uint64(int(n_paths))), "gvpm_accum_fold")
+
+    def accum_read(self, normalized=False):
+        """-> (acc [h,w,C] float32, have_smoke [h,w] uint8, emitted-path total)"""
+        h, w, c = getattr(self, "_accum_shape", (0, 0, 0))
+        acc = np.empty((h, w, c), dtype=np.float32)
+        smoke = np.empty((h, w), dtype=np.uint8)
+        total = C.c_uint64(0)
+        self._ck(self.lib.gvpm_accum_read(self.h, int(bool(normalized)), acc.ctypes.data_as(N.f32p),
+                                          smoke.ctypes.data_as(N.u8p), C.byref(total)), "gvpm_accum_read")
+        return acc, smoke, int(total.value)
+
+    def accum_device(self):
+        """-> (acc device pointer, have_smoke device pointer), owned by the context"""
+        a, s = C.c_void_p(), C.c_void_p()
+        self._ck(self.lib.gvpm_accum_device(self.h, C.byref(a), C.byref(s)), "gvpm_accum_device")
+        return a.value, s.value
+
+    def compute_gradient_accum(self, use_abs=False, reuse_primal=False, inv_emitted=1.0):
+        """compute_gradient on the device accumulators -> (throughput, gx, gy), [h, w, 3]"""
+        h, w, _ = getattr(self, "_accum_shape", (0, 0, 0))
+        thr, gx, gy = (np.empty((h, w, 3), dtype=np.float32) for _ in range(3))
+        self._ck(self.lib.gvpm_compute_gradient_accum(self.h, int(use_abs), int(reuse_primal), C.c_float(inv_emitted),
+                                                      thr.ctypes.data_as(N.f32p), gx.ctypes.data_as(N.f32p),
+                                                      gy.ctypes.data_as(N.f32p)), "gvpm_compute_gradient_accum")
+        return thr, gx, gy
+
+    def reconstruct_accum(self, direct=None, preset="L2D", use_abs=False, **params):
+        """reconstruct on the device accumulators -> (throughput, gx, gy, reconstruction), [h, w, 3]"""
+        p = poisson_params(preset, **params)
+        h, w, _ = getattr(self, "_accum_shape", (0, 0, 0))
+        d = None if direct is None else np.ascontiguousarray(direct, dtype=np.float32)
+        thr, gx, gy, rec = (np.empty((h, w, 3), dtype=np.float32) for _ in range(4))
+        self._ck(self.lib.gvpm_reconstruct_accum(self.h, int(use_abs), None if d is None else d.ctypes.data_as(N.f32p),
+                                                 C.byref(p), thr.ctypes.data_as(N.f32p), gx.ctypes.data_as(N.f32p),
+                                                 gy.ctypes.data_as(N.f32p), rec.ctypes.data_as(N.f32p)),
+                 "gvpm_reconstruct_accum")
+        return thr, gx, gy, rec
+
     def last_poisson_ms(self):
         return float(self.lib.gvpm_last_poisson_ms(self.h))
 

@@ -128,6 +128,7 @@ int dump_neighbours(gvpm_ctx *ctx, size_t rows, uint64_t *offsets, uint32_t *idx
   offsets[rows] = total;
   if (total > cap || (total && !idx)) return fail(ctx, GVPM_ERR_INVALID, "neighbour buffer too small");
   if (total == 0) return GVPM_OK;
+  ctx->out_state = gvpm_ctx::OUT_NONE;   // the fill pass may leave other values in the gather output
   if (pair_list) {   // the gather fills a flat list of (row, index) pairs: bucket it by row
     CK(ctx->nbr_idx.reserve(total * sizeof(uint2)));
     rc = fill(total);
@@ -281,6 +282,8 @@ static int gather_common(gvpm_ctx *ctx, float *out_dev, uint32_t *counts_dev, un
   }
   CK(cudaEventRecord(ctx->ev[3], ctx->stream));
   ctx->timed_gather = true;
+  if (out_dev == ctx->out.as<float>()) out_written(ctx);
+  else ctx->out_state = gvpm_ctx::OUT_ELSEWHERE;
   return GVPM_OK;
 }
 
@@ -474,6 +477,7 @@ int gvpm_gather_bre_host(gvpm_ctx *ctx, const gvpm_ray_soa *r, size_t n, float *
                        (r1 - r0) * GVPM_OUT_FLOATS * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
   }
+  out_written(ctx);
   return GVPM_OK;
 }
 
@@ -575,6 +579,7 @@ int gvpm_gather_vpm_device(gvpm_ctx *ctx, int nb_camera_samples, const float **o
   ctx->launches += total ? 1 : 0;
   CK(cudaEventRecord(ctx->ev[3], ctx->stream));
   ctx->timed_gather = true;
+  out_written(ctx);
   if (out_dev) *out_dev = ctx->out.as<float>();
   if (mvol_dev) *mvol_dev = ctx->mvol.as<uint32_t>();
   return GVPM_OK;

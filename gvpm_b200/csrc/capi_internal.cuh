@@ -105,6 +105,14 @@ long long poisson_solve_device(const float *tp, const float *dx, const float *dy
                                float alpha, int irlsIterMax, float irlsRegInit, float irlsRegIter, int cgIterMax,
                                int cgIterCheck, float cgTolerance, float *ws, float *host_rz, float *rec,
                                cudaStream_t st);
+void launch_accum_scatter(const float *out, uint32_t stride, const int32_t *px, const int32_t *py, uint32_t n, int w,
+                          int h, int C, float *dst, uint8_t *smoke, int sm_count, cudaStream_t st);
+void launch_accum_keys(const int32_t *px, const int32_t *py, uint32_t n, int w, int h, uint32_t *keys, uint32_t *vals,
+                       cudaStream_t st);
+void launch_accum_runs(const float *out, uint32_t stride, const uint32_t *skeys, const uint32_t *svals, uint32_t n,
+                       uint32_t npix, int C, float *dst, uint8_t *smoke, int sm_count, cudaStream_t st);
+void launch_accum_fold(float *acc, float *pix, size_t count, float itm1, float rnb, float rit, int sm_count,
+                       cudaStream_t st);
 }  // namespace gvpm
 
 using namespace gvpm;
@@ -273,6 +281,21 @@ struct gvpm_ctx {
   uint32_t n_samples = 0;
   bool samples_loaded = false;
   float sample_radius_max = 0.f;
+  // what `out` holds for gvpm_accum_add: OUT_READY = the per-ray results (out_stride floats per ray) of the last gather,
+  // run on ray set out_gen; OUT_ADDED = the same, already added; OUT_ELSEWHERE = the last gather wrote to caller memory
+  enum { OUT_NONE = 0, OUT_READY, OUT_ADDED, OUT_ELSEWHERE };
+  int out_state = OUT_NONE;
+  uint64_t out_gen = 0;
+  uint32_t out_stride = GVPM_OUT_FLOATS;
+  uint64_t pixel_rays_gen = ~0ull;   // rays_gen of a gvpm_generate_rays set: one ray per pixel of its rows
+  // per-pixel accumulators (gvpm_accum_*, capi_accum.cu): acc [w*h*channels], pix the iteration sum (APA mode),
+  // smoke one byte per pixel, keys four arrays of n_rays words + sort scratch (uploaded rays)
+  struct Accum {
+    bool ready = false, apa = false;
+    int w = 0, h = 0, channels = 0;
+    uint64_t total = 0;   // emitted paths (non-APA mode)
+    DevBuf acc, pix, smoke, keys;
+  } accum;
   DevBuf grad_in, grad_out;
   DevBuf poisson_io, poisson_ws;   // device copies of the four input planes + the result; solver workspace
   float poisson_ms = 0.f;
@@ -387,6 +410,12 @@ int copy_soa(gvpm_ctx *ctx, const typename S::Host &h, void *staging, size_t n_t
 // pair count a gather reports when its perspective grid is incomplete (bounded compaction overflow, build_frustum)
 constexpr unsigned long long kBuildOverflow = 1ull << 62;
 
+// a gather has queued its per-ray results for the current ray set into ctx->out, `stride` floats per ray
+inline void out_written(gvpm_ctx *ctx, uint32_t stride = GVPM_OUT_FLOATS) {
+  ctx->out_state = gvpm_ctx::OUT_READY;
+  ctx->out_gen = ctx->rays_gen;
+  ctx->out_stride = stride;
+}
 int grid_incomplete(gvpm_ctx *ctx);                                   // the failure a gather reports then
 // the checks and fields every gather shares: medium and config, its structure built, rays, counter block
 int gather_params(gvpm_ctx *ctx, GatherParams &P, bool built, const char *not_built);
@@ -416,3 +445,9 @@ int check_scene(gvpm_ctx *ctx, const gvpm_box_scene *s);
 // nullptr: the beams exist on the device only and the sum runs there)
 int begin_beam_set(gvpm_ctx *ctx, size_t n);
 int commit_beams(gvpm_ctx *ctx, const gvpm_beam_soa *host);
+// computeGradient / computeGradient + Poisson on [h*w*27] accumulators: host memory (uploaded first) or, acc_on_device,
+// device memory of this context read where it is (capi_image.cu)
+int compute_gradient_impl(gvpm_ctx *ctx, const float *acc, bool acc_on_device, int w, int h, int use_abs, int reuse,
+                          float inv_emitted, float *throughput, float *gx, float *gy);
+int reconstruct_impl(gvpm_ctx *ctx, const float *acc, bool acc_on_device, int w, int h, int use_abs, const float *direct,
+                     const gvpm_poisson_params *params, float *throughput, float *gx, float *gy, float *reconstruction);

@@ -134,6 +134,7 @@ int gvpm_gather_planes_device(gvpm_ctx *ctx, const float **out_dev, const uint32
   ctx->launches += ctx->n_rays ? 1 : 0;
   CK(cudaEventRecord(ctx->ev[3], ctx->stream));
   ctx->timed_gather = true;
+  out_written(ctx);
   if (out_dev) *out_dev = ctx->out.as<float>();
   if (counts_dev) *counts_dev = ctx->counts.as<uint32_t>();
   return GVPM_OK;
@@ -380,6 +381,7 @@ int gvpm_gather_beams_device(gvpm_ctx *ctx, const float **out_dev, const uint32_
   if (rc) return rc;
   CK(cudaEventRecord(ctx->ev[3], ctx->stream));
   ctx->timed_gather = true;
+  out_written(ctx);
   if (out_dev) *out_dev = ctx->out.as<float>();
   if (counts_dev) *counts_dev = ctx->counts.as<uint32_t>();
   return GVPM_OK;
@@ -439,6 +441,7 @@ int gvpm_gather_sppm_beams(gvpm_ctx *ctx, int technique, float *out, uint32_t *c
   if (rc) return rc;
   CK(cudaEventRecord(ctx->ev[3], ctx->stream));
   ctx->timed_gather = true;
+  out_written(ctx, 3);   // [n_rays][3]
   const size_t n = ctx->n_rays;
   return copy_back(ctx, out, n * 3 * sizeof(float), counts, n * 8);
 }

@@ -83,6 +83,7 @@ int gvpm_generate_rays(gvpm_ctx *ctx, const gvpm_box_scene *scene, const gvpm_pi
   }
   rc = gvpm_commit_rays(ctx);
   if (rc) return rc;
+  ctx->pixel_rays_gen = ctx->rays_gen;   // one ray per pixel of rows [y0, y1): gvpm_accum_add needs no sort
   // The rays of a pinhole are concurrent by construction: what analyse_rays would measure on the device (and read back)
   // follows from the camera.  Every ray is pos + t * dir up to the rounding of the entry point (a few ulp of the
   // coordinates, bounded here by 4e-6 * (1 + |pos|)); projected directions span [-tx, tx] x rows [y0, y1).

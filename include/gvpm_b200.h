@@ -492,6 +492,55 @@ int gvpm_reconstruct(gvpm_ctx *ctx, const float *acc, int w, int h, int use_abs,
 /* device time of the last gvpm_poisson_solve / gvpm_reconstruct, copies included (CUDA events, ms) */
 float gvpm_last_poisson_ms(const gvpm_ctx *ctx);
 
+/* ---- per-pixel accumulators on the device: the fold of every iteration of a progressive render -------------------
+ * GatherPoint's volume accumulators (gvpm_struct.h:421-455; sppm: GatherPoint::fluxVol) kept in the context's device
+ * memory across iterations, updated as GPMIntegrator (gvpm.cpp:1054-1069, G-VPM :1176-1181) and SPPMIntegrator
+ * (sppm.cpp:866-871) update them, and handed to the gradient and the Poisson solve without a host round trip.  The
+ * results are the host mirror's (VolumeGatherB200 / SPPMVolumeGatherB200 foldIteration) bit for bit, given the same
+ * per-ray gather output.  Per iteration:
+ *     gather (any of gvpm_gather_bre / _device / _host, gvpm_gather_sppm_bre, gvpm_gather_vpm / _device,
+ *             gvpm_gather_beams / _device, gvpm_gather_planes / _device, gvpm_gather_sppm_beams);
+ *     gvpm_accum_add;              (once per ray set: an iteration may come in several ray batches)
+ *     gvpm_accum_fold(it, n_paths);
+ * and after the last one gvpm_reconstruct_accum (or gvpm_accum_read for the image itself).
+ *
+ * gvpm_accum_reset: w x h pixels (w * h < 2^30) of `channels` floats - 27 for gvpm, 3 for sppm's fluxVol - zeroed,
+ *   with one have_smoke byte per pixel and the emitted-path total (grow-only allocations, like every context buffer).
+ *   apa = 1: the APA running mean (BRE, beams, planes, sppm); apa = 0: the plain sum of G-VPM, divided by the total
+ *   number of emitted paths when read normalised.
+ * gvpm_accum_add: the per-ray results the last gather left in the context's output, for the current ray set, added to
+ *   their pixels (px, py of the rays): into the iteration's sum (apa = 1) or straight into the accumulators (apa = 0).
+ *   Only the first `channels` floats of each ray's row are read.  Rays outside the film are skipped; every ray inside
+ *   it sets its pixel's have_smoke byte.  The rays of one pixel are added in ray order, and batches in call order add
+ *   up to the same bits as one batch holding their concatenation.  Rays of gvpm_generate_rays (one per pixel) are
+ *   scattered directly; other ray sets are first sorted by pixel.  Fails with GVPM_ERR_INVALID when no gather has run
+ *   on the current ray set (gvpm_ray_staging, gvpm_upload_rays and gvpm_generate_rays start a new one), when the last
+ *   gather's output has already been added, when the last gather wrote to caller memory (gvpm_gather_bre_into), or when
+ *   it wrote fewer floats per ray than there are channels (gvpm_gather_sppm_beams writes 3).  It first completes any
+ *   asynchronous gather still in flight (gvpm_gather_bre_device: waits for it, and re-runs it when its pair list
+ *   overflowed, as gvpm_sync does), so it never adds an incomplete result; this costs one wait per add while such a
+ *   gather is queued.  The work itself is queued on the context's stream.
+ * gvpm_accum_fold: the end of iteration `it` (1, 2, ...) whose light paths numbered n_paths.  apa = 1: for EVERY
+ *   pixel, reached or not, acc = (acc * (float)(it - 1) + sum * (1.0f / (float)n_paths)) * (1.0f / (float)it), then
+ *   the iteration's sum is cleared.  apa = 0: n_paths is added to the emitted total.  it >= 1, n_paths >= 1.
+ * gvpm_accum_read: host copies [h*w*channels] floats, [h*w] bytes and the emitted total; each pointer may be NULL.
+ *   normalized = 1 with apa = 0 multiplies by 1.0f / (float)total (the G-VPM image; nothing when total is 0).
+ * gvpm_accum_device: the device arrays themselves, read-only (valid until the next gvpm_accum_reset).  A sharded
+ *   render whose ranks own disjoint pixels (column bands) sums the ranks' arrays to the single-GPU result exactly.
+ * gvpm_compute_gradient_accum / gvpm_reconstruct_accum: gvpm_compute_gradient (reuse_primal = 0) or
+ *   gvpm_compute_gradient_reuse_primal (reuse_primal = 1, inv_emitted > 0), and gvpm_reconstruct, applied to the
+ *   accumulators as they are stored (27 channels only).
+ * Every call but gvpm_accum_reset fails with GVPM_ERR_INVALID before the first gvpm_accum_reset. */
+int gvpm_accum_reset(gvpm_ctx *ctx, int w, int h, int channels, int apa);
+int gvpm_accum_add(gvpm_ctx *ctx);
+int gvpm_accum_fold(gvpm_ctx *ctx, int it, uint64_t n_paths);
+int gvpm_accum_read(gvpm_ctx *ctx, int normalized, float *acc, uint8_t *have_smoke, uint64_t *total_emitted);
+int gvpm_accum_device(gvpm_ctx *ctx, const float **acc, const uint8_t **have_smoke);
+int gvpm_compute_gradient_accum(gvpm_ctx *ctx, int use_abs, int reuse_primal, float inv_emitted, float *throughput,
+                                float *gx, float *gy);
+int gvpm_reconstruct_accum(gvpm_ctx *ctx, int use_abs, const float *direct, const gvpm_poisson_params *params,
+                           float *throughput, float *gx, float *gy, float *reconstruction);
+
 
 /* ---- next rows (SURVEY.md 8 f-1, f-2): the two host stages on either side of the gather, on the device -------------
  * Scene class covered (the synthetic scenes of SURVEY.md 8d): an axis-aligned box filled with the homogeneous
