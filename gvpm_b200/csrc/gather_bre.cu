@@ -33,7 +33,8 @@ namespace gvpm {
 #define GVPM_SHADE_THREADS 128
 #endif
 #ifndef GVPM_SHADE_MIN_BLOCKS
-// 96 registers, no spills.  Tuned on cfg5 (B200, 1000 W): 4: 2.90 ms, 5: 2.63, 6: 2.69, 8: 2.82.  A phase A/B hand-off
+// 89 registers, no spills (6: 80 registers with 40 B spilled, 7: 72 with 64 B; profiles/r4_shade_code.md).  Tuned on cfg5
+// at 96 registers, before the scan and the near-occluder loop shrank (B200, 1000 W): 4: 2.90 ms, 5: 2.63, 6: 2.69, 8: 2.82.  A phase A/B hand-off
 // that re-reads the photon record in phase B instead of carrying it through shared memory fits 80 / 72 registers at 6 / 7
 // (with spills) but shades slower at every bound, 5 / 6 / 7: 2.75 / 2.75 / 2.78 ms against 2.44 (profiles/r3_shade_records.md)
 #define GVPM_SHADE_MIN_BLOCKS 5
@@ -539,7 +540,10 @@ k_bre_shade(const __grid_constant__ GatherParams P) {
   // software pipeline over the grid-stride loop: the pair of the NEXT iteration is already in registers, so its
   // 128-byte photon record (a random HBM line) is prefetched while the current pair is shaded, and the pair of the
   // iteration after that is requested
-  const unsigned long long first = (unsigned long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31);
+  // the warp's first pair, through a shuffle from lane 0 so that ptxas sees the loop bound as warp-uniform: it then
+  // knows the warp is converged at warp_run_sum and emits a single copy of its scan
+  const unsigned long long first =
+      (unsigned long long)blockIdx.x * blockDim.x + 32u * __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
   const uint2 none = make_uint2(0xffffffffu, 0u);
   uint2 cur = none, nxt = none;
   if (first + lane < total) cur = P.pairs[first + lane];

@@ -38,6 +38,18 @@ __device__ __forceinline__ sf ssqrt(sf a) { return sf(__fsqrt_rn(a.v)); }
 __device__ __forceinline__ sf smax(sf a, sf b) { return sf(fmaxf(a.v, b.v)); }
 __device__ __forceinline__ sf safe_sqrt(sf a) { return ssqrt(smax(sf(0.f), a)); }
 
+// __fdiv_rn(a, b) < 0 without the division, for |b| < 2 (the side tests' b is a dot product of two unit vectors, so
+// |b| <= 1 + rounding).  The quotient is negative exactly when a and b have opposite sign bits and it is neither NaN nor
+// a zero:
+//   a = +-0 gives +-0 or NaN (b = +-0) and a = NaN or b = NaN gives NaN: excluded by |a| > 0 and |b| < inf;
+//   b = +-inf gives +-0 or NaN: excluded by |b| < inf;
+//   b = +-0 with a != 0 gives +-inf, whose sign is the xor of the sign bits (-0 counts as negative), as here;
+//   a = +-inf with b finite gives +-inf, likewise;
+//   finite nonzero a over finite b with |b| < 2 has |a / b| > 2^-149 / 2, so it rounds to a nonzero value of that sign.
+__host__ __device__ __forceinline__ bool quotient_negative(float a, float b) {
+  return fabsf(a) > 0.f && fabsf(b) < INFINITY && (signbit(a) != signbit(b));
+}
+
 struct v3 {
   sf x, y, z;
   __device__ v3() {}

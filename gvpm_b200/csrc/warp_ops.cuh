@@ -105,13 +105,18 @@ struct BallotCounts {
 // last lane of the run (lanes with !valid take part in the scan but add nothing).  Inclusive shuffle-up scan, offsets
 // 1 .. 16, each lane adding the value `off` lanes below while that lane is in its run.  SKIP_ZERO: a run sum that
 // compares equal to 0 is not added (an atomic add of +0 would turn a -0 in `out` into +0).
+// Offsets at or above the warp's longest run are skipped (warp-uniform): no lane is `off` lanes into its run there, so
+// those levels add nothing and the sums are the same bits.  The caller must be converged in a way ptxas can see (a
+// warp-uniform loop around the call), or it emits a second, WARPSYNC-wrapped copy of the N x 5 shuffles.
 template <int N, bool SKIP_ZERO = false>
 __device__ __forceinline__ void warp_run_sum(uint32_t key, float (&a)[N], bool valid, float *out, int lane) {
   const uint32_t kprev = __shfl_up_sync(0xffffffffu, key, 1);
   const uint32_t heads = __ballot_sync(0xffffffffu, lane == 0 || kprev != key);
   const int start = 31 - __clz(heads & (0xffffffffu >> (31 - lane)));  // first lane of my run
+  const int runMax = (int)__reduce_max_sync(0xffffffffu, (uint32_t)(lane - start)) + 1;  // longest run, in lanes
 #pragma unroll
   for (int off = 1; off < 32; off <<= 1) {
+    if (off >= runMax) break;
     const bool same = lane - off >= start;
 #pragma unroll
     for (int j = 0; j < N; ++j) {
