@@ -58,11 +58,7 @@ int gvpm_ctx_create(int device, gvpm_ctx **out) {
   memset(ctx->pair_count_host, 0, 48 * sizeof(unsigned long long));
   for (auto &g : ctx->ring) cudaEventCreateWithFlags(&g.done, cudaEventDisableTiming);
   cudaHostAlloc((void **)&ctx->pin_host, 128, cudaHostAllocDefault);
-  cudaEventCreateWithFlags(&ctx->ev_hint, cudaEventDisableTiming);
   { const char *e = getenv("GVPM_ACCEL"); ctx->force_bvh = e && !strcmp(e, "bvh"); }
-  { const char *e = getenv("GVPM_FRUSTUM_SORT"); ctx->radix_frustum = e && !strcmp(e, "radix"); }
-  // side-stream dispatch: one CTA per SM by default (N = 8, cfg5: 32 CTAs 1.96 ms / step, 96: 1.11, one per chunk: 1.13)
-  { const char *e = getenv("GVPM_DISPATCH_CTAS"); ctx->dispatch_ctas = e ? std::max(0, atoi(e)) : -1; }
   cudaHostAlloc((void **)&ctx->sample_stats_host, 64, cudaHostAllocDefault);
   memset(ctx->sample_stats_host, 0, 64);
   ctx->bounds.reserve(256);
@@ -87,7 +83,6 @@ int gvpm_ctx_destroy(gvpm_ctx *ctx) {
   if (ctx->pair_count_host) cudaFreeHost(ctx->pair_count_host);
   if (ctx->sample_stats_host) cudaFreeHost(ctx->sample_stats_host);
   if (ctx->pin_host) cudaFreeHost(ctx->pin_host);
-  if (ctx->ev_hint) cudaEventDestroy(ctx->ev_hint);
   for (auto &g : ctx->ring) if (g.done) cudaEventDestroy(g.done);
   for (auto &ps : ctx->push_streams) if (ps) { cudaStreamSynchronize(ps); cudaStreamDestroy(ps); }
   if (ctx->push_kernel_stream) { cudaStreamSynchronize(ctx->push_kernel_stream); cudaStreamDestroy(ctx->push_kernel_stream); }

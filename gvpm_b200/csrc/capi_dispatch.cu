@@ -215,8 +215,9 @@ int gvpm_dispatch_photons(gvpm_ctx *ctx, int which, size_t n_total, size_t begin
     for (int d = 0; d < D.n_peers; ++d) P.pad_r_max = std::max(P.pad_r_max, P.grids[d].pad_r);
     P.pad_r_max += 2e-5f * (1.f + std::fabs(P.grids[0].C[0]) + std::fabs(P.grids[0].C[1]) + std::fabs(P.grids[0].C[2]));   // the centres agree to 1e-5
   }
-  // on the side stream: a small persistent grid (GVPM_DISPATCH_CTAS, default one CTA per SM); in-stream: one CTA per chunk
-  launch_dispatch(P, ks, ks == ctx->stream ? 0 : (ctx->dispatch_ctas < 0 ? ctx->sm_count : ctx->dispatch_ctas));
+  // on the side stream: a persistent grid of one CTA per SM (N = 8, cfg5: 32 CTAs 1.96 ms / step, 96: 1.11, one per
+  // chunk: 1.13); in-stream: one CTA per chunk
+  launch_dispatch(P, ks, ks == ctx->stream ? 0 : ctx->sm_count);
   launch_dispatch_signal(Sg, ks);
   ctx->launches += 4;
   CK(cudaGetLastError());
@@ -243,14 +244,10 @@ int gvpm_build_dispatched(gvpm_ctx *ctx, int which, float radius, uint32_t *n_ke
   ctx->launches += 1;
   replace_photon_set(ctx, (size_t)D.n_peers * D.region_cap, true, D.inbox[which].as<float4>(), D.region_cap,
                      ctrl + DC_COUNT + which * GVPM_MAX_PEERS);
-  if (gen == 1 && which == 0) {   // first build over an inbox: mostly empty regions; its exact count sizes the following ones
-    ctx->kept_fraction_hint = 0.25;
-    ctx->kept_hint_valid = false;
-  }
   rc = build_frustum(ctx, radius, n_kept);
   if (rc) return rc;
   // a peer that never signalled (k_flag_wait timed out) or a region overflow: the grid is incomplete, and the gather says
-  // so (the same device flag a bounded build sets when it overflows); gvpm_dispatch_status names the cause
+  // so (through the build's overflow flag, which the BRE traversal reads); gvpm_dispatch_status names the cause
   if (ctx->build_ovf) {
     launch_or_flag(const_cast<uint32_t *>(ctx->build_ovf), ctrl + DC_TIMEOUT, ctx->stream);
     launch_or_flag(const_cast<uint32_t *>(ctx->build_ovf), ctrl + DC_OVERFLOW, ctx->stream);

@@ -6,11 +6,9 @@
 static unsigned long long grown_pairs(unsigned long long total) { return total + total / 8 + 1024; }
 
 int grid_incomplete(gvpm_ctx *ctx) {
-  ctx->force_exact_build = true;
   return fail(ctx, GVPM_ERR_INVALID,
-              "the perspective grid is incomplete - it was sized from the previous iteration's photon count and this "
-              "iteration kept over 25 % more, or a peer's photon dispatch never arrived (gvpm_dispatch_status): the gather "
-              "did not run.  Build again (the next build reads its exact count) and gather again");
+              "the perspective grid is incomplete - a peer's photon dispatch never arrived or overflowed its region "
+              "(gvpm_dispatch_status names which): the gather did not run.  Build again and gather again");
 }
 
 int gather_params(gvpm_ctx *ctx, GatherParams &P, bool built, const char *not_built) {
@@ -245,7 +243,7 @@ int pending_check(gvpm_ctx *ctx, bool block) {
     --ctx->ring_n;
     ctx->last_pairs = total;
     if (total <= g.cap) continue;
-    if (total >= kBuildOverflow) return grid_incomplete(ctx);   // the bounded frustum build was too small: nothing was gathered
+    if (total >= kBuildOverflow) return grid_incomplete(ctx);   // a peer's dispatch timed out or overflowed: nothing was gathered
     // overflow: make the list large enough for the next one
     cudaStreamSynchronize(ctx->stream);
     int rc = reserve_pairs(ctx, grown_pairs(total));

@@ -31,8 +31,8 @@ size_t frustum_occ_bytes();
 void launch_frustum_keys(const float4 *rays, uint32_t n_rays, const float *pos, uint32_t stride, const uint32_t *par_src,
                          uint32_t par_stride, uint32_t par_shift, uint32_t n,
                          const FrustumGrid &G, uint32_t *occ, uint32_t *keys, uint32_t *vals, unsigned *coord_mag,
-                         uint32_t *keepmask, uint32_t *block_kept, int sm_count, cudaStream_t st, uint32_t region_cap = 0,
-                         const uint32_t *region_count = nullptr, uint32_t *cell_count = nullptr);
+                         uint32_t *keepmask, uint32_t *cell_count, uint32_t region_cap, const uint32_t *region_count,
+                         int sm_count, cudaStream_t st);
 size_t cell_scan_temp_bytes(uint32_t n_keys);
 cudaError_t launch_cell_scan(void *temp, size_t temp_bytes, const uint32_t *cell_count, uint32_t *cell_start, uint32_t n_keys,
                              cudaStream_t st);
@@ -47,15 +47,10 @@ void launch_flag_set(const FlagSetParams &P, cudaStream_t st);
 void launch_or_flag(uint32_t *dst, const uint32_t *src, cudaStream_t st);
 void launch_l2_read(const void *p, size_t bytes, int reps, unsigned *sink, int sm_count, cudaStream_t st);
 void launch_translate_idx(uint32_t *idx, unsigned long long n, const float4 *aos, cudaStream_t st);
-void launch_compact_kept(const uint32_t *keys, const uint32_t *keepmask, const uint32_t *block_off, uint32_t n,
-                         uint32_t *keys_c, uint32_t *vals_c, cudaStream_t st, uint32_t limit, uint32_t *overflow);
-void launch_fill_u32(uint32_t *p, uint32_t n, uint32_t value, cudaStream_t st);
+void launch_compact_kept(const uint32_t *keepmask, const uint32_t *block_off, uint32_t n, uint32_t *vals_c, cudaStream_t st);
 void launch_pack_sorted_kept(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *sorted, uint32_t m,
-                             float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st, bool records_ready);
+                             float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st);
 void launch_scan_u32(uint32_t *vals, uint32_t nb, uint32_t *total, cudaStream_t st);
-size_t cell_starts_scratch_bytes(uint32_t n_keys);
-void launch_cell_starts(const uint32_t *sorted_keys, uint32_t n, uint32_t n_keys, uint32_t *cell_start, void *scratch,
-                        int sm_count, cudaStream_t st);
 size_t ray_grid_bytes();
 size_t ray_mask_bytes();
 void launch_ray_region(const float4 *rays, uint32_t nRays, float radius, float *box, void *grid, uint32_t *mask,
@@ -189,7 +184,7 @@ struct gvpm_ctx {
   bool photons_direct = false;   // gvpm_trace_photons_direct: the 128-byte records in `aos` ARE the photon set (no staging, no packing)
   // dispatched photon set (gvpm_build_dispatched): the records live in an inbox the peers wrote; one region of
   // region_cap records per sender, region_count[s] (device) of them filled
-  const uint32_t *build_ovf = nullptr;   // device flag of the last frustum build (bounded compaction overflowed)
+  const uint32_t *build_ovf = nullptr;   // device flag of the last frustum build (a peer's dispatch timed out or overflowed)
   float4 *aos_override = nullptr;
   uint32_t region_cap = 0;
   const uint32_t *region_count = nullptr;
@@ -219,7 +214,7 @@ struct gvpm_ctx {
   float extent_hint = 1.f;  // diagonal of the photon AABB (host copy, refreshed lazily)
   // gvpm_build_points_for_rays: occupancy grid of the uploaded rays; the hierarchy then holds only the photons they can
   // reach and is valid for that ray set (rays_gen) alone
-  DevBuf ray_region;        // [0,32): ray box, [32,64): kept-photon counter, [64,..): RayGrid, the 32 KB cell mask, one keep bit per photon
+  DevBuf ray_region;        // [0,32): ray box, [32,..): RayGrid, the 32 KB cell mask, one keep bit per photon
   uint64_t rays_gen = 0, pruned_for_gen = 0;
   bool pruned = false;
   uint32_t n_kept = 0;
@@ -229,19 +224,10 @@ struct gvpm_ctx {
   bool force_bvh = false;            // GVPM_ACCEL=bvh: A/B switch for kernel experiments
   FrustumGrid grid{};
   DevBuf cell_start, grid_occ, pin_scratch, trace_scratch, keepmask, cell_count;
-  bool radix_frustum = false;        // GVPM_FRUSTUM_SORT=radix: the key sort of the perspective grid by radix sort (A/B switch)
-  double kept_fraction_hint = 1.0;   // share of the photons the last frustum build kept (sizes the next one's sort)
-  bool kept_hint_valid = false;      // the fraction comes from a count read back from a build over the same kind of set
-  bool force_exact_build = false;    // a bounded build overflowed: size the next one from its exact count (one host sync)
-  cudaEvent_t ev_hint = nullptr;
-  bool hint_pending = false;
-  uint32_t hint_n = 0;
-  uint32_t hint_rays = 0xffffffffu;   // ray count the hint belongs to
   double trace_photons_per_path = 0.0;   // running estimate (sizes the first batch of gvpm_trace_photons)
   double trace_beams_per_path = 0.0;     // the same for gvpm_trace_beams
   // pin_scratch: [0,64) fit floats, [64,96) stats words, [128,..) block partials (doubles)
   uint64_t pin_gen = ~0ull;          // rays_gen the ray analysis below belongs to
-  int dispatch_ctas = 0;             // side-stream dispatch: CTAs of its persistent grids (GVPM_DISPATCH_CTAS; 0 = one per chunk)
   bool have_view_dir = false;        // gvpm_set_view_direction: axis of the perspective grid's projection plane
   float view_dir[3] = {0.f, 0.f, 1.f};
   RayFit pin;
@@ -407,7 +393,7 @@ int copy_soa(gvpm_ctx *ctx, const typename S::Host &h, void *staging, size_t n_t
 }
 
 // ---- helpers shared between the units ----------------------------------------------------------------------------------
-// pair count a gather reports when its perspective grid is incomplete (bounded compaction overflow, build_frustum)
+// pair count a gather reports when its perspective grid is incomplete (build_ovf: a peer's dispatch timed out or overflowed)
 constexpr unsigned long long kBuildOverflow = 1ull << 62;
 
 // a gather has queued its per-ray results for the current ray set into ctx->out, `stride` floats per ray

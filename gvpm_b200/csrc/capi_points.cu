@@ -57,15 +57,13 @@ int build_pruned_bvh(gvpm_ctx *ctx, float radius, uint32_t *n_kept) {
   const uint32_t n = ctx->n_photons;
   cudaStream_t st = ctx->stream;
   CK(cudaEventRecord(ctx->ev[0], st));
-  const size_t gridOff = 64, maskOff = align256(gridOff + ray_grid_bytes()), keepOff = align256(maskOff + ray_mask_bytes());
+  const size_t gridOff = 32, maskOff = align256(gridOff + ray_grid_bytes()), keepOff = align256(maskOff + ray_mask_bytes());
   CK(ctx->ray_region.reserve(keepOff + 4 * ((size_t)n / 32 + 1)));
   char *rr = ctx->ray_region.as<char>();
   float *box = (float *)rr;
-  uint32_t *counter = (uint32_t *)(rr + 32);
   uint32_t *mask = (uint32_t *)(rr + maskOff), *keepmask = (uint32_t *)(rr + keepOff);
   const float boxInit[8] = {INFINITY, INFINITY, INFINITY, -INFINITY, -INFINITY, -INFINITY, 0.f, 0.f};
   CK(cudaMemcpyAsync(box, boxInit, sizeof(boxInit), cudaMemcpyHostToDevice, st));
-  CK(cudaMemsetAsync(counter, 0, 32, st));
   CK(cudaMemsetAsync(mask, 0, ray_mask_bytes(), st));
   launch_ray_region(ctx->rays.as<float4>(), ctx->n_rays, radius, box, rr + gridOff, mask, ctx->bounds.as<float>(),
                     ctx->sm_count, st);
@@ -84,7 +82,7 @@ int build_pruned_bvh(gvpm_ctx *ctx, float radius, uint32_t *n_kept) {
     uint32_t *block_kept = ctx->keepmask.as<uint32_t>();
     launch_keep_pruned(S.pos, n, rr + gridOff, mask, keepmask, block_kept, st);
     launch_scan_u32(block_kept, nb, block_kept + nb, st);
-    launch_compact_kept(nullptr, keepmask, block_kept, n, nullptr, ctx->vals_in.as<uint32_t>(), st, n, counter);
+    launch_compact_kept(keepmask, block_kept, n, ctx->vals_in.as<uint32_t>(), st);
     ctx->launches += 3;
     // the number of kept photons sizes the sort and the hierarchy levels: one 4-byte read-back
     CK(cudaMemcpyAsync(ctx->pair_count_host, block_kept + nb, 4, cudaMemcpyDeviceToHost, st));
@@ -104,7 +102,7 @@ int build_pruned_bvh(gvpm_ctx *ctx, float radius, uint32_t *n_kept) {
     CK(run_sort_bits(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
                      ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), kept, kHilbertBits, st));
     launch_pack_sorted_kept(S, n, keepmask, ctx->vals_out.as<uint32_t>(), kept, ctx->aos.as<float4>(),
-                            ctx->planes.as<float4>(), ctx->orig.as<uint32_t>(), st, false);
+                            ctx->planes.as<float4>(), ctx->orig.as<uint32_t>(), st);
     float4 *lo = ctx->box_lo.as<float4>(), *hi = ctx->box_hi.as<float4>();
     launch_leaf_boxes(ctx->planes.as<float4>(), kept, T.cnt[0], radius, lo, hi, st);
     for (int l = 1; l < levels; ++l)
@@ -198,125 +196,53 @@ int build_frustum(gvpm_ctx *ctx, float radius, uint32_t *n_kept) {
   const FrustumGrid G = make_frustum_grid(F, radius, ctx->have_cfg && ctx->cfg.path_set && !ctx->cfg.sppm_primal);
   const uint32_t total = G.n_cells;
   const uint32_t n_keys = (G.parity_split ? 2u : 1u) * total + 2;   // + NEAR + DROP
-  int bits = 1;
-  while ((1ull << bits) < (unsigned long long)n_keys) ++bits;
   CK(ctx->cell_start.reserve(((size_t)n_keys + 1) * 4));
-  // how much of the set did the previous build keep?  (read without blocking: sizes this build's sort)
-  if (ctx->hint_pending && cudaEventQuery(ctx->ev_hint) == cudaSuccess) {
-    ctx->hint_pending = false;
-    const uint32_t keptPrev = *(const uint32_t *)(ctx->pin_host + 30);
-    if (ctx->hint_n) { ctx->kept_fraction_hint = (double)keptPrev / (double)ctx->hint_n; ctx->kept_hint_valid = true; }
-  }
-  uint32_t m = n;   // sorted entries
   if (n > 0) {
-    const uint32_t nb = (n + 255) / 256;
-    int rc = reserve_sort(ctx, n);
-    if (rc) return rc;
+    CK(ctx->keys_in.reserve(4 * (size_t)n));
+    CK(ctx->vals_in.reserve(4 * (size_t)n));
+    CK(ctx->sort_temp.reserve(cell_scan_temp_bytes(n_keys)));
+    CK(ctx->cell_count.reserve(((size_t)n_keys + 2) * 4));
     CK(ctx->planes.reserve(16 * (size_t)n));
     CK(ctx->orig.reserve(4 * (size_t)n));
-    CK(ctx->keepmask.reserve(4 * ((size_t)n / 32 + 1) + 4 * ((size_t)nb + 4)));
+    CK(ctx->keepmask.reserve(4 * ((size_t)n / 32 + 2)));
     const bool direct = ctx->photons_direct;
     if (!direct) CK(ctx->aos.reserve(128 * (size_t)n));
-    CK(ctx->grid_occ.reserve(frustum_occ_bytes() + cell_starts_scratch_bytes(n_keys)));
-    uint32_t *keepmask = ctx->keepmask.as<uint32_t>(), *block_kept = keepmask + (n / 32 + 1);
+    CK(ctx->grid_occ.reserve(frustum_occ_bytes()));
+    uint32_t *keepmask = ctx->keepmask.as<uint32_t>(), *cell_count = ctx->cell_count.as<uint32_t>();
+    // the word after the keep bits: set when the build is incomplete (gvpm_build_dispatched: a peer's dispatch timed out
+    // or overflowed its region); the gather reports it instead of gathering
+    uint32_t *ovf = keepmask + (n / 32 + 1);
+    CK(cudaMemsetAsync(ovf, 0, 4, st));
     PhotonStaging S{};
     if (!direct) S = staging_ptrs<PhotonSoA>(ctx->ph_staging.p, n);
-    // Counting sort (default): the key pass counts the photons of every cell and gives each its rank in the cell; the
-    // exclusive scan of the counters IS cell_start; the packing pass (or a scatter pass over records that exist already)
-    // puts position plane entry and index at cell_start[key] + rank.  One streaming pass over the keys less than the
-    // radix sort takes for each of its three digits, no gather of the sorted plane, no cell-start search, and nothing
-    // to size from a count: dropped photons and the empty part of a dispatched inbox are simply never written.  The
-    // order inside a cell follows the atomics (the gather's float atomics are unordered anyway).
-    const bool counting = !ctx->radix_frustum;
-    uint32_t *cell_count = nullptr;
-    if (counting) {
-      CK(ctx->cell_count.reserve(((size_t)n_keys + 2) * 4));
-      cell_count = ctx->cell_count.as<uint32_t>();
-      CK(cudaMemsetAsync(cell_count, 0, ((size_t)n_keys + 2) * 4, st));
-      CK(ctx->sort_temp.reserve(std::max(sort_temp_bytes(n), cell_scan_temp_bytes(n_keys))));
-    }
+    // Counting sort: the key pass counts the photons of every cell and gives each its rank in the cell; the exclusive scan
+    // of the counters IS cell_start; the packing pass (or a scatter pass over records that exist already) puts position
+    // plane entry and index at cell_start[key] + rank.  Nothing to size from a count: dropped photons and the empty part
+    // of a dispatched inbox are simply never written.  The order inside a cell follows the atomics (the gather's float
+    // atomics are unordered anyway).
+    CK(cudaMemsetAsync(cell_count, 0, ((size_t)n_keys + 2) * 4, st));
     if (direct)   // position = first three floats of the record, path parity = bit 10 of its meta word
       launch_frustum_keys(ctx->rays.as<float4>(), ctx->n_rays, (const float *)ctx->records(), 32u, (const uint32_t *)ctx->records() + 3, 32u, 10u, n,
                           G, ctx->grid_occ.as<uint32_t>(), ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(),
-                          ctx->bounds.as<unsigned>() + 6, keepmask, block_kept, ctx->sm_count, st, ctx->region_cap, ctx->region_count,
-                          cell_count);
+                          ctx->bounds.as<unsigned>() + 6, keepmask, cell_count, ctx->region_cap, ctx->region_count, ctx->sm_count, st);
     else
       launch_frustum_keys(ctx->rays.as<float4>(), ctx->n_rays, S.pos, 3u, S.path_id, 1u, 0u, n, G, ctx->grid_occ.as<uint32_t>(),
                           ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), ctx->bounds.as<unsigned>() + 6, keepmask,
-                          block_kept, ctx->sm_count, st, 0, nullptr, cell_count);
-    const uint32_t *sortedKeys = nullptr, *sortedVals = nullptr;
-    uint32_t *ovf = block_kept + nb + 1;   // set when a bounded compaction meets more kept photons than it was sized for
-    CK(cudaMemsetAsync(ovf, 0, 4, st));
-    if (counting) {
-      CK(launch_cell_scan(ctx->sort_temp.p, ctx->sort_temp.cap, cell_count, ctx->cell_start.as<uint32_t>(), n_keys, st));
-      launch_pack_scatter(S, n, keepmask, ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), ctx->cell_start.as<uint32_t>(),
-                          ctx->records(), ctx->planes.as<float4>(), ctx->orig.as<uint32_t>(), st, direct,
-                          ctx->cell_start.as<uint32_t>() + n_keys - 1, ctx->sm_count);
-      sortedKeys = sortedVals = nullptr;
-      ctx->launches += 4;
-    } else if (ctx->kept_fraction_hint < 0.5) {
-      // sharded image: most photons are out of this rank's reach.  Compact the kept (key, index) pairs in index order
-      // (deterministic) and sort those only.  Their number sizes the sort: taken from the previous build's count (read
-      // back asynchronously) with a 25 % margin, the slots past the real count filled with DROP keys - no host round
-      // trip in the step.  Without a previous count (first build, or after an overflow) the exact count is read back.
-      launch_scan_u32(block_kept, nb, block_kept + nb, st);
-      const bool bounded = ctx->kept_hint_valid && !ctx->force_exact_build;
-      if (bounded) {
-        const uint32_t DROP = n_keys - 1;
-        m = (uint32_t)std::min<double>((double)n, ctx->kept_fraction_hint * 1.25 * (double)n + 65536.0);
-        launch_fill_u32(ctx->keys_out.as<uint32_t>(), m, DROP, st);
-        CK(cudaMemsetAsync(ctx->vals_out.p, 0, 4 * (size_t)m, st));
-        launch_compact_kept(ctx->keys_in.as<uint32_t>(), keepmask, block_kept, n, ctx->keys_out.as<uint32_t>(),
-                            ctx->vals_out.as<uint32_t>(), st, m, ovf);
-        CK(cudaMemcpyAsync(ctx->pin_host + 30, block_kept + nb, 4, cudaMemcpyDeviceToHost, st));
-        CK(cudaEventRecord(ctx->ev_hint, st));
-        ctx->hint_pending = true;
-        ctx->hint_n = n;
-        ctx->launches += 1;
-      } else {
-        launch_compact_kept(ctx->keys_in.as<uint32_t>(), keepmask, block_kept, n, ctx->keys_out.as<uint32_t>(),
-                            ctx->vals_out.as<uint32_t>(), st, n, ovf);
-        CK(cudaMemcpyAsync(ctx->pair_count_host, block_kept + nb, 4, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        m = *(const uint32_t *)ctx->pair_count_host;
-        ctx->kept_fraction_hint = (double)m / (double)n;
-        ctx->kept_hint_valid = true;
-        ctx->force_exact_build = false;
-        ctx->hint_pending = false;
-      }
-      if (m) CK(run_sort_bits(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_out.as<uint32_t>(), ctx->keys_in.as<uint32_t>(),
-                              ctx->vals_out.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), m, bits, st));
-      sortedKeys = ctx->keys_in.as<uint32_t>();
-      sortedVals = ctx->vals_in.as<uint32_t>();
-      ctx->launches += 2;
-    } else {
-      CK(run_sort_bits(ctx->sort_temp.p, ctx->sort_temp.cap, ctx->keys_in.as<uint32_t>(), ctx->keys_out.as<uint32_t>(),
-                       ctx->vals_in.as<uint32_t>(), ctx->vals_out.as<uint32_t>(), n, bits, st));
-      sortedKeys = ctx->keys_out.as<uint32_t>();
-      sortedVals = ctx->vals_out.as<uint32_t>();
-    }
+                          cell_count, 0, nullptr, ctx->sm_count, st);
+    CK(launch_cell_scan(ctx->sort_temp.p, ctx->sort_temp.cap, cell_count, ctx->cell_start.as<uint32_t>(), n_keys, st));
+    launch_pack_scatter(S, n, keepmask, ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), ctx->cell_start.as<uint32_t>(),
+                        ctx->records(), ctx->planes.as<float4>(), ctx->orig.as<uint32_t>(), st, direct,
+                        ctx->cell_start.as<uint32_t>() + n_keys - 1, ctx->sm_count);
     ctx->build_ovf = ovf;
-    if (!counting) {
-      launch_cell_starts(sortedKeys, m, n_keys, ctx->cell_start.as<uint32_t>(),
-                         ctx->grid_occ.as<char>() + frustum_occ_bytes(), ctx->sm_count, st);
-      launch_pack_sorted_kept(S, n, keepmask, sortedVals, m, ctx->records(), ctx->planes.as<float4>(),
-                              ctx->orig.as<uint32_t>(), st, direct);
-    }
     CK(cudaEventRecord(ctx->ev_free[ctx->ph_staging_sel], st));   // last read of the staging buffer
-    if (!counting && m == n) {   // kept count of this build -> hint of the next one (no blocking)
-      CK(cudaMemcpyAsync(ctx->pin_host + 30, ctx->cell_start.as<uint32_t>() + n_keys - 1, 4, cudaMemcpyDeviceToHost, st));
-      CK(cudaEventRecord(ctx->ev_hint, st));
-      ctx->hint_pending = true;
-      ctx->hint_n = n;
-    }
-    ctx->launches += 9 + 4;
+    ctx->launches += 17;
     CK(cudaGetLastError());
   } else {
     CK(cudaMemsetAsync(ctx->bounds.p, 0, 7 * sizeof(float), st));
     CK(cudaMemsetAsync(ctx->cell_start.p, 0, ((size_t)n_keys + 1) * 4, st));
   }
   Tree T{};
-  T.n = m;
+  T.n = n;
   ctx->grid = G;
   int rc = points_built(ctx, T, radius, gvpm_ctx::ACCEL_FRUSTUM, true, n);
   if (rc) return rc;

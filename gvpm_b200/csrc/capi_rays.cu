@@ -30,12 +30,6 @@ int gvpm_commit_rays(gvpm_ctx *ctx) {
     CK(cudaGetLastError());
   }
   ctx->rays_loaded = true;
-  if (n != ctx->hint_rays) {   // another ray set (not a re-jittered one): what the last build kept says nothing about the next
-    ctx->hint_rays = n;
-    ctx->kept_hint_valid = false;
-    ctx->hint_pending = false;
-    ctx->kept_fraction_hint = 1.0;
-  }
   return GVPM_OK;
 }
 

@@ -198,7 +198,7 @@ struct GatherParams {
   // frustum-grid variant of the point gather (tree_build.cu / gather_bre.cu k_bre_grid_traverse)
   FrustumGrid grid;
   const uint32_t *cell_start;   // [grids * n_cells + 3]
-  const uint32_t *build_ovf;    // frustum build sized from the previous iteration's count: set when it was too small
+  const uint32_t *build_ovf;    // frustum build over a dispatched inbox: set when a peer's dispatch timed out or overflowed
   const float4 *planes;  // [n] sorted P0 = pos.xyz, meta (the only per-photon data the traversal reads)
   const float4 *aos;     // [n][8] full records in the caller's order (shading reads aos[orig[slot]])
   const uint32_t *orig;  // [n] original photon index of sorted slot

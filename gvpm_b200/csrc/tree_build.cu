@@ -535,29 +535,23 @@ __global__ void __launch_bounds__(256) k_frustum_mark(const float4 *__restrict__
   for (int w = threadIdx.x; w < kOccWords; w += blockDim.x)
     if (mask[w]) atomicOr(occ + w, mask[w]);
 }
-// per photon: footprint class, cell, key (see FrustumGrid).  vals = photon index.  coord_mag: atomicMax of the largest
-// |coordinate| (float bits; the traversal's rounding pad).
+// per photon: footprint class, cell, key (see FrustumGrid).  vals = the photon's rank inside its cell (one atomic on the
+// cell's counter): cell_start is the exclusive scan of the counters, and k_scatter_index puts the photon's index at
+// cell_start[key] + rank.  coord_mag: atomicMax of the largest |coordinate| (float bits; the traversal's rounding pad).
 __global__ void __launch_bounds__(256) k_frustum_keys(const float *__restrict__ pos, uint32_t stride,
                                                        const uint32_t *__restrict__ par_src, uint32_t par_stride, uint32_t par_shift,
                                                        uint32_t n, const FrustumGrid G, const uint32_t *__restrict__ occ,
                                                        uint32_t *__restrict__ keys, uint32_t *__restrict__ vals,
                                                        unsigned *__restrict__ coord_mag, uint32_t *__restrict__ keepmask,
-                                                       uint32_t *__restrict__ block_kept, uint32_t region_cap,
-                                                       const uint32_t *__restrict__ region_count,
-                                                       uint32_t *__restrict__ cell_count) {
-  // cell_count != null: counting sort.  vals[i] becomes the photon's rank inside its cell (one atomic on the cell's
-  // counter), cell_start the exclusive scan of the counters, and k_scatter_index puts the photon's index at
-  // cell_start[key] + rank: no radix sort, no cell-start search.
+                                                       uint32_t *__restrict__ cell_count, uint32_t region_cap,
+                                                       const uint32_t *__restrict__ region_count) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   float mag = 0.f;
   bool keep = false;
   // dispatched photon sets (dispatch.cu): the index space is one region of region_cap records per sending rank, of which
   // the first region_count[sender] are filled
   const bool filled = i < n && (region_cap == 0u || (i % region_cap) < __ldg(region_count + i / region_cap));
-  if (i < n && !filled) {
-    keys[i] = (G.parity_split ? 2u : 1u) * G.n_cells + 1u;
-    vals[i] = i;
-  }
+  if (i < n && !filled) keys[i] = (G.parity_split ? 2u : 1u) * G.n_cells + 1u;
   if (filled) {
     const float px = pos[(size_t)stride * i], py = pos[(size_t)stride * i + 1], pz = pos[(size_t)stride * i + 2];
     mag = fmaxf(fmaxf(fabsf(px), fabsf(py)), fabsf(pz));
@@ -565,16 +559,11 @@ __global__ void __launch_bounds__(256) k_frustum_keys(const float *__restrict__ 
     const uint32_t DROP = (G.parity_split ? 2u : 1u) * G.n_cells + 1u;
     keys[i] = key;
     keep = key != DROP;
-    vals[i] = (cell_count && keep) ? atomicAdd(cell_count + key, 1u) : i;
+    if (keep) vals[i] = atomicAdd(cell_count + key, 1u);
   }
-  // one keep bit per photon (word = 32 consecutive photons) and the CTA's number of kept photons: the record packing and
-  // the compaction in front of the sort (sharded images keep a small part of the set) read them
-  __shared__ uint32_t wkept[8];
+  // one keep bit per photon (word = 32 consecutive photons): the record packing and the index scatter read them
   const uint32_t km = __ballot_sync(0xffffffffu, keep);
-  if ((threadIdx.x & 31) == 0) {
-    if (i < n) keepmask[i >> 5] = km;
-    wkept[threadIdx.x >> 5] = __popc(km);
-  }
+  if ((threadIdx.x & 31) == 0 && i < n) keepmask[i >> 5] = km;
   // one atomic per CTA, and only while the CTA's maximum beats what is already there (a single hot address otherwise
   // serialises hundreds of thousands of atomics)
   __shared__ float wmag[8];
@@ -583,9 +572,7 @@ __global__ void __launch_bounds__(256) k_frustum_keys(const float *__restrict__ 
   __syncthreads();
   if (threadIdx.x == 0) {
     float m = 0.f;
-    uint32_t tot = 0;
-    for (int k = 0; k < (int)(blockDim.x >> 5); ++k) { m = fmaxf(m, wmag[k]); tot += wkept[k]; }
-    block_kept[blockIdx.x] = tot;
+    for (int k = 0; k < (int)(blockDim.x >> 5); ++k) m = fmaxf(m, wmag[k]);
     if (m > __uint_as_float(*(volatile unsigned *)coord_mag)) atomicMax(coord_mag, __float_as_uint(m));
   }
 }
@@ -607,11 +594,9 @@ __global__ void k_gather_by_index(const float4 *__restrict__ aos, const uint32_t
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x)
     planes[i] = __ldg(aos + (size_t)__ldg(orig + i) * GVPM_AOS_FLOAT4);
 }
-// (key, index) of the kept photons, in index order, packed to the front: block_off = exclusive scan of block_kept
-__global__ void __launch_bounds__(256) k_compact_kept(const uint32_t *__restrict__ keys, const uint32_t *__restrict__ keepmask,
-                                                       const uint32_t *__restrict__ block_off, uint32_t n,
-                                                       uint32_t *__restrict__ keys_c, uint32_t *__restrict__ vals_c,
-                                                       uint32_t limit, uint32_t *__restrict__ overflow) {
+// indices of the kept photons, in index order, packed to the front: block_off = exclusive scan of block_kept
+__global__ void __launch_bounds__(256) k_compact_kept(const uint32_t *__restrict__ keepmask, const uint32_t *__restrict__ block_off,
+                                                       uint32_t n, uint32_t *__restrict__ vals_c) {
   __shared__ BallotCounts<8> kept;
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   const uint32_t km = i < n ? __ldg(keepmask + (i >> 5)) : 0u;   // i and its warp share the word (blockDim = 256, aligned)
@@ -619,57 +604,7 @@ __global__ void __launch_bounds__(256) k_compact_kept(const uint32_t *__restrict
   __syncthreads();
   const int lane = threadIdx.x & 31;
   if (!(km >> lane & 1u)) return;
-  const uint32_t pos = block_off[blockIdx.x] + kept.before() + __popc(km & ((1u << lane) - 1u));
-  if (pos >= limit) {   // more kept photons than the (bounded) sort was sized for: the build is incomplete, say so
-    *overflow = 1u;
-    return;
-  }
-  if (keys) keys_c[pos] = keys[i];
-  vals_c[pos] = i;
-}
-__global__ void k_fill_u32(uint32_t *__restrict__ p, uint32_t n, uint32_t value) {
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) p[i] = value;
-}
-// cell_start[k] = first sorted slot whose key is >= k, for k in [0, n_keys].  Lane i owns the gap of keys in front of
-// slot i; the warp fills its lanes' gaps one after the other with all 32 lanes writing (coalesced).  Gaps of 4096 cells
-// and more (whole empty classes) are left to the second pass, which spreads each of them over the whole grid.
-struct BigGap { uint32_t lo, hi, val; };
-__global__ void __launch_bounds__(256) k_cell_starts(const uint32_t *__restrict__ sorted_keys, uint32_t n, uint32_t n_keys,
-                                                      uint32_t *__restrict__ cell_start, BigGap *__restrict__ big,
-                                                      uint32_t *__restrict__ n_big, uint32_t big_cap) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  const int lane = threadIdx.x & 31;
-  uint32_t lo = 1u, hi = 0u;   // empty
-  if (i <= n) {
-    lo = i == 0 ? 0u : sorted_keys[i - 1] + 1u;
-    hi = i == n ? n_keys : min(sorted_keys[i], n_keys);   // inclusive
-  }
-  const bool has = lo <= hi;
-  if (has && hi - lo >= 4095u) {
-    const uint32_t slot = atomicAdd(n_big, 1u);
-    if (slot < big_cap) big[slot] = BigGap{lo, hi, i};
-    lo = 1u; hi = 0u;
-  } else if (has && hi == lo) {
-    cell_start[lo] = i;   // the common case: one cell per photon step
-    lo = 1u; hi = 0u;
-  }
-  uint32_t m = __ballot_sync(0xffffffffu, lo <= hi);
-  while (m) {
-    const int src = __ffs(m) - 1;
-    m &= m - 1;
-    const uint32_t glo = __shfl_sync(0xffffffffu, lo, src), ghi = __shfl_sync(0xffffffffu, hi, src),
-                   gv = __shfl_sync(0xffffffffu, i, src);
-    for (uint32_t k = glo + lane; k <= ghi; k += 32) cell_start[k] = gv;
-  }
-}
-__global__ void __launch_bounds__(256) k_cell_starts_big(uint32_t *__restrict__ cell_start, const BigGap *__restrict__ big,
-                                                          const uint32_t *__restrict__ n_big, uint32_t big_cap) {
-  const uint32_t nb = min(*n_big, big_cap);
-  const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, stride = gridDim.x * blockDim.x;
-  for (uint32_t g = 0; g < nb; ++g) {
-    const BigGap G = big[g];
-    for (uint32_t k = G.lo + tid; k <= G.hi; k += stride) cell_start[k] = G.val;
-  }
+  vals_c[block_off[blockIdx.x] + kept.before() + __popc(km & ((1u << lane) - 1u))] = i;
 }
 
 // raw ray SoA -> 5 x 64 B records per ray
@@ -728,7 +663,7 @@ void launch_pack_sorted(const PhotonStaging &S, float4 *aos, const uint32_t *sor
 }
 size_t ray_grid_bytes() { return sizeof(RayGrid); }
 size_t ray_mask_bytes() { return (size_t)kGridWords * 4; }
-// box: 6 floats (+inf x3, -inf x3 on entry); grid: RayGrid; mask: zeroed kGridWords words; counter: zeroed
+// box: 6 floats (+inf x3, -inf x3 on entry); grid: RayGrid; mask: zeroed kGridWords words
 void launch_ray_region(const float4 *rays, uint32_t nRays, float radius, float *box, void *grid, uint32_t *mask,
                        float *bounds, int sm_count, cudaStream_t st) {
   if (nRays) k_ray_box<<<std::min<uint32_t>((nRays + 255) / 256, 1024u), 256, 0, st>>>(rays, nRays, radius, box);
@@ -745,11 +680,10 @@ void launch_keep_pruned(const float *pos, uint32_t n, const void *grid, const ui
 void launch_keys_kept(const float *pos, const uint32_t *vals, uint32_t m, const void *grid, uint32_t *keys, cudaStream_t st) {
   if (m) k_keys_kept<<<(m + 255) / 256, 256, 0, st>>>(pos, vals, m, (const RayGrid *)grid, keys);
 }
-// records of the kept photons only (keepmask; skipped when they exist already), then the sorted position plane / index
-// map of the first m sorted slots
+// records of the kept photons only (keepmask), then the sorted position plane / index map of the first m sorted slots
 void launch_pack_sorted_kept(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *sorted, uint32_t m,
-                             float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st, bool records_ready) {
-  if (!records_ready && n) k_pack_aos_kept<<<(n + 255) / 256, 256, 0, st>>>(S, n, keepmask, aos);
+                             float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st) {
+  if (n) k_pack_aos_kept<<<(n + 255) / 256, 256, 0, st>>>(S, n, keepmask, aos);
   if (m) k_gather_sorted<<<(m + 255) / 256, 256, 0, st>>>(aos, sorted, m, planes, orig);
 }
 // in-place exclusive scan of nb words by one CTA (a few thousand entries, 8 per thread); total -> total[0]
@@ -770,25 +704,22 @@ void launch_pinhole_fit(const float4 *rays, uint32_t n, double *partial, float *
   k_pinhole_check<<<nb, 256, 0, st>>>(rays, n, fit, stats);
 }
 size_t frustum_occ_bytes() { return (size_t)kOccWords * 4; }
-void launch_compact_kept(const uint32_t *keys, const uint32_t *keepmask, const uint32_t *block_off, uint32_t n,
-                         uint32_t *keys_c, uint32_t *vals_c, cudaStream_t st, uint32_t limit, uint32_t *overflow) {
-  if (n) k_compact_kept<<<(n + 255) / 256, 256, 0, st>>>(keys, keepmask, block_off, n, keys_c, vals_c, limit, overflow);
+void launch_compact_kept(const uint32_t *keepmask, const uint32_t *block_off, uint32_t n, uint32_t *vals_c, cudaStream_t st) {
+  if (n) k_compact_kept<<<(n + 255) / 256, 256, 0, st>>>(keepmask, block_off, n, vals_c);
 }
-void launch_fill_u32(uint32_t *p, uint32_t n, uint32_t value, cudaStream_t st) {
-  if (n) k_fill_u32<<<std::min<uint32_t>((n + 255) / 256, 2048u), 256, 0, st>>>(p, n, value);
-}
-// occ: frustum_occ_bytes() (zeroed here); coord_mag: one word (zeroed here)
+// occ: frustum_occ_bytes() (zeroed here); coord_mag: one word (zeroed here); cell_count: n_keys + 1 words, zeroed
 // pos / stride: photon positions (stride in floats: 3 for the staged SoA plane, 32 for 128-byte records); parity of the
 // photon's path id = (par_src[par_stride * i] >> par_shift) & 1
+// region_cap / region_count: dispatched photon sets (0 / nullptr: every index up to n holds a photon)
 void launch_frustum_keys(const float4 *rays, uint32_t n_rays, const float *pos, uint32_t stride, const uint32_t *par_src,
                          uint32_t par_stride, uint32_t par_shift, uint32_t n,
                          const FrustumGrid &G, uint32_t *occ, uint32_t *keys, uint32_t *vals, unsigned *coord_mag,
-                         uint32_t *keepmask, uint32_t *block_kept, int sm_count, cudaStream_t st, uint32_t region_cap,
-                         const uint32_t *region_count, uint32_t *cell_count) {
+                         uint32_t *keepmask, uint32_t *cell_count, uint32_t region_cap, const uint32_t *region_count,
+                         int sm_count, cudaStream_t st) {
   cudaMemsetAsync(occ, 0, frustum_occ_bytes(), st);
   cudaMemsetAsync(coord_mag, 0, 4, st);
   if (n_rays) k_frustum_mark<<<std::min<uint32_t>((n_rays + 255) / 256, 2u * (uint32_t)sm_count), 256, 0, st>>>(rays, n_rays, G, occ);
-  if (n) k_frustum_keys<<<(n + 255) / 256, 256, 0, st>>>(pos, stride, par_src, par_stride, par_shift, n, G, occ, keys, vals, coord_mag, keepmask, block_kept, region_cap, region_count, cell_count);
+  if (n) k_frustum_keys<<<(n + 255) / 256, 256, 0, st>>>(pos, stride, par_src, par_stride, par_shift, n, G, occ, keys, vals, coord_mag, keepmask, cell_count, region_cap, region_count);
 }
 // counting sort: cell_start[0 .. n_keys] = exclusive scan of the per-cell counts (cell_count[n_keys] must be 0)
 size_t cell_scan_temp_bytes(uint32_t n_keys) {
@@ -813,17 +744,6 @@ void launch_pack_scatter(const PhotonStaging &S, uint32_t n, const uint32_t *kee
 void launch_frustum_mark(const float4 *rays, uint32_t n_rays, const FrustumGrid &G, uint32_t *occ, int sm_count, cudaStream_t st) {
   cudaMemsetAsync(occ, 0, frustum_occ_bytes(), st);
   if (n_rays) k_frustum_mark<<<std::min<uint32_t>((n_rays + 255) / 256, 2u * (uint32_t)sm_count), 256, 0, st>>>(rays, n_rays, G, occ);
-}
-// scratch: cell_starts_scratch_bytes(n_keys) bytes
-size_t cell_starts_scratch_bytes(uint32_t n_keys) { return 16 + ((size_t)n_keys / 4096 + 2) * sizeof(BigGap); }
-void launch_cell_starts(const uint32_t *sorted_keys, uint32_t n, uint32_t n_keys, uint32_t *cell_start, void *scratch,
-                        int sm_count, cudaStream_t st) {
-  uint32_t *n_big = (uint32_t *)scratch;
-  BigGap *big = (BigGap *)((char *)scratch + 16);
-  const uint32_t cap = n_keys / 4096 + 2;   // gaps of >= 4096 cells are disjoint: there cannot be more of them
-  cudaMemsetAsync(n_big, 0, 4, st);
-  k_cell_starts<<<(n + 1 + 255) / 256, 256, 0, st>>>(sorted_keys, n, n_keys, cell_start, big, n_big, cap);
-  k_cell_starts_big<<<2 * sm_count, 256, 0, st>>>(cell_start, big, n_big, cap);
 }
 void launch_leaf_boxes(const float4 *p0, uint32_t n, uint32_t nLeaves, float radius, float4 *lo, float4 *hi,
                        cudaStream_t st) {

@@ -44,10 +44,9 @@ def _oracle(case, rays):
     return ob.bre_gather(case.photons, rays, case.medium, case.config, case.tri, case.radius, mode="brute", neighbours=True)
 
 
-@pytest.mark.parametrize("world,cycles,view_dir,sort", [(2, 2, None, "counting"), (4, 1, None, "radix"), (4, 2, (0.0, 0.0, 1.0), "counting"),
-                                                        (8, 1, (0.05, -0.02, 1.0), "counting"), (8, 1, (0.0, 0.0, 1.0), "radix")])
-def test_dispatched_gather_equals_oracle(built, world, cycles, view_dir, sort, monkeypatch):
-    monkeypatch.setenv("GVPM_FRUSTUM_SORT", sort)
+@pytest.mark.parametrize("world,cycles,view_dir", [(2, 2, None), (4, 1, None), (4, 2, (0.0, 0.0, 1.0)), (8, 1, (0.05, -0.02, 1.0)),
+                                                   (8, 1, (0.0, 0.0, 1.0))])
+def test_dispatched_gather_equals_oracle(built, world, cycles, view_dir):
     case = H.make_case(n_photons=120000, w=256, h=64, scale=1.0)
     ctxs, rays, n_slice = _ranks(case, world, cycles, view_dir)
     n = case.photons.n

@@ -100,13 +100,10 @@ def test_vpm_after_frustum_build_rebuilds_the_hierarchy(built):
     ctx.close()
 
 
-@pytest.mark.parametrize("sort", ["counting", "radix"])
-def test_second_sharded_build_compacts_before_the_sort(built, sort, monkeypatch):
-    """Repeated builds of a sharded ray set.  Counting sort (default): dropped photons are never written.  Radix sort
-    (GVPM_FRUSTUM_SORT=radix, the A/B switch): the first build reports how few photons it kept, the next ones compact the
-    kept (key, index) pairs before sorting.  Same counts, same radiance either way."""
+def test_repeated_sharded_builds_keep_the_same_count(built):
+    """Repeated builds of a sharded ray set (each over a new upload of the photons): every build keeps the same number of
+    photons, a small part of the set, and gives the oracle's exact neighbour counts and its radiance."""
     from oracle import binding as ob
-    monkeypatch.setenv("GVPM_FRUSTUM_SORT", sort)
     case = H.make_case(n_photons=80000, w=64, h=64, scale=0.5)
     idx = shard.band_indices(case.rays.px, case.rays.py, 64, 64, 8, 3, 1)
     case.rays = case.rays.take(idx)
@@ -123,46 +120,6 @@ def test_second_sharded_build_compacts_before_the_sort(built, sort, monkeypatch)
         outs.append(kept)
     assert outs[0] == outs[1] == outs[2]
     ctx.close()
-
-
-def test_bounded_build_overflow_is_reported_and_recovered(built, monkeypatch):
-    """Radix-sort variant of the sharded build (GVPM_FRUSTUM_SORT=radix): it sizes its sort from the previous iteration's
-    kept count (+25 %, no host round trip).  When an iteration keeps far more, the gather must say so instead of
-    returning a partial result, and the next build (exact count) must give the right answer."""
-    from oracle import binding as ob
-    from gvpm_b200.api import GvpmError
-    monkeypatch.setenv("GVPM_FRUSTUM_SORT", "radix")
-    case = H.make_case(n_photons=1600000, w=64, h=64, scale=0.5)
-    idx = shard.band_indices(case.rays.px, case.rays.py, 64, 64, 8, 3, 1)
-    case.rays = case.rays.take(idx)
-    ctx = H.gpu_context(case)
-    assert ctx.build_points_for_rays(case.radius) > 65536 * 1.3     # what the set keeps for these rays
-    far = case.photons.copy()
-    far.view("pos")[:] += np.float32(40.0)         # an iteration whose photons no ray can reach
-    for _ in range(3):                              # full sort, then exact compaction, then a bounded one sized for ~0 kept
-        ctx.upload_photons(far)
-        assert ctx.build_points_for_rays(case.radius) == 0
-        out, counts = ctx.gather_bre()
-        assert not counts.any()
-    ctx.upload_photons(case.photons)                # ... followed by one that keeps > 65536 + 25 %
-    ctx.build_points_for_rays(case.radius, want_kept=False)
-    with pytest.raises(GvpmError, match="sized from the previous iteration"):   # ("... is incomplete - it was sized from ...")
-        ctx.gather_bre()
-    kept = ctx.build_points_for_rays(case.radius)   # exact count this time
-    assert kept > 65536 * 1.3
-    out, counts = ctx.gather_bre()
-    ref = ob.bre_gather(case.photons, case.rays, case.medium, case.config, case.tri, case.radius, mode="brute")
-    np.testing.assert_array_equal(counts, ref.counts)
-    H.assert_radiance_close(out, ref.out, 1e-4, "after the overflow")
-    ctx.close()
-
-
-def test_frustum_radix_sort_variant_matches_oracle(built, monkeypatch):
-    """GVPM_FRUSTUM_SORT=radix keeps the radix-sorted build of the perspective grid (stable order inside a cell)"""
-    monkeypatch.setenv("GVPM_FRUSTUM_SORT", "radix")
-    case = H.make_case(n_photons=60000, w=64, h=48, scale=2.0)
-    ref, kept = _check(case, "frustum, radix sort")
-    assert ref.counts[:, 0].sum() > 3000
 
 
 def test_view_direction_does_not_change_results(built):
