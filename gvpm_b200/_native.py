@@ -112,6 +112,7 @@ ABI_SYMBOLS = [
     "gvpm_gather_bre_device", "gvpm_gather_bre_into", "gvpm_gather_bre_host", "gvpm_dump_neighbours_bre",
     "gvpm_compute_gradient", "gvpm_compute_gradient_reuse_primal", "gvpm_poisson_preset", "gvpm_poisson_solve", "gvpm_reconstruct", "gvpm_last_poisson_ms", "gvpm_last_timings", "gvpm_last_gather_detail", "gvpm_launch_count",
     "gvpm_upload_vpm_samples", "gvpm_gather_vpm", "gvpm_gather_vpm_device", "gvpm_dump_neighbours_vpm",
+    "gvpm_generate_vpm_samples",
     "gvpm_upload_beams", "gvpm_build_beams", "gvpm_gather_beams", "gvpm_gather_beams_device", "gvpm_dump_neighbours_beams", "gvpm_beam_subbeam_count",
     "gvpm_gather_sppm_beams", "gvpm_dump_neighbours_sppm_beams",
     "gvpm_box_scene_default", "gvpm_generate_rays", "gvpm_trace_photons", "gvpm_trace_photons_direct", "gvpm_trace_beams", "gvpm_planes_from_beams", "gvpm_read_device", "gvpm_measure_read_bandwidth", "gvpm_staging_peek",
@@ -224,6 +225,8 @@ def load_lib():
     lib.gvpm_upload_vpm_samples.argtypes = [vp, C.POINTER(VpmSampleSoA), C.c_size_t]
     lib.gvpm_gather_vpm.argtypes = [vp, C.c_int, f32p, u32p, u32p]
     lib.gvpm_dump_neighbours_vpm.argtypes = [vp, C.c_int, u64p, u32p, C.c_size_t]
+    lib.gvpm_generate_vpm_samples.argtypes = [vp, C.c_int, C.c_int, C.c_uint64, C.c_float, C.c_float, vp,
+                                              C.POINTER(C.c_size_t)]
     lib.gvpm_launch_count.argtypes = [vp]
     lib.gvpm_launch_count.restype = C.c_uint64
     for name in ABI_SYMBOLS:

@@ -433,6 +433,37 @@ class Context:
         self._ck(self.lib.gvpm_upload_vpm_samples(self.h, C.byref(cs), samples.n), "gvpm_upload_vpm_samples")
         self.n_samples = samples.n
 
+    def generate_vpm_samples(self, nb_camera_samples=40, seed=0, radius=None, radius_per_ray=None, stratified=False,
+                             epsilon=1e-4):
+        """the distance samples of the current ray set drawn on the device (what synth_vpm_samples draws, in place of
+        upload_vpm_samples); radius: one radius for every ray, or radius_per_ray: a device pointer (int) or an object
+        with data_ptr(), such as a CUDA float32 tensor of n_rays.  -> number of samples drawn"""
+        ptr = None
+        if radius_per_ray is not None:
+            if hasattr(radius_per_ray, "data_ptr"):
+                if str(getattr(radius_per_ray, "dtype", "float32")).rsplit(".", 1)[-1] != "float32":
+                    raise ValueError("radius_per_ray must hold float32")
+                if getattr(radius_per_ray, "is_cuda", True) is False:
+                    raise ValueError("radius_per_ray must be in device memory")
+                if hasattr(radius_per_ray, "numel") and radius_per_ray.numel() < self.n_rays:
+                    raise ValueError(f"radius_per_ray holds {radius_per_ray.numel()} values for {self.n_rays} rays")
+                ptr = radius_per_ray.data_ptr()
+            else:
+                ptr = int(radius_per_ray)
+        n = C.c_size_t(0)
+        self._ck(self.lib.gvpm_generate_vpm_samples(self.h, int(nb_camera_samples), int(bool(stratified)),
+                                                    C.c_uint64(int(seed) & 0xFFFFFFFFFFFFFFFF),
+                                                    C.c_float(epsilon), C.c_float(0.0 if radius is None else radius),
+                                                    C.c_void_p(ptr) if ptr else None, C.byref(n)),
+                 "gvpm_generate_vpm_samples")
+        self.n_samples = int(n.value)
+        return self.n_samples
+
+    def download_vpm_samples(self):
+        """parity aid: the current distance samples (uploaded or drawn on the device) as a VpmSampleSet"""
+        from . import records as R
+        return self._download_staged(4, R.VpmSampleSet, R._VPM_FIELDS)
+
     def gather_vpm_device(self, nb_camera_samples):
         o, m = C.c_void_p(), C.c_void_p()
         self._ck(self.lib.gvpm_gather_vpm_device(self.h, nb_camera_samples, C.byref(o), C.byref(m)),

@@ -214,9 +214,9 @@ int gvpm_read_device(gvpm_ctx *ctx, const void *dev, void *host, size_t bytes) {
 }
 
 int gvpm_staging_peek(gvpm_ctx *ctx, int which, void **dev, size_t *count) {
-  if (!ctx || !dev || which < 0 || which > 3) return GVPM_ERR_INVALID;
-  const DevBuf *buf[4] = {&ctx->ph_staging, &ctx->ray_staging, &ctx->beam_staging, &ctx->plane_staging};
-  const size_t n[4] = {ctx->n_photons, ctx->n_rays, ctx->n_beams, ctx->n_planes};
+  if (!ctx || !dev || which < 0 || which > 4) return GVPM_ERR_INVALID;
+  const DevBuf *buf[5] = {&ctx->ph_staging, &ctx->ray_staging, &ctx->beam_staging, &ctx->plane_staging, &ctx->sample_staging};
+  const size_t n[5] = {ctx->n_photons, ctx->n_rays, ctx->n_beams, ctx->n_planes, ctx->n_samples};
   *dev = buf[which]->p;
   if (count) *count = n[which];
   return GVPM_OK;

@@ -335,6 +335,8 @@ static int vpm_params(gvpm_ctx *ctx, GatherParams &P, int nb_camera_samples) {
   int rc = fill_params(ctx, P, ctx->out.as<float>(), nullptr);
   if (rc) return rc;
   if (!ctx->samples_loaded) return fail(ctx, GVPM_ERR_INVALID, "no VPM samples uploaded");
+  if (ctx->samples_drawn && ctx->samples_rays_gen != ctx->rays_gen)
+    return fail(ctx, GVPM_ERR_INVALID, "VPM samples were drawn for another ray set: draw them again");
   if (nb_camera_samples <= 0) return fail(ctx, GVPM_ERR_INVALID, "nbCameraSamples must be positive");
   if (ctx->sample_radius_max > ctx->radius)
     return fail(ctx, GVPM_ERR_INVALID, "gvpm_build_points radius is smaller than a sample radius");
@@ -511,13 +513,38 @@ int gvpm_dump_neighbours_bre(gvpm_ctx *ctx, uint64_t *offsets, uint32_t *idx, si
       });
 }
 
-// The six arrays go up as they are and one kernel packs them (2 float4 per sample), finds the largest sample radius and
-// checks the ray indices (pack_prims.cu); both are looked at after the copy of two words at the end of this call.
+// The sample staging buffer holds a set of n samples (n_dev: a count known on the device only, n is then its bound):
+// one kernel packs them (2 float4 per sample), finds the largest sample radius and checks the ray indices and the
+// radii (pack_prims.cu); the host reads the stats (and the count) with one copy of three words and checks them.
+// Negative or non-finite radii are refused for drawn samples only (an uploaded set keeps the checks it always had).
+static int commit_samples(gvpm_ctx *ctx, uint32_t n, const uint32_t *n_dev, bool drawn) {
+  uint32_t *stats = ctx->work_counter.as<uint32_t>() + 8;   // words 8, 9 of the counter block (+ word 10: n_dev)
+  CK(cudaMemsetAsync(stats, 0, 8, ctx->stream));
+  launch_pack_samples(ctx->sample_staging.p, n, n_dev, ctx->n_rays, ctx->samples.as<float4>(), stats, ctx->stream);
+  ctx->launches += n ? 1 : 0;
+  CK(cudaGetLastError());
+  uint32_t *host = ctx->sample_stats_host + 8;
+  CK(cudaMemcpyAsync(host, stats, n_dev ? 12 : 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));   // the caller's arrays are only read during the call
+  ctx->n_samples = n_dev ? host[2] : n;
+  if (host[1] & 1u) {
+    ctx->samples_loaded = false;
+    return fail(ctx, GVPM_ERR_INVALID, "sample refers to a ray that is not uploaded");
+  }
+  if (drawn && (host[1] & 2u)) {
+    ctx->samples_loaded = false;
+    return fail(ctx, GVPM_ERR_INVALID, "per-ray radius must be finite and >= 0");
+  }
+  memcpy(&ctx->sample_radius_max, &host[0], 4);
+  return GVPM_OK;
+}
+
 int gvpm_upload_vpm_samples(gvpm_ctx *ctx, const gvpm_vpm_sample_soa *s, size_t n) {
   if (!ctx || (n && !s) || n > 0xfffffff0u) return GVPM_ERR_INVALID;
   cudaSetDevice(ctx->device);
   ctx->n_samples = (uint32_t)n;
   ctx->samples_loaded = true;
+  ctx->samples_drawn = false;
   ctx->sample_radius_max = 0.f;
   ++ctx->state_gen;
   if (n == 0) return GVPM_OK;
@@ -526,19 +553,62 @@ int gvpm_upload_vpm_samples(gvpm_ctx *ctx, const gvpm_vpm_sample_soa *s, size_t 
   CK(ctx->sample_counts.reserve(2 * n * sizeof(uint32_t)));
   int rc = copy_soa<SampleSoA>(ctx, *s, ctx->sample_staging.p, n, 0, 0, n, ctx->stream);
   if (rc) return rc;
-  uint32_t *stats = ctx->work_counter.as<uint32_t>() + 8;   // words 8, 9 of the counter block
-  CK(cudaMemsetAsync(stats, 0, 8, ctx->stream));
-  launch_pack_samples(staging_ptrs<SampleSoA>(ctx->sample_staging.p, n), (uint32_t)n, ctx->n_rays,
-                      ctx->samples.as<float4>(), stats, ctx->stream);
-  ctx->launches += 1;
+  return commit_samples(ctx, (uint32_t)n, nullptr, false);
+}
+
+// Count -> scan -> emit over the rays (generate.cu), then the upload's pack and checks on the drawn set.  The buffers
+// are sized for the bound n_rays * nb; the staging arrays are laid out for the count the scan finds, which the host
+// learns from the pack's stats read-back.
+int gvpm_generate_vpm_samples(gvpm_ctx *ctx, int nb_camera_samples, int stratified, uint64_t seed, float epsilon,
+                              float radius, const float *radius_per_ray_dev, size_t *n_samples) {
+  if (!ctx) return GVPM_ERR_INVALID;
+  if (!ctx->rays_loaded) return fail(ctx, GVPM_ERR_INVALID, "gvpm_generate_vpm_samples: no committed ray set");
+  if (!ctx->have_medium) return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_medium first");
+  if (nb_camera_samples <= 0) return fail(ctx, GVPM_ERR_INVALID, "nbCameraSamples must be positive");
+  if (!(epsilon > 0.f)) return fail(ctx, GVPM_ERR_INVALID, "epsilon must be > 0");
+  if (!radius_per_ray_dev && !(std::isfinite(radius) && radius > 0.f))
+    return fail(ctx, GVPM_ERR_INVALID, "radius must be finite and > 0 (or give a per-ray radius array)");
+  const uint32_t nr = ctx->n_rays;
+  const size_t bound = (size_t)nr * (size_t)nb_camera_samples;
+  if (bound > 0xfffffff0u) return fail(ctx, GVPM_ERR_INVALID, "n_rays * nb_camera_samples exceeds 0xfffffff0 samples");
+  cudaSetDevice(ctx->device);
+  ctx->n_samples = 0;
+  ctx->samples_loaded = true;
+  ctx->samples_drawn = true;
+  ctx->samples_rays_gen = ctx->rays_gen;
+  ctx->sample_radius_max = 0.f;
+  ++ctx->state_gen;
+  if (n_samples) *n_samples = 0;
+  if (nr == 0) return GVPM_OK;
+  const uint32_t tiles = (nr + 255) / 256;
+  CK(ctx->sample_staging.reserve(SoaLayout<SampleSoA>(bound).bytes));
+  CK(ctx->samples.reserve(2 * bound * sizeof(float4)));
+  CK(ctx->sample_counts.reserve(2 * bound * sizeof(uint32_t)));
+  CK(ctx->sample_scratch.reserve(4 * ((size_t)nr + tiles + 1)));
+  const RayStaging R = staging_ptrs<RaySoA>(ctx->ray_staging.p, nr);
+  uint32_t *total = ctx->work_counter.as<uint32_t>() + 10;   // word 10 of the counter block: read back by commit_samples
+  VpmGenParams P{};
+  P.o = R.o;
+  P.d = R.d;
+  P.edge_len = R.edge_len;
+  P.radius_per_ray = radius_per_ray_dev;
+  P.n_rays = nr;
+  P.nb = nb_camera_samples;
+  P.stratified = stratified ? 1 : 0;
+  P.seed = seed;
+  P.epsilon = epsilon;
+  P.radius = radius;
+  for (int c = 0; c < 3; ++c) P.sigma_t[c] = ctx->medium.sigma_s[c] + ctx->medium.sigma_a[c];
+  P.counts = ctx->sample_scratch.as<uint32_t>();
+  P.tile_tot = P.counts + nr;
+  P.n_total = total;
+  P.staging = ctx->sample_staging.p;
+  launch_vpm_samples(P, total, ctx->sm_count, ctx->stream);
+  ctx->launches += 3;
   CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(ctx->sample_stats_host, stats, 8, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));   // the caller's arrays are only read during the call
-  if (ctx->sample_stats_host[1]) {
-    ctx->samples_loaded = false;
-    return fail(ctx, GVPM_ERR_INVALID, "sample refers to a ray that is not uploaded");
-  }
-  memcpy(&ctx->sample_radius_max, &ctx->sample_stats_host[0], 4);
+  const int rc = commit_samples(ctx, (uint32_t)bound, total, true);
+  if (rc) return rc;
+  if (n_samples) *n_samples = ctx->n_samples;
   return GVPM_OK;
 }
 

@@ -94,7 +94,9 @@ void launch_sub_count(const float *len, uint32_t n, const float *subsize, uint32
 void launch_sub_emit(const float4 *rec, const float *len, uint32_t n, const float *subsize, const uint32_t *block_off,
                      uint32_t cap, float *sub_pos, float4 *sub_raw, cudaStream_t st);
 void launch_pack_planes(const PlaneStaging &S, uint32_t n, float4 *rec, float *centre, uint32_t *flag, cudaStream_t st);
-void launch_pack_samples(const SampleStaging &S, uint32_t n, uint32_t n_rays, float4 *packed, uint32_t *stats, cudaStream_t st);
+void launch_pack_samples(const void *staging, uint32_t n, const uint32_t *n_dev, uint32_t n_rays, float4 *packed,
+                         uint32_t *stats, cudaStream_t st);
+void launch_vpm_samples(const VpmGenParams &P, uint32_t *total, int sm_count, cudaStream_t st);
 size_t poisson_workspace_floats(size_t n);
 long long poisson_solve_device(const float *tp, const float *dx, const float *dy, const float *direct, int W, int H,
                                float alpha, int irlsIterMax, float irlsRegInit, float irlsRegIter, int cgIterMax,
@@ -262,11 +264,14 @@ struct gvpm_ctx {
   uint32_t n_planes = 0;
   bool planes_loaded = false, planes_built = false;
   DevBuf samples, sample_counts, mvol, sample_staging;  // G-VPM distance samples (+ their raw SoA arrays)
-  uint32_t *sample_stats_host = nullptr;  // pinned: [0] max sample radius (float bits), [1] bad ray index seen; [2] plane flag;
-                                          // [4] sub-beam size (float bits), [5] sub-beam count of traced beams
+  DevBuf sample_scratch;                  // gvpm_generate_vpm_samples: samples per ray, then per tile of 256 rays
+  uint32_t *sample_stats_host = nullptr;  // pinned: [2] plane flag; [4] sub-beam size (float bits), [5] sub-beam count of
+                                          // traced beams; [8..10] the sample pack's stats (commit_samples)
   uint32_t n_samples = 0;
   bool samples_loaded = false;
   float sample_radius_max = 0.f;
+  bool samples_drawn = false;             // the samples were drawn by gvpm_generate_vpm_samples, for ray set samples_rays_gen
+  uint64_t samples_rays_gen = 0;
   // what `out` holds for gvpm_accum_add: OUT_READY = the per-ray results (out_stride floats per ray) of the last gather,
   // run on ray set out_gen; OUT_ADDED = the same, already added; OUT_ELSEWHERE = the last gather wrote to caller memory
   enum { OUT_NONE = 0, OUT_READY, OUT_ADDED, OUT_ELSEWHERE };
@@ -340,6 +345,10 @@ struct SampleSoA {
   using Staging = SampleStaging;
   static constexpr const char *name = "gvpm_vpm_sample_soa";
 };
+
+// sample_staging_at (gvpm_device.cuh) states this layout for the device
+static_assert(SampleSoA::elt[0] == 4 && SampleSoA::elt[1] == 4 && SampleSoA::elt[2] == 12 && SampleSoA::elt[3] == 4 &&
+                  SampleSoA::elt[4] == 4 && SampleSoA::elt[5] == 4, "sample_staging_at");
 
 template <class S> struct SoaLayout {  // offsets of the arrays of n elements inside the staging buffer
   size_t off[S::N], bytes = 0;

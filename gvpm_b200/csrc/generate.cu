@@ -12,10 +12,15 @@
 //                     that does not escape, LTBeamMap::tryAppendLT (gvpm_beams.h:54-84).
 //   k_planes_from_beams   LTPhotonPlane::transformBeam (gvpm_plane.h:53-73) of every beam of the current set: one
 //                     thread per beam, photon planes written into the plane staging arrays.
-// Random numbers: PCG32 keyed by (seed, pixel index) / (seed, path index) / (seed ^ constant, beam index).  Arithmetic: strictly rounded fp32 in a fixed
+//   k_vpm_count / k_vpm_emit   the camera distance samples of G-VPM (computeVolumeGradientPhoton, gvpm.cpp:1141-1175,
+//                     as gvpm_synth_vpm_samples restates it) from the current ray set: one thread per ray, count ->
+//                     exclusive scan over tiles of rays -> emit into the sample staging arrays, so the samples land in
+//                     ray order.
+// Random numbers: PCG32 keyed by (seed, pixel index) / (seed, path index) / (seed ^ constant, beam or ray index).  Arithmetic: strictly rounded fp32 in a fixed
 // operation order; log, exp, sin and cos are polynomial routines (pm_*) built from +, -, *, / only, so a CPU
 // restatement compiled without FMA contraction reproduces every record bit for bit (tests/test_gpu_generate.py).
 #include "gvpm_device.cuh"
+#include "launch_sizing.cuh"
 #include "warp_ops.cuh"
 
 namespace gvpm {
@@ -474,6 +479,91 @@ __global__ void __launch_bounds__(256) k_planes_from_beams(const __grid_constant
   P.edge_id[i] = (int32_t)P.beams.depth[i];
 }
 
+// ---- G-VPM camera distance samples ----------------------------------------------------------------------------------
+// computeVolumeGradientPhoton's draws (gvpm.cpp:1141-1175) for a ray that is its gather point's only medium edge
+// (pdfSel = 1): nb uniforms, stratified or not, each turned into a distance by HomogeneousMedium::sampleDistance with
+// EDistanceAlwaysValid and the balance strategy (homogeneous.cpp:293-430), in gvpm_synth_vpm_samples' operation order.
+// Ray r draws from PCG32(seed ^ kVpmSeed, r), the synth's stream.  EMIT = false: returns the number of samples the ray
+// keeps.  EMIT = true: also stores them at slots first, first + 1, ... of S.
+constexpr unsigned long long kVpmSeed = 0xD1B54A32D192ED03ULL;
+template <bool EMIT>
+__device__ __forceinline__ uint32_t vpm_draws(const VpmGenParams &P, uint32_t r, uint32_t first, const SampleStaging &S) {
+  const sf eps(P.epsilon), len(P.edge_len[r]);
+  if (!(len > sf(4.f) * eps)) return 0u;
+  const sf mint = eps, maxt = len;
+  const sf density(P.sigma_t[1]);   // the sampling channel, min(int(0.5 * 3), 2) = 1
+  const sf maxDist = smax((maxt - mint) - eps, sf(0.f));
+  const sf norm = sf(1.f) - sf(pm_exp(((-density) * maxDist).v));
+  const sf distSurf = maxt - mint;
+  sf coef[3];   // sigma_t[c] / (1 - exp(-sigma_t[c] * distSurf)): pdfSuccess' normalisation of channel c
+#pragma unroll
+  for (int c = 0; c < 3; ++c) coef[c] = sf(P.sigma_t[c]) / (sf(1.f) - sf(pm_exp(((-sf(P.sigma_t[c])) * distSurf).v)));
+  const v3 o(P.o[3 * (size_t)r], P.o[3 * (size_t)r + 1], P.o[3 * (size_t)r + 2]);
+  const v3 d(P.d[3 * (size_t)r], P.d[3 * (size_t)r + 1], P.d[3 * (size_t)r + 2]);
+  const float rad = P.radius_per_ray ? P.radius_per_ray[r] : P.radius;
+  const sf normalization = sf(1.f) / sf((float)P.nb);
+  Pcg32 rng(P.seed ^ kVpmSeed, r);
+  uint32_t kept = 0;
+  for (int i = 0; i < P.nb; ++i) {
+    sf rand(rng.uniform());
+    if (P.stratified) rand = sf((float)i) * normalization + rand * normalization;
+    const sf dist = (-sf(pm_log((sf(1.f) - rand * norm).v))) / density;
+    if (!(dist < distSurf)) continue;   // "failed to sample the distance": the draw is skipped
+    const sf t = dist + mint;
+    const v3 p = o + d * t;
+    if (p.x == o.x && p.y == o.y && p.z == o.z) continue;
+    // exp(-sigma_t[c] * dist) is both pdfSuccess' factor and the transmittance: (-a) * b and a * (-b) round alike
+    sf tr[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) tr[c] = sf(pm_exp(((-sf(P.sigma_t[c])) * dist).v));
+    sf pdf(0.f);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) pdf = pdf + coef[c] * tr[c];
+    pdf = pdf / sf(3.f);
+    if (smax(tr[0], smax(tr[1], tr[2])).v < 1e-20f) tr[0] = tr[1] = tr[2] = sf(0.f);
+    if (EMIT) {
+      const size_t s = (size_t)first + kept;
+      const_cast<uint32_t *>(S.ray)[s] = r;
+      const_cast<float *>(S.t)[s] = t.v;
+      float *T = const_cast<float *>(S.transmittance) + 3 * s;
+      T[0] = tr[0].v; T[1] = tr[1].v; T[2] = tr[2].v;
+      const_cast<float *>(S.pdf_success)[s] = pdf.v;
+      const_cast<float *>(S.pdf_sel)[s] = 1.0f;
+      const_cast<float *>(S.radius)[s] = rad;
+    }
+    ++kept;
+  }
+  return kept;
+}
+// One thread per ray, CTAs stride over tiles of 256 rays.  Count pass: samples kept per ray and per tile.
+__global__ void __launch_bounds__(256) k_vpm_count(const __grid_constant__ VpmGenParams P) {
+  const uint32_t tiles = (P.n_rays + 255) / 256;
+  for (uint32_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+    const uint32_t r = tile * 256 + threadIdx.x;
+    uint32_t c = 0;
+    if (r < P.n_rays) {
+      c = vpm_draws<false>(P, r, 0u, SampleStaging{});
+      P.counts[r] = c;
+    }
+    const uint32_t t = block_total<8>(c);
+    if (threadIdx.x == 0) P.tile_tot[tile] = t;
+    __syncthreads();   // block_total's shared words are written again by the next tile
+  }
+}
+// Emit pass: the same draws, stored at the ray's offset in the staging arrays of the set of *n_total samples, so the
+// samples land ray by ray, draws in ascending order, whatever the launch geometry.
+__global__ void __launch_bounds__(256) k_vpm_emit(const __grid_constant__ VpmGenParams P) {
+  const uint32_t tiles = (P.n_rays + 255) / 256;
+  const SampleStaging S = sample_staging_at(P.staging, *P.n_total);
+  for (uint32_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+    const uint32_t r = tile * 256 + threadIdx.x;
+    const uint32_t c = r < P.n_rays ? P.counts[r] : 0u;
+    const uint32_t first = P.tile_tot[tile] + block_exclusive<8>(c);
+    if (c) vpm_draws<true>(P, r, first, S);
+    __syncthreads();   // block_exclusive's shared words are written again by the next tile
+  }
+}
+
 // ---- launchers ------------------------------------------------------------------------------------------------------
 void launch_generate_rays(const RayGenParams &P, cudaStream_t st) {
   const int bs = P.block;
@@ -500,6 +590,14 @@ void launch_trace_emit(const TraceParams &P, bool beams, const uint8_t *counts, 
 }
 void launch_planes_from_beams(const PlaneGenParams &P, cudaStream_t st) {
   if (P.n) k_planes_from_beams<<<(P.n + 255) / 256, 256, 0, st>>>(P);
+}
+// counts: [n_rays] words; tile_tot: [(n_rays + 255) / 256 + 1] words; total: the samples kept in all (one word, which
+// P.n_total of the emit pass points to)
+void launch_vpm_samples(const VpmGenParams &P, uint32_t *total, int sm_count, cudaStream_t st) {
+  const uint32_t tiles = (P.n_rays + 255) / 256;
+  if (tiles) k_vpm_count<<<stride_grid<k_vpm_count>(sm_count, 256, P.n_rays), 256, 0, st>>>(P);
+  k_scan_exclusive<uint32_t, 8><<<1, 1024, 0, st>>>(P.tile_tot, tiles, total, 0);
+  if (tiles) k_vpm_emit<<<stride_grid<k_vpm_emit>(sm_count, 256, P.n_rays), 256, 0, st>>>(P);
 }
 
 }  // namespace gvpm

@@ -156,6 +156,21 @@ struct SampleStaging { // raw gvpm_vpm_sample_soa arrays on the device
   const uint32_t *ray;
   const float *t, *transmittance, *pdf_success, *pdf_sel, *radius;
 };
+// The sample staging arrays of a set of n samples inside one buffer, laid out as capi_internal.cuh's SoaLayout<SampleSoA>
+// lays them out (element sizes 4, 4, 12, 4, 4, 4 bytes, each array on a 256-byte boundary).  For kernels that learn n
+// on the device (the samples gvpm_generate_vpm_samples draws).
+__host__ __device__ __forceinline__ SampleStaging sample_staging_at(const void *base, uint32_t n) {
+  const size_t a4 = (4 * (size_t)n + 255) & ~(size_t)255, a12 = (12 * (size_t)n + 255) & ~(size_t)255;
+  const char *b = (const char *)base;
+  SampleStaging S;
+  S.ray = (const uint32_t *)b;
+  S.t = (const float *)(b + a4);
+  S.transmittance = (const float *)(b + 2 * a4);
+  S.pdf_success = (const float *)(b + 2 * a4 + a12);
+  S.pdf_sel = (const float *)(b + 3 * a4 + a12);
+  S.radius = (const float *)(b + 4 * a4 + a12);
+  return S;
+}
 
 // implicit 32-ary hierarchy over Morton-sorted photons: level 0 = leaves of 32 photons,
 // level l+1 node j = union of level l nodes [32j, 32j+32).  Boxes already inflated by the radius
@@ -328,6 +343,20 @@ struct PlaneGenParams {
   // plane staging arrays (gvpm_plane_soa order)
   float *origin, *w0, *length0, *w1, *length1, *flux;
   int32_t *edge_id;
+};
+// G-VPM camera distance samples from the current ray set (generate.cu k_vpm_count / k_vpm_emit): one PCG32 stream per ray
+struct VpmGenParams {
+  const float *o, *d, *edge_len;   // ray staging arrays
+  const float *radius_per_ray;     // [n_rays], or null: `radius` for every ray
+  uint32_t n_rays;
+  int nb, stratified;
+  unsigned long long seed;
+  float epsilon, radius;
+  float sigma_t[3];
+  uint32_t *counts;                // [n_rays] samples kept per ray (count pass writes, emit pass reads)
+  uint32_t *tile_tot;              // [tiles + 1] samples per tile of 256 rays, scanned in place into tile offsets
+  const uint32_t *n_total;         // device: samples kept in all (the scan's total; the emit pass's staging layout)
+  void *staging;                   // the sample staging buffer
 };
 // ---- strictly rounded double (the reference's fp64 island: cylinderIntersection / solveQuadraticDouble,
 // photonmapper/beams_3d_intersections.h:100-137, src/libcore/util.cpp:487-525) ----------------------------

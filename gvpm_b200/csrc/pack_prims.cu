@@ -131,28 +131,33 @@ __global__ void __launch_bounds__(256) k_pack_planes(const PlaneStaging S, uint3
     centre[i3 + a] = __fadd_rn(__fadd_rn(o[a], __fmul_rn(0.5f, e0[a])), __fmul_rn(0.5f, e1[a]));
 }
 
-// distance samples: 2 float4 per sample; stats[0] = max radius (float bits; radii are positive), stats[1] |= 1 when a
-// sample refers to a ray that is not uploaded (the index is clamped so that the gather stays in bounds; the error
-// is reported by the gather)
-__global__ void __launch_bounds__(256) k_pack_samples(const SampleStaging S, uint32_t n, uint32_t n_rays,
-                                                       float4 *__restrict__ packed, uint32_t *__restrict__ stats) {
+// distance samples: 2 float4 per sample of the staging buffer holding n samples (n_dev: a count known on the device
+// only, n is then the grid's bound); stats[0] = max radius (float bits; radii are positive), stats[1] |= 1 when a sample
+// refers to a ray that is not uploaded (the index is clamped so that the gather stays in bounds; the error is reported
+// by the caller), |= 2 when a radius is negative or not finite
+__global__ void __launch_bounds__(256) k_pack_samples(const void *staging, uint32_t n, const uint32_t *n_dev,
+                                                       uint32_t n_rays, float4 *__restrict__ packed,
+                                                       uint32_t *__restrict__ stats) {
+  if (n_dev) n = *n_dev;
+  const SampleStaging S = sample_staging_at(staging, n);
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   float rad = 0.f;
-  bool bad = false;
+  bool bad = false, badRad = false;
   if (i < n) {
     uint32_t rb = S.ray[i];
     if (rb >= n_rays) { bad = true; rb = n_rays ? n_rays - 1 : 0u; }
     rad = S.radius[i];
+    badRad = !(rad >= 0.f && rad < INFINITY);
     packed[2 * (size_t)i] = make_float4(S.t[i], S.pdf_success[i], S.pdf_sel[i], rad);
     packed[2 * (size_t)i + 1] = make_float4(S.transmittance[3 * (size_t)i], S.transmittance[3 * (size_t)i + 1],
                                             S.transmittance[3 * (size_t)i + 2], __uint_as_float(rb));
   }
   rad = fmaxf(rad, 0.f);
   rad = warp_max(rad);
-  const uint32_t anyBad = __ballot_sync(0xffffffffu, bad);
+  const uint32_t anyBad = __ballot_sync(0xffffffffu, bad), anyBadRad = __ballot_sync(0xffffffffu, badRad);
   if ((threadIdx.x & 31) == 0) {
     atomicMax(stats, __float_as_uint(rad));
-    if (anyBad) atomicOr(stats + 1, 1u);
+    if (anyBad || anyBadRad) atomicOr(stats + 1, (anyBad ? 1u : 0u) | (anyBadRad ? 2u : 0u));
   }
 }
 
@@ -197,8 +202,9 @@ void launch_sub_emit(const float4 *rec, const float *len, uint32_t n, const floa
 void launch_pack_planes(const PlaneStaging &S, uint32_t n, float4 *rec, float *centre, uint32_t *flag, cudaStream_t st) {
   if (n) k_pack_planes<<<(n + 255) / 256, 256, 0, st>>>(S, n, rec, centre, flag);
 }
-void launch_pack_samples(const SampleStaging &S, uint32_t n, uint32_t n_rays, float4 *packed, uint32_t *stats, cudaStream_t st) {
-  if (n) k_pack_samples<<<(n + 255) / 256, 256, 0, st>>>(S, n, n_rays, packed, stats);
+void launch_pack_samples(const void *staging, uint32_t n, const uint32_t *n_dev, uint32_t n_rays, float4 *packed,
+                         uint32_t *stats, cudaStream_t st) {
+  if (n) k_pack_samples<<<(n + 255) / 256, 256, 0, st>>>(staging, n, n_dev, n_rays, packed, stats);
 }
 
 }  // namespace gvpm

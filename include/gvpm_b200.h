@@ -145,8 +145,8 @@ typedef struct gvpm_ray_soa {
  * (gvpm.cpp:1141-1175: edge selection by the discrete CDF, then
  * HomogeneousMedium::sampleDistance(ray, mRec, sampler, EDistanceAlwaysValid), homogeneous.cpp:293-430).
  * One entry per (pixel, camera sample); `ray` indexes the gvpm_ray_soa record of the chosen medium edge.
- * The distance is sampled on the host (it consumes the integrator's sampler and libm's logf), so the
- * query points are bit-identical inputs for the gather. */
+ * Uploaded, the distance is sampled on the host (it consumes the integrator's sampler and libm's logf), so the
+ * query points are bit-identical inputs for the gather; gvpm_generate_vpm_samples draws them on the device. */
 typedef struct gvpm_vpm_sample_soa {
   const uint32_t *ray;         /* [n]   index into the uploaded rays */
   const float *t;              /* [n]   mRec.t (the query point is o + t*d) */
@@ -444,7 +444,8 @@ int gvpm_dump_neighbours_planes(gvpm_ctx *ctx, uint64_t *offsets, uint32_t *idx,
 /* ---- G-VPM: replaces gradientPhotonMap->evaluate(gRec, p, querySize) over all camera distance
  *      samples, gvpm.cpp:1141-1185 + kdtree.h:675-731 + shift_volume_photon.cpp:489-655 ----------------
  * Call order: gvpm_upload_photons, gvpm_build_points(radius >= every sample radius), gvpm_upload_rays
- * (one record per (gather point, medium edge)), gvpm_upload_vpm_samples, gvpm_gather_vpm.
+ * (one record per (gather point, medium edge)), gvpm_upload_vpm_samples (or gvpm_generate_vpm_samples, below),
+ * gvpm_gather_vpm.
  * out: [n_rays*27] with the reference's 1/nbCameraSamples normalisation applied (gvpm.cpp:1177-1182);
  * mvol (may be NULL): [n_rays] the MVol of gvpm.cpp:1175 = photons found by the range queries of the
  * ray's samples (drives the per-pixel radius update :1191-1195, which stays on the host);
@@ -454,6 +455,25 @@ int gvpm_gather_vpm(gvpm_ctx *ctx, int nb_camera_samples, float *out, uint32_t *
 int gvpm_gather_vpm_device(gvpm_ctx *ctx, int nb_camera_samples, const float **out_dev, const uint32_t **mvol_dev);
 /* per-SAMPLE neighbour index sets, same CSR convention as gvpm_dump_neighbours_bre */
 int gvpm_dump_neighbours_vpm(gvpm_ctx *ctx, int nb_camera_samples, uint64_t *offsets, uint32_t *idx, size_t cap);
+/* The distance samples drawn on the device from the context's current ray set, in place of gvpm_upload_vpm_samples:
+ * what gvpm_synth_vpm_samples (the host restatement of gvpm.cpp:1141-1175 + HomogeneousMedium::sampleDistance with
+ * EDistanceAlwaysValid) draws, for rays that are each their gather point's only medium edge (pdf_sel = 1; the rays of
+ * gvpm_generate_rays are).  A ray draws only if edge_len > 4 * epsilon.  Ray r draws from
+ * PCG32(seed ^ 0xD1B54A32D192ED03, r), the synth's stream; draw i takes u (stratified: i * (1/nb) + u * (1/nb)) to
+ *   d = -log(1 - u * (1 - exp(-sigma_t[1] * max(edge_len - 2 epsilon, 0)))) / sigma_t[1],
+ * skipped unless d < edge_len - epsilon and o + (d + epsilon) * dir != o; t = d + epsilon,
+ * pdf_success = sum_c sigma_t[c] / (1 - exp(-sigma_t[c] (edge_len - epsilon))) * exp(-sigma_t[c] d) / 3,
+ * transmittance[c] = exp(-sigma_t[c] d) (all zero when all are below 1e-20), radius = radius_per_ray_dev[r] (device
+ * memory, n_rays floats) or, when that is NULL, `radius`.  Samples are stored ray by ray, draws in ascending order.
+ * Arithmetic is strictly rounded fp32 in the synth's operation order with the tracers' polynomial log / exp, so the
+ * samples are bit-reproducible (they differ from the synth's libm results in the last bits, DESIGN.md §6).  The context
+ * is left as gvpm_upload_vpm_samples of the same arrays leaves it; *n_samples (may be NULL) = the number drawn.  The
+ * gathers and gvpm_dump_neighbours_vpm refuse the drawn samples once another ray set has been committed.  Fails with
+ * GVPM_ERR_INVALID without a committed ray set or a medium, for nb_camera_samples <= 0, epsilon not > 0, a scalar
+ * radius that is not finite and > 0 (without a per-ray array), n_rays * nb_camera_samples > 0xfffffff0, or a per-ray
+ * radius of a drawing ray that is negative or not finite. */
+int gvpm_generate_vpm_samples(gvpm_ctx *ctx, int nb_camera_samples, int stratified, uint64_t seed, float epsilon,
+                              float radius, const float *radius_per_ray_dev, size_t *n_samples);
 
 /* ---- hand-off: computeGradient (gvpm.cpp:1205-1306) on the 27-float planes -------------
  * acc: device or host? -> host [h*w*27] APA-averaged accumulators in pixel order;
@@ -622,8 +642,8 @@ int gvpm_read_device(gvpm_ctx *ctx, const void *dev, void *host, size_t bytes);
  * gb_per_s = bytes * reps / time.  A buffer well below the 126 MB L2 gives the L2 read bandwidth, one far above it the
  * HBM read bandwidth. */
 int gvpm_measure_read_bandwidth(gvpm_ctx *ctx, size_t bytes, int reps, double *gb_per_s);
-/* parity aid: the selected photon staging buffer (which = 0), the ray staging buffer (1), the beam staging buffer (2)
- * or the plane staging buffer (3) as they are, without the side effects of gvpm_photon_staging / gvpm_ray_staging
+/* parity aid: the selected photon staging buffer (which = 0), the ray staging buffer (1), the beam staging buffer (2),
+ * the plane staging buffer (3) or the G-VPM sample staging buffer (4) as they are, without the side effects of gvpm_photon_staging / gvpm_ray_staging
  * (which invalidate the build / the committed rays).  Each holds its SoA's arrays back to back, every array starting
  * on a 256-byte boundary; count = the number of elements of the current set. */
 int gvpm_staging_peek(gvpm_ctx *ctx, int which, void **dev, size_t *count);
