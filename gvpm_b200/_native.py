@@ -102,6 +102,7 @@ BEAM_TECHNIQUES = {"beam1d": 0, "beam3d_naive": 1, "beam3d_egsr": 2, "beam3d": 3
 ABI_SYMBOLS = [
     "gvpm_abi_version", "gvpm_ctx_create", "gvpm_ctx_destroy", "gvpm_last_error", "gvpm_sync",
     "gvpm_stream", "gvpm_set_medium", "gvpm_set_config", "gvpm_set_occluders",
+    "gvpm_set_occluder_accel", "gvpm_occluder_accel_kind", "gvpm_occluded",
     "gvpm_upload_photons", "gvpm_photon_staging", "gvpm_build_points", "gvpm_build_points_for_rays", "gvpm_accel_kind", "gvpm_set_view_direction",
     "gvpm_photon_staging_select", "gvpm_photon_staging_layout", "gvpm_upload_photons_slice",
     "gvpm_peer_export", "gvpm_peer_connect", "gvpm_peer_push_photon_slice", "gvpm_peer_wait_photons", "gvpm_peer_push_mode",
@@ -147,6 +148,9 @@ def load_lib():
     lib.gvpm_set_medium.argtypes = [vp, C.POINTER(Medium)]
     lib.gvpm_set_config.argtypes = [vp, C.POINTER(Config)]
     lib.gvpm_set_occluders.argtypes = [vp, f32p, C.c_size_t]
+    lib.gvpm_set_occluder_accel.argtypes = [vp, C.c_int]
+    lib.gvpm_occluder_accel_kind.argtypes = [vp]
+    lib.gvpm_occluded.argtypes = [vp, f32p, f32p, f32p, f32p, C.c_size_t, C.POINTER(C.c_uint8)]
     lib.gvpm_upload_photons.argtypes = [vp, C.POINTER(PhotonSoA), C.c_size_t]
     lib.gvpm_photon_staging.argtypes = [vp, C.c_size_t, C.POINTER(vp), C.POINTER(C.c_size_t)]
     lib.gvpm_build_points.argtypes = [vp, C.c_float]

@@ -57,6 +57,33 @@ class Context:
         self._ck(self.lib.gvpm_set_occluders(self.h, tri.ctypes.data_as(N.f32p), tri.size // 9),
                  "gvpm_set_occluders")
 
+    _OCC_ACCEL = {"auto": 0, "list": 1, "bvh": 2}
+
+    def set_occluder_accel(self, mode):
+        """Any-hit path of the shadow rays: "auto" (list up to 32 triangles, BVH above), "list" or "bvh"."""
+        if mode not in self._OCC_ACCEL:
+            raise ValueError(f"occluder accel must be one of {sorted(self._OCC_ACCEL)}, not {mode!r}")
+        self._ck(self.lib.gvpm_set_occluder_accel(self.h, self._OCC_ACCEL[mode]), "gvpm_set_occluder_accel")
+
+    def occluder_accel(self):
+        """The path the gathers take for the current occluders: "list" or "bvh"."""
+        return {1: "list", 2: "bvh"}[self.lib.gvpm_occluder_accel_kind(self.h)]
+
+    def occluded(self, o, d, mint, maxt):
+        """Shadow-ray any-hit of n rays against the occluders (the gathers' own device code) -> bool[n]."""
+        o = np.ascontiguousarray(o, dtype=np.float32).reshape(-1, 3)
+        d = np.ascontiguousarray(d, dtype=np.float32).reshape(-1, 3)
+        n = o.shape[0]
+        mint = np.ascontiguousarray(np.broadcast_to(np.asarray(mint, dtype=np.float32), (n,)))
+        maxt = np.ascontiguousarray(np.broadcast_to(np.asarray(maxt, dtype=np.float32), (n,)))
+        if d.shape[0] != n:
+            raise ValueError("o and d must have the same number of rays")
+        hit = np.zeros(n, dtype=np.uint8)
+        self._ck(self.lib.gvpm_occluded(self.h, o.ctypes.data_as(N.f32p), d.ctypes.data_as(N.f32p),
+                                        mint.ctypes.data_as(N.f32p), maxt.ctypes.data_as(N.f32p), n,
+                                        hit.ctypes.data_as(N.u8p)), "gvpm_occluded")
+        return hit.astype(bool)
+
     # ---- photons
     def upload_photons(self, photons):
         cs = photons.as_c()

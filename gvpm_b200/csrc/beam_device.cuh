@@ -336,7 +336,7 @@ __device__ __forceinline__ v3 beam_shift_pos(const GatherParams &P, const BaseRa
 }
 
 // shiftBeam -> shiftBeamDiffuse + diffuseReconnectionPhotonBeam; S / weight keep (0, 1) on failure
-template <bool K1D>
+template <bool K1D, bool BVH>
 __device__ __forceinline__ void shift_beam_diffuse(const GatherParams &P, const BeamRec &beam, v3 ok, v3 dk, sf lenK,
                                                    v3 eyeK, sf sensor, sf shiftW, const BeamKernelRec &kRec,
                                                    v3 newPos, v3 &S, sf &weight) {
@@ -346,7 +346,7 @@ __device__ __forceinline__ void shift_beam_diffuse(const GatherParams &P, const 
   v3 newPBDir = newPos - beam.o;
   const sf newPBDist = length(newPBDir);
   newPBDir = newPBDir / newPBDist;
-  if (occluded(P, beam.o, newPBDir, sf(P.cfg.epsilon), newPBDist)) { weight = sf(1.f); return; }
+  if (occluded<BVH>(P, beam.o, newPBDir, sf(P.cfg.epsilon), newPBDist)) { weight = sf(1.f); return; }
   const v3 basePos = beam.o + beam.dir * kRec.v;
   const sf pdfKernelAndDist = kRec.pdf();
   v3 thr(1.f, 1.f, 1.f);
@@ -419,7 +419,7 @@ __device__ __forceinline__ void shift_beam_diffuse(const GatherParams &P, const 
 
 // BeamGradRadianceQuery::operator() for one (ray, beam) pair whose kernel record is valid and which
 // passed the filters
-template <bool K1D>
+template <bool K1D, bool BVH>
 __device__ __forceinline__ void beam_functor(const GatherParams &P, const float4 *__restrict__ rec, const BaseRay &R,
                                              const BeamRec &beam, const BeamKernelRec &kRec, float *a) {
   const sf r(P.radius);
@@ -461,14 +461,14 @@ __device__ __forceinline__ void beam_functor(const GatherParams &P, const float4
       }
       if (K1D && !alreadyShift && kRec.w <= lenK) {   // newShiftBeam, :311-317
         const v3 offsetPos = beam_shift_pos_1d(R, ok, dk, beam.o, beam.dir, kRec.w, kRec.u);
-        shift_beam_diffuse<K1D>(P, beam, ok, dk, lenK, eyeK, sensor, shiftW, kRec, offsetPos, S, weight);
+        shift_beam_diffuse<K1D, BVH>(P, beam, ok, dk, lenK, eyeK, sensor, shiftW, kRec, offsetPos, S, weight);
       } else if (!alreadyShift && kRec.w <= lenK) {
         const sf dd = dot(beam.o - ok, dk);
         const sf minDistSqr = length_sq(beam.o - (ok + dd * dk));
         if (minDistSqr.v > 0.f) {
           const v3 u = (beam.o + beam.dir * kRec.v) - (R.o + kRec.w * R.d);
           const v3 offsetPos = beam_shift_pos(P, R, ok, dk, kRec.w, u, shiftW);
-          shift_beam_diffuse<K1D>(P, beam, ok, dk, lenK, eyeK, sensor, shiftW, kRec, offsetPos, S, weight);
+          shift_beam_diffuse<K1D, BVH>(P, beam, ok, dk, lenK, eyeK, sensor, shiftW, kRec, offsetPos, S, weight);
         } else {
           weight = sf(1.f);
         }

@@ -5,13 +5,10 @@
 //   shiftNull / shiftPhotonDiffuse / getShiftPos    shift_volume_photon.cpp:119-158,382-486,858-896
 //   diffuseReconnection                         gvpm/shift/operation/shift_diffuse.cpp:11-134
 //   HomogeneousMedium::eval, phase eval         src/medium/homogeneous.cpp:432-513, src/phase/hg.cpp:107-110
-//   Triangle::rayIntersect                      include/mitsuba/core/triangle.h:109-145
 #pragma once
-#include "gvpm_device.cuh"
+#include "occluder_device.cuh"
 
 namespace gvpm {
-
-__device__ __forceinline__ float4 ldg4(const float4 *p) { return __ldg(p); }
 
 // conservative slab test of a box (inflated by the radius at build time) against the ray interval
 // [tlo, thi]; the rounding/packet pad is folded into the origin: (lo - pad) - o == lo - (o + pad)
@@ -59,79 +56,6 @@ __device__ __forceinline__ sf phase_eval(const GatherParams &P, v3 wi, v3 wo) {
   sf g(P.hg_g);
   sf temp = sf(1.f) + g * g + sf(2.f) * g * dot(wi, wo);
   return sf(GVPM_INV_FOURPI) * (sf(1.f) - g * g) / (temp * ssqrt(temp));
-}
-
-// any-hit over the occluder list.  Two conservative culls precede the strictly rounded Moller-Trumbore test
-// (|d| = 1): (1) the origin is farther from the triangle's plane than maxt; (2) the ray meets the plane at a
-// parameter that is outside [mint, maxt] by more than the rounding of the strict test (the parent vertex of a
-// reconnection usually lies ON a wall, whose plane it then meets at t ~ 0 < mint).  Single exit, so the lanes of a
-// warp reconverge right after the loop.
-__device__ __forceinline__ bool occluder_hit(const GatherParams &P, uint32_t t, v3 o, v3 d, sf mint, sf maxt,
-                                             float omag) {
-  const float4 pl = ldg4(P.tri_plane + t);
-  const float sdist = pl.x * o.x.v + pl.y * o.y.v + pl.z * o.z.v + pl.w;
-  if (fabsf(sdist) > maxt.v * 1.001f + 1e-5f) return false;
-  const float nd = pl.x * d.x.v + pl.y * d.y.v + pl.z * d.z.v;
-  const float and_ = fabsf(nd);
-  if (and_ > 1e-3f) {
-    // plane parameter tp = -sdist/nd; the strict tt differs from it by < aux.x * |o - p0| / |nd| (+ relative).
-    // Compared after multiplying through by |nd| (no division).
-    const float2 aux = __ldg(P.tri_aux + t);
-    const float num = nd < 0.f ? sdist : -sdist;  // tp * |nd|
-    const float slack = aux.x * (omag + aux.y + 1e-3f) * 1.7321f + 2e-6f * fabsf(num);
-    if (num + slack < mint.v * and_ || num - slack > maxt.v * and_) return false;
-  }
-  const float *tv = P.tri + 9 * t;
-  v3 p0(__ldg(tv), __ldg(tv + 1), __ldg(tv + 2)), p1(__ldg(tv + 3), __ldg(tv + 4), __ldg(tv + 5)),
-      p2(__ldg(tv + 6), __ldg(tv + 7), __ldg(tv + 8));
-  v3 edge1 = p1 - p0, edge2 = p2 - p0;
-  v3 pvec = cross(d, edge2);
-  sf det = dot(edge1, pvec);
-  if (det.v == 0.f) return false;
-  sf inv_det = sf(1.f) / det;
-  v3 tvec = o - p0;
-  sf u = dot(tvec, pvec) * inv_det;
-  if (u.v < 0.f || u.v > 1.f) return false;
-  v3 qvec = cross(tvec, edge1);
-  sf v = dot(d, qvec) * inv_det;
-  if (v.v >= 0.f && (u + v).v <= 1.f) {
-    sf tt = dot(edge2, qvec) * inv_det;
-    if (tt >= mint && tt <= maxt) return true;
-  }
-  return false;
-}
-__device__ __forceinline__ bool occluded(const GatherParams &P, v3 o, v3 d, sf mint, sf maxt) {
-  bool hit = false;
-  if (maxt < mint) return false;
-  const float omag = fmaxf(fmaxf(fabsf(o.x.v), fabsf(o.y.v)), fabsf(o.z.v));
-  for (uint32_t t = 0; t < P.n_tri && !hit; ++t) hit = occluder_hit(P, t, o, d, mint, maxt, omag);
-  return hit;
-}
-// Shadow rays of one (ray, photon) pair share their origin (the parent vertex): the triangles whose plane lies
-// within `bound` of it are found once per pair (bit t of the mask, n_tri <= 32); a shadow ray whose plane-distance
-// cull radius fits inside `bound` then visits only those.
-struct OccluderNear { uint32_t mask; float bound; };
-__device__ __forceinline__ OccluderNear occluders_near(const GatherParams &P, v3 o, float bound) {
-  OccluderNear n;
-  n.mask = 0u;
-  n.bound = P.n_tri <= 32u ? bound : -1.f;
-  // unrolled 4-fold, so 4 plane loads are in flight: nvcc's own choice (16-fold, all 16 loads in flight) made this loop
-  // the register peak of the shade kernels
-  if (P.n_tri <= 32u)
-#pragma unroll 4
-    for (uint32_t t = 0; t < P.n_tri; ++t) {
-      const float4 pl = ldg4(P.tri_plane + t);
-      if (fabsf(pl.x * o.x.v + pl.y * o.y.v + pl.z * o.z.v + pl.w) <= bound) n.mask |= 1u << t;
-    }
-  return n;
-}
-__device__ __forceinline__ bool occluded_near(const GatherParams &P, const OccluderNear &n, v3 o, v3 d, sf mint, sf maxt) {
-  if (!(maxt.v * 1.001f + 1e-5f <= n.bound)) return occluded(P, o, d, mint, maxt);
-  bool hit = false;
-  if (maxt < mint) return false;
-  const float omag = fmaxf(fmaxf(fabsf(o.x.v), fabsf(o.y.v)), fabsf(o.z.v));
-  for (uint32_t m = n.mask; m != 0u && !hit; m &= m - 1u) hit = occluder_hit(P, __ffs(m) - 1, o, d, mint, maxt, omag);
-  return hit;
 }
 
 // coordinateSystemCoherent, src/libcore/util.cpp:592-599
@@ -327,9 +251,13 @@ __device__ __forceinline__ v3 get_shift_pos(const GatherParams &P, sf rr2, v3 p,
 // Shadow rays run from the parent towards the offset photon over maxt = lProj * shadow_maxt_scale; twice the base edge
 // length bounds lProj for every coherent offset (longer ones fall back to the full occluder loop).  Built per pair, not
 // per photon: the occluders and shadow_maxt_scale may change between the build and the gather.
+// BVH: no mask, every shadow ray walks the occluder BVH.
+template <bool BVH>
 __device__ __forceinline__ OccluderNear pair_occluders(const GatherParams &P, v3 parent, sf lBase) {
+  if (BVH) return OccluderNear{0u, -1.f};
   return occluders_near(P, parent, 2.f * (lBase.v * P.cfg.shadow_maxt_scale * 1.001f + 1e-5f));
 }
+template <bool BVH>
 __device__ __forceinline__ void shift_photon_diffuse(const GatherParams &P, const PhotonRec &ph, const OccluderNear &near,
                                                      v3 offsetPos, v3 dk, v3 eyeK, sf sensor, sf Tshift, sf pdfBase,
                                                      sf pdfShift, v3 &S, sf &weight) {
@@ -339,7 +267,7 @@ __device__ __forceinline__ void shift_photon_diffuse(const GatherParams &P, cons
   dProj = dProj / lProj;
   // manifold shift (glossy parent): out of scope, fails like useManifold=false
   bool ok = ph.ptype != GVPM_PARENT_OTHER;
-  if (ok) ok = !occluded_near(P, near, ph.parent, dProj, sf(P.cfg.epsilon), lProj * sf(P.cfg.shadow_maxt_scale));
+  if (ok) ok = !occluded_near<BVH>(P, near, ph.parent, dProj, sf(P.cfg.epsilon), lProj * sf(P.cfg.shadow_maxt_scale));
   // type-specific terms of diffuseReconnection
   const v3 wiW = ph.wiW;
   const sf cosO = dot(ph.pn, dProj);
@@ -439,7 +367,7 @@ __device__ __forceinline__ void bre_photon(const GatherParams &P, const float4 *
 
   const MediumRec mShift = medium_eval(P, sf(P.cfg.epsilon), tBase);
   const v3 zBase = R.o + tBase * R.d;
-  const OccluderNear near = pair_occluders(P, ph.parent, ph.lBase);
+  const OccluderNear near = pair_occluders<false>(P, ph.parent, ph.lBase);
 
   // The offset loop is kept rolled (one copy of the shift code); k is warp-uniform, so the accumulation goes
   // through a switch with static register indices instead of a local-memory staging array.
@@ -471,7 +399,7 @@ __device__ __forceinline__ void bre_photon(const GatherParams &P, const float4 *
           sf ds = length_sq((ok + dd * dk) - offsetPos);
           pdfShift = chord_pdf(safe_sqrt(rr2 - ds));
         }
-        shift_photon_diffuse(P, ph, near, offsetPos, dk, eyeK, sensor, mShift.T, pdfCam, pdfShift, S, weight);
+        shift_photon_diffuse<false>(P, ph, near, offsetPos, dk, eyeK, sensor, mShift.T, pdfCam, pdfShift, S, weight);
       }
     }
     if ((k == 1 && R.px == P.cfg.film_w - 1) || (k == 2 && R.py == P.cfg.film_h - 1)) weight = sf(1.f);
@@ -506,6 +434,7 @@ enum {  // float slots of ctx[pair]
   CX_TBASE = 29, CX_PDFCAM = 30, CX_TSHIFT = 31, CX_RAY = 32
 };
 
+template <bool BVH>
 __device__ __forceinline__ void bre_pairs_warp(const GatherParams &P, uint2 pr, bool valid, float *a, ShadeShared &W,
                                                int lane) {
   const sf r(P.radius), rr2 = r * r;
@@ -537,7 +466,7 @@ __device__ __forceinline__ void bre_pairs_warp(const GatherParams &P, uint2 pr, 
     acc_add(a, 0, (baseContrib * recip) * rrG);
     Tshift = medium_eval(P, sf(P.cfg.epsilon), tBase).T;
     zBase = R.o + tBase * R.d;
-    const OccluderNear near = pair_occluders(P, ph.parent, ph.lBase);
+    const OccluderNear near = pair_occluders<BVH>(P, ph.parent, ph.lBase);
     float *c = W.ctx[lane];
     c[CX_P] = ph.p.x.v; c[CX_P + 1] = ph.p.y.v; c[CX_P + 2] = ph.p.z.v;
     c[CX_PARENT] = ph.parent.x.v; c[CX_PARENT + 1] = ph.parent.y.v; c[CX_PARENT + 2] = ph.parent.z.v;
@@ -631,7 +560,7 @@ __device__ __forceinline__ void bre_pairs_warp(const GatherParams &P, uint2 pr, 
       }
       sf weight(1.f);
       v3 S(0.f, 0.f, 0.f);
-      shift_photon_diffuse(P, q, near, offsetPos, dk, eyeK, sensor, Ts, pC, pdfShift, S, weight);
+      shift_photon_diffuse<BVH>(P, q, near, offsetPos, dk, eyeK, sensor, Ts, pC, pdfShift, S, weight);
       W.res[owner][k] = make_float4(S.x.v, S.y.v, S.z.v, weight.v);
     }
   }

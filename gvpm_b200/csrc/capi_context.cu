@@ -1,4 +1,5 @@
-// capi_context.cu — context lifetime, scene constants (medium, config, occluders), timings and small queries.
+// capi_context.cu — context lifetime, scene constants (medium, config, occluders and their any-hit path), timings and
+// small queries.
 #include "capi_internal.cuh"
 
 static std::string g_create_error;
@@ -145,8 +146,11 @@ int gvpm_set_config(gvpm_ctx *ctx, const gvpm_config *c) {
 
 int gvpm_set_occluders(gvpm_ctx *ctx, const float *tri_xyz, size_t n_tri) {
   if (!ctx || (n_tri && !tri_xyz)) return GVPM_ERR_INVALID;
+  if (n_tri > GVPM_MAX_OCCLUDERS)
+    return fail(ctx, GVPM_ERR_INVALID, "more than GVPM_MAX_OCCLUDERS (2^24) occluder triangles");
   cudaSetDevice(ctx->device);
   ctx->n_tri = (uint32_t)n_tri;
+  ctx->occ_built = false;
   ++ctx->state_gen;
   if (n_tri == 0) return GVPM_OK;
   std::vector<float> planes(4 * n_tri), aux(2 * n_tri);
@@ -182,6 +186,54 @@ int gvpm_set_occluders(gvpm_ctx *ctx, const float *tri_xyz, size_t n_tri) {
   CK(cudaMemcpyAsync(ctx->tri_aux.p, aux.data(), 2 * n_tri * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(ctx->tri.p, tri_xyz, 9 * n_tri * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(ctx->tri_plane.p, planes.data(), 4 * n_tri * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (occluder_use_bvh(ctx)) {
+    const int rc = build_occluder_bvh(ctx);
+    if (rc) ctx->n_tri = 0;   // no half-built set: the occluders are cleared
+    return rc;
+  }
+  return GVPM_OK;
+}
+
+int gvpm_set_occluder_accel(gvpm_ctx *ctx, int mode) {
+  if (!ctx) return GVPM_ERR_INVALID;
+  if (mode != GVPM_OCC_AUTO && mode != GVPM_OCC_LIST && mode != GVPM_OCC_BVH)
+    return fail(ctx, GVPM_ERR_INVALID, "occluder accel must be GVPM_OCC_AUTO, GVPM_OCC_LIST or GVPM_OCC_BVH");
+  ctx->occ_accel = mode;   // both paths give the same any-hit: the gathers' results do not change
+  if (occluder_use_bvh(ctx) && !ctx->occ_built) {
+    cudaSetDevice(ctx->device);
+    return build_occluder_bvh(ctx);
+  }
+  return GVPM_OK;
+}
+
+int gvpm_occluder_accel_kind(const gvpm_ctx *ctx) {
+  if (!ctx) return 0;
+  return occluder_use_bvh(ctx) ? GVPM_OCC_BVH : GVPM_OCC_LIST;
+}
+
+int gvpm_occluded(gvpm_ctx *ctx, const float *o, const float *d, const float *mint, const float *maxt, size_t n,
+                  uint8_t *hit) {
+  if (!ctx || (n && (!o || !d || !mint || !maxt || !hit))) return GVPM_ERR_INVALID;
+  if (n > 0xffffffffull) return fail(ctx, GVPM_ERR_INVALID, "more than 2^32 - 1 rays");
+  if (n == 0) return GVPM_OK;
+  cudaSetDevice(ctx->device);
+  const size_t o_d = align256(12 * n), o_mint = o_d + align256(12 * n), o_maxt = o_mint + align256(4 * n),
+               o_hit = o_maxt + align256(4 * n);
+  CK(ctx->occ_query.reserve(o_hit + n));
+  char *q = ctx->occ_query.as<char>();
+  CK(cudaMemcpyAsync(q, o, 12 * n, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(q + o_d, d, 12 * n, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(q + o_mint, mint, 4 * n, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(q + o_maxt, maxt, 4 * n, cudaMemcpyHostToDevice, ctx->stream));
+  GatherParams P;
+  memset(&P, 0, sizeof(P));
+  occluder_params(ctx, P);
+  launch_occluded(P, P.occ_nodes != nullptr, (const float *)q, (const float *)(q + o_d), (const float *)(q + o_mint),
+                  (const float *)(q + o_maxt), (uint32_t)n, (uint8_t *)(q + o_hit), ctx->stream);
+  CK(cudaGetLastError());
+  ++ctx->launches;
+  CK(cudaMemcpyAsync(hit, q + o_hit, n, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return GVPM_OK;
 }

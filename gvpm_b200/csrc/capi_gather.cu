@@ -27,6 +27,7 @@ int gather_params(gvpm_ctx *ctx, GatherParams &P, bool built, const char *not_bu
   P.sampling_weight = ctx->medium.sampling_weight;
   P.cfg = ctx->cfg;
   P.work_counter = ctx->work_counter.as<uint32_t>();
+  occluder_params(ctx, P);
   return GVPM_OK;
 }
 
@@ -53,10 +54,6 @@ int fill_params(gvpm_ctx *ctx, GatherParams &P, float *out_dev, uint32_t *counts
   else
     P.kernel_vol = (float)((double)GVPM_PI * std::pow((double)r, 2));
   P.bounds = ctx->bounds.as<float>();
-  P.tri = ctx->tri.as<float>();
-  P.tri_plane = ctx->tri_plane.as<float4>();
-  P.tri_aux = ctx->tri_aux.as<float2>();
-  P.n_tri = ctx->n_tri;
   P.out = out_dev;
   P.counts = counts_dev;
   P.pair_counter = (unsigned long long *)(ctx->work_counter.as<char>() + 8);

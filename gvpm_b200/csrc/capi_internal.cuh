@@ -165,8 +165,12 @@ struct gvpm_ctx {
   gvpm_config cfg{};
   bool have_cfg = false;
 
-  DevBuf tri, tri_plane, tri_aux;
+  DevBuf tri, tri_plane, tri_aux;   // in leaf order of the occluder BVH once it is built
   uint32_t n_tri = 0;
+  int occ_accel = GVPM_OCC_AUTO;     // gvpm_set_occluder_accel
+  bool occ_built = false;            // occ_nodes holds the BVH of the current set
+  uint32_t n_occ_nodes = 0;
+  DevBuf occ_nodes, occ_scratch, occ_query;   // BVH nodes; build scratch; gvpm_occluded's rays and hits
 
   DevBuf ph_staging, ph_staging_alt;  // the selected photon staging buffer and the other one (double buffering)
   int ph_staging_sel = 0;
@@ -435,6 +439,13 @@ FrustumGrid make_frustum_grid(const gvpm_ctx::RayFit &F, float radius, bool pari
 int build_frustum(gvpm_ctx *ctx, float radius, uint32_t *n_kept);
 int build_pruned_bvh(gvpm_ctx *ctx, float radius, uint32_t *n_kept);
 int check_scene(gvpm_ctx *ctx, const gvpm_box_scene *s);
+// occluder BVH (occluder_bvh.cu): whether the gathers walk it, building it for the current set (n_tri > 0), the
+// occluder fields of a gather's parameters, and the any-hit of gvpm_occluded on rays already on the device
+bool occluder_use_bvh(const gvpm_ctx *ctx);
+int build_occluder_bvh(gvpm_ctx *ctx);
+void occluder_params(const gvpm_ctx *ctx, GatherParams &P);
+void launch_occluded(const GatherParams &P, bool bvh, const float *o, const float *d, const float *mint, const float *maxt,
+                     uint32_t n, uint8_t *hit, cudaStream_t st);
 // a new beam set of n beams (staging sized, the old set and its build dropped); then fill the staging arrays and
 // commit_beams: records packed, sub-beam size and count known (host: the caller's arrays, for the host-side length sum;
 // nullptr: the beams exist on the device only and the sum runs there)

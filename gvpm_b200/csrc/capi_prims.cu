@@ -319,10 +319,6 @@ static int beam_params(gvpm_ctx *ctx, GatherParams &P) {
   P.weight_kernel = (float)(1.0 / P.kernel_vol);  // shift_volume_beams.h:272
   if (ctx->cfg.beam_kernel_1d) P.weight_kernel = 0.5f / r;  // :188
   P.bounds = ctx->beam_bounds.as<float>();
-  P.tri = ctx->tri.as<float>();
-  P.tri_plane = ctx->tri_plane.as<float4>();
-  P.tri_aux = ctx->tri_aux.as<float2>();
-  P.n_tri = ctx->n_tri;
   P.out = ctx->out.as<float>();
   P.counts = ctx->counts.as<uint32_t>();
   P.pair_counter = (unsigned long long *)(ctx->work_counter.as<char>() + 8);

@@ -318,7 +318,7 @@ struct BeamShadeShared {
   float t[32][GVPM_OUT_FLOATS + 2];   // a batch's results, transposed reduction (odd row stride: no bank conflicts)
 };
 
-template <bool K1D>
+template <bool K1D, bool BVH>
 __device__ __forceinline__ void beam_shade_batch(const GatherParams &P, BeamShadeShared &Q, uint32_t head, uint32_t cnt,
                                                  int lane) {
   float a[GVPM_OUT_FLOATS];
@@ -337,7 +337,7 @@ __device__ __forceinline__ void beam_shade_batch(const GatherParams &P, BeamShad
     kRec.weightKernel = sf(Q.f[4][e]); kRec.u = sf(Q.f[5][e]);
     kRec.contrib = v3(Q.f[6][e], Q.f[7][e], Q.f[8][e]);
     kRec.valid = true;
-    beam_functor<K1D>(P, rec, R, beam, kRec, a);
+    beam_functor<K1D, BVH>(P, rec, R, beam, kRec, a);
   }
   // per-ray sums over runs of equal ray id, transposed through shared memory: lane j walks column j of the 32 x 27
   // results in pair order and adds a run's sum with one coalesced atomic instruction (a rolled loop: the 27 x 5
@@ -362,7 +362,8 @@ __device__ __forceinline__ void beam_shade_batch(const GatherParams &P, BeamShad
   __syncwarp();
 }
 
-template <bool K1D>
+// BVH: shadow rays walk the occluder BVH (occluder_device.cuh)
+template <bool K1D, bool BVH>
 __global__ void __launch_bounds__(128, 3) k_beam_shade(const __grid_constant__ GatherParams P) {
   __shared__ BeamShadeShared ring[4];
   const int lane = threadIdx.x & 31;
@@ -442,7 +443,7 @@ __global__ void __launch_bounds__(128, 3) k_beam_shade(const __grid_constant__ G
     __syncwarp();
     if (qn >= 32u || (!more && qn > 0u)) {   // a full batch, or what is left once the pair list is exhausted
       const uint32_t take = min(qn, 32u);
-      beam_shade_batch<K1D>(P, Q, head, take, lane);
+      beam_shade_batch<K1D, BVH>(P, Q, head, take, lane);
       head = (head + take) & (kBeamRing - 1);
       qn -= take;
       __syncwarp();
@@ -517,10 +518,15 @@ cudaError_t launch_beam_traverse(const GatherParams &P, int sm_count, cudaStream
   k_beam_traverse<<<persistent_grid<k_beam_traverse>(sm_count, kBeamWarps * 32, need), kBeamWarps * 32, 0, stream>>>(P);
   return cudaGetLastError();
 }
+template <bool K1D> static void launch_beam_shade_k(const GatherParams &P, unsigned long long total, int sm_count,
+                                                    cudaStream_t stream) {
+  if (P.occ_nodes) k_beam_shade<K1D, true><<<stride_grid<k_beam_shade<K1D, true>>(sm_count, 128, total), 128, 0, stream>>>(P);
+  else k_beam_shade<K1D, false><<<stride_grid<k_beam_shade<K1D, false>>(sm_count, 128, total), 128, 0, stream>>>(P);
+}
 cudaError_t launch_beam_shade(const GatherParams &P, unsigned long long total, int sm_count, cudaStream_t stream) {
   if (total == 0) return cudaSuccess;
-  if (P.cfg.beam_kernel_1d) k_beam_shade<true><<<stride_grid<k_beam_shade<true>>(sm_count, 128, total), 128, 0, stream>>>(P);
-  else k_beam_shade<false><<<stride_grid<k_beam_shade<false>>(sm_count, 128, total), 128, 0, stream>>>(P);
+  if (P.cfg.beam_kernel_1d) launch_beam_shade_k<true>(P, total, sm_count, stream);
+  else launch_beam_shade_k<false>(P, total, sm_count, stream);
   return cudaGetLastError();
 }
 

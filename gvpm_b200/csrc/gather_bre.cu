@@ -528,7 +528,8 @@ k_bre_grid_traverse(const __grid_constant__ GatherParams P) {
   }
 }
 
-template <bool SPPM>
+// BVH: shadow rays walk the occluder BVH (occluder_device.cuh); SPPM casts none, so only <false, *> exist
+template <bool SPPM, bool BVH>
 __global__ void __launch_bounds__(GVPM_SHADE_THREADS, GVPM_SHADE_MIN_BLOCKS)
 k_bre_shade(const __grid_constant__ GatherParams P) {
   __shared__ ShadeShared shade_sh[SPPM ? 1 : GVPM_SHADE_THREADS / 32];
@@ -564,7 +565,7 @@ k_bre_shade(const __grid_constant__ GatherParams P) {
     if (SPPM) {
       if (valid) bre_photon<SPPM>(P, P.rays + (size_t)pr.x * GVPM_RAY_FLOAT4, pr.y, a);
     } else {
-      bre_pairs_warp(P, pr, valid, a, shade_sh[threadIdx.x >> 5], lane);
+      bre_pairs_warp<BVH>(P, pr, valid, a, shade_sh[threadIdx.x >> 5], lane);
     }
     // per-ray sums over RUNS of equal ray id (a ray's pairs arrive in contiguous runs, one per flush; the same ray
     // may own several runs, each adds its own partial sum)
@@ -585,12 +586,12 @@ template <int MODE> static void launch_traverse_mode(const GatherParams &P, int 
     k_bre_traverse<MODE><<<grid, kTravWarps * 32, 0, stream>>>(P);
   }
 }
-template <bool SPPM> static void launch_shade_mode(const GatherParams &P, unsigned long long total, int sm_count,
-                                                   cudaStream_t stream) {
+template <bool SPPM, bool BVH> static void launch_shade_mode(const GatherParams &P, unsigned long long total, int sm_count,
+                                                             cudaStream_t stream) {
   // total == ~0: the count is only known on the device (the kernel reads it): size the grid for a full pair list
   if (total == ~0ull || total > P.pair_cap) total = P.pair_cap;
-  const unsigned grid = stride_grid<k_bre_shade<SPPM>>(sm_count, GVPM_SHADE_THREADS, total);
-  k_bre_shade<SPPM><<<grid, GVPM_SHADE_THREADS, 0, stream>>>(P);
+  const unsigned grid = stride_grid<k_bre_shade<SPPM, BVH>>(sm_count, GVPM_SHADE_THREADS, total);
+  k_bre_shade<SPPM, BVH><<<grid, GVPM_SHADE_THREADS, 0, stream>>>(P);
 }
 
 cudaError_t launch_bre_traverse(const GatherParams &P, bool dump, int sm_count, cudaStream_t stream) {
@@ -603,8 +604,9 @@ cudaError_t launch_bre_traverse(const GatherParams &P, bool dump, int sm_count, 
 
 cudaError_t launch_bre_shade(const GatherParams &P, unsigned long long total, int sm_count, cudaStream_t stream) {
   if (total == 0) return cudaSuccess;
-  if (P.cfg.sppm_primal) launch_shade_mode<true>(P, total, sm_count, stream);
-  else launch_shade_mode<false>(P, total, sm_count, stream);
+  if (P.cfg.sppm_primal) launch_shade_mode<true, false>(P, total, sm_count, stream);
+  else if (P.occ_nodes) launch_shade_mode<false, true>(P, total, sm_count, stream);
+  else launch_shade_mode<false, false>(P, total, sm_count, stream);
   return cudaGetLastError();
 }
 

@@ -141,6 +141,7 @@ __global__ void __launch_bounds__(kVpmWarps * 32, 8) k_vpm_traverse(const __grid
 }
 
 // VolumeGradientPositionQuery::operator() for one (sample, photon) pair, after the filters.
+template <bool BVH>
 __device__ __forceinline__ void vpm_photon(const GatherParams &P, const float4 *__restrict__ rec, float4 s0,
                                            float4 s1, uint32_t pi, float *a) {
   const BaseRay R = load_base_ray(rec);
@@ -159,7 +160,7 @@ __device__ __forceinline__ void vpm_photon(const GatherParams &P, const float4 *
   const sf pdfBase = pdfSuccess * pdfSel;
   const sf recip = sf(1.f) / (kernelVol * pdfBase);
   acc_add(a, 0, baseContrib * recip);
-  const OccluderNear near = pair_occluders(P, ph.parent, ph.lBase);
+  const OccluderNear near = pair_occluders<BVH>(P, ph.parent, ph.lBase);
 
   float Sx[4], Sy[4], Sz[4], Wk[4];
 #pragma unroll 1
@@ -184,7 +185,7 @@ __device__ __forceinline__ void vpm_photon(const GatherParams &P, const float4 *
         shift_null(P, ph.flux, wi, dk, eyeK, sensor, Tk, pdfBase, pdfShift, S, weight);
       } else {  // :604-639
         const v3 offsetPos = get_shift_pos(P, rr2, ph.p, q, zShift, R.d, dk, false);
-        shift_photon_diffuse(P, ph, near, offsetPos, dk, eyeK, sensor, Tk, pdfBase, pdfShift, S, weight);
+        shift_photon_diffuse<BVH>(P, ph, near, offsetPos, dk, eyeK, sensor, Tk, pdfBase, pdfShift, S, weight);
       }
     }
     if ((k == 1 && R.px == P.cfg.film_w - 1) || (k == 2 && R.py == P.cfg.film_h - 1)) weight = sf(1.f);
@@ -198,6 +199,8 @@ __device__ __forceinline__ void vpm_photon(const GatherParams &P, const float4 *
   }
 }
 
+// BVH: shadow rays walk the occluder BVH (occluder_device.cuh)
+template <bool BVH>
 __global__ void __launch_bounds__(128, 4) k_vpm_shade(const __grid_constant__ GatherParams P) {
   const int lane = threadIdx.x & 31;
   unsigned long long total = *P.pair_counter;
@@ -216,7 +219,7 @@ __global__ void __launch_bounds__(128, 4) k_vpm_shade(const __grid_constant__ Ga
       const uint2 pr = P.pairs[i];
       const float4 s0 = ldg4(P.samples + 2 * (size_t)pr.x), s1 = ldg4(P.samples + 2 * (size_t)pr.x + 1);
       key = __float_as_uint(s1.w);
-      vpm_photon(P, P.rays + (size_t)key * GVPM_RAY_FLOAT4, s0, s1, pr.y, a);
+      vpm_photon<BVH>(P, P.rays + (size_t)key * GVPM_RAY_FLOAT4, s0, s1, pr.y, a);
 #pragma unroll
       for (int j = 0; j < GVPM_OUT_FLOATS; ++j) a[j] *= normalization;
     }
@@ -235,7 +238,8 @@ cudaError_t launch_vpm_traverse(const GatherParams &P, bool dump, int sm_count, 
 
 cudaError_t launch_vpm_shade(const GatherParams &P, unsigned long long total, int sm_count, cudaStream_t stream) {
   if (total == 0) return cudaSuccess;
-  k_vpm_shade<<<stride_grid<k_vpm_shade>(sm_count, 128, total), 128, 0, stream>>>(P);
+  if (P.occ_nodes) k_vpm_shade<true><<<stride_grid<k_vpm_shade<true>>(sm_count, 128, total), 128, 0, stream>>>(P);
+  else k_vpm_shade<false><<<stride_grid<k_vpm_shade<false>>(sm_count, 128, total), 128, 0, stream>>>(P);
   return cudaGetLastError();
 }
 

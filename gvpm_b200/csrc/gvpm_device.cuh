@@ -267,6 +267,9 @@ struct GatherParams {
   uint2 *dump_pairs;
   unsigned long long *dump_counter;
   unsigned long long dump_cap;
+  // occluder BVH (occluder_device.cuh): GVPM_OCC_NODE_FLOAT4 float4 per node; null when the shadow rays use the list
+  const float4 *occ_nodes;
+  uint32_t n_occ_nodes;
 };
 
 // ---- photon dispatch between ranks (dispatch.cu) -----------------------------------------------------------------------

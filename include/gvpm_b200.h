@@ -212,7 +212,24 @@ void *gvpm_stream(gvpm_ctx *ctx);
 /* ---- scene constants ----------------------------------------------------------------- */
 int gvpm_set_medium(gvpm_ctx *ctx, const gvpm_medium *m);
 int gvpm_set_config(gvpm_ctx *ctx, const gvpm_config *c);
+/* Occluders: the triangles the reconnection shadow rays test, typically every triangle of the
+ * scene (flattenOccluders).  n_tri = 0 clears them; more than GVPM_MAX_OCCLUDERS fails with
+ * GVPM_ERR_INVALID.  When the selected path (gvpm_set_occluder_accel) is the BVH, the call builds
+ * it on the device once for the set; the gathers then use it until the next call. */
+#define GVPM_MAX_OCCLUDERS (1u << 24)
 int gvpm_set_occluders(gvpm_ctx *ctx, const float *tri_xyz /* [n_tri*9] */, size_t n_tri);
+/* Path of the shadow-ray any-hit.  AUTO (the default): the flat list up to 32 triangles, the BVH
+ * above.  LIST and BVH force one path; both give the same answer for every ray.  Any other value
+ * fails with GVPM_ERR_INVALID.  Selecting the BVH for the current set builds it if needed. */
+enum gvpm_occluder_accel { GVPM_OCC_AUTO = 0, GVPM_OCC_LIST = 1, GVPM_OCC_BVH = 2 };
+int gvpm_set_occluder_accel(gvpm_ctx *ctx, int mode);
+/* the path the gathers take for the current set: GVPM_OCC_LIST or GVPM_OCC_BVH (0 for ctx = NULL) */
+int gvpm_occluder_accel_kind(const gvpm_ctx *ctx);
+/* Any-hit of n rays (host arrays: o, d [n*3], mint, maxt [n]) against the occluders, through the
+ * path the gathers take and the same device code as their shadow rays; hit[i] = 0 or 1.  A parity
+ * and timing aid; blocking. */
+int gvpm_occluded(gvpm_ctx *ctx, const float *o, const float *d, const float *mint, const float *maxt, size_t n,
+                  uint8_t *hit);
 
 /* ---- photon points: replaces GPhotonMap::tryAppend/build (gvpm_accel.h:119-203,
  *      include/mitsuba/core/kdtree.h:326-378) and the GradientBeamRadianceEstimator
