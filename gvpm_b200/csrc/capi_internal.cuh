@@ -28,17 +28,19 @@ int pinhole_blocks(uint32_t n);
 void launch_pinhole_fit(const float4 *rays, uint32_t n, double *partial, float *fit, unsigned *stats, cudaStream_t st,
                         const float *view_dir);
 size_t frustum_occ_bytes();
-void launch_frustum_keys(const float4 *rays, uint32_t n_rays, const float *pos, uint32_t stride, const uint32_t *par_src,
-                         uint32_t par_stride, uint32_t par_shift, uint32_t n,
-                         const FrustumGrid &G, uint32_t *occ, uint32_t *keys, uint32_t *vals, unsigned *coord_mag,
-                         uint32_t *keepmask, uint32_t *cell_count, uint32_t region_cap, const uint32_t *region_count,
-                         int sm_count, cudaStream_t st);
+void launch_frustum_keys(const float *pos, uint32_t stride, const uint32_t *par_src, uint32_t par_stride, uint32_t par_shift,
+                         uint32_t n, const FrustumGrid &G, const uint32_t *occ, uint32_t *keys, uint32_t *vals,
+                         unsigned *coord_mag, uint32_t *keepmask, uint32_t *cell_count, uint32_t region_cap,
+                         const uint32_t *region_count, cudaStream_t st);
+void launch_frustum_pack(const PhotonStaging &S, uint32_t n, const FrustumGrid &G, const uint32_t *occ, uint32_t *keys,
+                         uint32_t *vals, unsigned *coord_mag, uint32_t *keepmask, uint32_t *cell_count, float4 *aos,
+                         float4 *plane_src, cudaStream_t st);
 size_t cell_scan_temp_bytes(uint32_t n_keys);
 cudaError_t launch_cell_scan(void *temp, size_t temp_bytes, const uint32_t *cell_count, uint32_t *cell_start, uint32_t n_keys,
                              cudaStream_t st);
-void launch_pack_scatter(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *keys, const uint32_t *rank,
-                         const uint32_t *cell_start, float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st,
-                         bool records_ready, const uint32_t *kept_dev, int sm_count);
+void launch_scatter_gather(uint32_t n, const uint32_t *keepmask, const uint32_t *keys, const uint32_t *rank,
+                           const uint32_t *cell_start, const float4 *src, uint32_t stride, const uint32_t *kept_dev,
+                           float4 *planes, uint32_t *orig, int sm_count, cudaStream_t st);
 void launch_frustum_mark(const float4 *rays, uint32_t n_rays, const FrustumGrid &G, uint32_t *occ, int sm_count, cudaStream_t st);
 void launch_dispatch(const DispatchParams &P, cudaStream_t st, int ctas);
 void launch_dispatch_signal(const SignalParams &P, cudaStream_t st);
@@ -230,6 +232,8 @@ struct gvpm_ctx {
   bool force_bvh = false;            // GVPM_ACCEL=bvh: A/B switch for kernel experiments
   FrustumGrid grid{};
   DevBuf cell_start, grid_occ, pin_scratch, trace_scratch, keepmask, cell_count;
+  DevBuf plane_src;                  // first float4 of each kept photon's record, caller's order (staged frustum builds)
+  bool occ_ready = false;            // grid_occ holds the occupancy mask of the current RayFit (analyse_rays)
   double trace_photons_per_path = 0.0;   // running estimate (sizes the first batch of gvpm_trace_photons)
   double trace_beams_per_path = 0.0;     // the same for gvpm_trace_beams
   // pin_scratch: [0,64) fit floats, [64,96) stats words, [128,..) block partials (doubles)

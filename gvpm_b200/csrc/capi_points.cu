@@ -126,9 +126,8 @@ static float decode_max_key(unsigned key) {
   return f;
 }
 // Are the uploaded rays concurrent (do their lines meet in one point)?  Two reductions over the packed rays and one
-// read-back, cached until other rays are uploaded.
-int analyse_rays(gvpm_ctx *ctx) {
-  if (ctx->pin_gen == ctx->rays_gen) return GVPM_OK;
+// read-back.
+static int fit_rays(gvpm_ctx *ctx) {
   gvpm_ctx::RayFit &F = ctx->pin;
   F.concurrent = false;
   ctx->pin_gen = ctx->rays_gen;
@@ -152,6 +151,25 @@ int analyse_rays(gvpm_ctx *ctx) {
   F.ymin = -decode_max_key(st[4]); F.ymax = decode_max_key(st[5]);
   F.concurrent = std::isfinite(F.delta) && F.cosmin > 0.35f && std::isfinite(F.xmin) && std::isfinite(F.xmax) &&
                  std::isfinite(F.ymin) && std::isfinite(F.ymax) && F.xmin <= F.xmax && F.ymin <= F.ymax;
+  return GVPM_OK;
+}
+// The ray fit, cached until other rays are uploaded (or another view direction is set), and for concurrent rays the
+// occupancy mask of their projected directions that the perspective-grid builds test photons against.  The mask depends on
+// the fit alone (projection basis and bounds), never on the radius or the photons, so it is built once per fit.
+int analyse_rays(gvpm_ctx *ctx) {
+  if (ctx->pin_gen != ctx->rays_gen) {
+    ctx->occ_ready = false;
+    int rc = fit_rays(ctx);
+    if (rc) return rc;
+  }
+  if (ctx->pin.concurrent && !ctx->occ_ready) {
+    CK(ctx->grid_occ.reserve(frustum_occ_bytes()));
+    launch_frustum_mark(ctx->rays.as<float4>(), ctx->n_rays, make_frustum_grid(ctx->pin, 1.f, false),
+                        ctx->grid_occ.as<uint32_t>(), ctx->sm_count, ctx->stream);
+    ctx->launches += 2;
+    CK(cudaGetLastError());
+    ctx->occ_ready = true;
+  }
   return GVPM_OK;
 }
 
@@ -206,9 +224,12 @@ int build_frustum(gvpm_ctx *ctx, float radius, uint32_t *n_kept) {
     CK(ctx->orig.reserve(4 * (size_t)n));
     CK(ctx->keepmask.reserve(4 * ((size_t)n / 32 + 2)));
     const bool direct = ctx->photons_direct;
-    if (!direct) CK(ctx->aos.reserve(128 * (size_t)n));
-    CK(ctx->grid_occ.reserve(frustum_occ_bytes()));
+    if (!direct) {
+      CK(ctx->aos.reserve(128 * (size_t)n));
+      CK(ctx->plane_src.reserve(16 * (size_t)n));
+    }
     uint32_t *keepmask = ctx->keepmask.as<uint32_t>(), *cell_count = ctx->cell_count.as<uint32_t>();
+    const uint32_t *occ = ctx->grid_occ.as<uint32_t>();   // analyse_rays built it for this fit
     // the word after the keep bits: set when the build is incomplete (gvpm_build_dispatched: a peer's dispatch timed out
     // or overflowed its region); the gather reports it instead of gathering
     uint32_t *ovf = keepmask + (n / 32 + 1);
@@ -216,26 +237,27 @@ int build_frustum(gvpm_ctx *ctx, float radius, uint32_t *n_kept) {
     PhotonStaging S{};
     if (!direct) S = staging_ptrs<PhotonSoA>(ctx->ph_staging.p, n);
     // Counting sort: the key pass counts the photons of every cell and gives each its rank in the cell; the exclusive scan
-    // of the counters IS cell_start; the packing pass (or a scatter pass over records that exist already) puts position
-    // plane entry and index at cell_start[key] + rank.  Nothing to size from a count: dropped photons and the empty part
+    // of the counters IS cell_start; a scatter pass puts each kept photon's index at cell_start[key] + rank, and the
+    // position plane is gathered through that index map.  Nothing to size from a count: dropped photons and the empty part
     // of a dispatched inbox are simply never written.  The order inside a cell follows the atomics (the gather's float
-    // atomics are unordered anyway).
+    // atomics are unordered anyway).  Staged photons: the key pass also packs the kept photons' records (and their
+    // first float4 into plane_src, which the plane gather reads); records that exist already are read in place.
     CK(cudaMemsetAsync(cell_count, 0, ((size_t)n_keys + 2) * 4, st));
     if (direct)   // position = first three floats of the record, path parity = bit 10 of its meta word
-      launch_frustum_keys(ctx->rays.as<float4>(), ctx->n_rays, (const float *)ctx->records(), 32u, (const uint32_t *)ctx->records() + 3, 32u, 10u, n,
-                          G, ctx->grid_occ.as<uint32_t>(), ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(),
-                          ctx->bounds.as<unsigned>() + 6, keepmask, cell_count, ctx->region_cap, ctx->region_count, ctx->sm_count, st);
-    else
-      launch_frustum_keys(ctx->rays.as<float4>(), ctx->n_rays, S.pos, 3u, S.path_id, 1u, 0u, n, G, ctx->grid_occ.as<uint32_t>(),
+      launch_frustum_keys((const float *)ctx->records(), 32u, (const uint32_t *)ctx->records() + 3, 32u, 10u, n, G, occ,
                           ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), ctx->bounds.as<unsigned>() + 6, keepmask,
-                          cell_count, 0, nullptr, ctx->sm_count, st);
+                          cell_count, ctx->region_cap, ctx->region_count, st);
+    else
+      launch_frustum_pack(S, n, G, occ, ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), ctx->bounds.as<unsigned>() + 6,
+                          keepmask, cell_count, ctx->aos.as<float4>(), ctx->plane_src.as<float4>(), st);
     CK(launch_cell_scan(ctx->sort_temp.p, ctx->sort_temp.cap, cell_count, ctx->cell_start.as<uint32_t>(), n_keys, st));
-    launch_pack_scatter(S, n, keepmask, ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), ctx->cell_start.as<uint32_t>(),
-                        ctx->records(), ctx->planes.as<float4>(), ctx->orig.as<uint32_t>(), st, direct,
-                        ctx->cell_start.as<uint32_t>() + n_keys - 1, ctx->sm_count);
+    launch_scatter_gather(n, keepmask, ctx->keys_in.as<uint32_t>(), ctx->vals_in.as<uint32_t>(), ctx->cell_start.as<uint32_t>(),
+                          direct ? ctx->records() : ctx->plane_src.as<float4>(), direct ? 8u : 1u,   // record: 8 float4
+                          ctx->cell_start.as<uint32_t>() + n_keys - 1, ctx->planes.as<float4>(), ctx->orig.as<uint32_t>(),
+                          ctx->sm_count, st);
     ctx->build_ovf = ovf;
     CK(cudaEventRecord(ctx->ev_free[ctx->ph_staging_sel], st));   // last read of the staging buffer
-    ctx->launches += 17;
+    ctx->launches += 8;
     CK(cudaGetLastError());
   } else {
     CK(cudaMemsetAsync(ctx->bounds.p, 0, 7 * sizeof(float), st));

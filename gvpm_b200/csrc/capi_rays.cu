@@ -97,6 +97,7 @@ int gvpm_generate_rays(gvpm_ctx *ctx, const gvpm_box_scene *scene, const gvpm_pi
     F.count = (float)n;
     F.concurrent = n > 0 && F.cosmin > 0.35f;
     ctx->pin_gen = ctx->rays_gen;
+    ctx->occ_ready = false;
   }
   return GVPM_OK;
 }

@@ -576,8 +576,63 @@ __global__ void __launch_bounds__(256) k_frustum_keys(const float *__restrict__ 
     if (m > __uint_as_float(*(volatile unsigned *)coord_mag)) atomicMax(coord_mag, __float_as_uint(m));
   }
 }
+// k_frustum_keys and k_pack_aos_kept in one pass over the staged SoA (the path_id plane and the positions are read once):
+// one warp per 32 consecutive photons.  Each lane computes its photon's key; a kept photon takes its rank in the cell,
+// then loads the rest of its fields and builds its record in the warp's shared tile, which the warp writes out with the
+// transposed stores of k_pack_aos_kept.  plane_src[i] = the record's first float4 (pos, meta), kept photons only: the
+// sorted position plane is gathered from this compact copy (16 of every 128 bytes) instead of from the records.
+__global__ void __launch_bounds__(256) k_frustum_pack(const PhotonStaging S, uint32_t n, const FrustumGrid G,
+                                                       const uint32_t *__restrict__ occ, uint32_t *__restrict__ keys,
+                                                       uint32_t *__restrict__ vals, unsigned *__restrict__ coord_mag,
+                                                       uint32_t *__restrict__ keepmask, uint32_t *__restrict__ cell_count,
+                                                       float4 *__restrict__ aos, float4 *__restrict__ plane_src) {
+  __shared__ float4 tile[8][32 * 9];   // per warp: 32 records x 8 float4, row stride 9 float4 (conflict-free both ways)
+  __shared__ float wmag[8];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const uint32_t warpBase = blockIdx.x * blockDim.x + (w << 5);
+  const uint32_t i = warpBase + lane;
+  float4 *t = tile[w];
+  float mag = 0.f;
+  bool keep = false;
+  if (i < n) {
+    const size_t i3 = 3 * (size_t)i;
+    const v3 pos(__ldg(S.pos + i3), __ldg(S.pos + i3 + 1), __ldg(S.pos + i3 + 2));
+    const uint32_t pid = __ldg(S.path_id + i);
+    mag = fmaxf(fmaxf(fabsf(pos.x.v), fabsf(pos.y.v)), fabsf(pos.z.v));
+    const uint32_t key = frustum_key(G, occ, pos.x.v, pos.y.v, pos.z.v, [&]() { return pid; });
+    keys[i] = key;
+    keep = key != (G.parity_split ? 2u : 1u) * G.n_cells + 1u;
+    if (keep) {
+      vals[i] = atomicAdd(cell_count + key, 1u);
+      auto ld3 = [&](const float *p) { return v3(__ldg(p + i3), __ldg(p + i3 + 1), __ldg(p + i3 + 2)); };
+      const uint32_t meta = pack_meta(S.parent_type[i], S.depth[i], pid);
+      photon_record(t + lane * 9, pos, meta, ld3(S.flux), sf(__ldg(S.parent_pdf + i)), ld3(S.parent_pos),
+                    sf(__ldg(S.edge_pdf + i)), ld3(S.pred_pos), sf(__ldg(S.rr_weight + i)), ld3(S.parent_n),
+                    ld3(S.prefix_flux), ld3(S.parent_albedo), 0u);
+      plane_src[i] = make_float4(pos.x.v, pos.y.v, pos.z.v, __uint_as_float(meta));
+    }
+  }
+  const uint32_t km = __ballot_sync(0xffffffffu, keep);
+  if (lane == 0 && i < n) keepmask[i >> 5] = km;
+  __syncwarp();
+  float4 *dst = aos + (size_t)warpBase * GVPM_AOS_FLOAT4;
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const uint32_t q = 32u * j + lane;          // float4 index inside the warp's 4 KB of records
+    if (km >> (q >> 3) & 1u) dst[q] = t[(q >> 3) * 9 + (q & 7u)];
+  }
+  // coordinate magnitude: one atomic per CTA, as in k_frustum_keys
+  mag = warp_max(mag);
+  if (lane == 0) wmag[w] = mag;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float m = 0.f;
+    for (int k = 0; k < (int)(blockDim.x >> 5); ++k) m = fmaxf(m, wmag[k]);
+    if (m > __uint_as_float(*(volatile unsigned *)coord_mag)) atomicMax(coord_mag, __float_as_uint(m));
+  }
+}
 // counting sort: the index map alone (orig[cell_start[key] + rank] = photon).  4-byte random writes into an array that
-// stays in L2 (40 MB for 10 M photons); the position plane is then gathered with coalesced writes (k_gather_sorted).
+// stays in L2 (40 MB for 10 M photons); the position plane is then gathered with coalesced writes (k_gather_by_index).
 // Scattering the 16-byte plane entries directly costs more than both passes together: random partial-sector writes into
 // 160 MB are read-modify-write cycles in DRAM (measured: 0.40 ms against 0.06 + 0.24 ms).
 __global__ void __launch_bounds__(256) k_scatter_index(const uint32_t *__restrict__ keys, const uint32_t *__restrict__ rank,
@@ -587,12 +642,14 @@ __global__ void __launch_bounds__(256) k_scatter_index(const uint32_t *__restric
   if (i >= n || !(__ldg(keepmask + (i >> 5)) >> (i & 31u) & 1u)) return;
   orig[__ldg(cell_start + keys[i]) + rank[i]] = i;
 }
-// position plane from the index map; m = number of sorted slots, read from the device (cell_start[n_keys - 1] = kept photons)
-__global__ void k_gather_by_index(const float4 *__restrict__ aos, const uint32_t *__restrict__ orig, const uint32_t *__restrict__ m_dev,
-                                  float4 *__restrict__ planes) {
+// position plane from the index map: planes[s] = src[orig[s] * stride] (stride 1: k_frustum_pack's plane_src; 8: the
+// first float4 of 128-byte records); m = number of sorted slots, read from the device (cell_start[n_keys - 1] = kept
+// photons).  (Four independent loads in flight per thread measured no faster: profiles/r6_build.md.)
+__global__ void k_gather_by_index(const float4 *__restrict__ src, uint32_t stride, const uint32_t *__restrict__ orig,
+                                  const uint32_t *__restrict__ m_dev, float4 *__restrict__ planes) {
   const uint32_t m = __ldg(m_dev);
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x)
-    planes[i] = __ldg(aos + (size_t)__ldg(orig + i) * GVPM_AOS_FLOAT4);
+    planes[i] = __ldg(src + (size_t)__ldg(orig + i) * stride);
 }
 // indices of the kept photons, in index order, packed to the front: block_off = exclusive scan of block_kept
 __global__ void __launch_bounds__(256) k_compact_kept(const uint32_t *__restrict__ keepmask, const uint32_t *__restrict__ block_off,
@@ -707,19 +764,23 @@ size_t frustum_occ_bytes() { return (size_t)kOccWords * 4; }
 void launch_compact_kept(const uint32_t *keepmask, const uint32_t *block_off, uint32_t n, uint32_t *vals_c, cudaStream_t st) {
   if (n) k_compact_kept<<<(n + 255) / 256, 256, 0, st>>>(keepmask, block_off, n, vals_c);
 }
-// occ: frustum_occ_bytes() (zeroed here); coord_mag: one word (zeroed here); cell_count: n_keys + 1 words, zeroed
-// pos / stride: photon positions (stride in floats: 3 for the staged SoA plane, 32 for 128-byte records); parity of the
-// photon's path id = (par_src[par_stride * i] >> par_shift) & 1
+// occ: the occupancy mask of the rays (launch_frustum_mark); coord_mag: one word (zeroed here); cell_count: n_keys + 1
+// words, zeroed.  pos / stride: photon positions in 128-byte records (stride 32 floats); parity of the photon's path id
+// = (par_src[par_stride * i] >> par_shift) & 1
 // region_cap / region_count: dispatched photon sets (0 / nullptr: every index up to n holds a photon)
-void launch_frustum_keys(const float4 *rays, uint32_t n_rays, const float *pos, uint32_t stride, const uint32_t *par_src,
-                         uint32_t par_stride, uint32_t par_shift, uint32_t n,
-                         const FrustumGrid &G, uint32_t *occ, uint32_t *keys, uint32_t *vals, unsigned *coord_mag,
-                         uint32_t *keepmask, uint32_t *cell_count, uint32_t region_cap, const uint32_t *region_count,
-                         int sm_count, cudaStream_t st) {
-  cudaMemsetAsync(occ, 0, frustum_occ_bytes(), st);
+void launch_frustum_keys(const float *pos, uint32_t stride, const uint32_t *par_src, uint32_t par_stride, uint32_t par_shift,
+                         uint32_t n, const FrustumGrid &G, const uint32_t *occ, uint32_t *keys, uint32_t *vals,
+                         unsigned *coord_mag, uint32_t *keepmask, uint32_t *cell_count, uint32_t region_cap,
+                         const uint32_t *region_count, cudaStream_t st) {
   cudaMemsetAsync(coord_mag, 0, 4, st);
-  if (n_rays) k_frustum_mark<<<std::min<uint32_t>((n_rays + 255) / 256, 2u * (uint32_t)sm_count), 256, 0, st>>>(rays, n_rays, G, occ);
   if (n) k_frustum_keys<<<(n + 255) / 256, 256, 0, st>>>(pos, stride, par_src, par_stride, par_shift, n, G, occ, keys, vals, coord_mag, keepmask, cell_count, region_cap, region_count);
+}
+// the same outputs for the staged SoA, plus the records of the kept photons (aos) and their first float4 (plane_src)
+void launch_frustum_pack(const PhotonStaging &S, uint32_t n, const FrustumGrid &G, const uint32_t *occ, uint32_t *keys,
+                         uint32_t *vals, unsigned *coord_mag, uint32_t *keepmask, uint32_t *cell_count, float4 *aos,
+                         float4 *plane_src, cudaStream_t st) {
+  cudaMemsetAsync(coord_mag, 0, 4, st);
+  if (n) k_frustum_pack<<<(n + 255) / 256, 256, 0, st>>>(S, n, G, occ, keys, vals, coord_mag, keepmask, cell_count, aos, plane_src);
 }
 // counting sort: cell_start[0 .. n_keys] = exclusive scan of the per-cell counts (cell_count[n_keys] must be 0)
 size_t cell_scan_temp_bytes(uint32_t n_keys) {
@@ -731,16 +792,17 @@ cudaError_t launch_cell_scan(void *temp, size_t temp_bytes, const uint32_t *cell
                              cudaStream_t st) {
   return cub::DeviceScan::ExclusiveSum(temp, temp_bytes, cell_count, cell_start, (int)n_keys + 1, st);
 }
-// records of the kept photons, index map at cell_start[key] + rank, position plane gathered from it (kept_dev: slots in use)
-void launch_pack_scatter(const PhotonStaging &S, uint32_t n, const uint32_t *keepmask, const uint32_t *keys, const uint32_t *rank,
-                         const uint32_t *cell_start, float4 *aos, float4 *planes, uint32_t *orig, cudaStream_t st,
-                         bool records_ready, const uint32_t *kept_dev, int sm_count) {
+// index map at cell_start[key] + rank, then the position plane gathered through it from src (stride in float4: 1 for
+// plane_src, 8 for records); kept_dev: slots in use
+void launch_scatter_gather(uint32_t n, const uint32_t *keepmask, const uint32_t *keys, const uint32_t *rank,
+                           const uint32_t *cell_start, const float4 *src, uint32_t stride, const uint32_t *kept_dev,
+                           float4 *planes, uint32_t *orig, int sm_count, cudaStream_t st) {
   if (!n) return;
-  if (!records_ready) k_pack_aos_kept<<<(n + 255) / 256, 256, 0, st>>>(S, n, keepmask, aos);
   k_scatter_index<<<(n + 255) / 256, 256, 0, st>>>(keys, rank, keepmask, cell_start, n, orig);
-  k_gather_by_index<<<std::min<uint32_t>((n + 255) / 256, 16u * (uint32_t)sm_count), 256, 0, st>>>(aos, orig, kept_dev, planes);
+  k_gather_by_index<<<std::min<uint32_t>((n + 255) / 256, 16u * (uint32_t)sm_count), 256, 0, st>>>(src, stride, orig, kept_dev, planes);
 }
-// the occupancy mask alone (what a rank publishes to the ranks that send it photons)
+// the occupancy mask alone: the one the builds test against (analyse_rays, once per ray fit) and the copy a rank
+// publishes to the ranks that send it photons
 void launch_frustum_mark(const float4 *rays, uint32_t n_rays, const FrustumGrid &G, uint32_t *occ, int sm_count, cudaStream_t st) {
   cudaMemsetAsync(occ, 0, frustum_occ_bytes(), st);
   if (n_rays) k_frustum_mark<<<std::min<uint32_t>((n_rays + 255) / 256, 2u * (uint32_t)sm_count), 256, 0, st>>>(rays, n_rays, G, occ);
