@@ -6,8 +6,10 @@ synthetic-input generator.  There is no CPU fallback: see _native.load_lib().
 """
 from . import _native
 from .records import (BeamSet, PlaneSet, PhotonSet, RaySet, VpmSampleSet, synth_beams, synth_planes, bre_radius, make_config, make_medium, synth_occluders,
-                      synth_photons, synth_rays, synth_vpm_samples, box_scene_default, pinhole_camera)
+                      synth_photons, synth_rays, synth_vpm_samples, box_scene_default, pinhole_camera,
+                      lookat_camera, box_scene_as_mesh)
 
 __all__ = ["_native", "PhotonSet", "RaySet", "bre_radius", "make_config", "make_medium",
            "synth_occluders", "synth_photons", "synth_rays", "VpmSampleSet", "synth_vpm_samples",
-           "BeamSet", "PlaneSet", "synth_beams", "synth_planes", "box_scene_default", "pinhole_camera"]
+           "BeamSet", "PlaneSet", "synth_beams", "synth_planes", "box_scene_default", "pinhole_camera",
+           "lookat_camera", "box_scene_as_mesh"]

@@ -89,6 +89,16 @@ class PinholeCamera(C.Structure):
                 ("inside_medium", C.c_int32)]
 
 
+class MeshScene(C.Structure):
+    _fields_ = [("lo", C.c_float * 3), ("hi", C.c_float * 3), ("n_tri", C.c_size_t), ("tri", f32p), ("albedo", f32p),
+                ("emissive", u8p), ("light_power", C.c_float)]
+
+
+class LookatCamera(C.Structure):
+    _fields_ = [("pos", C.c_float * 3), ("forward", C.c_float * 3), ("up", C.c_float * 3), ("tan_half_fov_x", C.c_float),
+                ("film_w", C.c_int32), ("film_h", C.c_int32)]
+
+
 class PoissonParams(C.Structure):
     _fields_ = [("alpha", C.c_float), ("irls_iter_max", C.c_int32), ("irls_reg_init", C.c_float),
                 ("irls_reg_iter", C.c_float), ("cg_iter_max", C.c_int32), ("cg_iter_check", C.c_int32),
@@ -116,7 +126,9 @@ ABI_SYMBOLS = [
     "gvpm_generate_vpm_samples",
     "gvpm_upload_beams", "gvpm_build_beams", "gvpm_gather_beams", "gvpm_gather_beams_device", "gvpm_dump_neighbours_beams", "gvpm_beam_subbeam_count",
     "gvpm_gather_sppm_beams", "gvpm_dump_neighbours_sppm_beams",
-    "gvpm_box_scene_default", "gvpm_generate_rays", "gvpm_trace_photons", "gvpm_trace_photons_direct", "gvpm_trace_beams", "gvpm_planes_from_beams", "gvpm_read_device", "gvpm_measure_read_bandwidth", "gvpm_staging_peek",
+    "gvpm_box_scene_default", "gvpm_generate_rays", "gvpm_trace_photons", "gvpm_trace_photons_direct", "gvpm_trace_beams", "gvpm_planes_from_beams",
+    "gvpm_set_trace_mesh", "gvpm_trace_photons_mesh", "gvpm_trace_photons_direct_mesh", "gvpm_trace_beams_mesh",
+    "gvpm_generate_rays_mesh", "gvpm_read_device", "gvpm_measure_read_bandwidth", "gvpm_staging_peek",
     "gvpm_upload_planes", "gvpm_build_planes", "gvpm_gather_planes", "gvpm_gather_planes_device", "gvpm_dump_neighbours_planes",
     "gvpm_accum_reset", "gvpm_accum_add", "gvpm_accum_fold", "gvpm_accum_read", "gvpm_accum_device",
     "gvpm_compute_gradient_accum", "gvpm_reconstruct_accum",
@@ -163,6 +175,10 @@ def load_lib():
     lib.gvpm_trace_photons_direct.argtypes = [vp, C.POINTER(BoxScene), C.c_size_t, C.c_uint64, C.c_int, C.c_int, C.c_int, u64p]
     lib.gvpm_trace_beams.argtypes = [vp, C.POINTER(BoxScene), C.c_size_t, C.c_uint64, C.c_int, C.c_int, C.c_int, u64p]
     lib.gvpm_planes_from_beams.argtypes = [vp, C.c_uint64]
+    lib.gvpm_set_trace_mesh.argtypes = [vp, C.POINTER(MeshScene)]
+    for name in ("gvpm_trace_photons_mesh", "gvpm_trace_photons_direct_mesh", "gvpm_trace_beams_mesh"):
+        getattr(lib, name).argtypes = [vp, C.c_size_t, C.c_uint64, C.c_int, C.c_int, C.c_int, u64p]
+    lib.gvpm_generate_rays_mesh.argtypes = [vp, C.POINTER(LookatCamera), C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_float]
     lib.gvpm_read_device.argtypes = [vp, vp, vp, C.c_size_t]
     lib.gvpm_measure_read_bandwidth.argtypes = [vp, C.c_size_t, C.c_int, C.POINTER(C.c_double)]
     lib.gvpm_staging_peek.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(C.c_size_t)]

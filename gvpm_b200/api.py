@@ -243,6 +243,47 @@ class Context:
                                            C.byref(paths)), "gvpm_trace_beams")
         return int(paths.value)
 
+    # ---- the same generators on a triangle-mesh scene
+    def set_trace_mesh(self, tri, albedo, emissive, light_power, lo, hi):
+        """the mesh scene of the *_mesh generators: triangles [n, 9] inside the medium box lo / hi, albedo [n, 3],
+        emissive [n] flags (the area light of total power light_power); copied and its BVH built on the device"""
+        tri = np.ascontiguousarray(tri, dtype=np.float32).reshape(-1, 9)
+        n = tri.shape[0]
+        albedo = np.ascontiguousarray(albedo, dtype=np.float32).reshape(n, 3)
+        emissive = np.ascontiguousarray(emissive, dtype=np.uint8).reshape(n)
+        sc = N.MeshScene()
+        for a in range(3):
+            sc.lo[a], sc.hi[a] = float(lo[a]), float(hi[a])
+        sc.n_tri = n
+        sc.tri, sc.albedo = tri.ctypes.data_as(N.f32p), albedo.ctypes.data_as(N.f32p)
+        sc.emissive = emissive.ctypes.data_as(N.u8p)
+        sc.light_power = float(light_power)
+        self._ck(self.lib.gvpm_set_trace_mesh(self.h, C.byref(sc)), "gvpm_set_trace_mesh")
+
+    def trace_photons_mesh(self, n, seed, max_depth=12, rr_depth=1, min_depth=0, direct=False):
+        """trace_photons on the mesh scene; -> light paths traced"""
+        paths = C.c_uint64(0)
+        fn = self.lib.gvpm_trace_photons_direct_mesh if direct else self.lib.gvpm_trace_photons_mesh
+        self._ck(fn(self.h, n, C.c_uint64(seed), max_depth, rr_depth, min_depth, C.byref(paths)),
+                 "gvpm_trace_photons_mesh")
+        self.n_photons = n
+        return int(paths.value)
+
+    def trace_beams_mesh(self, n, seed, max_depth=12, rr_depth=1, min_depth=0):
+        """trace_beams on the mesh scene; -> light paths traced"""
+        paths = C.c_uint64(0)
+        self._ck(self.lib.gvpm_trace_beams_mesh(self.h, n, C.c_uint64(seed), max_depth, rr_depth, min_depth,
+                                                C.byref(paths)), "gvpm_trace_beams_mesh")
+        return int(paths.value)
+
+    def generate_rays_mesh(self, camera, seed, block=32, y0=0, y1=None, epsilon=1e-4):
+        """generate_rays on the mesh scene for a look-at pinhole (records.lookat_camera)"""
+        y1 = camera.film_h if y1 is None else y1
+        self._ck(self.lib.gvpm_generate_rays_mesh(self.h, C.byref(camera), C.c_uint64(seed), block, y0, y1,
+                                                  C.c_float(epsilon)), "gvpm_generate_rays_mesh")
+        self.n_rays = camera.film_w * (y1 - y0)
+        return self.n_rays
+
     def planes_from_beams(self, seed):
         """one photon plane per beam of the current beam set, made on the device (call build_planes next)"""
         self._ck(self.lib.gvpm_planes_from_beams(self.h, C.c_uint64(seed)), "gvpm_planes_from_beams")

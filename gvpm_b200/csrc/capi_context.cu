@@ -4,6 +4,37 @@
 
 static std::string g_create_error;
 
+void triangle_planes(const float *tri, size_t n_tri, std::vector<float> &planes, std::vector<float> &aux) {
+  planes.assign(4 * n_tri, 0.f);
+  aux.assign(2 * n_tri, 0.f);
+  for (size_t t = 0; t < n_tri; ++t) {
+    const float *p = tri + 9 * t;
+    double e1[3], e2[3], n[3];
+    for (int a = 0; a < 3; ++a) { e1[a] = (double)p[3 + a] - p[a]; e2[a] = (double)p[6 + a] - p[a]; }
+    n[0] = e1[1] * e2[2] - e1[2] * e2[1];
+    n[1] = e1[2] * e2[0] - e1[0] * e2[2];
+    n[2] = e1[0] * e2[1] - e1[1] * e2[0];
+    double len = std::sqrt(n[0] * n[0] + n[1] * n[1] + n[2] * n[2]);
+    {
+      // rounding slack of the strict ray-triangle parameter (bre_device.cuh occluded()): ~16 eps * |e1||e2|/|e1 x e2|
+      // per unit of |o - p0| / |n.d|; aux = (that coefficient, largest |vertex coordinate|)
+      const double l1 = std::sqrt(e1[0] * e1[0] + e1[1] * e1[1] + e1[2] * e1[2]),
+                   l2 = std::sqrt(e2[0] * e2[0] + e2[1] * e2[1] + e2[2] * e2[2]);
+      double vmag = 0;
+      for (int a = 0; a < 9; ++a) vmag = std::max(vmag, (double)std::fabs(p[a]));
+      aux[2 * t] = (float)(len > 0 ? 2e-6 * (l1 * l2 / len) : 0.0);
+      aux[2 * t + 1] = (float)vmag;
+    }
+    if (len > 0) {
+      for (int a = 0; a < 3; ++a) n[a] /= len;
+      planes[4 * t] = (float)n[0]; planes[4 * t + 1] = (float)n[1]; planes[4 * t + 2] = (float)n[2];
+      planes[4 * t + 3] = (float)(-(n[0] * p[0] + n[1] * p[1] + n[2] * p[2]));
+    } else {
+      planes[4 * t] = planes[4 * t + 1] = planes[4 * t + 2] = planes[4 * t + 3] = 0.f;  // never culled
+    }
+  }
+}
+
 extern "C" {
 
 int gvpm_abi_version(void) { return GVPM_ABI_VERSION; }
@@ -153,33 +184,8 @@ int gvpm_set_occluders(gvpm_ctx *ctx, const float *tri_xyz, size_t n_tri) {
   ctx->occ_built = false;
   ++ctx->state_gen;
   if (n_tri == 0) return GVPM_OK;
-  std::vector<float> planes(4 * n_tri), aux(2 * n_tri);
-  for (size_t t = 0; t < n_tri; ++t) {
-    const float *p = tri_xyz + 9 * t;
-    double e1[3], e2[3], n[3];
-    for (int a = 0; a < 3; ++a) { e1[a] = (double)p[3 + a] - p[a]; e2[a] = (double)p[6 + a] - p[a]; }
-    n[0] = e1[1] * e2[2] - e1[2] * e2[1];
-    n[1] = e1[2] * e2[0] - e1[0] * e2[2];
-    n[2] = e1[0] * e2[1] - e1[1] * e2[0];
-    double len = std::sqrt(n[0] * n[0] + n[1] * n[1] + n[2] * n[2]);
-    {
-      // rounding slack of the strict ray-triangle parameter (bre_device.cuh occluded()): ~16 eps * |e1||e2|/|e1 x e2|
-      // per unit of |o - p0| / |n.d|; aux = (that coefficient, largest |vertex coordinate|)
-      const double l1 = std::sqrt(e1[0] * e1[0] + e1[1] * e1[1] + e1[2] * e1[2]),
-                   l2 = std::sqrt(e2[0] * e2[0] + e2[1] * e2[1] + e2[2] * e2[2]);
-      double vmag = 0;
-      for (int a = 0; a < 9; ++a) vmag = std::max(vmag, (double)std::fabs(p[a]));
-      aux[2 * t] = (float)(len > 0 ? 2e-6 * (l1 * l2 / len) : 0.0);
-      aux[2 * t + 1] = (float)vmag;
-    }
-    if (len > 0) {
-      for (int a = 0; a < 3; ++a) n[a] /= len;
-      planes[4 * t] = (float)n[0]; planes[4 * t + 1] = (float)n[1]; planes[4 * t + 2] = (float)n[2];
-      planes[4 * t + 3] = (float)(-(n[0] * p[0] + n[1] * p[1] + n[2] * p[2]));
-    } else {
-      planes[4 * t] = planes[4 * t + 1] = planes[4 * t + 2] = planes[4 * t + 3] = 0.f;  // never culled
-    }
-  }
+  std::vector<float> planes, aux;
+  triangle_planes(tri_xyz, n_tri, planes, aux);
   CK(ctx->tri.reserve(9 * n_tri * sizeof(float)));
   CK(ctx->tri_plane.reserve(4 * n_tri * sizeof(float)));
   CK(ctx->tri_aux.reserve(2 * n_tri * sizeof(float)));

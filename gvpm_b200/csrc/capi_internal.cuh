@@ -85,9 +85,14 @@ cudaError_t launch_vpm_shade(const GatherParams &P, unsigned long long total, in
 void launch_gradient(const float *acc, int w, int h, int use_abs, float *thr, float *gx, float *gy,
                      cudaStream_t st, int reuse = 0, float inv_emitted = 1.f);
 void launch_generate_rays(const RayGenParams &P, cudaStream_t st);
+void launch_generate_rays(const MeshRayGenParams &P, cudaStream_t st);
 void launch_trace_count(const TraceParams &P, bool beams, uint8_t *counts, unsigned long long *block_tot,
                         unsigned long long *totals, cudaStream_t st);
+void launch_trace_count(const MeshTraceParams &P, bool beams, uint8_t *counts, unsigned long long *block_tot,
+                        unsigned long long *totals, cudaStream_t st);
 void launch_trace_emit(const TraceParams &P, bool beams, const uint8_t *counts, const unsigned long long *block_off,
+                       unsigned long long *last_path, cudaStream_t st);
+void launch_trace_emit(const MeshTraceParams &P, bool beams, const uint8_t *counts, const unsigned long long *block_off,
                        unsigned long long *last_path, cudaStream_t st);
 void launch_planes_from_beams(const PlaneGenParams &P, cudaStream_t st);
 void launch_pack_beams(const BeamStaging &S, uint32_t n, float4 *rec, float *len, cudaStream_t st);
@@ -173,6 +178,17 @@ struct gvpm_ctx {
   bool occ_built = false;            // occ_nodes holds the BVH of the current set
   uint32_t n_occ_nodes = 0;
   DevBuf occ_nodes, occ_scratch, occ_query;   // BVH nodes; build scratch; gvpm_occluded's rays and hits
+
+  // mesh scene of gvpm_set_trace_mesh (capi_photons.cu): triangles, planes, slack terms, albedos and the caller's index
+  // of each, in the leaf order of its BVH (build_mesh_bvh); emit = the emissive triangles' vertices, triangle indices
+  // and area running sum, back to back
+  struct TraceMesh {
+    bool ready = false;
+    uint32_t n_tri = 0, n_nodes = 0, n_emit = 0, emit_last = 0;
+    float emit_total = 0.f, lo[3] = {}, hi[3] = {}, light_power = 0.f;
+    size_t emit_idx_off = 0, emit_cdf_off = 0;
+    DevBuf tri, plane, aux, albedo, perm, nodes, emit, albedo_in;
+  } mesh;
 
   DevBuf ph_staging, ph_staging_alt;  // the selected photon staging buffer and the other one (double buffering)
   int ph_staging_sel = 0;
@@ -446,7 +462,16 @@ int check_scene(gvpm_ctx *ctx, const gvpm_box_scene *s);
 // occluder BVH (occluder_bvh.cu): whether the gathers walk it, building it for the current set (n_tri > 0), the
 // occluder fields of a gather's parameters, and the any-hit of gvpm_occluded on rays already on the device
 bool occluder_use_bvh(const gvpm_ctx *ctx);
+int build_tri_bvh(gvpm_ctx *ctx, DevBuf &tri, DevBuf &plane, DevBuf &aux, uint32_t n, DevBuf &nodes, uint32_t *n_nodes,
+                  DevBuf *perm);
 int build_occluder_bvh(gvpm_ctx *ctx);
+// the mesh scene's BVH over ctx->mesh.tri / plane / aux (n_tri set, in the caller's order), then its albedos
+// (ctx->mesh.albedo_in, the caller's order) into leaf order
+int build_mesh_bvh(gvpm_ctx *ctx);
+MeshScene mesh_view(const gvpm_ctx *ctx);   // the device view of ctx->mesh (capi_photons.cu)
+// plane (unit normal, offset; zeros for a zero-area triangle) and rounding-slack terms (coefficient, largest |vertex
+// coordinate|) of each triangle, as the BVH walks and their culls read them
+void triangle_planes(const float *tri, size_t n_tri, std::vector<float> &planes, std::vector<float> &aux);
 void occluder_params(const gvpm_ctx *ctx, GatherParams &P);
 void launch_occluded(const GatherParams &P, bool bvh, const float *o, const float *d, const float *mint, const float *maxt,
                      uint32_t n, uint8_t *hit, cudaStream_t st);

@@ -1,4 +1,6 @@
 // capi_photons.cu — photon staging and upload, peer exchange of photon slices, on-device photon and beam tracing.
+#include <type_traits>
+
 #include "capi_internal.cuh"
 
 // A new photon set replaces the old one: staged (direct = false), traced straight into the gather records, or
@@ -243,16 +245,26 @@ int gvpm_box_scene_default(gvpm_box_scene *s) {
   return GVPM_OK;
 }
 
+}  // extern "C"
+
 // The checks every tracer shares and the walk parameters of the medium: a non-zero return is the error to report.
+// `scene` is the box (Params = TraceParams) or null (the mesh scene of gvpm_set_trace_mesh).
+template <class Params>
 static int trace_setup(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
-                       int min_depth, TraceParams &P) {
-  if (!ctx || !scene || n > 0xfffffff0u) return GVPM_ERR_INVALID;
+                       int min_depth, Params &P) {
+  constexpr bool mesh = std::is_same<Params, MeshTraceParams>::value;
+  if (!ctx || (!mesh && !scene) || n > 0xfffffff0u) return GVPM_ERR_INVALID;
   if (!ctx->have_medium) return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_medium first");
   cudaSetDevice(ctx->device);
-  int rc = check_scene(ctx, scene);
-  if (rc) return rc;
-  P = TraceParams{};
-  P.scene = *scene;
+  P = Params{};
+  if constexpr (mesh) {
+    if (!ctx->mesh.ready) return fail(ctx, GVPM_ERR_INVALID, "no mesh scene: gvpm_set_trace_mesh first");
+    P.scene = mesh_view(ctx);
+  } else {
+    int rc = check_scene(ctx, scene);
+    if (rc) return rc;
+    P.scene = *scene;
+  }
   P.sigma_s = ctx->medium.sigma_s[0];
   P.sigma_a = ctx->medium.sigma_a[0];
   P.hg_g = ctx->medium.hg_g;
@@ -269,7 +281,8 @@ static int trace_setup(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uin
 // sized from the records-per-path ratio seen so far (`per_path`, updated); `barren` is the error when 64 batches do not
 // fill the set.  n_paths: paths up to and including the
 // one that stored the last record.
-static int trace_batches(gvpm_ctx *ctx, TraceParams &P, bool beams, double &per_path, const char *barren,
+template <class Params>
+static int trace_batches(gvpm_ctx *ctx, Params &P, bool beams, double &per_path, const char *barren,
                          uint64_t *n_paths) {
   const unsigned long long n = P.n_total;
   cudaStream_t st = ctx->stream;
@@ -308,9 +321,10 @@ static int trace_batches(gvpm_ctx *ctx, TraceParams &P, bool beams, double &per_
   return GVPM_OK;
 }
 
+template <class Params>
 static int trace_impl(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
                       int min_depth, uint64_t *n_paths, bool direct) {
-  TraceParams P;
+  Params P;
   int rc = trace_setup(ctx, scene, n, seed, max_depth, rr_depth, min_depth, P);
   if (rc) return rc;
   void *dev = nullptr;
@@ -332,21 +346,13 @@ static int trace_impl(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint
                        "gvpm_trace_photons: the light paths store (almost) no photon in this scene", n_paths);
 }
 
-int gvpm_trace_photons(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
-                       int min_depth, uint64_t *n_paths) {
-  return trace_impl(ctx, scene, n, seed, max_depth, rr_depth, min_depth, n_paths, false);
-}
-int gvpm_trace_photons_direct(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth,
-                              int rr_depth, int min_depth, uint64_t *n_paths) {
-  return trace_impl(ctx, scene, n, seed, max_depth, rr_depth, min_depth, n_paths, true);
-}
-
-int gvpm_trace_beams(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
-                     int min_depth, uint64_t *n_paths) {
+template <class Params>
+static int trace_beams_impl(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth,
+                            int rr_depth, int min_depth, uint64_t *n_paths) {
   if (ctx && max_depth > 255)   // per-path counts are bytes: a path stores at most max_depth - 1 beams
     return fail(ctx, GVPM_ERR_INVALID, "gvpm_trace_beams: max_depth must be <= 255");
   if (n > 0x0ffffff0u) return GVPM_ERR_INVALID;   // the bound of gvpm_upload_beams
-  TraceParams P;
+  Params P;
   int rc = trace_setup(ctx, scene, n, seed, max_depth, rr_depth, min_depth, P);
   if (rc) return rc;
   rc = begin_beam_set(ctx, n);
@@ -359,6 +365,152 @@ int gvpm_trace_beams(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint6
                      "gvpm_trace_beams: the light paths store (almost) no beam in this scene", n_paths);
   if (rc) return rc;
   return commit_beams(ctx, nullptr);
+}
+
+// ---- mesh scene (gvpm_set_trace_mesh) -------------------------------------------------------------------------------
+// the box grown by 2e-6 of its extent (MeshScene::glo / ghi), each operation rounded on its own
+__attribute__((optimize("fp-contract=off"))) static void grown_box(float lo, float hi, float &glo, float &ghi) {
+  const float m = 2e-6f * (hi - lo);
+  glo = lo - m;
+  ghi = hi + m;
+}
+
+MeshScene mesh_view(const gvpm_ctx *ctx) {
+  const gvpm_ctx::TraceMesh &M = ctx->mesh;
+  MeshScene V{};
+  V.tri = M.tri.as<float>();
+  V.plane = M.plane.as<float4>();
+  V.aux = M.aux.as<float2>();
+  V.albedo = M.albedo.as<float>();
+  V.perm = M.perm.as<uint32_t>();
+  V.nodes = M.nodes.as<float4>();
+  V.n_tri = M.n_tri;
+  V.n_nodes = M.n_nodes;
+  V.emit_tri = M.emit.as<float>();
+  V.emit_idx = (const uint32_t *)(M.emit.as<char>() + M.emit_idx_off);
+  V.emit_cdf = (const float *)(M.emit.as<char>() + M.emit_cdf_off);
+  V.n_emit = M.n_emit;
+  V.emit_last = M.emit_last;
+  V.emit_total = M.emit_total;
+  for (int a = 0; a < 3; ++a) { V.lo[a] = M.lo[a]; V.hi[a] = M.hi[a]; grown_box(M.lo[a], M.hi[a], V.glo[a], V.ghi[a]); }
+  V.light_power = M.light_power;
+  return V;
+}
+
+// area of a triangle in fp32, each operation rounded on its own in this order (the CPU restatement forms the same)
+__attribute__((optimize("fp-contract=off"))) static float triangle_area(const float *p) {
+  const float e1x = p[3] - p[0], e1y = p[4] - p[1], e1z = p[5] - p[2];
+  const float e2x = p[6] - p[0], e2y = p[7] - p[1], e2z = p[8] - p[2];
+  const float cx = e1y * e2z - e1z * e2y, cy = e1z * e2x - e1x * e2z, cz = e1x * e2y - e1y * e2x;
+  return 0.5f * std::sqrt((cx * cx + cy * cy) + cz * cz);
+}
+
+static int set_trace_mesh(gvpm_ctx *ctx, const gvpm_mesh_scene *s) {
+  if (!s) return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: null scene");
+  const size_t n = s->n_tri;
+  if (n > GVPM_MAX_OCCLUDERS) return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: more than 2^24 triangles");
+  if (n && (!s->tri || !s->albedo || !s->emissive))
+    return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: null tri, albedo or emissive array");
+  float tol[3];
+  for (int a = 0; a < 3; ++a) {
+    if (!std::isfinite(s->lo[a]) || !std::isfinite(s->hi[a]))
+      return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: the box is not finite");
+    if (!(s->lo[a] < s->hi[a])) return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: empty box");
+    tol[a] = 1e-6f * (s->hi[a] - s->lo[a]);
+  }
+  if (!std::isfinite(s->light_power)) return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: light_power is not finite");
+  std::vector<float> etri;
+  std::vector<uint32_t> eidx;
+  std::vector<float> ecdf;
+  float total = 0.f;
+  uint32_t last = 0;
+  bool any = false;
+  for (size_t t = 0; t < n; ++t) {
+    const float *p = s->tri + 9 * t;
+    for (int k = 0; k < 9; ++k) {
+      const int a = k % 3;
+      if (!std::isfinite(p[k]))
+        return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: triangle " + std::to_string(t) + " has a non-finite coordinate");
+      if (p[k] < s->lo[a] - tol[a] || p[k] > s->hi[a] + tol[a])
+        return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: triangle " + std::to_string(t) + " lies outside the box");
+    }
+    for (int c = 0; c < 3; ++c)
+      if (!std::isfinite(s->albedo[3 * t + c]))
+        return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: triangle " + std::to_string(t) + " has a non-finite albedo");
+    if (!s->emissive[t]) continue;
+    const float area = triangle_area(p);
+    total = total + area;
+    if (area > 0.f) { last = (uint32_t)eidx.size(); any = true; }
+    etri.insert(etri.end(), p, p + 9);
+    eidx.push_back((uint32_t)t);
+    ecdf.push_back(total);
+  }
+  if (!any) return fail(ctx, GVPM_ERR_INVALID, "gvpm_set_trace_mesh: no emissive triangle of positive area");
+  gvpm_ctx::TraceMesh &M = ctx->mesh;
+  std::vector<float> planes, aux;
+  triangle_planes(s->tri, n, planes, aux);
+  cudaStream_t st = ctx->stream;
+  CK(M.tri.reserve(36 * n));
+  CK(M.plane.reserve(16 * n));
+  CK(M.aux.reserve(8 * n));
+  CK(M.albedo.reserve(12 * n));
+  CK(M.albedo_in.reserve(12 * n));
+  const size_t m = eidx.size();
+  M.emit_idx_off = align256(36 * m);
+  M.emit_cdf_off = M.emit_idx_off + align256(4 * m);
+  CK(M.emit.reserve(M.emit_cdf_off + 4 * m));
+  CK(cudaMemcpyAsync(M.tri.p, s->tri, 36 * n, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(M.plane.p, planes.data(), 16 * n, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(M.aux.p, aux.data(), 8 * n, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(M.albedo_in.p, s->albedo, 12 * n, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(M.emit.p, etri.data(), 36 * m, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(M.emit.as<char>() + M.emit_idx_off, eidx.data(), 4 * m, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(M.emit.as<char>() + M.emit_cdf_off, ecdf.data(), 4 * m, cudaMemcpyHostToDevice, st));
+  CK(cudaStreamSynchronize(st));
+  M.n_tri = (uint32_t)n;
+  const int rc = build_mesh_bvh(ctx);
+  if (rc) return rc;
+  M.n_emit = (uint32_t)m;
+  M.emit_last = last;
+  M.emit_total = total;
+  for (int a = 0; a < 3; ++a) { M.lo[a] = s->lo[a]; M.hi[a] = s->hi[a]; }
+  M.light_power = s->light_power;
+  M.ready = true;
+  return GVPM_OK;
+}
+
+extern "C" {
+
+int gvpm_trace_photons(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
+                       int min_depth, uint64_t *n_paths) {
+  return trace_impl<TraceParams>(ctx, scene, n, seed, max_depth, rr_depth, min_depth, n_paths, false);
+}
+int gvpm_trace_photons_direct(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth,
+                              int rr_depth, int min_depth, uint64_t *n_paths) {
+  return trace_impl<TraceParams>(ctx, scene, n, seed, max_depth, rr_depth, min_depth, n_paths, true);
+}
+int gvpm_trace_beams(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint64_t seed, int max_depth, int rr_depth,
+                     int min_depth, uint64_t *n_paths) {
+  return trace_beams_impl<TraceParams>(ctx, scene, n, seed, max_depth, rr_depth, min_depth, n_paths);
+}
+
+int gvpm_set_trace_mesh(gvpm_ctx *ctx, const gvpm_mesh_scene *scene) {
+  if (!ctx) return GVPM_ERR_INVALID;
+  cudaSetDevice(ctx->device);
+  ctx->mesh.ready = false;   // a failed call leaves no mesh scene
+  return set_trace_mesh(ctx, scene);
+}
+int gvpm_trace_photons_mesh(gvpm_ctx *ctx, size_t n, uint64_t seed, int max_depth, int rr_depth, int min_depth,
+                            uint64_t *n_paths) {
+  return trace_impl<MeshTraceParams>(ctx, nullptr, n, seed, max_depth, rr_depth, min_depth, n_paths, false);
+}
+int gvpm_trace_photons_direct_mesh(gvpm_ctx *ctx, size_t n, uint64_t seed, int max_depth, int rr_depth, int min_depth,
+                                   uint64_t *n_paths) {
+  return trace_impl<MeshTraceParams>(ctx, nullptr, n, seed, max_depth, rr_depth, min_depth, n_paths, true);
+}
+int gvpm_trace_beams_mesh(gvpm_ctx *ctx, size_t n, uint64_t seed, int max_depth, int rr_depth, int min_depth,
+                          uint64_t *n_paths) {
+  return trace_beams_impl<MeshTraceParams>(ctx, nullptr, n, seed, max_depth, rr_depth, min_depth, n_paths);
 }
 
 }  // extern "C"

@@ -103,3 +103,74 @@ int gvpm_generate_rays(gvpm_ctx *ctx, const gvpm_box_scene *scene, const gvpm_pi
 }
 
 }  // extern "C"
+
+// The look-at frame: f = normalize(forward), r = normalize(cross(up, f)), u = cross(f, r), each operation rounded on its own
+// in this order (the CPU restatement forms the same).  False when forward is zero or parallel to up.
+__attribute__((optimize("fp-contract=off"))) static bool lookat_frame(const gvpm_lookat_camera &c, LookatCam &L) {
+  auto unit = [](float &x, float &y, float &z) {
+    const float l = std::sqrt((x * x + y * y) + z * z);
+    if (!(l > 0.f) || !std::isfinite(l)) return false;
+    const float il = 1.0f / l;
+    x = x * il; y = y * il; z = z * il;
+    return true;
+  };
+  float f[3] = {c.forward[0], c.forward[1], c.forward[2]};
+  if (!unit(f[0], f[1], f[2])) return false;
+  float r[3] = {c.up[1] * f[2] - c.up[2] * f[1], c.up[2] * f[0] - c.up[0] * f[2], c.up[0] * f[1] - c.up[1] * f[0]};
+  if (!unit(r[0], r[1], r[2])) return false;
+  const float u[3] = {f[1] * r[2] - f[2] * r[1], f[2] * r[0] - f[0] * r[2], f[0] * r[1] - f[1] * r[0]};
+  for (int a = 0; a < 3; ++a) { L.pos[a] = c.pos[a]; L.f[a] = f[a]; L.r[a] = r[a]; L.u[a] = u[a]; }
+  return true;
+}
+
+extern "C" {
+
+int gvpm_generate_rays_mesh(gvpm_ctx *ctx, const gvpm_lookat_camera *cam, uint64_t seed, int block, int y0, int y1,
+                            float epsilon) {
+  if (!ctx || !cam) return GVPM_ERR_INVALID;
+  cudaSetDevice(ctx->device);
+  if (!ctx->mesh.ready) return fail(ctx, GVPM_ERR_INVALID, "no mesh scene: gvpm_set_trace_mesh first");
+  const bool zorder = block < 0;
+  const int bs = zorder ? -block : block;
+  if (bs < 1 || bs > 32 || (zorder && (bs & (bs - 1)))) return fail(ctx, GVPM_ERR_INVALID, "block must be in [1, 32] (a power of two for Z-order)");
+  if (cam->film_w <= 0 || cam->film_h <= 0 || y0 < 0 || y1 > cam->film_h || y0 > y1)
+    return fail(ctx, GVPM_ERR_INVALID, "bad film size / row range");
+  if (!(cam->tan_half_fov_x > 0.f) || !std::isfinite(cam->tan_half_fov_x))
+    return fail(ctx, GVPM_ERR_INVALID, "gvpm_lookat_camera: tan_half_fov_x must be positive and finite");
+  MeshRayGenParams P{};
+  for (int a = 0; a < 3; ++a)
+    if (!std::isfinite(cam->pos[a])) return fail(ctx, GVPM_ERR_INVALID, "gvpm_lookat_camera: pos is not finite");
+  if (!lookat_frame(*cam, P.cam))
+    return fail(ctx, GVPM_ERR_INVALID, "gvpm_lookat_camera: forward is zero or parallel to up");
+  const gvpm_ctx::TraceMesh &M = ctx->mesh;
+  bool inside = true;
+  for (int a = 0; a < 3; ++a) inside = inside && cam->pos[a] > M.lo[a] && cam->pos[a] < M.hi[a];
+  P.cam.tan_half_fov_x = cam->tan_half_fov_x;
+  P.cam.film_w = cam->film_w;
+  P.cam.film_h = cam->film_h;
+  P.cam.inside_medium = inside ? 1 : 0;
+  const size_t n = (size_t)cam->film_w * (size_t)(y1 - y0);
+  void *dev = nullptr;
+  int rc = gvpm_ray_staging(ctx, n, &dev, nullptr);
+  if (rc) return rc;
+  if (n) {
+    P.scene = mesh_view(ctx);
+    P.seed = seed;
+    P.block = bs;
+    P.zorder = zorder ? 1 : 0;
+    P.y0 = y0;
+    P.y1 = y1;
+    P.epsilon = epsilon;
+    writable_view<RaySoA>(P.o, staging_ptrs<RaySoA>(dev, n));
+    launch_generate_rays(P, ctx->stream);
+    ctx->launches += 1;
+    CK(cudaGetLastError());
+  }
+  rc = gvpm_commit_rays(ctx);
+  if (rc) return rc;
+  ctx->pixel_rays_gen = ctx->rays_gen;   // one ray per pixel of rows [y0, y1): gvpm_accum_add needs no sort
+  // the ray fit of the perspective grid is measured on the device (analyse_rays), as for uploaded rays
+  return GVPM_OK;
+}
+
+}  // extern "C"

@@ -1,5 +1,7 @@
 // generate.cu — the two host stages on either side of the gather, on the device (SURVEY.md §8 rows f-1, f-2), for the
-// box scene class of include/gvpm_b200.h (gvpm_box_scene):
+// box scene class of include/gvpm_b200.h (gvpm_box_scene) and the mesh scene class (gvpm_mesh_scene: triangles in the
+// medium's box, walked through their BVH by closest_hit_bvh).  The walk, the camera rays and their kernels are
+// templates on the scene (its parameter struct); the box instantiations are the code they were before the mesh existed:
 //   k_generate_rays   camera-ray medium segments + 4 offset segments of a pinhole sensor: what GatherPointMap::generate
 //                     (gvpm/gvpm_gatherpoint.h:259-486), ShiftGatherPoint::generate (gvpm/shift/shift_cameraPath.h:146-413)
 //                     and sensorMIS (gvpm_struct.h:608-631) produce per pixel, written straight into the ray staging
@@ -19,8 +21,11 @@
 // Random numbers: PCG32 keyed by (seed, pixel index) / (seed, path index) / (seed ^ constant, beam or ray index).  Arithmetic: strictly rounded fp32 in a fixed
 // operation order; log, exp, sin and cos are polynomial routines (pm_*) built from +, -, *, / only, so a CPU
 // restatement compiled without FMA contraction reproduces every record bit for bit (tests/test_gpu_generate.py).
+#include <type_traits>
+
 #include "gvpm_device.cuh"
 #include "launch_sizing.cuh"
+#include "occluder_device.cuh"
 #include "warp_ops.cuh"
 
 namespace gvpm {
@@ -99,6 +104,7 @@ __device__ __forceinline__ void pm_sincos2pi(float u, float &sn, float &cs) {   
 
 // ---- scene ---------------------------------------------------------------------------------------------------------
 struct SceneHit { sf t; v3 n, albedo; bool escaped; };
+struct MeshSceneHit : SceneHit { uint32_t tri; };   // tri: the triangle hit (caller's index)
 __device__ __forceinline__ float comp(const v3 &a, int axis) { return axis == 0 ? a.x.v : (axis == 1 ? a.y.v : a.z.v); }
 // nearest of the five walls, the open face and the rectangles, in this order (ties keep the earlier one)
 __device__ __forceinline__ SceneHit intersect_scene(const gvpm_box_scene &S, v3 o, v3 d) {
@@ -138,8 +144,96 @@ __device__ __forceinline__ SceneHit intersect_scene(const gvpm_box_scene &S, v3 
   return h;
 }
 __device__ __forceinline__ v3 unit(v3 a) { return a * (sf(1.0f) / length(a)); }
+// the box has no triangles to skip
+__device__ __forceinline__ SceneHit intersect_scene(const gvpm_box_scene &S, v3 o, v3 d, uint32_t) {
+  return intersect_scene(S, o, d);
+}
+
+// ---- mesh scene (gvpm_set_trace_mesh) -----------------------------------------------------------------------------------
+// parameter of the exit of a ray from inside the box lo / hi: the nearest of the three far planes, strictly rounded
+__device__ __forceinline__ sf box_exit(const float *lo, const float *hi, v3 o, v3 d) {
+  sf t(INFINITY);
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    const float dc = comp(d, a);
+    if (dc == 0.f) continue;
+    const sf ta = (sf(dc > 0.f ? hi[a] : lo[a]) - sf(comp(o, a))) / sf(dc);
+    if (ta < t) t = ta;
+  }
+  return t;
+}
+// winding normal of the triangle at leaf slot s / of 9 floats
+__device__ __forceinline__ v3 tri_normal(const float *p) {
+  const v3 p0(p[0], p[1], p[2]), p1(p[3], p[4], p[5]), p2(p[6], p[7], p[8]);
+  return unit(cross(p1 - p0, p2 - p0));
+}
+// the nearest triangle (closest_hit_bvh, never `skip`) up to the exit of the grown box, else the box exit (escaped):
+// a triangle at t <= t_exit wins, and so does one on a face of the box that rounding puts just beyond it
+__device__ __forceinline__ MeshSceneHit intersect_scene(const MeshScene &M, v3 o, v3 d, uint32_t skip) {
+  const sf texit = box_exit(M.lo, M.hi, o, d);
+  const MeshHit c = closest_hit_bvh(M, o, d, box_exit(M.glo, M.ghi, o, d), skip);
+  MeshSceneHit h;
+  h.tri = c.idx;
+  if (c.slot == kMeshNone) {
+    h.t = texit; h.escaped = true;
+    h.n = v3(0.f, 0.f, 0.f); h.albedo = v3(0.f, 0.f, 0.f);
+    return h;
+  }
+  h.t = sf(c.t);
+  h.escaped = false;
+  const v3 n = tri_normal(M.tri + 9 * (size_t)c.slot);
+  h.n = dot(n, d).v > 0.f ? -n : n;   // facing the incoming ray
+  const float *a = M.albedo + 3 * (size_t)c.slot;
+  h.albedo = v3(a[0], a[1], a[2]);
+  return h;
+}
 
 // ---- f-2: camera rays --------------------------------------------------------------------------------------------------
+__device__ __forceinline__ bool make_ray(const MeshRayGenParams &P, sf tx, sf ty, sf sx, sf sy, v3 &ro, v3 &rd, sf &rl) {
+  const MeshScene &M = P.scene;
+  const LookatCam &C = P.cam;
+  const sf w((float)C.film_w), h((float)C.film_h);
+  const sf x = ((sx / w - sf(0.5f)) * sf(2.f)) * tx, y = ((sy / h - sf(0.5f)) * sf(2.f)) * ty;
+  const v3 r(C.r[0], C.r[1], C.r[2]), u(C.u[0], C.u[1], C.u[2]), f(C.f[0], C.f[1], C.f[2]);
+  const v3 dir = unit((r * x + u * y) + f);
+  const v3 cam(C.pos[0], C.pos[1], C.pos[2]);
+  rd = dir;
+  if (C.inside_medium) {
+    ro = cam;
+  } else {
+    // slab test: the entry face is the axis of the largest near parameter (the first such axis on ties)
+    sf tIn(-INFINITY), tOut(INFINITY);
+    int face = -1;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      const float dc = comp(dir, a), oc = comp(cam, a);
+      if (dc == 0.f) {
+        if (oc < M.lo[a] || oc > M.hi[a]) { tOut = sf(-INFINITY); }
+        continue;
+      }
+      const sf t0 = (sf(M.lo[a]) - sf(oc)) / sf(dc), t1 = (sf(M.hi[a]) - sf(oc)) / sf(dc);
+      const sf tn = t0 < t1 ? t0 : t1, tf = t0 < t1 ? t1 : t0;
+      if (tn > tIn) { tIn = tn; face = a; }
+      if (tf < tOut) tOut = tf;
+    }
+    if (face < 0 || !(tIn <= tOut) || !(tIn.v > 0.f)) { ro = cam; rl = sf(0.f); return false; }
+    ro = cam + dir * tIn;
+    const float plane = comp(dir, face) > 0.f ? M.lo[face] : M.hi[face];
+    if (face == 0) ro.x = sf(plane); else if (face == 1) ro.y = sf(plane); else ro.z = sf(plane);
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+      if (a != face && (comp(ro, a) <= M.lo[a] || comp(ro, a) >= M.hi[a])) { rl = sf(0.f); return false; }
+    // a triangle in front of the entry or on the entry face (up to the grown box's tolerance inside it) hides the
+    // medium: the bound is where the ray crosses the face moved inwards by that tolerance
+    const float inner = comp(dir, face) > 0.f ? (sf(M.lo[face]) + (sf(M.lo[face]) - sf(M.glo[face]))).v
+                                              : (sf(M.hi[face]) - (sf(M.ghi[face]) - sf(M.hi[face]))).v;
+    const sf tBlock = (sf(inner) - sf(comp(cam, face))) / sf(comp(dir, face));
+    if (closest_hit_bvh(M, cam, dir, tBlock, kMeshNone).slot != kMeshNone) { rl = sf(0.f); return false; }
+  }
+  const SceneHit hit = intersect_scene(M, ro, rd, kMeshNone);
+  rl = hit.t;
+  return hit.t.v > (sf(4.f) * sf(P.epsilon)).v;   // a segment that reaches the box exit ends there
+}
 __device__ __forceinline__ bool make_ray(const RayGenParams &P, sf tx, sf ty, sf sx, sf sy, v3 &ro, v3 &rd, sf &rl) {
   const gvpm_box_scene &S = P.scene;
   const sf w((float)P.cam.film_w), h((float)P.cam.film_h);
@@ -170,7 +264,8 @@ __device__ __forceinline__ void put3(float *dst, size_t i, v3 v) { dst[3 * i] = 
 
 // one CTA per block x block pixel block (block <= 32: 1024 threads); the pixels of a block that fall inside the image
 // are compacted in block order (row-major or Z-order), blocks follow each other row by row
-__global__ void __launch_bounds__(1024) k_generate_rays(const __grid_constant__ RayGenParams P) {
+template <class Params>
+__global__ void __launch_bounds__(1024) k_generate_rays(const __grid_constant__ Params P) {
   __shared__ uint32_t warpTot[32];
   const int w = P.cam.film_w, bs = P.block;
   const int blocksX = (w + bs - 1) / bs;
@@ -253,21 +348,47 @@ __device__ __forceinline__ sf hg_eval(sf g, sf cosWiWo) {   // phase/hg.cpp:107-
   return (sf(GVPM_INV_FOURPI) * (sf(1.f) - g * g)) / (temp * ssqrt(temp));
 }
 
+// ---- emitter sample of the mesh scene: vertex 1 of a light path; returns the triangle it lies on --------------------
+// u0 picks the first emissive triangle whose running area sum exceeds u0 * total (clamped to the last one of
+// non-zero area), u1, u2 a uniform point on it (p0 + e1 (1 - sqrt u1) + e2 u2 sqrt u1); the normal is the winding
+// normal, the side the triangle emits on
+__device__ __forceinline__ uint32_t sample_emitter(const MeshScene &M, Pcg32 &rng, v3 &pos, v3 &n) {
+  const float target = (sf(rng.uniform()) * sf(M.emit_total)).v;
+  uint32_t lo = 0, hi = M.n_emit;
+  while (lo < hi) {
+    const uint32_t mid = (lo + hi) >> 1;
+    if (M.emit_cdf[mid] > target) hi = mid; else lo = mid + 1;
+  }
+  const uint32_t k = min(lo, M.emit_last);
+  const float u1 = rng.uniform(), u2 = rng.uniform();
+  const float *p = M.emit_tri + 9 * (size_t)k;
+  const v3 p0(p[0], p[1], p[2]), e1 = v3(p[3], p[4], p[5]) - p0, e2 = v3(p[6], p[7], p[8]) - p0;
+  const sf su = ssqrt(sf(u1));
+  pos = p0 + (e1 * (sf(1.f) - su) + e2 * (sf(u2) * su));
+  n = unit(cross(e1, e2));
+  return M.emit_idx[k];
+}
+
+template <class Scene> constexpr bool kIsMesh = std::is_same<Scene, MeshScene>::value;
+
 // What a light path stores: volume photons (GPhotonMap::tryAppend) or photon beams (LTBeamMap::tryAppendLT).
 enum class EmitKind { Photons, Beams };
 
 // The walk of light path `pathIdx`.  EMIT = false: returns the number of records it would store.  EMIT = true: stores
 // them at slots first, first + 1, ... (< n_total) with path id `pid`.  The RNG draws, the arithmetic and the
 // termination do not depend on KIND; only which records are written does.
-template <EmitKind KIND, bool EMIT>
-__device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned long long pathIdx, unsigned long long first,
-                                              uint32_t pid) {
-  const gvpm_box_scene &S = P.scene;
+template <class Scene, EmitKind KIND, bool EMIT>
+__device__ __forceinline__ uint32_t walk_path(const TraceParamsT<Scene> &P, unsigned long long pathIdx,
+                                              unsigned long long first, uint32_t pid) {
+  const Scene &S = P.scene;
   Pcg32 rng(P.seed, pathIdx);
   const sf sigS(P.sigma_s), sigT = sf(P.sigma_s) + sf(P.sigma_a);
   // vertex 0 = emitter supernode (weight = power), vertex 1 = emitter sample
   v3 curPos, curN(0.f, -1.f, 0.f), curAlbedo(0.f, 0.f, 0.f), curWeight(1.f, 1.f, 1.f), prevPos(1.f, 1.f, 1.f);
-  {
+  uint32_t curTri = kMeshNone;   // the mesh triangle the current vertex lies on
+  if constexpr (kIsMesh<Scene>) {
+    curTri = sample_emitter(S, rng, curPos, curN);   // one more draw (the triangle pick) before the point's two
+  } else {   // a point of the light rectangle, normal -y
     const float u1 = rng.uniform(), u2 = rng.uniform();
     curPos = v3(sf(S.light_x0) + (sf(S.light_x1) - sf(S.light_x0)) * sf(u1), sf(S.light_y),
                 sf(S.light_z0) + (sf(S.light_z1) - sf(S.light_z0)) * sf(u2));
@@ -285,7 +406,7 @@ __device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned lon
   uint32_t appended = 0;
   const int firstStored = max(2, P.min_depth + 1), firstBeam = max(1, P.min_depth);
   for (;;) {
-    const SceneHit h = intersect_scene(S, curPos, dir);
+    const auto h = intersect_scene(S, curPos, dir, curTri);
     const sf t = (-sf(pm_log((sf(1.0f) - sf(rng.uniform())).v))) / sigT;
     const bool inMedium = t < h.t;
     const sf L = inMedium ? t : h.t;
@@ -348,6 +469,7 @@ __device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned lon
     thr = flux;
     prevPos = curPos;
     curPos = nvPos; curN = nvN; curAlbedo = nvAlbedo; curWeight = nvWeight; curType = nvType; curRr = sf(1.f);
+    if constexpr (kIsMesh<Scene>) curTri = inMedium ? kMeshNone : h.tri;
     ci = ni;
     if (ci >= P.max_depth) break;   // path length bound
     // russian roulette before sampling the next direction (vertex.cpp:291-302)
@@ -386,21 +508,21 @@ __device__ __forceinline__ uint32_t walk_path(const TraceParams &P, unsigned lon
 }
 
 // pass 1: records per path; block totals of (records, contributing paths) packed as (paths << 40 | records)
-template <EmitKind KIND>
-__global__ void __launch_bounds__(256) k_trace_count(const __grid_constant__ TraceParams P, uint8_t *__restrict__ counts,
+template <class Scene, EmitKind KIND>
+__global__ void __launch_bounds__(256) k_trace_count(const __grid_constant__ TraceParamsT<Scene> P, uint8_t *__restrict__ counts,
                                                       unsigned long long *__restrict__ block_tot) {
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
   uint32_t c = 0;
   if (k < P.n_paths) {
-    c = walk_path<KIND, false>(P, P.path_base + k, 0ull, 0u);
+    c = walk_path<Scene, KIND, false>(P, P.path_base + k, 0ull, 0u);
     counts[k] = (uint8_t)c;
   }
   const unsigned long long t = block_total<8>((unsigned long long)c | ((unsigned long long)(c ? 1u : 0u) << 40));
   if (threadIdx.x == 0) block_tot[blockIdx.x] = t;
 }
 // pass 2: the same walks, stored.  last_path[0] = 1 + index of the path that stored record n_total - 1.
-template <EmitKind KIND>
-__global__ void __launch_bounds__(256) k_trace_emit(const __grid_constant__ TraceParams P, const uint8_t *__restrict__ counts,
+template <class Scene, EmitKind KIND>
+__global__ void __launch_bounds__(256) k_trace_emit(const __grid_constant__ TraceParamsT<Scene> P, const uint8_t *__restrict__ counts,
                                                      const unsigned long long *__restrict__ block_off,
                                                      unsigned long long *__restrict__ last_path) {
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -411,7 +533,7 @@ __global__ void __launch_bounds__(256) k_trace_emit(const __grid_constant__ Trac
   const unsigned long long first = P.slot_base + (excl & ((1ull << 40) - 1ull));
   const uint32_t pid = P.path_id_base + (uint32_t)(excl >> 40);
   if (first >= P.n_total) return;
-  walk_path<KIND, true>(P, P.path_base + k, first, pid);
+  walk_path<Scene, KIND, true>(P, P.path_base + k, first, pid);
   if (first + c >= P.n_total) last_path[0] = P.path_base + k + 1ull;   // exactly one path crosses the end of the set
 }
 
@@ -565,28 +687,48 @@ __global__ void __launch_bounds__(256) k_vpm_emit(const __grid_constant__ VpmGen
 }
 
 // ---- launchers ------------------------------------------------------------------------------------------------------
-void launch_generate_rays(const RayGenParams &P, cudaStream_t st) {
+template <class Params> void generate_rays(const Params &P, cudaStream_t st) {
   const int bs = P.block;
   const int blocksX = (P.cam.film_w + bs - 1) / bs, blocksY = (P.y1 - P.y0 + bs - 1) / bs;
-  if (blocksX > 0 && blocksY > 0) k_generate_rays<<<blocksX * blocksY, 1024, 0, st>>>(P);
+  if (blocksX > 0 && blocksY > 0) k_generate_rays<Params><<<blocksX * blocksY, 1024, 0, st>>>(P);
 }
+void launch_generate_rays(const RayGenParams &P, cudaStream_t st) { generate_rays(P, st); }
+void launch_generate_rays(const MeshRayGenParams &P, cudaStream_t st) { generate_rays(P, st); }
 // counts: [n_paths] bytes; block_tot: [(n_paths + 255) / 256 + 1] words; totals: [0] batch total (paths << 40 | photons)
 // beams: the beam emission kind (b_* arrays) instead of photons
-void launch_trace_count(const TraceParams &P, bool beams, uint8_t *counts, unsigned long long *block_tot,
-                        unsigned long long *totals, cudaStream_t st) {
+template <class Scene>
+void trace_count(const TraceParamsT<Scene> &P, bool beams, uint8_t *counts, unsigned long long *block_tot,
+                 unsigned long long *totals, cudaStream_t st) {
   const uint32_t nb = (P.n_paths + 255) / 256;
   if (nb) {
-    if (beams) k_trace_count<EmitKind::Beams><<<nb, 256, 0, st>>>(P, counts, block_tot);
-    else k_trace_count<EmitKind::Photons><<<nb, 256, 0, st>>>(P, counts, block_tot);
+    if (beams) k_trace_count<Scene, EmitKind::Beams><<<nb, 256, 0, st>>>(P, counts, block_tot);
+    else k_trace_count<Scene, EmitKind::Photons><<<nb, 256, 0, st>>>(P, counts, block_tot);
   }
   k_scan_exclusive<unsigned long long, 1><<<1, 1024, 0, st>>>(block_tot, nb, totals, 0);
 }
-void launch_trace_emit(const TraceParams &P, bool beams, const uint8_t *counts, const unsigned long long *block_off,
-                       unsigned long long *last_path, cudaStream_t st) {
+template <class Scene>
+void trace_emit(const TraceParamsT<Scene> &P, bool beams, const uint8_t *counts, const unsigned long long *block_off,
+                unsigned long long *last_path, cudaStream_t st) {
   const uint32_t nb = (P.n_paths + 255) / 256;
   if (!nb) return;
-  if (beams) k_trace_emit<EmitKind::Beams><<<nb, 256, 0, st>>>(P, counts, block_off, last_path);
-  else k_trace_emit<EmitKind::Photons><<<nb, 256, 0, st>>>(P, counts, block_off, last_path);
+  if (beams) k_trace_emit<Scene, EmitKind::Beams><<<nb, 256, 0, st>>>(P, counts, block_off, last_path);
+  else k_trace_emit<Scene, EmitKind::Photons><<<nb, 256, 0, st>>>(P, counts, block_off, last_path);
+}
+void launch_trace_count(const TraceParams &P, bool beams, uint8_t *counts, unsigned long long *block_tot,
+                        unsigned long long *totals, cudaStream_t st) {
+  trace_count(P, beams, counts, block_tot, totals, st);
+}
+void launch_trace_count(const MeshTraceParams &P, bool beams, uint8_t *counts, unsigned long long *block_tot,
+                        unsigned long long *totals, cudaStream_t st) {
+  trace_count(P, beams, counts, block_tot, totals, st);
+}
+void launch_trace_emit(const TraceParams &P, bool beams, const uint8_t *counts, const unsigned long long *block_off,
+                       unsigned long long *last_path, cudaStream_t st) {
+  trace_emit(P, beams, counts, block_off, last_path, st);
+}
+void launch_trace_emit(const MeshTraceParams &P, bool beams, const uint8_t *counts, const unsigned long long *block_off,
+                       unsigned long long *last_path, cudaStream_t st) {
+  trace_emit(P, beams, counts, block_off, last_path, st);
 }
 void launch_planes_from_beams(const PlaneGenParams &P, cudaStream_t st) {
   if (P.n) k_planes_from_beams<<<(P.n + 255) / 256, 256, 0, st>>>(P);

@@ -303,9 +303,39 @@ struct SignalParams {
 struct FlagSetParams { int n; uint32_t value; uint32_t *dst[GVPM_MAX_PEERS]; };
 
 // ---- on-device generators (generate.cu) -------------------------------------------------------------------------------
-struct RayGenParams {
-  gvpm_box_scene scene;
-  gvpm_pinhole_camera cam;
+// The mesh scene of gvpm_set_trace_mesh on the device.  The triangles, their planes and slack terms (as the occluders'
+// tri_plane / tri_aux) and the albedos are in the leaf order of the scene's BVH (occluder_device.cuh layout); perm maps
+// a leaf-order slot to the caller's triangle index.  The emissive triangles are kept apart, in the caller's order.
+struct MeshScene {
+  const float *tri;
+  const float4 *plane;
+  const float2 *aux;
+  const float *albedo;
+  const uint32_t *perm;
+  const float4 *nodes;
+  uint32_t n_tri, n_nodes;
+  const float *emit_tri;        // [n_emit*9]
+  const uint32_t *emit_idx;     // [n_emit] caller's triangle index
+  const float *emit_cdf;        // [n_emit] fp32 running sum of the areas, in index order
+  uint32_t n_emit, emit_last;   // emit_last: the last emissive triangle of non-zero area
+  float emit_total;             // emit_cdf[n_emit - 1]
+  float lo[3], hi[3];
+  // the box grown by 2e-6 of its extent on each axis (twice the tolerance of gvpm_set_trace_mesh): every triangle lies
+  // inside it, so a triangle on a face of the box is found whatever the rounding of its parameter and of the exit's
+  float glo[3], ghi[3];
+  float light_power;
+};
+// gvpm_lookat_camera with its frame (right, up, forward: capi_rays.cu forms it) and the field names of
+// gvpm_pinhole_camera that k_generate_rays reads
+struct LookatCam {
+  float pos[3], r[3], u[3], f[3];
+  float tan_half_fov_x;
+  int32_t film_w, film_h;
+  int32_t inside_medium;
+};
+template <class Scene, class Cam> struct RayGenParamsT {
+  Scene scene;
+  Cam cam;
   unsigned long long seed;
   int block, zorder, y0, y1;
   float epsilon;
@@ -315,8 +345,10 @@ struct RayGenParams {
   uint8_t *off_valid;
   float *off_o, *off_d, *off_len, *off_eye, *off_sensor;
 };
-struct TraceParams {
-  gvpm_box_scene scene;
+using RayGenParams = RayGenParamsT<gvpm_box_scene, gvpm_pinhole_camera>;
+using MeshRayGenParams = RayGenParamsT<MeshScene, LookatCam>;
+template <class Scene> struct TraceParamsT {
+  Scene scene;
   float sigma_s, sigma_a, hg_g;
   int phase_type, max_depth, rr_depth, min_depth;
   unsigned long long seed, path_base;
@@ -336,6 +368,8 @@ struct TraceParams {
   uint8_t *b_parent_type, *b_end_on_surface, *b_depth;
   uint32_t *b_path_id;
 };
+using TraceParams = TraceParamsT<gvpm_box_scene>;
+using MeshTraceParams = TraceParamsT<MeshScene>;
 // photon planes from the current beam set (generate.cu k_planes_from_beams): one PCG32 stream per beam
 struct PlaneGenParams {
   BeamStaging beams;

@@ -214,8 +214,11 @@ void occluder_params(const gvpm_ctx *ctx, GatherParams &P) {
   P.n_occ_nodes = bvh ? ctx->n_occ_nodes : 0u;
 }
 
-int build_occluder_bvh(gvpm_ctx *ctx) {
-  const uint32_t n = ctx->n_tri;
+// The build of one triangle set in place: tri / plane / aux (n entries) are permuted into leaf order, the nodes written
+// to `nodes` (*n_nodes of them); perm, when given, receives the permutation (leaf slot -> index the set had before).
+// The occluders and the mesh scene each call it on their own arrays.
+int build_tri_bvh(gvpm_ctx *ctx, DevBuf &tri, DevBuf &plane, DevBuf &aux, uint32_t n, DevBuf &nodes, uint32_t *n_nodes,
+                  DevBuf *perm) {
   const uint32_t nL = (n + GVPM_OCC_LEAF - 1) / GVPM_OCC_LEAF, nI = nL - 1, nNodes = 2 * nL - 1;
   cudaStream_t st = ctx->stream;
   // scratch: centroids, keys / values in and out, sort scratch, bounds, permuted triangles, the radix tree
@@ -230,21 +233,22 @@ int build_occluder_bvh(gvpm_ctx *ctx) {
   const size_t sort_bytes = sort_temp_bytes(n);
   const size_t o_sort = carve(sort_bytes);
   CK(ctx->occ_scratch.reserve(off));
-  CK(ctx->occ_nodes.reserve((size_t)nNodes * GVPM_OCC_NODE_FLOAT4 * sizeof(float4)));
+  CK(nodes.reserve((size_t)nNodes * GVPM_OCC_NODE_FLOAT4 * sizeof(float4)));
+  if (perm) CK(perm->reserve(4ull * n));
   char *S = ctx->occ_scratch.as<char>();
   auto u32 = [&](size_t o) { return (uint32_t *)(S + o); };
   float *cen = (float *)(S + o_cen);
   const unsigned b = 256, g = (n + b - 1) / b;
-  k_occ_centroids<<<g, b, 0, st>>>(ctx->tri.as<float>(), n, cen);
+  k_occ_centroids<<<g, b, 0, st>>>(tri.as<float>(), n, cen);
   launch_bounds(cen, n, (float *)(S + o_part), (float *)(S + o_bounds), st, 3);
   launch_morton(cen, n, (float *)(S + o_bounds), u32(o_kin), u32(o_vin), st, 3);
   CK(run_sort_bits(S + o_sort, sort_bytes, u32(o_kin), u32(o_kout), u32(o_vin), u32(o_vout), n, kHilbertBits, st));
-  k_occ_permute<<<g, b, 0, st>>>(u32(o_vout), n, ctx->tri.as<float>(), ctx->tri_plane.as<float4>(),
-                                 ctx->tri_aux.as<float2>(), (float *)(S + o_tri), (float4 *)(S + o_plane),
-                                 (float2 *)(S + o_aux));
-  CK(cudaMemcpyAsync(ctx->tri.p, S + o_tri, 36ull * n, cudaMemcpyDeviceToDevice, st));
-  CK(cudaMemcpyAsync(ctx->tri_plane.p, S + o_plane, 16ull * n, cudaMemcpyDeviceToDevice, st));
-  CK(cudaMemcpyAsync(ctx->tri_aux.p, S + o_aux, 8ull * n, cudaMemcpyDeviceToDevice, st));
+  k_occ_permute<<<g, b, 0, st>>>(u32(o_vout), n, tri.as<float>(), plane.as<float4>(), aux.as<float2>(),
+                                 (float *)(S + o_tri), (float4 *)(S + o_plane), (float2 *)(S + o_aux));
+  CK(cudaMemcpyAsync(tri.p, S + o_tri, 36ull * n, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(plane.p, S + o_plane, 16ull * n, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(aux.p, S + o_aux, 8ull * n, cudaMemcpyDeviceToDevice, st));
+  if (perm) CK(cudaMemcpyAsync(perm->p, S + o_vout, 4ull * n, cudaMemcpyDeviceToDevice, st));
   CK(cudaMemsetAsync(S + o_parent, 0xff, 4ull * nL, st));
   CK(cudaMemsetAsync(S + o_lparent, 0xff, 4ull * nL, st));
   CK(cudaMemsetAsync(S + o_arrived, 0, 4ull * nL, st));
@@ -252,14 +256,46 @@ int build_occluder_bvh(gvpm_ctx *ctx) {
                                                        u32(o_parent), u32(o_lparent));
   k_occ_pos<<<(nI + nL + b - 1) / b, b, 0, st>>>(nL, u32(o_first), u32(o_split), u32(o_parent), u32(o_lparent),
                                                  u32(o_pin), u32(o_pleaf));
-  k_occ_boxes<<<(nL + b - 1) / b, b, 0, st>>>(n, nL, ctx->tri.as<float>(), ctx->tri_plane.as<float4>(),
-                                             ctx->tri_aux.as<float2>(), u32(o_first), u32(o_last), u32(o_split),
-                                             u32(o_parent), u32(o_lparent), u32(o_pin), u32(o_pleaf), u32(o_arrived),
-                                             ctx->occ_nodes.as<float4>());
+  k_occ_boxes<<<(nL + b - 1) / b, b, 0, st>>>(n, nL, tri.as<float>(), plane.as<float4>(), aux.as<float2>(), u32(o_first),
+                                             u32(o_last), u32(o_split), u32(o_parent), u32(o_lparent), u32(o_pin),
+                                             u32(o_pleaf), u32(o_arrived), nodes.as<float4>());
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(st));
   ctx->launches += 8 + (nI ? 1 : 0);
-  ctx->n_occ_nodes = nNodes;
+  *n_nodes = nNodes;
+  return GVPM_OK;
+}
+
+int build_occluder_bvh(gvpm_ctx *ctx) {
+  const int rc = build_tri_bvh(ctx, ctx->tri, ctx->tri_plane, ctx->tri_aux, ctx->n_tri, ctx->occ_nodes,
+                               &ctx->n_occ_nodes, nullptr);
+  if (rc) return rc;
   ctx->occ_built = true;
+  return GVPM_OK;
+}
+
+// the mesh scene's albedos into the leaf order of its BVH
+namespace gvpm {
+namespace {
+__global__ void k_mesh_albedo(const uint32_t *__restrict__ perm, uint32_t n, const float *__restrict__ in,
+                              float *__restrict__ out) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t s = perm[i];
+#pragma unroll
+  for (int a = 0; a < 3; ++a) out[3 * (size_t)i + a] = in[3 * (size_t)s + a];
+}
+}  // namespace
+}  // namespace gvpm
+
+int build_mesh_bvh(gvpm_ctx *ctx) {
+  gvpm_ctx::TraceMesh &M = ctx->mesh;
+  int rc = build_tri_bvh(ctx, M.tri, M.plane, M.aux, M.n_tri, M.nodes, &M.n_nodes, &M.perm);
+  if (rc) return rc;
+  k_mesh_albedo<<<(M.n_tri + 255) / 256, 256, 0, ctx->stream>>>(M.perm.as<uint32_t>(), M.n_tri,
+                                                                  M.albedo_in.as<float>(), M.albedo.as<float>());
+  CK(cudaGetLastError());
+  CK(cudaStreamSynchronize(ctx->stream));
+  ctx->launches += 1;
   return GVPM_OK;
 }

@@ -125,6 +125,103 @@ __device__ __forceinline__ bool occluded_bvh(const GatherParams &P, v3 o, v3 d, 
   return hit;
 }
 
+// ---- closest hit on the mesh scene (MeshScene, gvpm_set_trace_mesh) ------------------------------------------------------
+// occluder_hit's culls and strict test on triangle s of the mesh, returning the strict parameter tt when the test
+// accepts it in [mint, maxt], else +inf.  The culls are occluder_hit's, so they never reject a triangle whose strict tt
+// lies in [mint, maxt].
+__device__ __forceinline__ float mesh_tri_t(const MeshScene &M, uint32_t s, v3 o, v3 d, sf mint, sf maxt, float omag) {
+  const float4 pl = ldg4(M.plane + s);
+  const float sdist = pl.x * o.x.v + pl.y * o.y.v + pl.z * o.z.v + pl.w;
+  if (fabsf(sdist) > maxt.v * 1.001f + 1e-5f) return INFINITY;
+  const float nd = pl.x * d.x.v + pl.y * d.y.v + pl.z * d.z.v;
+  const float and_ = fabsf(nd);
+  if (and_ > 1e-3f) {
+    const float2 aux = __ldg(M.aux + s);
+    const float num = nd < 0.f ? sdist : -sdist;
+    const float slack = aux.x * (omag + aux.y + 1e-3f) * 1.7321f + 2e-6f * fabsf(num);
+    if (num + slack < mint.v * and_ || num - slack > maxt.v * and_) return INFINITY;
+  }
+  const float *tv = M.tri + 9 * (size_t)s;
+  v3 p0(__ldg(tv), __ldg(tv + 1), __ldg(tv + 2)), p1(__ldg(tv + 3), __ldg(tv + 4), __ldg(tv + 5)),
+      p2(__ldg(tv + 6), __ldg(tv + 7), __ldg(tv + 8));
+  v3 edge1 = p1 - p0, edge2 = p2 - p0;
+  v3 pvec = cross(d, edge2);
+  sf det = dot(edge1, pvec);
+  if (det.v == 0.f) return INFINITY;
+  sf inv_det = sf(1.f) / det;
+  v3 tvec = o - p0;
+  sf u = dot(tvec, pvec) * inv_det;
+  if (u.v < 0.f || u.v > 1.f) return INFINITY;
+  v3 qvec = cross(tvec, edge1);
+  sf v = dot(d, qvec) * inv_det;
+  if (v.v >= 0.f && (u + v).v <= 1.f) {
+    sf tt = dot(edge2, qvec) * inv_det;
+    if (tt >= mint && tt <= maxt) return tt.v;
+  }
+  return INFINITY;
+}
+
+// Closest hit: the triangle with the smallest strict tt in (1e-6, bound], ties to the smaller caller index, never the
+// triangle `skip` (the one the ray starts on); slot = kMeshNone when there is none.  The brute-force loop over all
+// triangles with the same rule gives the same answer.
+constexpr uint32_t kMeshNone = 0xffffffffu;
+struct MeshHit { float t; uint32_t slot, idx; };
+// The stackless walk of occluded_bvh with a shrinking upper bound: maxt = the best tt found so far (the box exit at
+// first).  occluded_bvh's argument holds for any interval [mint, maxt]: a node is skipped only when no triangle below
+// it can pass the culls and strict test of occluder_hit (here mesh_tri_t) with a tt in [mint, maxt].  Here the interval
+// at the time of the skip is [1e-6, B], B the best tt so far, and B only decreases: a skipped triangle has no tt in
+// [1e-6, B], so it cannot beat B, nor the final answer <= B, nor tie with it (a tie needs tt = final <= B).  The pad uses
+// T from the first bound, which is >= every later one, so it is never smaller than the argument needs.  Skipping
+// `skip` and keeping the smaller index on equal tt are decisions on triangles that the walk did reach, in any order.
+__device__ __forceinline__ MeshHit closest_hit_bvh(const MeshScene &M, v3 o, v3 d, sf bound, uint32_t skip) {
+  MeshHit best{bound.v, kMeshNone, kMeshNone};
+  const sf mint(1e-6f);
+  if (bound < mint) return best;
+  const float omag = fmaxf(fmaxf(fabsf(o.x.v), fabsf(o.y.v)), fabsf(o.z.v));
+  const float T = fmaxf(fabsf(mint.v), fabsf(bound.v));
+  const float dx = fabsf(d.x.v) < 1e-20f ? copysignf(1e-20f, d.x.v) : d.x.v;
+  const float dy = fabsf(d.y.v) < 1e-20f ? copysignf(1e-20f, d.y.v) : d.y.v;
+  const float dz = fabsf(d.z.v) < 1e-20f ? copysignf(1e-20f, d.z.v) : d.z.v;
+  const float ix = 1.f / dx, iy = 1.f / dy, iz = 1.f / dz;
+  uint32_t i = 0;
+  while (i < M.n_nodes) {
+    const float4 *nd = M.nodes + (size_t)GVPM_OCC_NODE_FLOAT4 * i;
+    const float4 a = ldg4(nd), b = ldg4(nd + 1), c = ldg4(nd + 2);
+    const uint32_t w = __float_as_uint(a.w);
+    const bool leaf = (w & GVPM_OCC_LEAF_BIT) != 0u;
+    bool enter = true;
+    float sphi, cphi;
+    __sincosf(c.w, &sphi, &cphi);
+    const float ad = fabsf(c.x * d.x.v + c.y * d.y.v + c.z * d.z.v);
+    const float cmin = ad * cphi - sqrtf(fmaxf(0.f, 1.f - ad * ad)) * sphi - 1e-5f;
+    if (cmin > 1.001e-3f) {
+      const float V = fmaxf(fmaxf(fmaxf(fabsf(a.x), fabsf(b.x)), fmaxf(fabsf(a.y), fabsf(b.y))),
+                            fmaxf(fabsf(a.z), fabsf(b.z)));
+      const float St = (b.w * 1.7321f * (omag + V + 1e-3f) / cmin + 2e-6f * T) * 1.00001f;
+      const float pad = 4.f * St + 9.5367431640625e-7f * (V + omag + T) + 1e-30f;
+      float t1 = ((a.x - pad) - o.x.v) * ix, t2 = ((b.x + pad) - o.x.v) * ix;
+      float tn = fminf(t1, t2), tf = fmaxf(t1, t2);
+      t1 = ((a.y - pad) - o.y.v) * iy; t2 = ((b.y + pad) - o.y.v) * iy;
+      tn = fmaxf(tn, fminf(t1, t2)); tf = fminf(tf, fmaxf(t1, t2));
+      t1 = ((a.z - pad) - o.z.v) * iz; t2 = ((b.z + pad) - o.z.v) * iz;
+      tn = fmaxf(tn, fminf(t1, t2)); tf = fminf(tf, fmaxf(t1, t2));
+      enter = tn <= tf && tf >= mint.v - pad && tn <= best.t + pad;
+    }
+    if (enter && leaf) {
+      const uint32_t first = w & ~GVPM_OCC_LEAF_BIT;
+      const uint32_t last = min(first + GVPM_OCC_LEAF, M.n_tri);
+      for (uint32_t s = first; s < last; ++s) {
+        const uint32_t idx = __ldg(M.perm + s);
+        if (idx == skip) continue;
+        const float tt = mesh_tri_t(M, s, o, d, mint, sf(best.t), omag);
+        if (tt > 1e-6f && (tt < best.t || (tt == best.t && idx < best.idx))) best = MeshHit{tt, s, idx};
+      }
+    }
+    i = (enter || leaf) ? i + 1 : w;
+  }
+  return best;
+}
+
 // BVH: compile-time variant of the shade kernels (the list instantiations carry none of the walk)
 template <bool BVH>
 __device__ __forceinline__ bool occluded(const GatherParams &P, v3 o, v3 d, sf mint, sf maxt) {

@@ -247,3 +247,48 @@ def pinhole_camera(w, h, cam_dist=1.5, cover=0.96):
     cam.tan_half_fov_x = np.float32(cover) if inside else np.float32(0.5) * np.float32(cover) / np.float32(cam_dist)
     cam.film_w, cam.film_h, cam.inside_medium = w, h, int(inside)
     return cam
+
+
+def lookat_camera(w, h, pos, forward=(0.0, 0.0, 1.0), up=(0.0, 1.0, 0.0), tan_half_fov_x=0.32):
+    """A pinhole with a look-at frame (gvpm_lookat_camera) for the mesh generators: forward = +z, up = +y is the frame of
+    pinhole_camera()."""
+    cam = N.LookatCamera()
+    for a in range(3):
+        cam.pos[a], cam.forward[a], cam.up[a] = float(pos[a]), float(forward[a]), float(up[a])
+    cam.tan_half_fov_x = float(np.float32(tan_half_fov_x))
+    cam.film_w, cam.film_h = w, h
+    return cam
+
+
+def box_scene_as_mesh(scene):
+    """A gvpm_box_scene as mesh-scene arrays: two triangles per wall (the open face z = lo stays open), per rectangle and
+    for the light (emissive, wound so that its normal points down, with the ceiling's albedo).  -> dict of the keyword
+    arguments of Context.set_trace_mesh."""
+    lo = np.array(scene.lo[:], dtype=np.float32)
+    hi = np.array(scene.hi[:], dtype=np.float32)
+    quads, alb, emit = [], [], []
+
+    def quad(a, b, c, d, albedo, e=0):
+        # a b c d in order around the quad: triangles (a, b, c) and (a, c, d) share its winding
+        quads.extend([(a, b, c), (a, c, d)])
+        alb.extend([albedo, albedo])
+        emit.extend([e, e])
+
+    x0, y0, z0 = lo
+    x1, y1, z1 = hi
+    fa = [tuple(scene.face_albedo[i][:]) for i in range(5)]
+    quad((x0, y0, z0), (x0, y1, z0), (x0, y1, z1), (x0, y0, z1), fa[0])   # x = lo
+    quad((x1, y0, z0), (x1, y0, z1), (x1, y1, z1), (x1, y1, z0), fa[1])   # x = hi
+    quad((x0, y0, z0), (x0, y0, z1), (x1, y0, z1), (x1, y0, z0), fa[2])   # y = lo
+    quad((x0, y1, z0), (x1, y1, z0), (x1, y1, z1), (x0, y1, z1), fa[3])   # y = hi
+    quad((x0, y0, z1), (x0, y1, z1), (x1, y1, z1), (x1, y0, z1), fa[4])   # z = hi
+    for r in range(scene.n_rects):
+        R = scene.rect[r]
+        quad((R.x0, R.y, R.z0), (R.x1, R.y, R.z0), (R.x1, R.y, R.z1), (R.x0, R.y, R.z1), tuple(R.albedo[:]))
+    ly = scene.light_y
+    # winding (x0, z0) -> (x1, z0) -> (x1, z1): the normal cross((dx, 0, 0), (dx, 0, dz)) = (0, -dx dz, 0) points down
+    quad((scene.light_x0, ly, scene.light_z0), (scene.light_x1, ly, scene.light_z0), (scene.light_x1, ly, scene.light_z1),
+         (scene.light_x0, ly, scene.light_z1), fa[3], 1)
+    tri = np.array(quads, dtype=np.float32).reshape(-1, 9)
+    return dict(tri=tri, albedo=np.array(alb, dtype=np.float32).reshape(-1, 3), emissive=np.array(emit, dtype=np.uint8),
+                light_power=float(scene.light_power), lo=lo, hi=hi)

@@ -585,8 +585,8 @@ int gvpm_reconstruct_accum(gvpm_ctx *ctx, int use_abs, const float *direct, cons
  * boundary towards the sensor: light paths leave through it, camera rays enter through it), up to 4 two-sided
  * diffuse rectangles parallel to the xz plane inside the box, and a rectangular diffuse area light on the plane
  * y = light_y pointing down (-y).  gvpm_box_scene_default() is the Cornell box of the bench / test workloads.
- * Everything else (arbitrary meshes, glossy BSDFs, other emitters) stays with the host renderer and the upload entry
- * points above. */
+ * Triangle meshes inside the medium's box have entry points of their own (gvpm_mesh_scene below); glossy BSDFs and
+ * other emitters stay with the host renderer and the upload entry points above. */
 typedef struct gvpm_box_scene {
   float lo[3], hi[3];           /* the medium's box */
   float face_albedo[5][3];      /* x = lo, x = hi, y = lo, y = hi, z = hi (z = lo is open) */
@@ -651,6 +651,66 @@ int gvpm_trace_beams(gvpm_ctx *ctx, const gvpm_box_scene *scene, size_t n, uint6
  * The context is left as gvpm_upload_planes of the same arrays leaves it: call gvpm_build_planes next.  Fails when
  * there is no beam set, no medium, or the medium's sampling_weight is not 1. */
 int gvpm_planes_from_beams(gvpm_ctx *ctx, uint64_t seed);
+
+/* ---- rows f-1 / f-2 on triangle-mesh scenes ---------------------------------------------------------------------------
+ * Scene class: the homogeneous medium of gvpm_set_medium fills the axis-aligned box lo / hi, whose boundary is
+ * index-matched everywhere (a ray that reaches it before any triangle leaves the scene: the light path ends there, a
+ * camera segment ends there).  Inside the box: n_tri triangles (tri = 9 floats each, p0 p1 p2), each with one diffuse
+ * albedo, two-sided; the shading normal is normalize(cross(p1 - p0, p2 - p0)) turned to face the incoming ray.  Every
+ * vertex must lie in the box, up to 1e-6 of the box extent on each axis.  The triangles flagged emissive (emissive[i] !=
+ * 0) are also one diffuse area light of total power light_power, emitting on the side of their winding normal only;
+ * they are surfaces too, with their own albedo (0 absorbs).
+ * Emitter sampling (a restatement, not Mitsuba's shape-sampling sequence): the areas of the emissive triangles are
+ * summed in fp32 in triangle index order on the host; a light path draws u0 and picks the first emissive triangle whose
+ * running sum exceeds u0 * total (the last emissive triangle of non-zero area when none does), then u1, u2 for the
+ * point p0 + (e1 * (1 - sqrt(u1)) + e2 * (u2 * sqrt(u1))), then the cosine direction about the winding normal as the
+ * box tracer draws it.  u0 is the only draw the box walk does not make; every later draw is the box walk's.
+ * Intersection: the nearest triangle with a strictly rounded Moller-Trumbore parameter t > 1e-6 (Triangle::rayIntersect,
+ * include/mitsuba/core/triangle.h:109-145), ties to the smaller triangle index, skipping the triangle the ray starts
+ * on, searched up to the exit of the box grown by 2e-6 of its extent (strictly rounded slab tests): a triangle wins over
+ * the box exit when t <= t_exit, and so does a wall on a face of the box that rounding puts just beyond it.  The walk
+ * goes down a BVH built on the device once per scene; its answer is that of the brute-force loop over all triangles.
+ * This scene does not change the occluders: pass the same triangles to gvpm_set_occluders for the shadow rays. */
+typedef struct gvpm_mesh_scene {
+  float lo[3], hi[3];           /* the medium's box */
+  size_t n_tri;                 /* <= GVPM_MAX_OCCLUDERS (2^24) */
+  const float *tri;             /* [n_tri*9] */
+  const float *albedo;          /* [n_tri*3] */
+  const uint8_t *emissive;      /* [n_tri] */
+  float light_power;
+} gvpm_mesh_scene;
+/* Copies the arrays to the device and builds the scene's BVH there; the mesh entries below then use it until the next
+ * call.  Fails with GVPM_ERR_INVALID (and the reason in gvpm_last_error) on a null array, an empty or non-finite box,
+ * more than 2^24 triangles, a non-finite coordinate, albedo or power, a vertex outside the box, or no emissive
+ * triangle of positive area; the context then has no mesh scene. */
+int gvpm_set_trace_mesh(gvpm_ctx *ctx, const gvpm_mesh_scene *scene);
+/* gvpm_trace_photons / gvpm_trace_photons_direct / gvpm_trace_beams on the mesh scene: the same walk, random numbers
+ * (plus the emitter pick), records, batching and limits, and the context is left as they leave it.  Fail with
+ * GVPM_ERR_INVALID when there is no mesh scene or no medium. */
+int gvpm_trace_photons_mesh(gvpm_ctx *ctx, size_t n, uint64_t seed, int max_depth, int rr_depth, int min_depth,
+                            uint64_t *n_paths);
+int gvpm_trace_photons_direct_mesh(gvpm_ctx *ctx, size_t n, uint64_t seed, int max_depth, int rr_depth, int min_depth,
+                                   uint64_t *n_paths);
+int gvpm_trace_beams_mesh(gvpm_ctx *ctx, size_t n, uint64_t seed, int max_depth, int rr_depth, int min_depth,
+                          uint64_t *n_paths);
+/* A pinhole with a look-at frame: f = normalize(forward), r = normalize(cross(up, f)), u = cross(f, r); the ray of
+ * film point (sx, sy) has direction normalize((r * x + u * y) + f) with x = ((sx / film_w - 0.5) * 2) * tan_half_fov_x,
+ * y = ((sy / film_h - 0.5) * 2) * tan_half_fov_x * film_h / film_w (forward = +z, up = +y is gvpm_pinhole_camera's
+ * frame).  A camera strictly inside the box starts its segments at pos (edge 1); one outside starts them where the ray
+ * enters the box (edge 2): the entry face is the slab test's, the entry point is snapped onto that face's plane and
+ * must lie inside the face, and no triangle may be hit before the face moved inwards by that 2e-6 margin. */
+typedef struct gvpm_lookat_camera {
+  float pos[3], forward[3], up[3];
+  float tan_half_fov_x;
+  int32_t film_w, film_h;
+} gvpm_lookat_camera;
+/* gvpm_generate_rays on the mesh scene: the same pixels, PCG32 draws, segments (ending at the nearest triangle or at
+ * the box exit), offsets, edge_id, eye_contrib and off_sensor = 1.  Fails with GVPM_ERR_INVALID without a mesh scene,
+ * on a bad block, film or row range, or a camera whose forward is zero, parallel to up, or whose field of view is not
+ * positive and finite. */
+int gvpm_generate_rays_mesh(gvpm_ctx *ctx, const gvpm_lookat_camera *cam, uint64_t seed, int block, int y0, int y1,
+                            float epsilon);
+
 /* parity aid: copy `bytes` bytes at `dev` (a pointer handed out by this library, e.g. gvpm_photon_staging /
  * gvpm_ray_staging) to host memory, after the work queued on the context's stream */
 int gvpm_read_device(gvpm_ctx *ctx, const void *dev, void *host, size_t bytes);
