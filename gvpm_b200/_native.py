@@ -105,6 +105,19 @@ class PoissonParams(C.Structure):
                 ("cg_precond", C.c_int32), ("cg_tolerance", C.c_float)]
 
 
+# gvpm_device.cuh FrustumGrid (gvpm_frustum_grid copies it out as raw bytes)
+GVPM_GRID_CLASSES = 16
+
+
+class FrustumGrid(C.Structure):
+    _fields_ = [("C", C.c_float * 3), ("m", C.c_float * 3), ("u", C.c_float * 3), ("v", C.c_float * 3),
+                ("gx0", C.c_float), ("gy0", C.c_float), ("csize", C.c_float * GVPM_GRID_CLASSES),
+                ("xmin", C.c_float), ("xmax", C.c_float), ("ymin", C.c_float), ("ymax", C.c_float), ("pad_r", C.c_float),
+                ("nx", C.c_uint32 * GVPM_GRID_CLASSES), ("ny", C.c_uint32 * GVPM_GRID_CLASSES),
+                ("base", C.c_uint32 * GVPM_GRID_CLASSES), ("n_cells", C.c_uint32), ("classes", C.c_int32),
+                ("parity_split", C.c_int32)]
+
+
 # gvpm_beam_technique (volTechnique strings of sppm.cpp:208-209)
 BEAM_TECHNIQUES = {"beam1d": 0, "beam3d_naive": 1, "beam3d_egsr": 2, "beam3d": 3}
 
@@ -113,7 +126,7 @@ ABI_SYMBOLS = [
     "gvpm_abi_version", "gvpm_ctx_create", "gvpm_ctx_destroy", "gvpm_last_error", "gvpm_sync",
     "gvpm_stream", "gvpm_set_medium", "gvpm_set_config", "gvpm_set_occluders",
     "gvpm_set_occluder_accel", "gvpm_occluder_accel_kind", "gvpm_occluded",
-    "gvpm_upload_photons", "gvpm_photon_staging", "gvpm_build_points", "gvpm_build_points_for_rays", "gvpm_accel_kind", "gvpm_set_view_direction",
+    "gvpm_upload_photons", "gvpm_photon_staging", "gvpm_build_points", "gvpm_build_points_for_rays", "gvpm_accel_kind", "gvpm_frustum_grid", "gvpm_set_view_direction",
     "gvpm_photon_staging_select", "gvpm_photon_staging_layout", "gvpm_upload_photons_slice",
     "gvpm_peer_export", "gvpm_peer_connect", "gvpm_peer_push_photon_slice", "gvpm_peer_wait_photons", "gvpm_peer_push_mode",
     "gvpm_dispatch_export", "gvpm_dispatch_connect", "gvpm_dispatch_photons", "gvpm_build_dispatched", "gvpm_dispatch_release",
@@ -168,6 +181,7 @@ def load_lib():
     lib.gvpm_build_points.argtypes = [vp, C.c_float]
     lib.gvpm_build_points_for_rays.argtypes = [vp, C.c_float, u32p]
     lib.gvpm_accel_kind.argtypes = [vp]
+    lib.gvpm_frustum_grid.argtypes = [vp, vp, C.c_size_t, u32p, C.c_size_t, C.POINTER(C.c_size_t)]
     lib.gvpm_box_scene_default.argtypes = [C.POINTER(BoxScene)]
     lib.gvpm_generate_rays.argtypes = [vp, C.POINTER(BoxScene), C.POINTER(PinholeCamera), C.c_uint64, C.c_int, C.c_int,
                                        C.c_int, C.c_float]

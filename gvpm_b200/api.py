@@ -216,6 +216,15 @@ class Context:
         """'bvh' or 'frustum': what the last point build produced"""
         return {0: "bvh", 1: "frustum"}[int(self.lib.gvpm_accel_kind(self.h))]
 
+    def frustum_grid(self):
+        """(FrustumGrid, cell_start) of the perspective grid the last build made (read-only copy, for diagnostics)"""
+        grid, n = N.FrustumGrid(), C.c_size_t(0)
+        self._ck(self.lib.gvpm_frustum_grid(self.h, C.byref(grid), C.sizeof(grid), None, 0, C.byref(n)), "gvpm_frustum_grid")
+        cell_start = np.empty(n.value, dtype=np.uint32)
+        self._ck(self.lib.gvpm_frustum_grid(self.h, None, C.sizeof(grid), cell_start.ctypes.data_as(N.u32p), n.value, None),
+                 "gvpm_frustum_grid")
+        return grid, cell_start
+
     # ---- on-device generators (rows f-1, f-2)
     def generate_rays(self, scene, camera, seed, block=32, y0=0, y1=None, epsilon=1e-4):
         """camera-ray medium segments + offsets of a pinhole sensor, generated and committed on the device"""

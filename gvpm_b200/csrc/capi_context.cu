@@ -282,6 +282,24 @@ int gvpm_staging_peek(gvpm_ctx *ctx, int which, void **dev, size_t *count) {
 
 int gvpm_accel_kind(const gvpm_ctx *ctx) { return ctx ? ctx->accel : 0; }
 
+int gvpm_frustum_grid(gvpm_ctx *ctx, void *grid, size_t grid_bytes, uint32_t *cell_start, size_t cap, size_t *n_entries) {
+  if (!ctx) return GVPM_ERR_INVALID;
+  if (grid_bytes != sizeof(FrustumGrid)) return fail(ctx, GVPM_ERR_INVALID, "grid_bytes is not sizeof(FrustumGrid)");
+  if (!ctx->built || ctx->accel != gvpm_ctx::ACCEL_FRUSTUM)
+    return fail(ctx, GVPM_ERR_INVALID, "no perspective grid built (gvpm_build_points_for_rays over concurrent rays)");
+  const FrustumGrid &G = ctx->grid;
+  const size_t n = (size_t)(G.parity_split ? 2u : 1u) * G.n_cells + 3;   // + NEAR, DROP and the end
+  if (grid) memcpy(grid, &G, sizeof(FrustumGrid));
+  if (n_entries) *n_entries = n;
+  if (cell_start) {
+    if (cap < n) return fail(ctx, GVPM_ERR_INVALID, "cell_start holds fewer than *n_entries entries");
+    cudaSetDevice(ctx->device);
+    CK(cudaMemcpyAsync(cell_start, ctx->cell_start.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+  }
+  return GVPM_OK;
+}
+
 int gvpm_set_view_direction(gvpm_ctx *ctx, const float dir[3]) {
   if (!ctx) return GVPM_ERR_INVALID;
   if (dir) {

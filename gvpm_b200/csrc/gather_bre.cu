@@ -388,11 +388,30 @@ k_bre_traverse(const __grid_constant__ GatherParams P) {
 // slot ranges per class, one per cell row), and each candidate costs one 128-bit load (neighbouring pixels read the
 // same cells: L1) plus the relaxed pre-test.  Candidate queues, the strict predicate and the pair emission are the ones
 // of k_bre_traverse (flush_candidates), so the neighbour sets are bit-identical.
+// A tile first takes a census in one round of loads: lane i tests census entry i (class i / grids, grid i % grids) over
+// the tile's window in that class, the bounding box of its lanes' 3x3 windows, and one ballot lists the entries that
+// hold a photon there.  Photon footprints are about a pixel, so most classes hold photons somewhere in the image but
+// none near a given tile; those cost nothing.  Each lane then lists the non-empty row ranges of its own windows in the
+// listed entries (and NEAR) in shared memory, kGridItems entries at a time, and walks them as one candidate stream:
+// ceil(max_lane(candidates) / kTileBatch) batches per chunk of entries, not a round of batches per class.
 #ifndef GVPM_GRID_MIN_BLOCKS
 #define GVPM_GRID_MIN_BLOCKS 6
 #endif
+#ifndef GVPM_GRID_LOADS
+#define GVPM_GRID_LOADS 4   // candidate loads a lane issues together
+#endif
+#ifndef GVPM_GRID_ITEMS
+#define GVPM_GRID_ITEMS 2   // census entries whose ranges are listed (and their row loads issued) together
+#endif
+constexpr int kGridLoads = GVPM_GRID_LOADS;
+constexpr int kGridItems = GVPM_GRID_ITEMS;
+constexpr int kGridRanges = 3 * kGridItems;   // one range per cell row of a 3x3 window (NEAR: one)
+constexpr int kCensusRows = 8;                 // a taller tile window is tested as one span of cells (conservative)
+static_assert(kTileBatch % kGridLoads == 0, "a batch is a whole number of load groups");
 struct GridShared {
   uint32_t queue[kTileQ][32];
+  // [range][lane]: slot ranges [rbeg, rend) of the lane's current chunk; two spare rows for the walk's read-ahead
+  uint32_t rbeg[kGridRanges + 2][32], rend[kGridRanges + 2][32];
 };
 template <int MODE>
 __global__ void __launch_bounds__(kTravWarps * 32, GVPM_GRID_MIN_BLOCKS)
@@ -405,11 +424,13 @@ k_bre_grid_traverse(const __grid_constant__ GatherParams P) {
   const uint32_t nTiles = (P.ray_end - P.ray_begin + 31) / 32;
   const float coordMag = __ldg(P.bounds + 6);
   const bool prefilter = !DUMP && !SPPM && P.counts == nullptr;
-  const uint32_t nGridsBuilt = G.parity_split ? 2u : 1u;
+  const uint32_t gShift = G.parity_split ? 1u : 0u, nGridsBuilt = 1u << gShift;
   const uint32_t nearBeg = __ldg(P.cell_start + nGridsBuilt * G.n_cells), nearEnd = __ldg(P.cell_start + nGridsBuilt * G.n_cells + 1);
   // with the pathSet prefilter a ray only ever pairs with photons of its pixel's parity: it scans that grid alone
   const bool onlyMine = G.parity_split && prefilter && P.cfg.path_set;
-  const uint32_t nPass = onlyMine ? 1u : nGridsBuilt;
+  const bool censusLane = (uint32_t)lane < ((uint32_t)G.classes << gShift);
+  const int censusClass = censusLane ? lane >> gShift : 0;
+  const uint32_t censusBase = ((uint32_t)lane & (nGridsBuilt - 1u)) * G.n_cells + G.base[censusClass];
   if (P.build_ovf && __ldg(P.build_ovf)) {   // incomplete grid (capi_points.cu build_frustum): report it instead of gathering
     if (blockIdx.x == 0 && threadIdx.x == 0) *P.pair_counter = 1ull << 62;
     return;
@@ -461,64 +482,117 @@ k_bre_grid_traverse(const __grid_constant__ GatherParams P) {
         x = (L.dx * G.u[0] + L.dy * G.u[1] + L.dz * G.u[2]) * iz;
         y = (L.dx * G.v[0] + L.dy * G.v[1] + L.dz * G.v[2]) * iz;
       }
-      // One loop over the footprint classes, then the NEAR bucket (photons too close to C for any class: every ray
-      // tests them), then one empty round that flushes what is left: a single copy of the candidate loop and of
-      // flush_candidates (this kernel's instruction-fetch stalls grow with its code size).
-      for (int c = 0; c <= G.classes + 1; ++c) {
-        const bool isNear = c == G.classes, isLast = c == G.classes + 1;
-        const int cc = min(c, G.classes - 1);
-        const uint32_t nx = G.nx[cc], ny = G.ny[cc], base = G.base[cc];
-        if (!isNear && !isLast) {
-          // empty class (in every grid): nothing to do (warp-uniform)
-          bool empty = true;
-          for (uint32_t g = 0; g < nGridsBuilt; ++g)
-            empty = empty && __ldg(P.cell_start + g * G.n_cells + base) == __ldg(P.cell_start + g * G.n_cells + base + nx * ny);
-          if (empty) continue;
-        }
-        int x0 = 0, x1 = 0, y0 = 0, y1 = -1;
-        if (active && !isNear && !isLast) {
-          const float ic = 1.f / G.csize[cc];
-          int cx = (int)floorf((x - G.gx0) * ic), cy = (int)floorf((y - G.gy0) * ic);
-          cx = min(max(cx, 0), (int)nx - 1);
-          cy = min(max(cy, 0), (int)ny - 1);
-          x0 = max(cx - 1, 0); x1 = min(cx + 1, (int)nx - 1);
-          y0 = max(cy - 1, 0); y1 = min(cy + 1, (int)ny - 1);
-        }
-        const uint32_t nPassC = (isNear || isLast) ? 1u : nPass;
-        for (uint32_t pass = 0; pass < nPassC; ++pass) {
-          const uint32_t gbase = (onlyMine ? (uint32_t)parity : pass) * G.n_cells + base;
-          uint32_t s0 = 0u, s1 = 0u, s2 = 0u, n0 = 0u, n1 = 0u, n2 = 0u;
-          auto row = [&](int yy, uint32_t &sr, uint32_t &nr) {
-            const uint32_t rowBase = gbase + (uint32_t)yy * nx;
-            sr = __ldg(P.cell_start + rowBase + x0);
-            nr = __ldg(P.cell_start + rowBase + x1 + 1) - sr;
-          };
-          if (y0 <= y1) row(y0, s0, n0);
-          if (y0 + 1 <= y1) row(y0 + 1, s1, n1);
-          if (y0 + 2 <= y1) row(y0 + 2, s2, n2);
-          if (isNear && active) { s0 = nearBeg; n0 = nearEnd - nearBeg; }
-          const uint32_t n01 = n0 + n1, tot = n01 + n2;
-          const uint32_t wmax = isLast ? 1u : __reduce_max_sync(0xffffffffu, tot);
-          // four candidates per step: their loads are issued together (each lane reads its own cells; neighbouring
-          // pixels share them, so most of these hit L1)
-          for (uint32_t j0 = 0; j0 < wmax; j0 += kTileBatch) {
-            if (__any_sync(0xffffffffu, qn + (uint32_t)kTileBatch > (uint32_t)kTileQ || (isLast && qn > 0u))) flush();
+      // ---- census.  A lane's cell floor((x - gx0) / cell) is monotone in x, so the cells of the lanes' extreme
+      // coordinates bound every lane's window (a NaN coordinate, cell 0 after the clamp, widens the box to the grid's edge).
+      const float inf = __int_as_float(0x7f800000);
+      const float txlo = warp_min(active ? (isnan(x) ? -inf : x) : inf), txhi = warp_max(active ? (isnan(x) ? inf : x) : -inf);
+      const float tylo = warp_min(active ? (isnan(y) ? -inf : y) : inf), tyhi = warp_max(active ? (isnan(y) ? inf : y) : -inf);
+      bool hit = false;
+      if (censusLane) {
+        const int nx = (int)G.nx[censusClass], ny = (int)G.ny[censusClass];
+        const float ic = 1.f / G.csize[censusClass];
+        const int tx0 = max(min(max((int)floorf((txlo - G.gx0) * ic), 0), nx - 1) - 1, 0);
+        const int tx1 = min(min(max((int)floorf((txhi - G.gx0) * ic), 0), nx - 1) + 1, nx - 1);
+        const int ty0 = max(min(max((int)floorf((tylo - G.gy0) * ic), 0), ny - 1) - 1, 0);
+        const int ty1 = min(min(max((int)floorf((tyhi - G.gy0) * ic), 0), ny - 1) + 1, ny - 1);
+        uint32_t n = 0;
+        if (ty1 - ty0 < kCensusRows) {
 #pragma unroll
-            for (uint32_t u0 = 0; u0 < (uint32_t)kTileBatch; u0 += 4) {
-              float4 ph[4];
-              uint32_t sl[4];
+          for (int r = 0; r < kCensusRows; ++r) {
+            const uint32_t rowBase = censusBase + (uint32_t)(ty0 + r) * (uint32_t)nx;
+            if (ty0 + r <= ty1) n += __ldg(P.cell_start + rowBase + tx1 + 1) - __ldg(P.cell_start + rowBase + tx0);
+          }
+        } else {   // every cell of the window lies between these two in the key order
+          n = __ldg(P.cell_start + censusBase + (uint32_t)ty1 * nx + tx1 + 1) - __ldg(P.cell_start + censusBase + (uint32_t)ty0 * nx + tx0);
+        }
+        hit = n != 0u;
+      }
+      uint32_t todo = __ballot_sync(0xffffffffu, hit);
+      // a lane that scans its own parity's grid only visits class c when either grid has photons there: one entry per class
+      if (onlyMine) todo = (todo | todo >> 1) & 0x55555555u;
+      bool nearTodo = nearEnd > nearBeg;   // NEAR: every active ray tests the whole bucket
+
+      // ---- chunks of kGridItems entries: every lane lists its non-empty ranges, then walks them as one stream
+      for (;;) {
+        uint32_t nr = 0u, tot = 0u;
 #pragma unroll
-              for (int u = 0; u < 4; ++u) {
-                const uint32_t j = j0 + u0 + u;
-                sl[u] = j < n0 ? s0 + j : (j < n01 ? s1 + (j - n0) : s2 + (j - n01));
-                if (j < tot) ph[u] = ldg4(P.planes + sl[u]);
+        for (int t = 0; t < kGridItems; ++t) {
+          if (todo) {
+            const int i = __ffs(todo) - 1;
+            todo &= todo - 1u;
+            if (active) {
+              const int c = i >> gShift;
+              const uint32_t g = onlyMine ? (uint32_t)parity : ((uint32_t)i & (nGridsBuilt - 1u));
+              const uint32_t nx = G.nx[c], ny = G.ny[c];
+              const float ic = 1.f / G.csize[c];
+              int cx = (int)floorf((x - G.gx0) * ic), cy = (int)floorf((y - G.gy0) * ic);
+              cx = min(max(cx, 0), (int)nx - 1);
+              cy = min(max(cy, 0), (int)ny - 1);
+              const int x0 = max(cx - 1, 0), x1 = min(cx + 1, (int)nx - 1);
+              const int y0 = max(cy - 1, 0), y1 = min(cy + 1, (int)ny - 1);
+              const uint32_t gbase = g * G.n_cells + G.base[c];
+              uint32_t sr[3], er[3];
+#pragma unroll
+              for (int r = 0; r < 3; ++r) {
+                sr[r] = er[r] = 0u;
+                if (y0 + r <= y1) {
+                  const uint32_t rowBase = gbase + (uint32_t)(y0 + r) * nx;
+                  sr[r] = __ldg(P.cell_start + rowBase + x0);
+                  er[r] = __ldg(P.cell_start + rowBase + x1 + 1);
+                }
               }
 #pragma unroll
-              for (int u = 0; u < 4; ++u)
-                if (j0 + u0 + u < tot) test(ph[u], sl[u]);
+              for (int r = 0; r < 3; ++r)
+                if (er[r] > sr[r]) {
+                  S.rbeg[nr][lane] = sr[r];
+                  S.rend[nr][lane] = er[r];
+                  ++nr;
+                  tot += er[r] - sr[r];
+                }
+            }
+          } else if (nearTodo) {
+            nearTodo = false;
+            if (active) {
+              S.rbeg[nr][lane] = nearBeg;
+              S.rend[nr][lane] = nearEnd;
+              ++nr;
+              tot += nearEnd - nearBeg;
             }
           }
         }
+        const bool last = !todo && !nearTodo;
+        const uint32_t wmax = __reduce_max_sync(0xffffffffu, tot);
+        // the walk: [s, e) is the current range, [ns, ne) the next one (read ahead), k the range after that
+        uint32_t s = S.rbeg[0][lane], e = S.rend[0][lane], ns = S.rbeg[1][lane], ne = S.rend[1][lane], k = 2u;
+        // the closing batch of the tile's last chunk only flushes: one call site of flush_candidates (this kernel's
+        // instruction-fetch stalls grow with its code size)
+        const uint32_t nBatch = (wmax + kTileBatch - 1) / kTileBatch + (last ? 1u : 0u);
+        for (uint32_t b = 0, j0 = 0; b < nBatch; ++b, j0 += kTileBatch) {
+          const bool fin = last && b + 1u == nBatch;
+          if (__any_sync(0xffffffffu, qn + (uint32_t)kTileBatch > (uint32_t)kTileQ || (fin && qn > 0u))) flush();
+          if (fin) break;
+#pragma unroll
+          for (uint32_t u0 = 0; u0 < (uint32_t)kTileBatch; u0 += kGridLoads) {
+            float4 ph[kGridLoads];
+            uint32_t sl[kGridLoads];
+#pragma unroll
+            for (int u = 0; u < kGridLoads; ++u) {
+              sl[u] = s;
+              if (j0 + u0 + u < tot) {
+                ph[u] = ldg4(P.planes + s);
+                if (++s == e) {
+                  s = ns; e = ne;
+                  ns = S.rbeg[k][lane]; ne = S.rend[k][lane];
+                  ++k;
+                }
+              }
+            }
+#pragma unroll
+            for (int u = 0; u < kGridLoads; ++u)
+              if (j0 + u0 + u < tot) test(ph[u], sl[u]);
+          }
+        }
+        if (last) break;
       }
     }
     if (P.counts && have) {

@@ -347,6 +347,12 @@ int gvpm_build_points_for_rays(gvpm_ctx *ctx, float radius, uint32_t *n_kept);
  * around its own direction - no traversal.  Same neighbour sets, same results.  n_kept (photons some ray can reach)
  * then costs one device read-back: pass NULL when it is not needed.  gvpm_accel_kind: 0 = box hierarchy, 1 = grid. */
 int gvpm_accel_kind(const gvpm_ctx *ctx);
+/* Read-only view of the perspective grid the last build made (diagnostics, e.g. tools/trav_census.py): the grid's
+ * parameters as the device sees them (struct FrustumGrid of gvpm_device.cuh, all 4-byte fields; grid_bytes must be its
+ * size) and, when cell_start is not NULL, its cell_start array (first sorted slot of every key, NEAR and DROP included,
+ * then the end: *n_entries values; cap = room in cell_start).  Either output may be NULL.  Fails when the last build
+ * made a box hierarchy. */
+int gvpm_frustum_grid(gvpm_ctx *ctx, void *grid, size_t grid_bytes, uint32_t *cell_start, size_t cap, size_t *n_entries);
 /* Optional: the axis of the perspective grid's projection plane (default: the mean direction of the uploaded rays).
  * The sensor's viewing direction is the natural choice; ranks of a sharded image that all pass the same vector project
  * on the same plane, which lets gvpm_dispatch_photons classify a photon once for all receivers.  NULL: back to the
